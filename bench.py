@@ -17,7 +17,7 @@ The same line also carries the two multi-GPU modes BASELINE.json names:
                two small NCCL all-gathers per generation (lambda fitness scalars, then (n + 4) floats per rank), the
                generation captured in one CUDA graph; with the 1-GPU whole-population time beside it.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--skip c3,c4,cpu]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--skip c3,c4,cpu] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -116,6 +116,18 @@ def sampler_roofline(n, lam, live, ms, peak_gbs):
                     "algorithmic_bytes_per_launch": nbytes}}
 
 
+def dump_outputs(path, opt):
+    """What a caller of the timed generation holds after its last step (1.7 MB in all): the best path and cost so far,
+    the population that generation sampled for the next one, the fitness and collision counts of the population it
+    evaluated, and the mean and step size it updated.  The inputs are seeded, so two builds can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    best_x, best_f = opt.best()
+    arrays = {"best_x": best_x, "best_f": best_f, "X": opt.get("X"), "fit": opt.get("fit"),
+              "ncoll": opt.get("ncoll").astype(np.float32), "xmean": opt.get("xmean"), "sigma": opt.get("sigma")}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_b200(args):
     import torch
     import lmcma_path_planner_b200 as L
@@ -179,6 +191,8 @@ def run_b200(args):
     nsamp_mean = float(opt.get("nsamp").mean())
     live1, sigma1 = int(opt.get("live")[0]), float(opt.get("sigma")[0])
     ncoll_best = int(opt.get("ncoll")[0].min())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, opt)
 
     # steady state: back-to-back graph replays, L2 warm (the deployment mode: the map stays L2-resident)
     e0, e1 = torch.cuda.Event(True), torch.cuda.Event(True)
@@ -672,7 +686,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--skip", default="", help="comma list of c3,c4,cpu (development runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed generation computed as DIR/<name>.npy (rank 0, --impl b200)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

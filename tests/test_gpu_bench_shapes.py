@@ -334,3 +334,34 @@ def test_rows_sampler_streams_pairs_that_do_not_fit(po, monkeypatch):
 def weighted_sphere_np(X):
     X = np.atleast_2d(X)
     return np.sum((1.0 + np.arange(X.shape[1])) * X * X, axis=1)
+
+
+def test_bench_dumps_the_last_timed_generation(tmp_path):
+    """bench.py --dump-outputs DIR: after the timed steps, the arrays of the last timed generation land in DIR as float32 /
+    float64 .npy files, they are the state the JSON line of the same run reports after its timed region, and a second
+    run with the same arguments writes the same bits (what makes the files comparable from build to build)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(out):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1",
+                            "--skip", "c3,c4,cpu", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        j = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        return j, {p[:-len(".npy")]: np.load(out / p) for p in os.listdir(out)}
+
+    j, d = run(tmp_path / "a")
+    assert j["steps"] == 3
+    assert sorted(d) == ["X", "best_f", "best_x", "fit", "ncoll", "sigma", "xmean"]
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+    assert d["X"].shape == (1, 1024, 400) and d["fit"].shape == (1, 1024) and d["best_x"].shape == d["xmean"].shape == (1, 400)
+    assert d["sigma"][0] == j["config"]["sigma_in_timed_region"][1]
+    assert d["ncoll"].min() == j["config"]["min_collisions_in_last_population"]
+    assert np.isfinite(d["fit"]).all() and np.isfinite(d["X"]).all()
+    _, d2 = run(tmp_path / "b")
+    assert sorted(d2) == sorted(d)
+    for name in d:
+        assert d2[name].dtype == d[name].dtype and np.array_equal(d2[name], d[name]), name
