@@ -245,7 +245,24 @@ enum {
     LMCMA_B200_I32_LIVE = 5,       /* batch       (LMCMA::iterator_sz) */
     LMCMA_B200_I32_COUNTEVAL = 6,  /* batch       (CMABase::counteval) */
     LMCMA_B200_I32_NCOLL = 7,      /* batch x pop_count colliding samples of the last evaluated population */
-    LMCMA_B200_I32_NSAMP = 8       /* batch x pop_count map samples of the last evaluated population */
+    LMCMA_B200_I32_NSAMP = 8,      /* batch x pop_count map samples of the last evaluated population */
+    LMCMA_B200_I32_LAUNCH = 9      /* LMCMA_B200_LAUNCH_FIELDS values per HANDLE (not per instance), read-only: the launch
+                                      configuration chosen at create, indexed by LMCMA_B200_LAUNCH_* below */
+};
+/* fields of LMCMA_B200_I32_LAUNCH.  Sampler kernels: 0 = k_sample<NV> (narrow), 1 = k_sample_wide<RBW> (a row split over CW
+ * column-warps, R row groups per CTA), 2 = k_sample_rows<QW, RL> (rows on lanes).  KC / STAGES are those of the chosen
+ * sampler.  The update is k_update<NVB, RMAX, ROWS_IN_SMEM, OVERLAP, WARPS> (SWEEP_WARPS of them sweep), or with GRAM the
+ * Gram-matrix recompute whose k_coef keeps COEF_ELEMS elements per lane (0 without GRAM).  The overlapped k_update build
+ * is the one of the fused generations and of tell_all when OVERLAP is 1. */
+enum {
+    LMCMA_B200_LAUNCH_SAMPLER = 0, LMCMA_B200_LAUNCH_SMP_NV, LMCMA_B200_LAUNCH_SMP_SPEC, LMCMA_B200_LAUNCH_SMP_THREADS,
+    LMCMA_B200_LAUNCH_SMP_RBW, LMCMA_B200_LAUNCH_SMP_CW, LMCMA_B200_LAUNCH_SMP_R, LMCMA_B200_LAUNCH_SMP_ROWS_QW,
+    LMCMA_B200_LAUNCH_SMP_ROWS_RL, LMCMA_B200_LAUNCH_SMP_KC, LMCMA_B200_LAUNCH_SMP_STAGES,
+    LMCMA_B200_LAUNCH_UPD_NVB, LMCMA_B200_LAUNCH_UPD_RMAX, LMCMA_B200_LAUNCH_UPD_ROWS_IN_SMEM, LMCMA_B200_LAUNCH_UPD_GRAM,
+    LMCMA_B200_LAUNCH_UPD_WARPS, LMCMA_B200_LAUNCH_UPD_SWEEP_WARPS, LMCMA_B200_LAUNCH_COEF_ELEMS,
+    LMCMA_B200_LAUNCH_RANK_THREADS, LMCMA_B200_LAUNCH_RANK_FTILE, LMCMA_B200_LAUNCH_RANK_TILE_SORTED,
+    LMCMA_B200_LAUNCH_PROGRESSIVE, LMCMA_B200_LAUNCH_OVERLAP,
+    LMCMA_B200_LAUNCH_FIELDS
 };
 int lmcma_b200_get_f64(lmcma_b200_opt* opt, int32_t which, double* out, int64_t capacity);
 int lmcma_b200_get_f32(lmcma_b200_opt* opt, int32_t which, float* out, int64_t capacity);

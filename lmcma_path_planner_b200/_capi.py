@@ -15,6 +15,12 @@ MAP_F32, MAP_U8 = 0, 1
 F64 = {"xmean": 0, "sigma": 1, "s": 2, "best_f": 3, "consts": 4, "weights": 5, "Nj": 6, "Lj": 7}
 F32 = {"X": 0, "pc": 1, "V": 2, "P": 3, "fit": 4, "fit_sorted": 5, "prev_fit": 6, "Z": 7}
 I32 = {"t": 0, "vec": 1, "arindex": 2, "rank": 3, "itr": 4, "live": 5, "counteval": 6, "ncoll": 7, "nsamp": 8}
+I32_LAUNCH = 9
+# the fields of LMCMA_B200_I32_LAUNCH in order (LMCMA_B200_LAUNCH_*)
+LAUNCH_FIELDS = ("sampler", "smp_nv", "smp_spec", "smp_threads", "smp_RBW", "smp_CW", "smp_R", "smp_rows_qw", "smp_rows_rl",
+                 "smp_kc", "smp_stages", "upd_nvb", "upd_rmax", "upd_rows_in_smem", "upd_gram", "upd_warps",
+                 "upd_sweep_warps", "coef_elems", "rank_threads", "rank_ftile", "rank_tile_sorted", "progressive", "overlap")
+SAMPLERS = ("narrow", "wide", "rows")
 
 
 class LmcmaError(RuntimeError):

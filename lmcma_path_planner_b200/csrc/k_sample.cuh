@@ -327,13 +327,16 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
     const int nchunks = (live + kc - 1) / kc;
     SMP_STAMP(2);
     const float Mf = (float)o.M, Minv = 1.0f / Mf;
-    const int live8 = (live + SAMPLE_G - 1) & ~(SAMPLE_G - 1);
-    if (!progressive)
-        for (int k = threadIdx.x; k < live8; k += blockDim.x) {
-            float sc8 = Minv;                                       // M^-((k mod 8) + 1)
-            for (int c = 0; c < (k & 7); ++c) sc8 *= Minv;
+    // the groups of 8 start at chunk boundaries: with kc < 8 (rows longer than ~1600) pair k is element (k mod kc) of its
+    // group, and the last group reads up to 7 entries past its last live pair (zeros: they scale dots of zero pairs)
+    if (!progressive) {
+        const int gmask = min(kc, SAMPLE_G) - 1;                    // kc is 1, 2, 4 or 8
+        for (int k = threadIdx.x; k < live + SAMPLE_G - 1; k += blockDim.x) {
+            float sc8 = Minv;                                       // M^-((k mod min(kc, 8)) + 1)
+            for (int c = 0; c < (k & gmask); ++c) sc8 *= Minv;
             nj_s[k] = (k < live) ? o.Njs[(size_t)b * o.m + k] * sc8 : 0.f;
         }
+    }
     // progressive (warp 0, all lanes): chunk c = pairs [c kc, c kc + cnt) — poll their flags, stage Nj, request the copy
     int next_issue = 0;                                         // warp 0: chunks [0, next_issue) have been requested
     auto chunk_ready = [&](int c) -> bool {

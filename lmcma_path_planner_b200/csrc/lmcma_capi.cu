@@ -287,7 +287,7 @@ int launch_update(lmcma_b200_opt* o, const UpdateArgs& a_in, bool pdl, cudaStrea
         const int tiles = (d.m + GRAM_TILE - 1) / GRAM_TILE;
         k_gram<<<dim3(tiles, tiles, d.B * GRAM_KS), 256, 0, st>>>(d);
         const int coef_threads = std::min(1024, (8 * d.m + 31) & ~31);    // 8 lanes per basis row (m <= 128)
-        auto coef = d.m <= 40 ? k_coef<5> : (d.m <= 80 ? k_coef<10> : (d.m <= 96 ? k_coef<12> : k_coef<16>));   // elements per lane: ceil(m / 8)
+        auto coef = o->coef_elems == 5 ? k_coef<5> : (o->coef_elems == 10 ? k_coef<10> : (o->coef_elems == 12 ? k_coef<12> : k_coef<16>));
         if (o->coef_smem > 48 * 1024) CU(cudaFuncSetAttribute(coef, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->coef_smem));
         coef<<<d.B, coef_threads, o->coef_smem, st>>>(d);
         k_combine<<<dim3((d.ns / 4 + 127) / 128, (d.m + COMBINE_ROWS - 1) / COMBINE_ROWS, d.B), 128, 0, st>>>(d);
@@ -345,6 +345,8 @@ int configure_update(lmcma_b200_opt* o) {
     o->coef_smem = (size_t)2 * o->d.m * (o->d.m | 1) * sizeof(double) + (size_t)2 * o->d.m * sizeof(double);
     o->upd_gram = (!o->upd_rows_in_smem || o->tune.update_gram) && o->d.m <= 128 && o->coef_smem <= budget && !o->tune.update_streaming;
     if (o->upd_gram) { o->upd_rows_in_smem = false; o->upd_smem = fixed; }
+    // k_coef elements per lane: ceil(m / 8), rounded up to a compiled build (m <= 128)
+    o->coef_elems = !o->upd_gram ? 0 : (o->d.m <= 40 ? 5 : (o->d.m <= 80 ? 10 : (o->d.m <= 96 ? 12 : 16)));
     // pending rows in registers when they fit: m <= 8 warps x RMAX rows of <= 128 float4 columns
     o->upd_rmax = 0;
     o->upd_warps = UPD_WARPS;

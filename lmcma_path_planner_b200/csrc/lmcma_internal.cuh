@@ -229,6 +229,7 @@ struct lmcma_b200_opt {
     long long* graph_dbg = nullptr;   // LMCMA_B200_GRAPH_DBG: k_update's timeline inside the fused generation, printed by lmcma_b200_sync
     int upd_nvb = 4, upd_rmax = 0, upd_sweep_warps = 16, upd_warps = 16;
     bool upd_gram = false; size_t coef_smem = 0;   // Gram-matrix recompute (k_gram.cuh) for rows that fit neither registers nor smem
+    int coef_elems = 0;                            // k_coef<coef_elems>: elements per lane, ceil(m / 8) rounded up to a build
     bool upd_rows_in_smem = true;
     size_t upd_smem = 0, rank_smem = 0;
     int rank_threads = 1024;

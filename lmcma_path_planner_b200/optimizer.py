@@ -271,6 +271,15 @@ class Optimizer:
             a = np.ascontiguousarray(np.broadcast_to(np.asarray(value, np.int32), shp))
             K.check(K.lib().lmcma_b200_set_i32(self._h, K.I32[name], K.iptr(a), a.size))
 
+    def launch(self):
+        """The kernel configuration this handle's launches use (chosen at create from n, lambda, m, batch and the device):
+        a dict over _capi.LAUNCH_FIELDS; "sampler" is "narrow", "wide" or "rows"."""
+        v = np.zeros(len(K.LAUNCH_FIELDS), np.int32)
+        K.check(K.lib().lmcma_b200_get_i32(self._h, K.I32_LAUNCH, K.iptr(v), v.size))
+        out = dict(zip(K.LAUNCH_FIELDS, (int(x) for x in v)))
+        out["sampler"] = K.SAMPLERS[out["sampler"]]
+        return out
+
     def load_state(self, st):
         """Teacher forcing: load a state dict as produced by oracle.pyoracle._Base.state()."""
         self.set("xmean", st["xmean"]); self.set("sigma", st["sigma"]); self.set("s", st["s"])

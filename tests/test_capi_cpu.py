@@ -30,6 +30,17 @@ def test_every_declared_symbol_is_exported_and_bound():
     assert lib.lmcma_b200_abi_version() == 1
 
 
+def test_launch_query_fields_follow_the_header():
+    """Optimizer.launch() names the values of LMCMA_B200_I32_LAUNCH in the order of the header's LMCMA_B200_LAUNCH_* enum."""
+    hdr = open(os.path.join(ROOT, "include", "lmcma_b200.h")).read()
+    assert int(re.search(r"LMCMA_B200_I32_LAUNCH\s*=\s*(\d+)", hdr).group(1)) == K.I32_LAUNCH
+    assert K.I32_LAUNCH not in K.I32.values()
+    body = re.search(r"enum\s*\{\s*(LMCMA_B200_LAUNCH_SAMPLER\s*=\s*0[^}]*)\}", hdr).group(1)
+    names = re.findall(r"LMCMA_B200_LAUNCH_([A-Z0-9_]+)", body)
+    assert names[-1] == "FIELDS"
+    assert [s.lower() for s in names[:-1]] == [f.lower() for f in K.LAUNCH_FIELDS]
+
+
 def test_header_cites_the_reference_for_every_entry_point_group():
     hdr = open(os.path.join(ROOT, "include", "lmcma_b200.h")).read()
     for cite in ("lmcma.hpp:131", "lmcma.cpp:172-182", "lmcma.cpp:184-205", "lmcma.cpp:313-424", "lmcma.cpp:301-311",

@@ -143,7 +143,10 @@ def test_cost_full_size_properties(po):
 # optimiser: teacher-forced generations against the FP64 oracle (SURVEY 7.2 #3)
 # ------------------------------------------------------------------------------------------------
 def _teacher_forced(po, n, lam, m, gens, seed, lo=None, hi=None, sigma=1.0, fobj=weighted_sphere, x0=None,
-                    tol=2e-5, tol_v=None):
+                    tol=2e-5, tol_v=None, warm=None):
+    """`gens` teacher-forced generations.  warm: an oracle state of the same (n, m) (OracleLMCMA.state(), e.g. from a cheap
+    small-population run) to start from instead of the empty state, so that a few generations have every slot live and
+    being recycled; the previous fitness is then the sorted fitness of the first population."""
     rng = np.random.default_rng(seed)
     x0 = np.full(n, 0.5) if x0 is None else x0
     dev = L.Optimizer(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma0=sigma, rng="inject")
@@ -151,6 +154,12 @@ def _teacher_forced(po, n, lam, m, gens, seed, lo=None, hi=None, sigma=1.0, fobj
     zs = rng.standard_normal((gens + 1, lam, n)).astype(np.float32)
     ora = po.OracleLMCMA(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma=sigma, seed=1, Z0=zs[0].astype(np.float64))
     dev.inject_z(zs[0])
+    if warm is not None:
+        ora.load_state(warm, np.zeros(lam), zs[0].astype(np.float64))
+        prev = np.sort(fobj(ora.array("X")).astype(np.float32))
+        ora.load_state(warm, prev.astype(np.float64), zs[0].astype(np.float64))
+        dev.load_state(dict(warm, prev_fit=prev))
+        dev.resample()
     worst = {}
     for g in range(gens):
         Xo = ora.array("X")
@@ -226,7 +235,9 @@ def test_lmcma_teacher_forced_eight_warp_update(po, monkeypatch):
 
 
 def test_lmcma_teacher_forced_large_n(po):
-    """C4-like row length: n = 1500, m = 77 (multi-chunk bulk-copy pipeline, NV = 12)."""
+    """C4-like row length: n = 1500, m = 77 (narrow sampler k_sample<12>; the 77 rows of 1500 fit neither registers nor
+    shared memory, so the update is the Gram-matrix recompute with k_coef<10>).  The streaming update that keeps the rows
+    in global memory is tested in tests/test_gpu_dispatch_variants.py."""
     _teacher_forced(po, 1500, 32, 77, 6, seed=4, sigma=0.3)
 
 
