@@ -1050,8 +1050,8 @@ int lmcma_b200_sync(lmcma_b200_opt* o) {
     if (o->graph_dbg) {
         long long h[64];
         cudaMemcpy(h, o->graph_dbg, sizeof(h), cudaMemcpyDeviceToHost);
-        fprintf(stderr, "fused generation, k_update (ns since its start): bookkeeping=%lld prologue=%lld sweep: warp 0 done=%lld, all done + ranks seen=%lld post start=%lld mean=%lld newest row=%lld tail=%lld end=%lld",
-                h[1] - h[0], h[2] - h[0], h[7] - h[0], h[8] - h[0], h[3] - h[0], h[4] - h[0], h[9] - h[0], h[5] - h[0], h[6] - h[0]);
+        fprintf(stderr, "fused generation, k_update (ns since its start): bookkeeping=%lld prologue=%lld sweep: warp 0 done=%lld, all done + ranks seen=%lld post start=%lld mean=%lld progress[0]=%lld newest row=%lld tail=%lld end=%lld",
+                h[1] - h[0], h[2] - h[0], h[7] - h[0], h[8] - h[0], h[3] - h[0], h[4] - h[0], h[22] - h[0], h[9] - h[0], h[5] - h[0], h[6] - h[0]);
         fprintf(stderr, " chain blocks:");
         for (int i = 12; i < 21; ++i) fprintf(stderr, " %lld", (h[i] - h[0]) / 100);
         fprintf(stderr, " rows:");
