@@ -82,13 +82,17 @@ int lmcma_b200_map_create(int device, int dims, const int32_t* shape_xyz, const 
 /* Occupancy grid (1 = obstacle; row-major [ny][nx] / [nz][ny][nx]) -> exact Euclidean distance field in cells, on the
  * device (separable, integer-exact; k_edt.cuh).  Replaces the reference's ways of obtaining EDT_Matrix from a map:
  * the in-file 8SSEDT on a fixed 100 x 100 grid (planner.cpp:403-490) and dynamicEDT3D (planner.cpp:81-87, 305-307).
- * clamp > 0 limits the distance (dynamicEDT3D's maxdist); clamp <= 0 leaves it unbounded. */
+ * clamp > 0 limits the distance (dynamicEDT3D's maxdist); clamp <= 0 leaves it unbounded.  A grid without any obstacle
+ * gives the clamp everywhere, or FLT_MAX when unclamped.  Every axis must be at most 32767 cells long (else
+ * LMCMA_B200_ERR_ARG); the distances are exact for every such grid. */
 int lmcma_b200_edt(int device, int dims, const int32_t* shape_xyz, const uint8_t* occ_host, float clamp, float* dist_host_out);
 /* map_create fed by an occupancy grid: distance transform + conversion to the map storage, all on the device */
 int lmcma_b200_map_create_from_occupancy(int device, int dims, const int32_t* shape_xyz, const uint8_t* occ_host, float clamp,
                                          int storage, float u8_scale, float c_min, lmcma_b200_map** map_out);
 int lmcma_b200_map_destroy(lmcma_b200_map* map);
-/* the distance field the evaluator effectively uses, back on the host (identity for F32 storage) */
+/* the distance field the evaluator effectively uses, back on the host: U8 storage gives E_q = q * u8_scale; F32 storage
+ * gives 1 / (1 / max(E, c_min)) in FP32, i.e. the clearance with the c_min floor (up to the rounding of the two
+ * reciprocals), and 0 on obstacles */
 int lmcma_b200_map_dequantized(const lmcma_b200_map* map, float* dist_host_out);
 /* pin the map in L2 (cudaAccessPolicyWindow, persisting) for the launches of this library */
 int lmcma_b200_map_set_l2_persist(lmcma_b200_map* map, int enable);

@@ -7,43 +7,48 @@
 // then dist = sqrt(d2) (FP64 sqrt, rounded once to FP32 — what scipy's exact EDT gives), optional clamp, and the
 // conversion to the bricked map storage k_cost reads (k_brick) without a host round trip.
 #pragma once
+#include <cfloat>
 #include "lmcma_common.cuh"
 
 namespace lmcma {
 
-constexpr int EDT_INF = 1 << 29;      // "no obstacle on this line yet": above any real squared distance
+// Squared distances are unsigned 32-bit: the largest one an accepted grid holds (axes <= 32767 cells) is 3 * 32766^2 =
+// 3 220 832 268, past INT_MAX but below EDT_NONE, the "no obstacle" sentinel.  Envelope arithmetic is 64-bit.
+constexpr unsigned EDT_NONE = 0xffffffffu;   // no obstacle on this line / in this grid: above any real squared distance
+constexpr int EDT_FAR = 1 << 29;             // obstacle index of "none" in pass x's scans: farther than any real index
+constexpr float EDT_EMPTY = FLT_MAX;         // distance where the grid holds no obstacle at all, unless clamped
 
 // ---- pass x: one warp per line of nx cells (lines = ny * nz), d2[x] = (distance to the nearest obstacle along x)^2
-__global__ void __launch_bounds__(256) k_edt_x(const unsigned char* __restrict__ occ, int* __restrict__ d2, int nx, long long nlines) {
+__global__ void __launch_bounds__(256) k_edt_x(const unsigned char* __restrict__ occ, unsigned* __restrict__ d2, int nx, long long nlines) {
     const int lane = threadIdx.x & 31;
     const long long line = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (line >= nlines) return;
     const unsigned char* src = occ + line * nx;
-    int* dst = d2 + line * nx;
+    unsigned* dst = d2 + line * nx;
     // forward: index of the last obstacle at or before x (max-scan), chunk by chunk with a carry
-    int carry = -EDT_INF;
+    int carry = -EDT_FAR;
     for (int x0 = 0; x0 < nx; x0 += 32) {
         const int x = x0 + lane;
-        int v = (x < nx && src[x]) ? x : -EDT_INF;
+        int v = (x < nx && src[x]) ? x : -EDT_FAR;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v = max(v, u); }
         v = max(v, carry);
         carry = __shfl_sync(0xffffffffu, v, 31);
-        if (x < nx) dst[x] = (v <= -EDT_INF) ? EDT_INF : x - v;        // plain distance for now
+        if (x < nx) dst[x] = (v <= -EDT_FAR) ? EDT_FAR : x - v;        // plain distance for now
     }
     // backward: index of the first obstacle at or after x (min-scan from the right)
-    carry = EDT_INF;
+    carry = EDT_FAR;
     for (int x0 = ((nx - 1) / 32) * 32; x0 >= 0; x0 -= 32) {
         const int x = x0 + lane;
-        int v = (x < nx && src[x]) ? x : EDT_INF;
+        int v = (x < nx && src[x]) ? x : EDT_FAR;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_down_sync(0xffffffffu, v, o); if (lane + o < 32) v = min(v, u); }
         v = min(v, carry);
         carry = __shfl_sync(0xffffffffu, v, 0);
         if (x < nx) {
-            const int fwd = dst[x], bwd = (v >= EDT_INF) ? EDT_INF : v - x;
+            const int fwd = (int)dst[x], bwd = (v >= EDT_FAR) ? EDT_FAR : v - x;
             const int d = min(fwd, bwd);
-            dst[x] = d >= 32768 ? EDT_INF : d * d;                     // lines longer than 32767 cells are refused at the ABI
+            dst[x] = d >= 32768 ? EDT_NONE : (unsigned)(d * d);       // lines longer than 32767 cells are refused at the ABI
         }
     }
 }
@@ -51,16 +56,16 @@ __global__ void __launch_bounds__(256) k_edt_x(const unsigned char* __restrict__
 // ---- pass along an axis of length m with element stride `stride`: lines are enumerated by (inner, outer) with
 //      address = outer * outer_stride + inner, inner < n_inner consecutive in memory (coalesced across threads).
 //      s / t / gh: scratch of m entries per line, laid out [position][line] for the same reason.
-__global__ void __launch_bounds__(128) k_edt_axis(int* __restrict__ d2, int m, long long stride, int n_inner, long long n_outer,
-                                                  long long outer_stride, int* __restrict__ s, int* __restrict__ t, int* __restrict__ gh) {
+__global__ void __launch_bounds__(128) k_edt_axis(unsigned* __restrict__ d2, int m, long long stride, int n_inner, long long n_outer,
+                                                  long long outer_stride, int* __restrict__ s, int* __restrict__ t, unsigned* __restrict__ gh) {
     const long long line = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long nlines = (long long)n_inner * n_outer;
     if (line >= nlines) return;
     const long long inner = line % n_inner, outer = line / n_inner;
-    int* base = d2 + outer * outer_stride + inner;
+    unsigned* base = d2 + outer * outer_stride + inner;
     auto S = [&](int q) -> int& { return s[(long long)q * nlines + line]; };
     auto T = [&](int q) -> int& { return t[(long long)q * nlines + line]; };
-    auto G = [&](int q) -> int& { return gh[(long long)q * nlines + line]; };
+    auto G = [&](int q) -> unsigned& { return gh[(long long)q * nlines + line]; };
     // lower envelope: hull point q is the parabola centred at S(q) with height G(q), dominant from T(q) on
     int q = 0;
     S(0) = 0; T(0) = 0; G(0) = base[0];
@@ -71,7 +76,7 @@ __global__ void __launch_bounds__(128) k_edt_axis(int* __restrict__ d2, int m, l
             const long long f_old = (tq - sq) * (tq - sq) + gq, f_new = (tq - u) * (tq - u) + gu;
             if (f_old > f_new) --q; else break;
         }
-        if (q < 0) { q = 0; S(0) = u; T(0) = 0; G(0) = (int)gu; }
+        if (q < 0) { q = 0; S(0) = u; T(0) = 0; G(0) = (unsigned)gu; }
         else {
             const long long sq = S(q), gq = G(q);
             // Sep(i, u) = (u^2 - i^2 + G(u) - G(i)) div (2 (u - i)), floor division (numerator may be negative)
@@ -79,23 +84,23 @@ __global__ void __launch_bounds__(128) k_edt_axis(int* __restrict__ d2, int m, l
             long long sep = num / den;
             if ((num % den != 0) && ((num < 0) != (den < 0))) --sep;
             const long long w = 1 + sep;
-            if (w < m) { ++q; S(q) = u; T(q) = (int)max(w, 0LL); G(q) = (int)gu; }
+            if (w < m) { ++q; S(q) = u; T(q) = (int)max(w, 0LL); G(q) = (unsigned)gu; }
         }
     }
     for (int u = m - 1; u >= 0; --u) {
         const long long sq = S(q), gq = G(q);
         const long long d = ((long long)u - sq) * ((long long)u - sq) + gq;
-        base[(long long)u * stride] = d >= EDT_INF ? EDT_INF : (int)d;
+        base[(long long)u * stride] = d >= (long long)EDT_NONE ? EDT_NONE : (unsigned)d;
         if (u == T(q)) --q;
     }
 }
 
-// ---- d2 -> distance in cells (FP32), optional clamp; no obstacle anywhere -> clamp (or FLT_MAX when unclamped)
-__global__ void __launch_bounds__(256) k_edt_finish(const int* __restrict__ d2, float* __restrict__ dist, long long cells, float clamp) {
+// ---- d2 -> distance in cells (FP32), optional clamp; no obstacle anywhere -> clamp (or EDT_EMPTY = FLT_MAX when unclamped)
+__global__ void __launch_bounds__(256) k_edt_finish(const unsigned* __restrict__ d2, float* __restrict__ dist, long long cells, float clamp) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= cells) return;
-    const int v = d2[i];
-    float d = v >= EDT_INF ? 3.4e38f : (float)sqrt((double)v);
+    const unsigned v = d2[i];
+    float d = v == EDT_NONE ? EDT_EMPTY : (float)sqrt((double)v);
     if (clamp > 0.f) d = fminf(d, clamp);
     dist[i] = d;
 }

@@ -193,7 +193,8 @@ static int edt_device(int dims, const int32_t* shape, const unsigned char* d_occ
     const int nx = shape[0], ny = shape[1], nz = dims == 3 ? shape[2] : 1;
     ARG(nx <= 32767 && ny <= 32767 && nz <= 32767, "axis longer than 32767 cells");
     const size_t cells = (size_t)nx * ny * nz;
-    int *d2 = nullptr, *s = nullptr, *t = nullptr, *gh = nullptr;
+    unsigned *d2 = nullptr, *gh = nullptr;   // squared distances (k_edt.cuh)
+    int *s = nullptr, *t = nullptr;
     int rc = dmalloc(&d2, cells);
     if (!rc) rc = dmalloc(&s, cells);
     if (!rc) rc = dmalloc(&t, cells);
