@@ -208,7 +208,8 @@ int lmcma_b200_attach_cost(lmcma_b200_opt* opt, lmcma_b200_map* map, const lmcma
  * host round trip (the loop of example_lmcma.cpp:49-55 with the cost on the device). Asynchronous. */
 int lmcma_b200_run(lmcma_b200_opt* opt, int32_t generations);
 int lmcma_b200_sync(lmcma_b200_opt* opt);
-/* number of kernels this library has launched so far (all handles, this process) */
+/* number of kernels this library has launched so far (all handles, this process).  A replay of one of its CUDA graphs
+ * (lmcma_b200_run, lmcma_b200_tell_all) counts the kernels the graph holds; building a graph counts none. */
 int64_t lmcma_b200_launch_count(void);
 /* CUDA-event timing of everything enqueued by the last lmcma_b200_run on this handle (ms) */
 int lmcma_b200_last_run_ms(lmcma_b200_opt* opt, float* ms_out);

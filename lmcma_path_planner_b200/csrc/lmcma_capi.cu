@@ -15,6 +15,7 @@ using namespace lmcma_capi;
 namespace lmcma_capi {
 thread_local std::string g_err;
 std::atomic<long long> g_launches{0};
+thread_local long long* g_capture_launches = nullptr;
 DeviceProps g_props[64];
 }  // namespace lmcma_capi
 namespace lmcma {
@@ -33,54 +34,21 @@ int set_error(int code, const char* fmt, ...) {
 namespace {
 template <int NV, int RB, int MAXT, bool SPEC = false>
 int launch_sample_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
-    auto kern = k_sample<NV, RB, MAXT, SPEC>;
-    if (o->smp_smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->smp_smem));
     const int rows_per_cta = (o->smp_threads / 32) * RB;
     const int ctas = (o->d.pop_count + rows_per_cta - 1) / rows_per_cta;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(ctas, o->d.B); cfg.blockDim = dim3(o->smp_threads); cfg.dynamicSmemBytes = o->smp_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&cfg, kern, d, o->smp_kc, o->smp_stages));
-    g_launches++;
-    return 0;
+    return launch(k_sample<NV, RB, MAXT, SPEC>, dim3(ctas, o->d.B), o->smp_threads, o->smp_smem, st, pdl, d, o->smp_kc, o->smp_stages);
 }
 
 template <int RBW, int MAXT>
 int launch_sample_wide_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st, int progressive) {
-    auto kern = k_sample_wide<RBW, MAXT>;
-    if (o->smp_smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->smp_smem));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
     const int rows_per_cta = o->smp_R * RBW;
-    cfg.gridDim = dim3((o->d.pop_count + rows_per_cta - 1) / rows_per_cta, o->d.B); cfg.blockDim = dim3(32 * o->smp_R * o->smp_CW);
-    cfg.dynamicSmemBytes = o->smp_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&cfg, kern, d, o->smp_kc, o->smp_stages, o->smp_R, o->smp_CW, o->smp_qpw, progressive));
-    g_launches++;
-    return 0;
+    return launch(k_sample_wide<RBW, MAXT>, dim3((o->d.pop_count + rows_per_cta - 1) / rows_per_cta, o->d.B), 32 * o->smp_R * o->smp_CW,
+                  o->smp_smem, st, pdl, d, o->smp_kc, o->smp_stages, o->smp_R, o->smp_CW, o->smp_qpw, progressive);
 }
 template <int QW, int RL>
 int launch_sample_rows_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
-    auto kern = k_sample_rows<QW, RL>;
-    if (o->smp_rows_smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->smp_rows_smem));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((d.pop_count + 32 * RL - 1) / (32 * RL), d.B); cfg.blockDim = dim3(512);
-    cfg.dynamicSmemBytes = o->smp_rows_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&cfg, kern, d, o->smp_rows_kc, o->smp_rows_stages, o->smp_rows_region));
-    g_launches++;
-    return 0;
+    return launch(k_sample_rows<QW, RL>, dim3((d.pop_count + 32 * RL - 1) / (32 * RL), d.B), 512, o->smp_rows_smem, st, pdl,
+                  d, o->smp_rows_kc, o->smp_rows_stages, o->smp_rows_region);
 }
 int launch_sample_rows(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
     const bool two = o->smp_rows_rl == 2;
@@ -103,9 +71,8 @@ int launch_sample_wide(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_
 // setter it is rebuilt from the slot-indexed arrays
 int ensure_mirror(lmcma_b200_opt* o, cudaStream_t st) {
     if (!o->mirror_dirty) return 0;
-    k_pack_pairs<<<dim3(o->d.m, o->d.B), 128, 0, st>>>(o->d);
-    g_launches++;
-    CU(cudaGetLastError());
+    int rc = launch(k_pack_pairs, dim3(o->d.m, o->d.B), 128, 0, st, false, o->d);
+    if (rc) return rc;
     o->mirror_dirty = false;
     return 0;
 }
@@ -116,14 +83,11 @@ int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool pro
     if (o->mirror_dirty) { int rc = ensure_mirror(o, st); if (rc) return rc; pdl = false; }
     if (o->d_Lf) {   // smoothness prior: z <- L z for the whole population before computeAz (lmcma.cpp:216-217)
         const OptDev& d = o->d;
-        if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) {
-            k_gauss<<<dim3((d.ns / 4 + 127) / 128, d.pop_count, d.B), 128, 0, st>>>(d);
-            g_launches++;
-        }
+        int rc = 0;
+        if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) rc = launch(k_gauss, dim3((d.ns / 4 + 127) / 128, d.pop_count, d.B), 128, 0, st, false, d);
         const int rows = d.B * d.pop_count;
-        k_prior<<<dim3((d.ns + 63) / 64, (rows + 63) / 64), 256, 0, st>>>(d.Z, o->d_Lf, d.Zc, rows, d.n, d.ns);
-        g_launches++;
-        CU(cudaGetLastError());
+        if (!rc) rc = launch(k_prior, dim3((d.ns + 63) / 64, (rows + 63) / 64), 256, 0, st, false, d.Z, o->d_Lf, d.Zc, rows, d.n, d.ns);
+        if (rc) return rc;
         pdl = false;
     }
     // the host mirror of X (lmcma_b200_ask_all_view) is written by the samplers of the host-buffer protocol only: the fused
@@ -233,45 +197,16 @@ int configure_sample(lmcma_b200_opt* o) {
 // pdl: launched as a programmatic dependent of the kernel enqueued just before it on `st` (k_cost)
 int launch_rank(lmcma_b200_opt* o, const float* f_all, int mode, float* payload, cudaStream_t st, bool pdl = false) {
     if (o->d.tile_sorted) {                                       // lambda > 4096, unsplit: sort the fitness tiles first (k_rank.cuh)
-        cudaLaunchConfig_t c0;
-        memset(&c0, 0, sizeof(c0));
-        c0.gridDim = dim3((o->d.lambda + TELL_FTILE - 1) / TELL_FTILE, o->d.B); c0.blockDim = dim3(1024); c0.stream = st;
-        cudaLaunchAttribute a0[1];
-        a0[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        a0[0].val.programmaticStreamSerializationAllowed = 1;
-        c0.attrs = a0; c0.numAttrs = pdl ? 1 : 0;
-        CU(cudaLaunchKernelEx(&c0, k_rank_tiles, o->d, f_all));
-        g_launches++;
+        int rc = launch(k_rank_tiles, dim3((o->d.lambda + TELL_FTILE - 1) / TELL_FTILE, o->d.B), 1024, 0, st, pdl, o->d, f_all);
+        if (rc) return rc;
         pdl = false;                                              // k_rank itself follows in stream order
     }
-    auto kern = k_rank<1024>;
-    if (o->rank_smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->rank_smem));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(o->d.RS, o->d.B); cfg.blockDim = dim3(o->rank_threads); cfg.dynamicSmemBytes = o->rank_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&cfg, kern, o->d, f_all, mode, payload));
-    g_launches++;
-    return 0;
+    return launch(k_rank<1024>, dim3(o->d.RS, o->d.B), o->rank_threads, o->rank_smem, st, pdl, o->d, f_all, mode, payload);
 }
 
 template <int NVB, int RMAX, bool SMEM, bool OVERLAP = false, int WARPS = UPD_WARPS>
 int launch_update_t(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream_t st) {
-    auto kern = k_update<NVB, RMAX, SMEM, OVERLAP, WARPS>;
-    if (o->upd_smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->upd_smem));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(o->d.B); cfg.blockDim = dim3(32 * WARPS); cfg.dynamicSmemBytes = o->upd_smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&cfg, kern, o->d, a));
-    g_launches++;
-    return 0;
+    return launch(k_update<NVB, RMAX, SMEM, OVERLAP, WARPS>, o->d.B, 32 * WARPS, o->upd_smem, st, pdl, o->d, a);
 }
 
 // the serial part of update() (k_update.cuh).  pdl: launched as a programmatic dependent of the kernel enqueued just
@@ -285,15 +220,11 @@ int launch_update(lmcma_b200_opt* o, const UpdateArgs& a_in, bool pdl, cudaStrea
         if (rc) return rc;
         const OptDev& d = o->d;
         const int tiles = (d.m + GRAM_TILE - 1) / GRAM_TILE;
-        k_gram<<<dim3(tiles, tiles, d.B * GRAM_KS), 256, 0, st>>>(d);
+        if ((rc = launch(k_gram, dim3(tiles, tiles, d.B * GRAM_KS), 256, 0, st, false, d))) return rc;
         const int coef_threads = std::min(1024, (8 * d.m + 31) & ~31);    // 8 lanes per basis row (m <= 128)
         auto coef = o->coef_elems == 5 ? k_coef<5> : (o->coef_elems == 10 ? k_coef<10> : (o->coef_elems == 12 ? k_coef<12> : k_coef<16>));
-        if (o->coef_smem > 48 * 1024) CU(cudaFuncSetAttribute(coef, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->coef_smem));
-        coef<<<d.B, coef_threads, o->coef_smem, st>>>(d);
-        k_combine<<<dim3((d.ns / 4 + 127) / 128, (d.m + COMBINE_ROWS - 1) / COMBINE_ROWS, d.B), 128, 0, st>>>(d);
-        g_launches += 3;
-        CU(cudaGetLastError());
-        return 0;
+        if ((rc = launch(coef, d.B, coef_threads, o->coef_smem, st, false, d))) return rc;
+        return launch(k_combine, dim3((d.ns / 4 + 127) / 128, (d.m + COMBINE_ROWS - 1) / COMBINE_ROWS, d.B), 128, 0, st, false, d);
     }
     if (o->upd_nvb == 4) {
         if (a.overlap) {                                         // the overlapped generation (ensure_graph): register sweep only
@@ -406,6 +337,52 @@ int generation_tail(lmcma_b200_opt* o, cudaStream_t st) {
     return host_rng_and_sample(o, st, prog);
 }
 
+// ---- CUDA graphs: built by capture(), replayed by replay(), freed by drop_fused_graphs / drop_tell_graphs ----
+void drop(Graph& g) {
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+    g = Graph{};
+}
+void drop_fused_graphs(lmcma_b200_opt* o) {
+    drop(o->graph);
+    drop(o->graph_multi);
+}
+// the tell graphs, and with them what their speculative pass left behind
+void drop_tell_graphs(lmcma_b200_opt* o) {
+    drop(o->tell_graph);
+    drop(o->tell_graph_resume);
+    o->spec_valid = false;
+}
+
+// Records what body() enqueues on `st` (and on the streams it forks from `st`) into *g, which is empty.  Capture enqueues
+// nothing: the kernels the body launches are counted in g->launches, and each replay adds them to g_launches.
+template <class Body>
+int capture(cudaStream_t st, Body&& body, Graph* g) {
+    cudaGraph_t graph = nullptr;
+    long long launches = 0;
+    CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+    g_capture_launches = &launches;
+    int rc = body();
+    g_capture_launches = nullptr;
+    cudaError_t e = cudaStreamEndCapture(st, &graph);
+    if (!rc && e == cudaSuccess) e = cudaGraphInstantiate(&g->exec, graph, 0);
+    if (graph) cudaGraphDestroy(graph);
+    if (!rc && e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "graph capture / instantiate failed: %s", cudaGetErrorString(e));
+    if (rc) g->exec = nullptr;
+    else g->launches = (int)launches;
+    return rc;
+}
+
+int replay(const Graph& g, cudaStream_t st) {
+    CU(cudaGraphLaunch(g.exec, st));
+    g_launches += g.launches;
+    return 0;
+}
+
+// LMCMA_B200_GRAPH_DBG: k_update's timeline inside the graphs, printed by lmcma_b200_sync (best effort)
+void ensure_graph_dbg(lmcma_b200_opt* o) {
+    if (o->tune.graph_dbg && !o->graph_dbg && cudaMalloc(&o->graph_dbg, 64 * sizeof(long long)) == cudaSuccess) { cudaMemset(o->graph_dbg, 0, 64 * sizeof(long long)); cudaDeviceSynchronize(); }
+}
+
 // Do the two branches of a forked CUDA graph really run concurrently on this device, in this process?  (Not under a
 // profiler / sanitizer that serialises kernels, not when someone else holds the SMs.)  Probed once per device with two
 // one-thread kernels that shake hands within 5 ms; the second of two launches counts (the first pays module loading).
@@ -413,28 +390,22 @@ int probe_coschedule(lmcma_b200_opt* o) {
     if (o->props->cosched >= 0) return o->props->cosched;
     int result = 0;
     int* d = nullptr;
-    cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr;
+    Graph probe;
     cudaStream_t st = o->own_stream;
     if (cudaMalloc(&d, 4 * sizeof(int)) != cudaSuccess) { cudaGetLastError(); return 0; }
-    bool ok = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
-    if (ok) {
-        ok = cudaEventRecord(o->ev_fork, st) == cudaSuccess && cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) == cudaSuccess;
-        if (ok) { k_probe<<<1, 1, 0, o->side_stream>>>(d, d + 2, 0, 5000000ll); ok = cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess; }
-        if (ok) { k_probe<<<1, 1, 0, st>>>(d, d + 2, 1, 5000000ll); ok = cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess; }
-        cudaError_t e = cudaStreamEndCapture(st, &graph);
-        ok = ok && e == cudaSuccess && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess;
+    bool ok = capture(st, [&] {
+        bool ok2 = cudaEventRecord(o->ev_fork, st) == cudaSuccess && cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) == cudaSuccess;
+        if (ok2) ok2 = launch(k_probe, 1, 1, 0, o->side_stream, false, d, d + 2, 0, 5000000ll) == 0 && cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess;
+        if (ok2) ok2 = launch(k_probe, 1, 1, 0, st, false, d, d + 2, 1, 5000000ll) == 0 && cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
+        return ok2 ? 0 : LMCMA_B200_ERR_CUDA;
+    }, &probe) == 0;
+    for (int attempt = 0; attempt < 2 && ok; ++attempt) {
+        int h[4] = {0, 0, 0, 0};
+        ok = cudaMemcpyAsync(d, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess && replay(probe, st) == 0 &&
+             cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, st) == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+        result = ok && h[2] == 1 && h[3] == 1;
     }
-    if (ok) {
-        for (int attempt = 0; attempt < 2 && ok; ++attempt) {
-            int h[4] = {0, 0, 0, 0};
-            ok = cudaMemcpyAsync(d, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess && cudaGraphLaunch(exec, st) == cudaSuccess &&
-                 cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, st) == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
-            result = ok && h[2] == 1 && h[3] == 1;
-        }
-        g_launches += 4;
-    }
-    if (exec) cudaGraphExecDestroy(exec);
-    if (graph) cudaGraphDestroy(graph);
+    drop(probe);
     cudaFree(d);
     cudaGetLastError();
     o->props->cosched = result;
@@ -451,11 +422,8 @@ int lmcma_capi::check_lost(lmcma_b200_opt* o) {
     *reinterpret_cast<volatile int*>(o->err_host) = 0;
     o->overlap = false;
     o->props->cosched = 0;
-    if (o->graph_exec) { cudaGraphExecDestroy(o->graph_exec); o->graph_exec = nullptr; }
-    if (o->graph_exec_multi) { cudaGraphExecDestroy(o->graph_exec_multi); o->graph_exec_multi = nullptr; }
-    if (o->tell_graph) { cudaGraphExecDestroy(o->tell_graph); o->tell_graph = nullptr; }
-    if (o->tell_graph_resume) { cudaGraphExecDestroy(o->tell_graph_resume); o->tell_graph_resume = nullptr; }
-    o->spec_valid = false;
+    drop_fused_graphs(o);
+    drop_tell_graphs(o);
     o->tell_graph_failed = true;
     o->mirror_dirty = true;
     return fail(LMCMA_B200_ERR_CUDA, "overlapped generation lost co-scheduling (%s): the branches of the CUDA graph did not run "
@@ -466,22 +434,17 @@ int lmcma_capi::check_lost(lmcma_b200_opt* o) {
 namespace {
 
 int ensure_graph(lmcma_b200_opt* o) {
-    if (o->graph_exec && o->graph_built_for == o->stream) return 0;
-    if (o->graph_exec) { cudaGraphExecDestroy(o->graph_exec); o->graph_exec = nullptr; }
-    if (o->graph_exec_multi) { cudaGraphExecDestroy(o->graph_exec_multi); o->graph_exec_multi = nullptr; }
+    if (o->graph.exec && o->graph_built_for == o->stream) return 0;
+    drop_fused_graphs(o);
     CostArgs ca;
     int rc = cost_args_for(o, &ca);
     if (rc) return rc;
     cudaStream_t st = o->stream;
     if ((rc = ensure_mirror(o, st))) return rc;
-    const long long before = g_launches.load();
-    if (o->tune.graph_dbg && !o->graph_dbg && cudaMalloc(&o->graph_dbg, 64 * sizeof(long long)) == cudaSuccess) { cudaMemset(o->graph_dbg, 0, 64 * sizeof(long long)); cudaDeviceSynchronize(); }
+    ensure_graph_dbg(o);
     // `reps` generations in ONE graph: between two graph launches the device idles for the launch latency of the next one
     // (~5 us of a 52 us generation); inside a graph a generation follows the previous one as a plain dependency
-    auto capture = [&](int reps, cudaGraphExec_t* out) -> int {
-        cudaGraph_t graph = nullptr;
-        CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-        o->mirror_suppressed = true;                             // fused generations keep the candidates on the device
+    auto body = [&](int reps) -> int {
         UpdateArgs ua = update_args_local(o);
         ua.progressive = o->progressive ? 1 : 0;                 // ensure_mirror above: the mirror is clean
         ua.dbg = o->graph_dbg;
@@ -494,7 +457,7 @@ int ensure_graph(lmcma_b200_opt* o) {
                 if (cudaEventRecord(o->ev_fork, st) != cudaSuccess || cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph fork failed");
                 if (!rc2) rc2 = launch_update(o, ua, false, o->side_stream);
                 if (!rc2 && cudaEventRecord(o->ev_join, o->side_stream) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph join record failed");
-                if (!rc2) { k_gate<<<(o->d.B + 31) / 32, 32, 0, st>>>(o->d); g_launches++; }
+                if (!rc2) rc2 = launch(k_gate, (o->d.B + 31) / 32, 32, 0, st, false, o->d);
                 if (!rc2) rc2 = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
                 if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN | RANK_KEEP_FLAGS | (o->tune.rank_late ? 0 : 4), nullptr, st, true);
                 if (!rc2) rc2 = launch_sample(o, st, true, true, 2);
@@ -506,27 +469,17 @@ int ensure_graph(lmcma_b200_opt* o) {
                 if (!rc2) rc2 = launch_sample(o, st, true, o->progressive);
             }
         }
-        cudaError_t e = cudaStreamEndCapture(st, &graph);
-        o->mirror_suppressed = false;
-        if (!rc2 && e == cudaSuccess) {
-            e = cudaGraphInstantiate(out, graph, 0);
-            if (e != cudaSuccess) *out = nullptr;
-        }
-        if (graph) cudaGraphDestroy(graph);
-        if (!rc2 && e != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph capture / instantiate failed: %s", cudaGetErrorString(e));
         return rc2;
     };
-    rc = capture(1, &o->graph_exec);
-    if (!rc && o->tune.graph_unroll > 1 && capture(o->tune.graph_unroll, &o->graph_exec_multi) != 0) {   // optional: the single one still works
-        cudaGetLastError();
-        o->graph_exec_multi = nullptr;
-    }
-    g_launches.store(before);   // capture enqueues nothing
+    o->mirror_suppressed = true;                                 // fused generations keep the candidates on the device
+    rc = capture(st, [&] { return body(1); }, &o->graph);
+    if (!rc && o->tune.graph_unroll > 1 && capture(st, [&] { return body(o->tune.graph_unroll); }, &o->graph_multi) != 0)
+        cudaGetLastError();                                      // optional: the single one still works
+    o->mirror_suppressed = false;
     if (rc && o->overlap) {
         // the forked graph could not be built here (capture / instantiation of the side branch): fall back to the linear one
         cudaGetLastError();
-        if (o->graph_exec) { cudaGraphExecDestroy(o->graph_exec); o->graph_exec = nullptr; }
-    if (o->graph_exec_multi) { cudaGraphExecDestroy(o->graph_exec_multi); o->graph_exec_multi = nullptr; }
+        drop_fused_graphs(o);
         o->overlap = false;
         return ensure_graph(o);
     }
@@ -537,10 +490,8 @@ int ensure_graph(lmcma_b200_opt* o) {
 
 // tell_all of one query as a forked graph (see lmcma_b200_tell_all); on failure the caller takes the stream-ordered path
 int ensure_tell_graph(lmcma_b200_opt* o) {
-    if (o->tell_graph && o->tell_graph_for == o->stream) return ensure_mirror(o, o->stream);
-    if (o->tell_graph) { cudaGraphExecDestroy(o->tell_graph); o->tell_graph = nullptr; }
-    if (o->tell_graph_resume) { cudaGraphExecDestroy(o->tell_graph_resume); o->tell_graph_resume = nullptr; }
-    o->spec_valid = false;
+    if (o->tell_graph.exec && o->tell_graph_for == o->stream) return ensure_mirror(o, o->stream);
+    drop_tell_graphs(o);
     cudaStream_t st = o->stream;
     const OptDev& d = o->d;
     int rc = ensure_mirror(o, st);
@@ -548,18 +499,15 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
     if (!o->f_pinned && cudaHostAlloc(&o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaHostAllocDefault) != cudaSuccess) {
         cudaGetLastError(); o->f_pinned = nullptr; o->tell_graph_failed = true; return 0;
     }
-    const long long before = g_launches.load();
     // the speculative pass pays only where something hides it: with the host mirror on, the candidates' trip across PCIe
     // (35 us behind the sampler).  Without the mirror tell_all returns when the sampler is done, and a 25 us kernel behind
     // k_update would be the longer branch of the graph (measured: tell_all 57 -> 69 us)
     const bool spec = o->d_spec != nullptr && o->mirror_on && !o->mirror_suppressed;
     o->tell_graph_spec = spec;
-    if (o->tune.graph_dbg && !o->graph_dbg && cudaMalloc(&o->graph_dbg, 64 * sizeof(long long)) == cudaSuccess) { cudaMemset(o->graph_dbg, 0, 64 * sizeof(long long)); cudaDeviceSynchronize(); }
+    ensure_graph_dbg(o);
     // resume = 0: the whole update; resume = 1: k_update picks up the rows the last graph's speculative pass left.  With the
     // scratch both graphs END with that pass for the next generation, on the side branch behind k_update
-    auto capture = [&](int resume, cudaGraphExec_t* out) -> int {
-        cudaGraph_t graph = nullptr;
-        CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+    auto body = [&](int resume) -> int {
         UpdateArgs ua = update_args_local(o);
         ua.progressive = 1;
         ua.overlap = 1;
@@ -572,24 +520,20 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
         o->spec_valid = valid_before;                            // capture enqueues nothing
         if (ok) ok = cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess;
         if (ok) ok = cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st) == cudaSuccess;
-        if (ok) { k_gate<<<(d.B + 31) / 32, 32, 0, st>>>(d); ok = cudaGetLastError() == cudaSuccess; }   // k_update has reset the flags and holds its SM
+        if (ok) ok = launch(k_gate, (d.B + 31) / 32, 32, 0, st, false, d) == 0;   // k_update has reset the flags and holds its SM
         // the sampler is released when k_rank starts: the pairs it needs first are final (resume: at once; else as the sweep goes)
         if (ok) ok = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS | (o->tune.rank_late ? 0 : 4), nullptr, st, false) == 0;
         if (ok) ok = launch_sample(o, st, true, true, 2) == 0;
         if (ok) ok = cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
-        cudaError_t e = cudaStreamEndCapture(st, &graph);
-        if (ok && e == cudaSuccess && cudaGraphInstantiate(out, graph, 0) != cudaSuccess) *out = nullptr;
-        if (graph) cudaGraphDestroy(graph);
-        return 0;
+        return ok ? 0 : LMCMA_B200_ERR_CUDA;
     };
-    rc = capture(0, &o->tell_graph);
-    if (!rc && o->tell_graph && spec) rc = capture(1, &o->tell_graph_resume);
-    g_launches.store(before);   // capture enqueues nothing
-    if (rc) return rc;
-    if (!o->tell_graph || (spec && !o->tell_graph_resume)) {
+    rc = capture(st, [&] { return body(0); }, &o->tell_graph);
+    if (!rc && spec) rc = capture(st, [&] { return body(1); }, &o->tell_graph_resume);
+    if (rc) {
         cudaGetLastError();
-        if (o->tell_graph) { cudaGraphExecDestroy(o->tell_graph); o->tell_graph = nullptr; }
-        o->tell_graph_failed = true; return 0;
+        drop_tell_graphs(o);
+        o->tell_graph_failed = true;
+        return 0;
     }
     o->tell_graph_for = st;
     return 0;
@@ -806,10 +750,8 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     void* ptrs[] = {d.prev_sorted, d.tile_sorted, d.tile_pos, d.X, d.D, d.Z, d.Zc, o->d_Lf, d.fit, d.fit_sorted, d.prev_fit, d.rank, d.arindex, d.ncoll, d.nsamp, d.xmean, d.pc, d.V, d.P,
                     d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends};
     for (void* p : ptrs) cudaFree(p);
-    if (o->graph_exec) cudaGraphExecDestroy(o->graph_exec);
-    if (o->graph_exec_multi) cudaGraphExecDestroy(o->graph_exec_multi);
-    if (o->tell_graph) cudaGraphExecDestroy(o->tell_graph);
-    if (o->tell_graph_resume) cudaGraphExecDestroy(o->tell_graph_resume);
+    drop_fused_graphs(o);
+    drop_tell_graphs(o);
     cudaFree(o->d_spec);
     if (o->f_pinned) cudaFreeHost(o->f_pinned);
     if (o->err_host) cudaFreeHost(o->err_host);
@@ -894,9 +836,7 @@ int lmcma_b200_ask_all_view(lmcma_b200_opt* o, const float** X_view, int64_t* ld
         o->xh_fresh = false;
         register_mirror(o->x_mirror, floats * sizeof(float), d.X, d.ns, o->cfg.device);
         // the captured graphs carry the old kernel parameters (OptDev by value): rebuild them on next use
-        if (o->tell_graph) { cudaGraphExecDestroy(o->tell_graph); o->tell_graph = nullptr; }
-        if (o->tell_graph_resume) { cudaGraphExecDestroy(o->tell_graph_resume); o->tell_graph_resume = nullptr; }
-        o->spec_valid = false;
+        drop_tell_graphs(o);
     }
     if (!o->xh_fresh) {                                  // first use / after a fused run or a state setter: one ordinary copy
         CU(cudaMemcpyAsync(o->x_mirror, d.X, floats * sizeof(float), cudaMemcpyDeviceToHost, o->stream));
@@ -922,12 +862,11 @@ int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
         // k_sample follows its hand-over flags.  Same kernels and arithmetic as the fused generation (bit-identical to the
         // serial order), replayed as one CUDA graph: launched kernel by kernel, the fork / join costs more host time than
         // the overlap saves.
-        if ((rc = ensure_tell_graph(o)) == 0 && o->tell_graph) {
+        if ((rc = ensure_tell_graph(o)) == 0 && o->tell_graph.exec) {
             memcpy(o->f_pinned, f, (size_t)d.B * d.lambda * sizeof(float));
-            const bool resume = o->spec_valid && o->tell_graph_resume;   // the last tell_all graph left the next update's rows behind
-            CU(cudaGraphLaunch(resume ? o->tell_graph_resume : o->tell_graph, o->stream));
+            const bool resume = o->spec_valid && o->tell_graph_resume.exec;   // the last tell_all graph left the next update's rows behind
+            if ((rc = replay(resume ? o->tell_graph_resume : o->tell_graph, o->stream))) return rc;
             o->spec_valid = o->tell_graph_spec;                   // ... and so does this one
-            g_launches += 4 + (o->d.tile_sorted ? 1 : 0) + (o->tell_graph_spec ? 1 : 0);   // k_update, k_gate, (k_rank_tiles,) k_rank, k_sample, (speculative k_update)
             o->xh_fresh = o->mirror_on;                          // the captured sampler writes the host mirror when it is on
             o->x_cache_valid = false;
             o->sample_idx = 0;
@@ -998,8 +937,7 @@ int lmcma_b200_attach_cost(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b
     if (!o->d_ends) DM(o->d_ends, (size_t)o->d.B * 6);
     CU(cudaMemcpy(o->d_ends, e6.data(), e6.size() * sizeof(float), cudaMemcpyHostToDevice));
     o->cost_shape = pick_cost_shape(obj->waypoints, ends[0].start, ends[0].goal, map->dev.dims, o->tune);
-    if (o->graph_exec) { cudaGraphExecDestroy(o->graph_exec); o->graph_exec = nullptr; }
-    if (o->graph_exec_multi) { cudaGraphExecDestroy(o->graph_exec_multi); o->graph_exec_multi = nullptr; }
+    drop_fused_graphs(o);
     return 0;
 }
 
@@ -1016,13 +954,11 @@ int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
         if ((rc = ensure_graph(o))) return rc;
         if ((rc = ensure_mirror(o, o->stream))) return rc;       // a state setter since the last run: the graph's sampler reads the mirror
         CU(cudaEventRecord(o->ev0, o->stream));                  // after the (host-side) graph build: last_run_ms is device time
-        const int unroll = o->graph_exec_multi ? o->tune.graph_unroll : 0;
+        const int unroll = o->graph_multi.exec ? o->tune.graph_unroll : 0;
         for (int g = 0; g < generations;) {
             const bool multi = unroll > 1 && generations - g >= unroll;
-            CU(cudaGraphLaunch(multi ? o->graph_exec_multi : o->graph_exec, o->stream));
-            const int done = multi ? unroll : 1;
-            g_launches += (long long)done * (4 + (o->d_Lf ? (o->cfg.rng == LMCMA_B200_RNG_PHILOX ? 2 : 1) : 0) + (o->upd_gram ? 3 : 0) + (o->overlap ? 1 : 0) + (o->d.tile_sorted ? 1 : 0));
-            g += done;
+            if ((rc = replay(multi ? o->graph_multi : o->graph, o->stream))) return rc;
+            g += multi ? unroll : 1;
         }
     } else {
         if (o->cfg.rng == LMCMA_B200_RNG_INJECT && generations > 1)

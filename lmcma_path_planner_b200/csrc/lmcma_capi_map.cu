@@ -17,12 +17,7 @@ int launch_cost_t(const MapDev& mp, const CostArgs& a0, int rows, int B, CostSha
     // + the candidate row (16-byte aligned)
     const size_t smem = (size_t)36 * (a.W + 1) + sizeof(int) * (a.W + 2) + 28 + (size_t)8 * shape.cb + (STORAGE == 1 ? 1024 : 0) +
                         sizeof(float) * DIMS * ((size_t)a.W + 2) + 16;
-    auto kern = k_cost<DIMS, STORAGE, TRACE, MINB>;
-    if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<dim3(rows, B), shape.tpt, smem, st>>>(mp, a);
-    g_launches++;
-    CU(cudaGetLastError());
-    return 0;
+    return launch(k_cost<DIMS, STORAGE, TRACE, MINB>, dim3(rows, B), shape.tpt, smem, st, false, mp, a);
 }
 
 }  // namespace
@@ -176,16 +171,8 @@ static int map_alloc(int device, int dims, const int32_t* shape, int storage, fl
 static int map_fill_from_dist_dev(lmcma_b200_map* m, const float* d_dist, cudaStream_t st) {
     const MapDev& d = m->dev;
     const unsigned blocks = (unsigned)((m->cells + 255) / 256);
-    if (d.dims == 2) {
-        if (m->storage == 0) k_brick<2, 0><<<blocks, 256, 0, st>>>(d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
-        else k_brick<2, 1><<<blocks, 256, 0, st>>>(d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
-    } else {
-        if (m->storage == 0) k_brick<3, 0><<<blocks, 256, 0, st>>>(d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
-        else k_brick<3, 1><<<blocks, 256, 0, st>>>(d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
-    }
-    g_launches++;
-    CU(cudaGetLastError());
-    return 0;
+    auto kern = d.dims == 2 ? (m->storage == 0 ? k_brick<2, 0> : k_brick<2, 1>) : (m->storage == 0 ? k_brick<3, 0> : k_brick<3, 1>);
+    return launch(kern, blocks, 256, 0, st, false, d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
 }
 
 // exact Euclidean distance transform on the device (k_edt.cuh): d_occ (1 = obstacle) -> d_dist, both row-major [z][y][x]
@@ -200,24 +187,13 @@ static int edt_device(int dims, const int32_t* shape, const unsigned char* d_occ
     if (!rc) rc = dmalloc(&t, cells);
     if (!rc) rc = dmalloc(&gh, cells);
     if (!rc) {
-        const long long nlines = (long long)ny * nz;
-        k_edt_x<<<(unsigned)((nlines + 7) / 8), 256, 0, st>>>(d_occ, d2, nx, nlines);
-        g_launches++;
-        if (ny > 1) {
-            const long long lines = (long long)nx * nz;
-            k_edt_axis<<<(unsigned)((lines + 127) / 128), 128, 0, st>>>(d2, ny, nx, nx, nz, (long long)nx * ny, s, t, gh);
-            g_launches++;
-        }
-        if (nz > 1) {
-            const long long lines = (long long)nx * ny;
-            k_edt_axis<<<(unsigned)((lines + 127) / 128), 128, 0, st>>>(d2, nz, (long long)nx * ny, nx * ny, 1, 0, s, t, gh);
-            g_launches++;
-        }
-        k_edt_finish<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(d2, d_dist, (long long)cells, clamp);
-        g_launches++;
+        const long long nlines = (long long)ny * nz, ylines = (long long)nx * nz, zlines = (long long)nx * ny;
+        rc = launch(k_edt_x, (unsigned)((nlines + 7) / 8), 256, 0, st, false, d_occ, d2, nx, nlines);
+        if (!rc && ny > 1) rc = launch(k_edt_axis, (unsigned)((ylines + 127) / 128), 128, 0, st, false, d2, ny, nx, nx, nz, (long long)nx * ny, s, t, gh);
+        if (!rc && nz > 1) rc = launch(k_edt_axis, (unsigned)((zlines + 127) / 128), 128, 0, st, false, d2, nz, (long long)nx * ny, nx * ny, 1, 0, s, t, gh);
+        if (!rc) rc = launch(k_edt_finish, (unsigned)((cells + 255) / 256), 256, 0, st, false, d2, d_dist, (long long)cells, clamp);
         cudaError_t e = cudaStreamSynchronize(st);
-        if (e == cudaSuccess) e = cudaGetLastError();
-        if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "distance transform: %s", cudaGetErrorString(e));
+        if (!rc && e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "distance transform: %s", cudaGetErrorString(e));
     }
     cudaFree(d2); cudaFree(s); cudaFree(t); cudaFree(gh);
     return rc;

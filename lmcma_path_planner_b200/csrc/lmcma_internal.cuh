@@ -15,6 +15,7 @@
 #include <limits>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 #include "../../include/lmcma_b200.h"
 #include "lmcma_host.hpp"
@@ -25,6 +26,7 @@ using namespace lmcma;
 
 extern thread_local std::string g_err;     // lmcma_capi.cu
 extern std::atomic<long long> g_launches;
+extern thread_local long long* g_capture_launches;   // while this thread captures a graph: its count of the kernels captured
 
 inline int fail(int code, const char* fmt, ...) {
     char buf[512];
@@ -63,6 +65,31 @@ inline int dmalloc(T** p, size_t count) {
         int rc__ = dmalloc(&(ptr), (count));        \
         if (rc__) return rc__;                      \
     } while (0)
+
+// Every kernel of the library is launched here.  Dynamic shared memory above 48 KiB is opted into; pdl makes the kernel a
+// programmatic dependent of the kernel enqueued just before it on `st`.  The launch is counted in g_launches, or, while
+// this thread captures a graph, in the graph's own count, which each replay adds (lmcma_capi.cu: capture / replay).
+template <class... P, class... A>
+int launch(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, A&&... args) {
+    if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
+    CU(cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...));
+    if (g_capture_launches) ++*g_capture_launches;
+    else g_launches++;
+    return 0;
+}
+
+// an instantiated CUDA graph and the number of kernels it holds (what one replay adds to lmcma_b200_launch_count)
+struct Graph {
+    cudaGraphExec_t exec = nullptr;
+    int launches = 0;
+};
 
 
 inline int env_int(const char* name, int dflt) {
@@ -194,16 +221,16 @@ struct lmcma_b200_opt {
     lmcma_b200_objective obj{};
     float* d_ends = nullptr;
     // graph
-    cudaGraphExec_t graph_exec = nullptr;
-    cudaGraphExec_t graph_exec_multi = nullptr;   // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)
+    lmcma_capi::Graph graph;                  // one fused generation (lmcma_b200_run)
+    lmcma_capi::Graph graph_multi;            // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)
     cudaStream_t graph_built_for = nullptr;
-    cudaGraphExec_t tell_graph = nullptr;     // tell_all of one query: H2D fitness -> k_rank -> k_sample, k_update on a side branch
+    lmcma_capi::Graph tell_graph;             // tell_all of one query: H2D fitness -> k_rank -> k_sample, k_update on a side branch
     cudaStream_t tell_graph_for = nullptr;
     bool tell_graph_failed = false;
     // speculative update (k_update.cuh, UpdateArgs::phase): every tell_all graph ends with the fitness-independent part of the
     // NEXT generation's update (into d_spec, beside the sampler's tail and the candidates' trip across PCIe); the next tell_all
     // resumes from it (tell_graph_resume) unless anything else touched the optimiser's state in between
-    cudaGraphExec_t tell_graph_resume = nullptr;
+    lmcma_capi::Graph tell_graph_resume;
     float* d_spec = nullptr; size_t spec_stride = 0;
     bool spec_valid = false;
     bool tell_graph_spec = false;             // the tell graphs were captured with the speculative pass (host mirror on)
