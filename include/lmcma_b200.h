@@ -256,9 +256,11 @@ enum {
 };
 /* fields of LMCMA_B200_I32_LAUNCH.  Sampler kernels: 0 = k_sample<NV> (narrow), 1 = k_sample_wide<RBW> (a row split over CW
  * column-warps, R row groups per CTA), 2 = k_sample_rows<QW, RL> (rows on lanes).  KC / STAGES are those of the chosen
- * sampler.  The update is k_update<NVB, RMAX, ROWS_IN_SMEM, OVERLAP, WARPS> (SWEEP_WARPS of them sweep), or with GRAM the
- * Gram-matrix recompute whose k_coef keeps COEF_ELEMS elements per lane (0 without GRAM).  The overlapped k_update build
- * is the one of the fused generations and of tell_all when OVERLAP is 1. */
+ * sampler.  The update is k_update<NVB, RMAX, ROWS_IN_SMEM, OVERLAP, WARPS>, or with GRAM the Gram-matrix recompute whose
+ * k_coef keeps COEF_ELEMS elements per lane (0 without GRAM).  The overlapped k_update build is the one of the fused
+ * generations and of tell_all when OVERLAP is 1.  Two fields no longer vary and keep their place: SMP_SPEC is always 1
+ * (the NV = 4 narrow sampler runs full groups of pairs without per-pair predicates), and SWEEP_WARPS equals UPD_WARPS
+ * (every warp of k_update's CTA owns rows of the register sweep). */
 enum {
     LMCMA_B200_LAUNCH_SAMPLER = 0, LMCMA_B200_LAUNCH_SMP_NV, LMCMA_B200_LAUNCH_SMP_SPEC, LMCMA_B200_LAUNCH_SMP_THREADS,
     LMCMA_B200_LAUNCH_SMP_RBW, LMCMA_B200_LAUNCH_SMP_CW, LMCMA_B200_LAUNCH_SMP_R, LMCMA_B200_LAUNCH_SMP_ROWS_QW,

@@ -8,7 +8,7 @@
 // ever waits on another — folds the partials into the all-gather payload.
 // Every CTA also adds one ticket to OptDev::rank_ticket after its last store: the overlapped generation's k_update is not
 // a stream successor of this grid and waits for RS tickets (RANK_KEEP_FLAGS: the hand-over flags are then k_update's to
-// reset, and the dependent grid — the sampler — is released when the CTA is done, not after the wait on k_cost).
+// reset, and the dependent grid is the sampler).
 #pragma once
 #include "lmcma_common.cuh"
 
@@ -284,12 +284,10 @@ __global__ void __launch_bounds__(MAXT, 2) k_rank(OptDev o, const float* __restr
     const bool prev_staged = o.lambda <= TELL_FTILE;              // one tile, one pass: staged once, ahead of the wait
     tell_prologue(o, blockIdx.y, blockIdx.x, smem_raw);
     griddep_wait();
-    // overlapped generation (RANK_KEEP_FLAGS): the dependent is k_sample.  mode & 4 (the fused generation's default): released
-    // here, so that it works through the pairs k_update has already finished while this grid ranks (its 128 CTAs share SMs
-    // with this grid: the ranks arrive ~1 us later, the sampler is done 8 us earlier).  Otherwise (tell_all, where the sweep is
-    // the longer branch; LMCMA_B200_RANK_LATE=1) it is released when this CTA is done
-    const bool late_release = (mode & RANK_KEEP_FLAGS) && !(mode & 4);
-    if (!late_release) griddep_launch_dependents();
+    // The dependent is released here, as soon as the fitness is there.  In the overlapped generation and tell_all
+    // (RANK_KEEP_FLAGS) it is k_sample, which then works through the pairs k_update has already finished while this grid
+    // ranks (its CTAs share SMs with this grid: the ranks arrive ~1 us later, the sampler is done 8 us earlier)
+    griddep_launch_dependents();
     const int b = blockIdx.y;
     // the hand-over flags of this generation's k_update -> k_sample (both start after this grid has completed)
     if (blockIdx.x == 0 && !(mode & RANK_KEEP_FLAGS)) for (int i = threadIdx.x; i < o.m + 2; i += blockDim.x) o.progress[(size_t)b * (o.m + 2) + i] = 0;
@@ -302,7 +300,6 @@ __global__ void __launch_bounds__(MAXT, 2) k_rank(OptDev o, const float* __restr
         atomicAdd(o.rank_ticket + b, 1u);
         if (o.dbg && b == 0 && blockIdx.x == gridDim.x - 1) o.dbg[21] = gtime();
     }
-    if (late_release) griddep_launch_dependents();
     if (!(mode & RANK_PACK)) return;
     __threadfence();
     __syncthreads();

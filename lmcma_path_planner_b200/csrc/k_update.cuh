@@ -36,8 +36,6 @@ struct UpdateArgs {
     long long slice_stride, inst_stride;
     int payload_mode;          // slices are all-gather payloads (S rides in the 2 floats after ns)
     long long* dbg;            // optional: globaltimer stamps (LMCMA_B200_UPDATE_DBG)
-    int blocked;               // register sweep: a warp owns R CONSECUTIVE rows (else rows w, w + sweep_warps, ...)
-    int sweep_warps;           // register sweep: warps that own rows (<= UPD_WARPS; every warp pays a fixed cost per step)
     int overlap;               // fused single-query generation: this kernel runs on a side branch of the graph, CONCURRENTLY
                                // with k_cost and k_rank.  Everything that does not depend on this generation's fitness —
                                // bookkeeping, and the sweep over every pending row but the newest — comes first; then it
@@ -52,7 +50,6 @@ struct UpdateArgs {
                                // Same arithmetic on the same inputs: bit-identical to phase 0
     float* spec;               // phase 1 / 2 scratch of one instance x spec_stride floats (layout: spec_* below)
     long long spec_stride;
-    int no_dry;                // overlapped generation: skip the pre-execution pass of the post-rank code (LMCMA_B200_UPDATE_DRY=0)
     int progressive;           // publish OptDev::progress flags as the outputs become final: k_sample (launched as a
                                // programmatic dependent) consumes the pairs while the sweep is still producing them
 };
@@ -70,7 +67,7 @@ __host__ __device__ __forceinline__ size_t spec_floats(int m, int ns) { return s
 template <bool SMEM> __device__ __forceinline__ float4 ld_row4(const float4* p) { return SMEM ? *p : __ldcg(p); }
 
 // NVB  = float4 column slots per lane (ns <= 128 * NVB)
-// RMAX = pending rows a warp can hold in registers (m <= UPD_WARPS * RMAX); 0 = streaming sweep (rows stay in
+// RMAX = pending rows a warp can hold in registers (m <= WARPS * RMAX); 0 = streaming sweep (rows stay in
 //        shared memory, or in HBM/L2 when SMEM is false); -1 = no sweep here: the recompute is done by the Gram-matrix
 //        kernels (k_gram.cuh) for shapes whose rows fit neither registers nor shared memory; this kernel then only
 //        hands them {first_stale, live}
@@ -443,14 +440,13 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     if (RMAX < 0) {
         // the Gram-matrix kernels take it from here (they also write Nj / Lj)
     } else if (RMAX > 0) {
-        // ---------------- register sweep: warp w owns rows first_stale + w + r * UPD_WARPS ----------------
+        // ---------------- register sweep: warp w owns rows first_stale + w + r * WARPS ----------------
         constexpr int R = RMAX > 0 ? RMAX : 1;
-        const int sw = a.sweep_warps;
-        const int rstride = a.blocked ? 1 : sw;
+        constexpr int rstride = WARPS;
         // The newest row (this generation's evolution path) is not part of the sweep: it takes its factors a BLOCK at a time
         // (newest_row below).  In the overlapped generation it does not even exist yet when the sweep starts.
         const int hi = live - 1;
-        const int base = (warp < sw && phase != 2) ? first_stale + (a.blocked ? warp * R : warp) : hi;     // warps >= sw own nothing; phase 2: no sweep
+        const int base = phase != 2 ? first_stale + warp : hi;      // phase 2: no sweep
         float4 y[R][NVB];
 #pragma unroll
         for (int r = 0; r < R; ++r) {
@@ -793,7 +789,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
             for (int step = 0; step < 4; ++step) {
                 const bool dry = step < 2;
                 if (dry) {
-                    if (tid == 32) sh_dry = (*reinterpret_cast<const volatile int*>(o.rank_ticket + b) != (int)need && !a.no_dry) ? 1 : 0;
+                    if (tid == 32) sh_dry = *reinterpret_cast<const volatile int*>(o.rank_ticket + b) != (int)need ? 1 : 0;
                     __syncthreads();
                     if (!sh_dry) { step = 1; continue; }
                 } else if (step == 2) {

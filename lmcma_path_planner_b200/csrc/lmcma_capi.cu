@@ -60,11 +60,7 @@ int launch_sample_rows(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_
 }
 
 int launch_sample_wide(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st, int progressive) {
-    switch (o->smp_RBW) {
-        case 1: return launch_sample_wide_t<1, 1024>(o, d, pdl, st, progressive);
-        case 2: return launch_sample_wide_t<2, 1024>(o, d, pdl, st, progressive);
-        default: return launch_sample_wide_t<4, 512>(o, d, pdl, st, progressive);
-    }
+    return o->smp_RBW == 2 ? launch_sample_wide_t<2, 1024>(o, d, pdl, st, progressive) : launch_sample_wide_t<4, 512>(o, d, pdl, st, progressive);
 }
 
 // the sequence-ordered (v, pc) mirror k_sample streams from is maintained by k_update; after create or a state
@@ -100,7 +96,7 @@ int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool pro
     switch (o->smp_nv) {
         case 1: return launch_sample_t<1, 4, 512>(o, d, pdl, st);
         case 2: return launch_sample_t<2, 4, 512>(o, d, pdl, st);
-        case 4: return o->tune.sample_spec ? launch_sample_t<4, 2, 512, true>(o, d, pdl, st) : launch_sample_t<4, 2, 512>(o, d, pdl, st);
+        case 4: return launch_sample_t<4, 2, 512, true>(o, d, pdl, st);
         case 8: return launch_sample_t<8, 1, 512>(o, d, pdl, st);
         case 12: return launch_sample_t<12, 1, 256>(o, d, pdl, st);
         case 16: return launch_sample_t<16, 1, 256>(o, d, pdl, st);
@@ -120,43 +116,36 @@ int configure_sample(lmcma_b200_opt* o) {
     const int maxt = o->smp_nv >= 12 ? 256 : 512;
     // as many warps per CTA as keeps >= ~1 CTA per SM
     int threads = maxt;
-    const int forced = o->tune.sample_threads;
-    if (forced >= 32 && forced <= maxt && forced % 32 == 0) threads = forced;
-    else
-        while (threads > 64) {
-            const int rows_per_cta = (threads / 32) * o->smp_rb;
-            const long long ctas = (long long)((o->d.pop_count + rows_per_cta - 1) / rows_per_cta) * o->d.B;
-            if (ctas * 4 >= (long long)o->props->sm_count * 3) break;   // bigger tiles re-read the pairs less often
-            threads >>= 1;
-        }
+    while (threads > 64) {
+        const int rows_per_cta = (threads / 32) * o->smp_rb;
+        const long long ctas = (long long)((o->d.pop_count + rows_per_cta - 1) / rows_per_cta) * o->d.B;
+        if (ctas * 4 >= (long long)o->props->sm_count * 3) break;   // bigger tiles re-read the pairs less often
+        threads >>= 1;
+    }
     o->smp_threads = threads;
     const size_t pair_bytes = (size_t)2 * o->d.ns * sizeof(float);
     // pairs per stage: one group of 8 when it fits (else 4 / 2 / 1); as many stages as the live pairs need, within
-    // ~160 KB, so that for the common shapes every pair is requested up front and nothing is re-issued
-    const size_t budget = (size_t)o->tune.sample_smem_kb * 1024;
+    // 160 KB, so that for the common shapes every pair is requested up front and nothing is re-issued
+    const size_t budget = (size_t)160 * 1024;
     int kc = (int)(budget / 2 / pair_bytes);
     kc = kc >= 8 ? 8 : (kc >= 4 ? 4 : (kc >= 2 ? 2 : 1));
     // long rows (C4: 12 KB per pair): two stages of a FULL group of 8 still fit one SM (192 KB), and a 4-pair stage runs the
     // 8-wide group code half empty
-    if (kc == 4 && 2 * 8 * pair_bytes + 24 * 1024 <= o->props->smem_optin && o->tune.sample_smem_kb_set == 0) kc = 8;
+    if (kc == 4 && 2 * 8 * pair_bytes + 24 * 1024 <= o->props->smem_optin) kc = 8;
     o->smp_kc = kc;
     const int max_chunks = (o->d.m + kc - 1) / kc;
     o->smp_stages = (int)std::max<size_t>(2, std::min<size_t>(std::min(max_chunks, SAMPLE_MAX_STAGES), budget / (kc * pair_bytes)));   // >= 2 even beyond the budget
     o->smp_smem = (size_t)o->smp_stages * kc * pair_bytes + SAMPLE_MAX_STAGES * 8 + (size_t)(2 * o->d.m + 16) * sizeof(float);
     // one large population: split every row over CW column-warps (k_sample_wide) for occupancy
     o->smp_wide = false;
-    if (o->d.pop_count >= 256 && nq > 32 && !o->tune.sample_narrow) {
+    if (o->d.pop_count >= 256 && nq > 32) {
         o->smp_wide = true;
         o->smp_CW = (nq + 31) / 32;
         o->smp_qpw = (nq + o->smp_CW - 1) / o->smp_CW;
         // rows per warp: 2 (4 for very large populations); row-groups per CTA so that the grid still covers the SMs
-        o->smp_RBW = o->tune.sample_rbw ? o->tune.sample_rbw : (o->d.pop_count >= 1024 ? 4 : 2);
-        if (o->smp_RBW != 1 && o->smp_RBW != 2) o->smp_RBW = 4;
+        o->smp_RBW = o->d.pop_count >= 1024 ? 4 : 2;
         int R = std::max(1, std::min(15, (o->smp_RBW == 4 ? 16 : 32) / o->smp_CW));
-        const int forced_R = o->tune.sample_r;
-        if (forced_R >= 1 && forced_R <= R) R = forced_R;
-        else
-            while (R > 1 && (long long)((o->d.pop_count + R * o->smp_RBW - 1) / (R * o->smp_RBW)) * o->d.B * 4 < (long long)o->props->sm_count * 3) R >>= 1;
+        while (R > 1 && (long long)((o->d.pop_count + R * o->smp_RBW - 1) / (R * o->smp_RBW)) * o->d.B * 4 < (long long)o->props->sm_count * 3) R >>= 1;
         o->smp_R = R;
         o->smp_smem += (size_t)o->smp_stages * ((kc + SAMPLE_G - 1) / SAMPLE_G) * o->smp_R * o->smp_CW * o->smp_RBW * SAMPLE_G * sizeof(float);
     }
@@ -168,7 +157,7 @@ int configure_sample(lmcma_b200_opt* o) {
     // generation (wide sampler only) is given up (fused generation 0.271 -> 0.253 ms at 8192, 1.71 -> 1.41 ms at 65536)
     const bool many = total_rows >= 4096 && o->d.pop_count >= 32 &&
                       (o->d.B > 1 || o->tune.sample_rows == 1 || (o->d.pop_count >= 8192 && o->d.pop_count == o->d.lambda));
-    if (o->tune.sample_rows != 0 && many && nq <= 128 && o->d.m <= 256 && !o->d_Lf) {
+    if (many && nq <= 128 && o->d.m <= 256 && !o->d_Lf) {
         const int NW = 16;
         const int qper = (nq + NW - 1) / NW;
         o->smp_rows_qw = qper <= 4 ? 4 : (qper <= 7 ? 7 : 8);
@@ -211,9 +200,7 @@ int launch_update_t(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream
 
 // the serial part of update() (k_update.cuh).  pdl: launched as a programmatic dependent of the kernel enqueued just
 // before it on `st` (k_rank), so that its prologue overlaps that kernel
-int launch_update(lmcma_b200_opt* o, const UpdateArgs& a_in, bool pdl, cudaStream_t st) {
-    UpdateArgs a = a_in;
-    if (a.sweep_warps <= 0) a.sweep_warps = o->upd_sweep_warps;     // callers that build UpdateArgs from scratch
+int launch_update(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream_t st) {
     if (a.phase == 0) o->spec_valid = false;                        // a whole update: whatever the speculative pass left is stale
     if (o->upd_gram) {
         int rc = o->upd_nvb == 4 ? launch_update_t<4, -1, false>(o, a, pdl, st) : launch_update_t<16, -1, false>(o, a, pdl, st);
@@ -248,9 +235,6 @@ UpdateArgs update_args_local(lmcma_b200_opt* o) {
     memset(&a, 0, sizeof(a));
     a.f_all = o->d.fit;
     a.slices = o->d.partial; a.n_slices = o->d.RS; a.slice_stride = o->d.ns; a.inst_stride = (long long)o->d.RS * o->d.ns;
-    a.blocked = o->tune.update_blocked;
-    a.sweep_warps = o->upd_sweep_warps;
-    a.no_dry = o->tune.update_dry ? 0 : 1;
     a.spec = o->d_spec; a.spec_stride = (long long)o->spec_stride;
     return a;
 }
@@ -274,24 +258,21 @@ int configure_update(lmcma_b200_opt* o) {
     if (o->upd_smem > budget) return fail(LMCMA_B200_ERR_ARG, "k_update needs %zu B shared memory (m = %d too large)", o->upd_smem, o->d.m);
     // rows that fit neither the registers nor the shared memory of one SM: Gram-matrix recompute (k_gram.cuh)
     o->coef_smem = (size_t)2 * o->d.m * (o->d.m | 1) * sizeof(double) + (size_t)2 * o->d.m * sizeof(double);
-    o->upd_gram = (!o->upd_rows_in_smem || o->tune.update_gram) && o->d.m <= 128 && o->coef_smem <= budget && !o->tune.update_streaming;
+    o->upd_gram = (!o->upd_rows_in_smem || o->tune.update_gram) && o->d.m <= 128 && o->coef_smem <= budget;
     if (o->upd_gram) { o->upd_rows_in_smem = false; o->upd_smem = fixed; }
     // k_coef elements per lane: ceil(m / 8), rounded up to a compiled build (m <= 128)
     o->coef_elems = !o->upd_gram ? 0 : (o->d.m <= 40 ? 5 : (o->d.m <= 80 ? 10 : (o->d.m <= 96 ? 12 : 16)));
     // pending rows in registers when they fit: m <= 8 warps x RMAX rows of <= 128 float4 columns
     o->upd_rmax = 0;
     o->upd_warps = UPD_WARPS;
-    if (o->upd_nvb == 4 && o->upd_rows_in_smem && !o->upd_gram && !o->tune.update_streaming) {
+    if (o->upd_nvb == 4 && o->upd_rows_in_smem && !o->upd_gram) {
         // batched instances (more than one wave of one-CTA-per-SM launches: two 8-warp CTAs per SM take ~1.3x the time of one
         // 16-warp CTA, so a second wave is what they beat) whose rows fit 8 warps x 5: CTAs of 8 warps, two per
         // SM — the sweep of one instance is a chain of dependent steps that leaves its SM two thirds idle (k_update.cuh)
         const bool two_per_sm = 2 * o->upd_smem + 4096 <= o->props->smem_optin && o->d.m <= 8 * 5;
         if (o->tune.update_warps == 8 ? two_per_sm : (o->tune.update_warps == 0 && two_per_sm && o->d.B > o->props->sm_count)) o->upd_warps = 8;
-        o->upd_sweep_warps = o->upd_warps;
-        const int forced_sw = o->tune.update_sweep_warps;
-        if (forced_sw >= 1 && forced_sw <= o->upd_warps) o->upd_sweep_warps = forced_sw;
-        if (o->d.m <= o->upd_sweep_warps * 3) o->upd_rmax = 3;
-        else if (o->d.m <= o->upd_sweep_warps * 5) o->upd_rmax = 5;
+        if (o->d.m <= o->upd_warps * 3) o->upd_rmax = 3;
+        else if (o->d.m <= o->upd_warps * 5) o->upd_rmax = 5;
     }
     return 0;
 }
@@ -459,7 +440,7 @@ int ensure_graph(lmcma_b200_opt* o) {
                 if (!rc2 && cudaEventRecord(o->ev_join, o->side_stream) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph join record failed");
                 if (!rc2) rc2 = launch(k_gate, (o->d.B + 31) / 32, 32, 0, st, false, o->d);
                 if (!rc2) rc2 = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
-                if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN | RANK_KEEP_FLAGS | (o->tune.rank_late ? 0 : 4), nullptr, st, true);
+                if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, true);
                 if (!rc2) rc2 = launch_sample(o, st, true, true, 2);
                 if (!rc2 && cudaStreamWaitEvent(st, o->ev_join, 0) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph join failed");
             } else {
@@ -522,7 +503,7 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
         if (ok) ok = cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st) == cudaSuccess;
         if (ok) ok = launch(k_gate, (d.B + 31) / 32, 32, 0, st, false, d) == 0;   // k_update has reset the flags and holds its SM
         // the sampler is released when k_rank starts: the pairs it needs first are final (resume: at once; else as the sweep goes)
-        if (ok) ok = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS | (o->tune.rank_late ? 0 : 4), nullptr, st, false) == 0;
+        if (ok) ok = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, false) == 0;
         if (ok) ok = launch_sample(o, st, true, true, 2) == 0;
         if (ok) ok = cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
         return ok ? 0 : LMCMA_B200_ERR_CUDA;
@@ -653,7 +634,7 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     }
     DM(d.fit, B * lam); DM(d.fit_sorted, B * lam); DM(d.prev_fit, B * lam);
     DM(d.rank, B * lam); DM(d.arindex, B * lam);
-    if (d.lambda > TELL_FTILE && d.pop_count == d.lambda && o->tune.rank_sorted) {
+    if (d.lambda > TELL_FTILE && d.pop_count == d.lambda) {
         DM(d.prev_sorted, B * lam); DM(d.tile_sorted, B * lam); DM(d.tile_pos, B * lam);
     }
     DM(d.ncoll, B * pc); DM(d.nsamp, B * pc);

@@ -101,7 +101,7 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
             int32_t* v = out;
             v[LMCMA_B200_LAUNCH_SAMPLER] = o->smp_rows ? 2 : (o->smp_wide ? 1 : 0);
             v[LMCMA_B200_LAUNCH_SMP_NV] = o->smp_nv;
-            v[LMCMA_B200_LAUNCH_SMP_SPEC] = o->tune.sample_spec ? 1 : 0;
+            v[LMCMA_B200_LAUNCH_SMP_SPEC] = 1;
             v[LMCMA_B200_LAUNCH_SMP_THREADS] = o->smp_rows ? 512 : (o->smp_wide ? 32 * o->smp_R * o->smp_CW : o->smp_threads);
             v[LMCMA_B200_LAUNCH_SMP_RBW] = o->smp_wide ? o->smp_RBW : 0;
             v[LMCMA_B200_LAUNCH_SMP_CW] = o->smp_wide ? o->smp_CW : 0;
@@ -115,7 +115,7 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
             v[LMCMA_B200_LAUNCH_UPD_ROWS_IN_SMEM] = o->upd_rows_in_smem ? 1 : 0;
             v[LMCMA_B200_LAUNCH_UPD_GRAM] = o->upd_gram ? 1 : 0;
             v[LMCMA_B200_LAUNCH_UPD_WARPS] = o->upd_warps;
-            v[LMCMA_B200_LAUNCH_UPD_SWEEP_WARPS] = o->upd_sweep_warps;
+            v[LMCMA_B200_LAUNCH_UPD_SWEEP_WARPS] = o->upd_warps;
             v[LMCMA_B200_LAUNCH_COEF_ELEMS] = o->coef_elems;
             v[LMCMA_B200_LAUNCH_RANK_THREADS] = o->rank_threads;
             v[LMCMA_B200_LAUNCH_RANK_FTILE] = d.rank_ftile;

@@ -98,20 +98,15 @@ inline int env_int(const char* name, int dflt) {
 }
 
 // Every LMCMA_B200_* environment knob, read ONCE when a handle (map or optimiser) is created and kept on the handle:
-// nothing on a launch path calls getenv.  All of them are experiment / debugging switches; the defaults are the product.
+// nothing on a launch path calls getenv.  The defaults are the product; each switch is a serial-order reference of the
+// bit-identity tests, a test seam, an operational override or a diagnostic (INTEGRATION.md section 5 lists them all).
 struct Tuning {
     int cost_minb = 0 /* 0 = by launch size */, cost_tpt = 0, cost_cb = 0, zerocopy = 1;
-    int sample_rows = -1;   // k_sample_rows: -1 = where it pays (many rows), 0 = never, 1 = also for one large population
-    int sample_spec = 1, sample_threads = 0, sample_smem_kb = 160, sample_smem_kb_set = 0, sample_narrow = 0, sample_rbw = 0, sample_r = 0;
-    int update_blocked = 0, update_gram = 0, update_streaming = 0, update_sweep_warps = 0;
-    int progressive = 1, overlap = 1, tell_overlap = 1, rank_sorted = 1;
-    int rank_late = 0;      // fused generation: 1 = k_sample is released when k_rank's CTAs are done, 0 = when k_rank starts (it then works
-                            // through the finished pairs beside the ranking: 66.5 -> 63.2 us per C2 generation once the newest row's
-                            // chain stopped being the longer branch)
+    int sample_rows = 0;    // 1: k_sample_rows also for one large population (else only where it pays: many rows)
+    int update_gram = 0, progressive = 1, overlap = 1, tell_overlap = 1;
     int tell_spec = 1;      // tell_all: speculative update of the next generation at the end of the graph (LMCMA_B200_TELL_SPEC=0: off)
     int graph_unroll = 8;   // fused generations per CUDA graph for runs of at least that many (LMCMA_B200_GRAPH_UNROLL, 1 = off)
     int update_warps = 0;   // k_update CTA size: 0 = by batch size, 8 / 16 forced (LMCMA_B200_UPDATE_WARPS)
-    int update_dry = 1;     // overlapped generation: pre-execute the post-rank code while k_rank is busy (k_update.cuh)
     int graph_dbg = 0, dbg = 0, update_dbg = 0, cost_dbg = 0;
     static Tuning from_env() {
         Tuning t;
@@ -119,28 +114,15 @@ struct Tuning {
         t.cost_tpt = env_int("LMCMA_B200_COST_TPT", 0);
         t.cost_cb = env_int("LMCMA_B200_COST_CB", 0);
         t.zerocopy = env_int("LMCMA_B200_ZEROCOPY", 1);
-        t.sample_spec = env_int("LMCMA_B200_SAMPLE_SPEC", 1);
-        t.sample_rows = env_int("LMCMA_B200_SAMPLE_ROWS", -1);
-        t.sample_threads = env_int("LMCMA_B200_SAMPLE_THREADS", 0);
-        t.sample_smem_kb_set = env_int("LMCMA_B200_SAMPLE_SMEM_KB", 0);
-        t.sample_smem_kb = t.sample_smem_kb_set ? t.sample_smem_kb_set : 160;
-        t.sample_narrow = env_int("LMCMA_B200_SAMPLE_NARROW", 0);
-        t.sample_rbw = env_int("LMCMA_B200_SAMPLE_RBW", 0);
-        t.sample_r = env_int("LMCMA_B200_SAMPLE_R", 0);
-        t.update_blocked = env_int("LMCMA_B200_UPDATE_BLOCKED", 0);
+        t.sample_rows = env_int("LMCMA_B200_SAMPLE_ROWS", 0);
         t.update_gram = env_int("LMCMA_B200_UPDATE_GRAM", 0);
-        t.update_streaming = env_int("LMCMA_B200_UPDATE_STREAMING", 0);
-        t.update_sweep_warps = env_int("LMCMA_B200_UPDATE_SWEEP_WARPS", 0);
         t.progressive = env_int("LMCMA_B200_PROGRESSIVE", 1);
         t.overlap = env_int("LMCMA_B200_OVERLAP", 1);
         t.tell_overlap = env_int("LMCMA_B200_TELL_OVERLAP", 1);
-        t.rank_late = env_int("LMCMA_B200_RANK_LATE", 0);
-        t.update_dry = env_int("LMCMA_B200_UPDATE_DRY", 1);
         t.tell_spec = env_int("LMCMA_B200_TELL_SPEC", 1);
         t.update_warps = env_int("LMCMA_B200_UPDATE_WARPS", 0);
         t.graph_unroll = env_int("LMCMA_B200_GRAPH_UNROLL", 8);
         if (t.graph_unroll < 1 || t.graph_unroll > 64) t.graph_unroll = 1;
-        t.rank_sorted = env_int("LMCMA_B200_RANK_SORTED", 1);
         t.graph_dbg = env_int("LMCMA_B200_GRAPH_DBG", 0);
         t.dbg = getenv("LMCMA_B200_DBG") ? 1 : 0;
         t.update_dbg = getenv("LMCMA_B200_UPDATE_DBG") ? 1 : 0;
@@ -254,7 +236,7 @@ struct lmcma_b200_opt {
     bool mirror_on = false, mirror_suppressed = false, xh_fresh = false;
     int* err_host = nullptr;          // page-locked, mapped: OptDev::err (a kernel of the overlapped generation gave up on its partner)
     long long* graph_dbg = nullptr;   // LMCMA_B200_GRAPH_DBG: k_update's timeline inside the fused generation, printed by lmcma_b200_sync
-    int upd_nvb = 4, upd_rmax = 0, upd_sweep_warps = 16, upd_warps = 16;
+    int upd_nvb = 4, upd_rmax = 0, upd_warps = 16;
     bool upd_gram = false; size_t coef_smem = 0;   // Gram-matrix recompute (k_gram.cuh) for rows that fit neither registers nor smem
     int coef_elems = 0;                            // k_coef<coef_elems>: elements per lane, ceil(m / 8) rounded up to a build
     bool upd_rows_in_smem = true;

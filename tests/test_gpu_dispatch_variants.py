@@ -90,22 +90,15 @@ CASES = {
                          where="test_gpu_bench_shapes.py::test_rows_sampler_teacher_forced_single_population"),
 }
 
-# builds reached only through an environment knob (experiments), never by the launcher's own choice
-EXCLUDED = {
-    "launch_sample_t<4,2,512>": "the non-speculative nv = 4 sampler: LMCMA_B200_SAMPLE_SPEC=0 only",
-    "launch_sample_wide_t<1,1024>": "one row per warp in the wide sampler: LMCMA_B200_SAMPLE_RBW=1 only",
-}
-
 
 def _instantiations(l):
     """The template instantiations (spelled as in lmcma_capi.cu, without spaces) a handle with launch() == l runs."""
     if l["sampler"] == "rows":
         smp = "launch_sample_rows_t<%d,%d>" % (l["smp_rows_qw"], l["smp_rows_rl"])
     elif l["sampler"] == "wide":
-        smp = {1: "launch_sample_wide_t<1,1024>", 2: "launch_sample_wide_t<2,1024>"}.get(l["smp_RBW"], "launch_sample_wide_t<4,512>")
+        smp = {2: "launch_sample_wide_t<2,1024>", 4: "launch_sample_wide_t<4,512>"}[l["smp_RBW"]]
     else:
-        smp = {1: "<1,4,512>", 2: "<2,4,512>", 4: "<4,2,512,true>" if l["smp_spec"] else "<4,2,512>", 8: "<8,1,512>",
-               12: "<12,1,256>", 16: "<16,1,256>"}[l["smp_nv"]]
+        smp = {1: "<1,4,512>", 2: "<2,4,512>", 4: "<4,2,512,true>", 8: "<8,1,512>", 12: "<12,1,256>", 16: "<16,1,256>"}[l["smp_nv"]]
         smp = "launch_sample_t" + smp
     nvb, rmax = l["upd_nvb"], l["upd_rmax"]
     if l["upd_gram"]:
@@ -377,7 +370,6 @@ def test_every_launcher_instantiation_has_a_case(monkeypatch):
             assert hasattr(importlib.import_module(mod[:-3]), name), c.where
     in_source = _source_instantiations()
     assert len(in_source) >= 30, sorted(in_source)                 # the patterns still match the launcher's spelling
-    assert set(EXCLUDED) <= in_source, sorted(set(EXCLUDED) - in_source)
     assert set(reached) <= in_source, sorted(set(reached) - in_source)
-    unreached = in_source - set(reached) - set(EXCLUDED)
+    unreached = in_source - set(reached)
     assert not unreached, sorted(unreached)
