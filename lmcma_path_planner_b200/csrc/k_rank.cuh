@@ -11,13 +11,11 @@
 // reset, and the dependent grid is the sampler).
 #pragma once
 #include "lmcma_common.cuh"
+#include "lmcma_plan.hpp"
 
 namespace lmcma {
 
 enum { RANK_PLAIN = 0, RANK_PACK = 1, RANK_KEEP_FLAGS = 2 };   // bit 1: the hand-over flags belong to a concurrently running k_update
-
-constexpr int TELL_FTILE = 4096;       // fitness values staged per shared-memory tile
-constexpr int TELL_MAX_ROWS = 256;     // rows per slice upper bound (rows_per = max(32, ceil(pop/256)))
 
 // ------------------------------------------------------------------------------------------------
 // Large unsplit populations (lambda > TELL_FTILE): counting costs lambda^2 compares (1.4 ms at lambda = 65536, half of

@@ -1,10 +1,9 @@
 // k_sample.cuh — offspring sampling kernel.
 #pragma once
 #include "lmcma_common.cuh"
+#include "lmcma_plan.hpp"
 
 namespace lmcma {
-
-constexpr int SAMPLE_G = 8;   // direction pairs per group: their dots are independent, reduced together
 
 // Sum v[g] over the 32 lanes for 8 values with 9 shuffles instead of 40: three exchange-and-halve stages
 // (each lane gives away the half of the values it will not own), then two butterfly stages.  On return
@@ -71,8 +70,6 @@ __device__ __forceinline__ void sample_finish(const OptDev& o, const double* __r
     reinterpret_cast<float4*>(drow)[q] = make_float4(dd[0], dd[1], dd[2], dd[3]);
     if (hrow) __stcs(reinterpret_cast<float4*>(hrow) + q, make_float4(xx[0], xx[1], xx[2], xx[3]));   // host mirror (OptDev::Xh)
 }
-
-constexpr int SAMPLE_MAX_STAGES = 8;
 
 // SPEC: full groups of 8 pairs run a copy of the two group loops without the per-pair `g < gcnt` predicates
 template <int NV, int RB, int MAXT, bool SPEC = false>

@@ -20,14 +20,12 @@
 //    then the rest.  Same operations in the same order as the serial launch order, bit for bit (DESIGN.md 4.2, 4.3).
 #pragma once
 #include "lmcma_common.cuh"
+#include "lmcma_plan.hpp"
 #include <type_traits>
 
 namespace lmcma {
 
-constexpr int UPD_WARPS = 16;
-constexpr int UPD_GROUPS = UPD_WARPS / 4;   // 128-thread groups of the mean phase
 constexpr int UPD_THREADS = 32 * UPD_WARPS;
-constexpr int UPD_BLK = 8;            // factors per block of the newest row's chain (k_update: newest_row)
 
 struct UpdateArgs {
     const float* f_all;        // B x lambda fitness of this generation (global candidate order)

@@ -1,5 +1,6 @@
-// lmcma_capi.cu — the C ABI declared in include/lmcma_b200.h: library / device queries, the optimiser entry points, launch
-// configuration of the sampler / rank / update kernels, the per-generation CUDA graphs, the split-population stages.
+// lmcma_capi.cu — the C ABI declared in include/lmcma_b200.h: library / device queries, the optimiser entry points, the
+// launchers of the sampler / rank / update kernels (their configuration: the handle's plan, lmcma_plan.cpp), the
+// per-generation CUDA graphs, the split-population stages.
 // No CPU fallback: every compute entry point needs a CUDA device.  Cost map + evaluator: lmcma_capi_map.cu; state
 // access + host-side reference pieces: lmcma_capi_state.cu; shared declarations: lmcma_internal.cuh.
 #include "lmcma_internal.cuh"
@@ -32,27 +33,27 @@ int set_error(int code, const char* fmt, ...) {
 }  // namespace lmcma
 
 namespace {
-template <int NV, int RB, int MAXT, bool SPEC = false>
+// the three sampler families; block, grid and shared memory of every launch: o->plan.sample
+template <int NV>
 int launch_sample_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
-    const int rows_per_cta = (o->smp_threads / 32) * RB;
-    const int ctas = (o->d.pop_count + rows_per_cta - 1) / rows_per_cta;
-    return launch(k_sample<NV, RB, MAXT, SPEC>, dim3(ctas, o->d.B), o->smp_threads, o->smp_smem, st, pdl, d, o->smp_kc, o->smp_stages);
+    const auto& s = o->plan.sample;
+    return launch(k_sample<NV, narrow_rb(NV), narrow_maxt(NV), narrow_spec(NV)>, dim3(s.ctas, d.B), s.threads, s.smem, st, pdl,
+                  d, s.kc, s.stages);
 }
-
-template <int RBW, int MAXT>
+template <int RBW>
 int launch_sample_wide_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st, int progressive) {
-    const int rows_per_cta = o->smp_R * RBW;
-    return launch(k_sample_wide<RBW, MAXT>, dim3((o->d.pop_count + rows_per_cta - 1) / rows_per_cta, o->d.B), 32 * o->smp_R * o->smp_CW,
-                  o->smp_smem, st, pdl, d, o->smp_kc, o->smp_stages, o->smp_R, o->smp_CW, o->smp_qpw, progressive);
+    const auto& s = o->plan.sample;
+    return launch(k_sample_wide<RBW, wide_maxt(RBW)>, dim3(s.ctas, d.B), s.threads, s.smem, st, pdl, d, s.kc, s.stages, s.R, s.CW,
+                  s.qpw, progressive);
 }
 template <int QW, int RL>
 int launch_sample_rows_t(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
-    return launch(k_sample_rows<QW, RL>, dim3((d.pop_count + 32 * RL - 1) / (32 * RL), d.B), 512, o->smp_rows_smem, st, pdl,
-                  d, o->smp_rows_kc, o->smp_rows_stages, o->smp_rows_region);
+    const auto& s = o->plan.sample;
+    return launch(k_sample_rows<QW, RL>, dim3(s.ctas, d.B), s.threads, s.smem, st, pdl, d, s.kc, s.stages, s.region);
 }
 int launch_sample_rows(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st) {
-    const bool two = o->smp_rows_rl == 2;
-    switch (o->smp_rows_qw) {
+    const bool two = o->plan.sample.rl == 2;
+    switch (o->plan.sample.qw) {
         case 4: return two ? launch_sample_rows_t<4, 2>(o, d, pdl, st) : launch_sample_rows_t<4, 1>(o, d, pdl, st);
         case 7: return two ? launch_sample_rows_t<7, 2>(o, d, pdl, st) : launch_sample_rows_t<7, 1>(o, d, pdl, st);
         default: return two ? launch_sample_rows_t<8, 2>(o, d, pdl, st) : launch_sample_rows_t<8, 1>(o, d, pdl, st);
@@ -60,7 +61,7 @@ int launch_sample_rows(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_
 }
 
 int launch_sample_wide(lmcma_b200_opt* o, const OptDev& d, bool pdl, cudaStream_t st, int progressive) {
-    return o->smp_RBW == 2 ? launch_sample_wide_t<2, 1024>(o, d, pdl, st, progressive) : launch_sample_wide_t<4, 512>(o, d, pdl, st, progressive);
+    return o->plan.sample.RBW == 2 ? launch_sample_wide_t<2>(o, d, pdl, st, progressive) : launch_sample_wide_t<4>(o, d, pdl, st, progressive);
 }
 
 // the sequence-ordered (v, pc) mirror k_sample streams from is maintained by k_update; after create or a state
@@ -91,143 +92,68 @@ int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool pro
     OptDev d = o->d;
     if (!o->mirror_on || o->mirror_suppressed) d.Xh = nullptr;
     o->xh_fresh = d.Xh != nullptr;
-    if (o->smp_rows) return launch_sample_rows(o, d, pdl, st);
-    if (o->smp_wide) return launch_sample_wide(o, d, pdl, st, (pdl && progressive && o->progressive) ? progressive_mode : 0);
-    switch (o->smp_nv) {
-        case 1: return launch_sample_t<1, 4, 512>(o, d, pdl, st);
-        case 2: return launch_sample_t<2, 4, 512>(o, d, pdl, st);
-        case 4: return launch_sample_t<4, 2, 512, true>(o, d, pdl, st);
-        case 8: return launch_sample_t<8, 1, 512>(o, d, pdl, st);
-        case 12: return launch_sample_t<12, 1, 256>(o, d, pdl, st);
-        case 16: return launch_sample_t<16, 1, 256>(o, d, pdl, st);
+    if (o->plan.sample.kind == Sampler::ROWS) return launch_sample_rows(o, d, pdl, st);
+    if (o->plan.sample.kind == Sampler::WIDE)
+        return launch_sample_wide(o, d, pdl, st, (pdl && progressive && o->plan.progressive) ? progressive_mode : 0);
+    switch (o->plan.sample.nv) {
+        case 1: return launch_sample_t<1>(o, d, pdl, st);
+        case 2: return launch_sample_t<2>(o, d, pdl, st);
+        case 4: return launch_sample_t<4>(o, d, pdl, st);
+        case 8: return launch_sample_t<8>(o, d, pdl, st);
+        case 12: return launch_sample_t<12>(o, d, pdl, st);
+        case 16: return launch_sample_t<16>(o, d, pdl, st);
     }
-    return fail(LMCMA_B200_ERR_ARG, "unsupported n for k_sample (nv=%d)", o->smp_nv);
-}
-
-int configure_sample(lmcma_b200_opt* o) {
-    const int nq = o->d.ns / 4;
-    const int need = (nq + 31) / 32;
-    static const int nvs[] = {1, 2, 4, 8, 12, 16};
-    o->smp_nv = 0;
-    for (int v : nvs)
-        if (v >= need) { o->smp_nv = v; break; }
-    if (!o->smp_nv) return fail(LMCMA_B200_ERR_ARG, "n = %d too large (max 2048)", o->d.n);
-    o->smp_rb = o->smp_nv <= 2 ? 4 : (o->smp_nv <= 4 ? 2 : 1);
-    const int maxt = o->smp_nv >= 12 ? 256 : 512;
-    // as many warps per CTA as keeps >= ~1 CTA per SM
-    int threads = maxt;
-    while (threads > 64) {
-        const int rows_per_cta = (threads / 32) * o->smp_rb;
-        const long long ctas = (long long)((o->d.pop_count + rows_per_cta - 1) / rows_per_cta) * o->d.B;
-        if (ctas * 4 >= (long long)o->props->sm_count * 3) break;   // bigger tiles re-read the pairs less often
-        threads >>= 1;
-    }
-    o->smp_threads = threads;
-    const size_t pair_bytes = (size_t)2 * o->d.ns * sizeof(float);
-    // pairs per stage: one group of 8 when it fits (else 4 / 2 / 1); as many stages as the live pairs need, within
-    // 160 KB, so that for the common shapes every pair is requested up front and nothing is re-issued
-    const size_t budget = (size_t)160 * 1024;
-    int kc = (int)(budget / 2 / pair_bytes);
-    kc = kc >= 8 ? 8 : (kc >= 4 ? 4 : (kc >= 2 ? 2 : 1));
-    // long rows (C4: 12 KB per pair): two stages of a FULL group of 8 still fit one SM (192 KB), and a 4-pair stage runs the
-    // 8-wide group code half empty
-    if (kc == 4 && 2 * 8 * pair_bytes + 24 * 1024 <= o->props->smem_optin) kc = 8;
-    o->smp_kc = kc;
-    const int max_chunks = (o->d.m + kc - 1) / kc;
-    o->smp_stages = (int)std::max<size_t>(2, std::min<size_t>(std::min(max_chunks, SAMPLE_MAX_STAGES), budget / (kc * pair_bytes)));   // >= 2 even beyond the budget
-    o->smp_smem = (size_t)o->smp_stages * kc * pair_bytes + SAMPLE_MAX_STAGES * 8 + (size_t)(2 * o->d.m + 16) * sizeof(float);
-    // one large population: split every row over CW column-warps (k_sample_wide) for occupancy
-    o->smp_wide = false;
-    if (o->d.pop_count >= 256 && nq > 32) {
-        o->smp_wide = true;
-        o->smp_CW = (nq + 31) / 32;
-        o->smp_qpw = (nq + o->smp_CW - 1) / o->smp_CW;
-        // rows per warp: 2 (4 for very large populations); row-groups per CTA so that the grid still covers the SMs
-        o->smp_RBW = o->d.pop_count >= 1024 ? 4 : 2;
-        int R = std::max(1, std::min(15, (o->smp_RBW == 4 ? 16 : 32) / o->smp_CW));
-        while (R > 1 && (long long)((o->d.pop_count + R * o->smp_RBW - 1) / (R * o->smp_RBW)) * o->d.B * 4 < (long long)o->props->sm_count * 3) R >>= 1;
-        o->smp_R = R;
-        o->smp_smem += (size_t)o->smp_stages * ((kc + SAMPLE_G - 1) / SAMPLE_G) * o->smp_R * o->smp_CW * o->smp_RBW * SAMPLE_G * sizeof(float);
-    }
-    if (o->smp_smem > o->props->smem_optin) return fail(LMCMA_B200_ERR_ARG, "k_sample needs %zu B shared memory", o->smp_smem);
-    // many rows (batched queries, or one very large population): rows on lanes, column slices on warps (k_sample_rows)
-    o->smp_rows = false;
-    const long long total_rows = (long long)o->d.B * o->d.pop_count;
-    // one population: from lambda = 8192 on it beats the wide sampler even though the progressive hand-over / overlapped
-    // generation (wide sampler only) is given up (fused generation 0.271 -> 0.253 ms at 8192, 1.71 -> 1.41 ms at 65536)
-    const bool many = total_rows >= 4096 && o->d.pop_count >= 32 &&
-                      (o->d.B > 1 || o->tune.sample_rows == 1 || (o->d.pop_count >= 8192 && o->d.pop_count == o->d.lambda));
-    if (many && nq <= 128 && o->d.m <= 256 && !o->d_Lf) {
-        const int NW = 16;
-        const int qper = (nq + NW - 1) / NW;
-        o->smp_rows_qw = qper <= 4 ? 4 : (qper <= 7 ? 7 : 8);
-        // two rows per lane when an instance has them and the grid still fills the SMs
-        o->smp_rows_rl = (o->d.pop_count >= 64 && total_rows / 64 >= 2LL * o->props->sm_count) ? 2 : 1;
-        const int rows = 32 * o->smp_rows_rl, kc2 = 8;
-        const int chunks = (o->d.m + kc2 - 1) / kc2;
-        const size_t stage_bytes = (size_t)kc2 * pair_bytes;
-        const size_t fixed2 = SAMPLE_MAX_STAGES * 8 + (size_t)((o->d.m + kc2 + 3) & ~3) * 4 + (size_t)chunks * kc2 * rows * 4 + (size_t)NW * kc2 * rows * 4;
-        const size_t tile_bytes = (size_t)rows * (o->d.ns + 4) * 4;
-        if (fixed2 + std::max(2 * stage_bytes, tile_bytes) + 1024 <= o->props->smem_optin) {
-            const size_t room = o->props->smem_optin - 1024 - fixed2;
-            int stages = (int)std::min<size_t>(std::min(chunks, SAMPLE_MAX_STAGES), room / stage_bytes);
-            stages = std::max(stages, 2);
-            const size_t region = std::max((size_t)stages * stage_bytes, tile_bytes);
-            o->smp_rows_kc = kc2; o->smp_rows_stages = stages; o->smp_rows_region = (int)(region / 4);
-            o->smp_rows_smem = region + fixed2;
-            o->smp_rows = true;
-            o->smp_wide = false;
-        }
-    }
-    return 0;
+    return fail(LMCMA_B200_ERR_ARG, "unsupported n for k_sample (nv=%d)", o->plan.sample.nv);
 }
 
 // ranks + recombination partial sums (k_rank.cuh); RANK_PACK is the split-population stage
 // pdl: launched as a programmatic dependent of the kernel enqueued just before it on `st` (k_cost)
 int launch_rank(lmcma_b200_opt* o, const float* f_all, int mode, float* payload, cudaStream_t st, bool pdl = false) {
-    if (o->d.tile_sorted) {                                       // lambda > 4096, unsplit: sort the fitness tiles first (k_rank.cuh)
+    const auto& r = o->plan.rank;
+    if (r.tile_sorted) {                                          // lambda > 4096, unsplit: sort the fitness tiles first (k_rank.cuh)
         int rc = launch(k_rank_tiles, dim3((o->d.lambda + TELL_FTILE - 1) / TELL_FTILE, o->d.B), 1024, 0, st, pdl, o->d, f_all);
         if (rc) return rc;
         pdl = false;                                              // k_rank itself follows in stream order
     }
-    return launch(k_rank<1024>, dim3(o->d.RS, o->d.B), o->rank_threads, o->rank_smem, st, pdl, o->d, f_all, mode, payload);
+    return launch(k_rank<1024>, dim3(r.slices, o->d.B), r.threads, r.smem, st, pdl, o->d, f_all, mode, payload);
 }
 
 template <int NVB, int RMAX, bool SMEM, bool OVERLAP = false, int WARPS = UPD_WARPS>
 int launch_update_t(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream_t st) {
-    return launch(k_update<NVB, RMAX, SMEM, OVERLAP, WARPS>, o->d.B, 32 * WARPS, o->upd_smem, st, pdl, o->d, a);
+    return launch(k_update<NVB, RMAX, SMEM, OVERLAP, WARPS>, o->d.B, 32 * WARPS, o->plan.update.smem, st, pdl, o->d, a);
 }
 
 // the serial part of update() (k_update.cuh).  pdl: launched as a programmatic dependent of the kernel enqueued just
 // before it on `st` (k_rank), so that its prologue overlaps that kernel
 int launch_update(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream_t st) {
     if (a.phase == 0) o->spec_valid = false;                        // a whole update: whatever the speculative pass left is stale
-    if (o->upd_gram) {
-        int rc = o->upd_nvb == 4 ? launch_update_t<4, -1, false>(o, a, pdl, st) : launch_update_t<16, -1, false>(o, a, pdl, st);
+    const auto& u = o->plan.update;
+    if (u.gram) {
+        int rc = u.nvb == 4 ? launch_update_t<4, -1, false>(o, a, pdl, st) : launch_update_t<16, -1, false>(o, a, pdl, st);
         if (rc) return rc;
         const OptDev& d = o->d;
         const int tiles = (d.m + GRAM_TILE - 1) / GRAM_TILE;
         if ((rc = launch(k_gram, dim3(tiles, tiles, d.B * GRAM_KS), 256, 0, st, false, d))) return rc;
-        const int coef_threads = std::min(1024, (8 * d.m + 31) & ~31);    // 8 lanes per basis row (m <= 128)
-        auto coef = o->coef_elems == 5 ? k_coef<5> : (o->coef_elems == 10 ? k_coef<10> : (o->coef_elems == 12 ? k_coef<12> : k_coef<16>));
-        if ((rc = launch(coef, d.B, coef_threads, o->coef_smem, st, false, d))) return rc;
+        const auto& c = o->plan.coef;
+        auto coef = c.elems == 5 ? k_coef<5> : (c.elems == 10 ? k_coef<10> : (c.elems == 12 ? k_coef<12> : k_coef<16>));
+        if ((rc = launch(coef, d.B, c.threads, c.smem, st, false, d))) return rc;
         return launch(k_combine, dim3((d.ns / 4 + 127) / 128, (d.m + COMBINE_ROWS - 1) / COMBINE_ROWS, d.B), 128, 0, st, false, d);
     }
-    if (o->upd_nvb == 4) {
+    if (u.nvb == 4) {
         if (a.overlap) {                                         // the overlapped generation (ensure_graph): register sweep only
-            if (o->upd_rmax == 3) return launch_update_t<4, 3, true, true>(o, a, pdl, st);
-            if (o->upd_rmax == 5) return launch_update_t<4, 5, true, true>(o, a, pdl, st);
+            if (u.rmax == 3) return launch_update_t<4, 3, true, true>(o, a, pdl, st);
+            if (u.rmax == 5) return launch_update_t<4, 5, true, true>(o, a, pdl, st);
             return fail(LMCMA_B200_ERR_STATE, "overlapped generation without the register sweep");
         }
-        if (o->upd_warps == 8) {                                 // batched instances: two CTAs of 8 warps per SM (configure_update)
-            if (o->upd_rmax == 3) return launch_update_t<4, 3, true, false, 8>(o, a, pdl, st);
-            if (o->upd_rmax == 5) return launch_update_t<4, 5, true, false, 8>(o, a, pdl, st);
+        if (u.warps == 8) {                                      // batched instances: two CTAs of 8 warps per SM (plan_launch)
+            if (u.rmax == 3) return launch_update_t<4, 3, true, false, 8>(o, a, pdl, st);
+            if (u.rmax == 5) return launch_update_t<4, 5, true, false, 8>(o, a, pdl, st);
         }
-        if (o->upd_rmax == 3) return launch_update_t<4, 3, true>(o, a, pdl, st);
-        if (o->upd_rmax == 5) return launch_update_t<4, 5, true>(o, a, pdl, st);
-        return o->upd_rows_in_smem ? launch_update_t<4, 0, true>(o, a, pdl, st) : launch_update_t<4, 0, false>(o, a, pdl, st);
+        if (u.rmax == 3) return launch_update_t<4, 3, true>(o, a, pdl, st);
+        if (u.rmax == 5) return launch_update_t<4, 5, true>(o, a, pdl, st);
+        return u.rows_in_smem ? launch_update_t<4, 0, true>(o, a, pdl, st) : launch_update_t<4, 0, false>(o, a, pdl, st);
     }
-    return o->upd_rows_in_smem ? launch_update_t<16, 0, true>(o, a, pdl, st) : launch_update_t<16, 0, false>(o, a, pdl, st);
+    return u.rows_in_smem ? launch_update_t<16, 0, true>(o, a, pdl, st) : launch_update_t<16, 0, false>(o, a, pdl, st);
 }
 
 UpdateArgs update_args_local(lmcma_b200_opt* o) {
@@ -237,44 +163,6 @@ UpdateArgs update_args_local(lmcma_b200_opt* o) {
     a.slices = o->d.partial; a.n_slices = o->d.RS; a.slice_stride = o->d.ns; a.inst_stride = (long long)o->d.RS * o->d.ns;
     a.spec = o->d_spec; a.spec_stride = (long long)o->spec_stride;
     return a;
-}
-
-int configure_update(lmcma_b200_opt* o) {
-    const int nq = o->d.ns / 4;
-    if (nq > 512) return fail(LMCMA_B200_ERR_ARG, "n = %d too large (max 2048)", o->d.n);
-    o->upd_nvb = nq <= 128 ? 4 : 16;
-    // k_rank: small populations (lambda <= 256) take CTAs of 256 threads and tiles of lambda values — the choice depends on
-    // lambda alone, so that a batched instance and the same instance run alone sum their partial sums in the same order
-    o->rank_threads = o->d.lambda <= 256 ? 256 : 1024;
-    o->d.rank_ftile = o->d.lambda <= 256 ? ((o->d.lambda + 3) & ~3) : TELL_FTILE;
-    o->rank_smem = (size_t)2 * o->d.rank_ftile * 4 + (size_t)3 * TELL_MAX_ROWS * 4 + (size_t)7 * 128 * 16;
-    const size_t fixed = (((size_t)o->d.m * 36 + 8 + 127) & ~(size_t)127) + (size_t)2048 * (UPD_GROUPS - 1);
-    // + the block Gram entries, and the stages of the newest row's multi-warp chain (k_update.cuh: chain_part)
-    const size_t rows = (size_t)o->d.m * o->d.ns * sizeof(float) + (size_t)o->d.m * (UPD_BLK + 1) * sizeof(float) +
-                        (o->upd_nvb == 4 ? (size_t)(2 * 4 * UPD_BLK * 32 + 16) * sizeof(float) + 16 : 0);
-    const size_t budget = o->props->smem_optin - 2048;            // static shared + slack
-    o->upd_rows_in_smem = fixed + rows <= budget;
-    o->upd_smem = fixed + (o->upd_rows_in_smem ? rows : 0);
-    if (o->upd_smem > budget) return fail(LMCMA_B200_ERR_ARG, "k_update needs %zu B shared memory (m = %d too large)", o->upd_smem, o->d.m);
-    // rows that fit neither the registers nor the shared memory of one SM: Gram-matrix recompute (k_gram.cuh)
-    o->coef_smem = (size_t)2 * o->d.m * (o->d.m | 1) * sizeof(double) + (size_t)2 * o->d.m * sizeof(double);
-    o->upd_gram = (!o->upd_rows_in_smem || o->tune.update_gram) && o->d.m <= 128 && o->coef_smem <= budget;
-    if (o->upd_gram) { o->upd_rows_in_smem = false; o->upd_smem = fixed; }
-    // k_coef elements per lane: ceil(m / 8), rounded up to a compiled build (m <= 128)
-    o->coef_elems = !o->upd_gram ? 0 : (o->d.m <= 40 ? 5 : (o->d.m <= 80 ? 10 : (o->d.m <= 96 ? 12 : 16)));
-    // pending rows in registers when they fit: m <= 8 warps x RMAX rows of <= 128 float4 columns
-    o->upd_rmax = 0;
-    o->upd_warps = UPD_WARPS;
-    if (o->upd_nvb == 4 && o->upd_rows_in_smem && !o->upd_gram) {
-        // batched instances (more than one wave of one-CTA-per-SM launches: two 8-warp CTAs per SM take ~1.3x the time of one
-        // 16-warp CTA, so a second wave is what they beat) whose rows fit 8 warps x 5: CTAs of 8 warps, two per
-        // SM — the sweep of one instance is a chain of dependent steps that leaves its SM two thirds idle (k_update.cuh)
-        const bool two_per_sm = 2 * o->upd_smem + 4096 <= o->props->smem_optin && o->d.m <= 8 * 5;
-        if (o->tune.update_warps == 8 ? two_per_sm : (o->tune.update_warps == 0 && two_per_sm && o->d.B > o->props->sm_count)) o->upd_warps = 8;
-        if (o->d.m <= o->upd_warps * 3) o->upd_rmax = 3;
-        else if (o->d.m <= o->upd_warps * 5) o->upd_rmax = 5;
-    }
-    return 0;
 }
 
 int cost_args_for(lmcma_b200_opt* o, CostArgs* a) {
@@ -307,7 +195,7 @@ int generation_tail(lmcma_b200_opt* o, cudaStream_t st) {
     int rc;
     if ((rc = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st))) return rc;
     // device RNG: k_sample follows k_update directly and can take its outputs as they become final
-    const bool prog = o->progressive && o->cfg.rng == LMCMA_B200_RNG_PHILOX && !o->mirror_dirty;
+    const bool prog = o->plan.progressive && o->cfg.rng == LMCMA_B200_RNG_PHILOX && !o->mirror_dirty;
     UpdateArgs ua = update_args_local(o);
     ua.progressive = prog ? 1 : 0;
     if ((rc = launch_update(o, ua, true, st))) return rc;
@@ -427,7 +315,7 @@ int ensure_graph(lmcma_b200_opt* o) {
     // (~5 us of a 52 us generation); inside a graph a generation follows the previous one as a plain dependency
     auto body = [&](int reps) -> int {
         UpdateArgs ua = update_args_local(o);
-        ua.progressive = o->progressive ? 1 : 0;                 // ensure_mirror above: the mirror is clean
+        ua.progressive = o->plan.progressive ? 1 : 0;            // ensure_mirror above: the mirror is clean
         ua.dbg = o->graph_dbg;
         int rc2 = 0;
         for (int g = 0; g < reps && !rc2; ++g) {
@@ -447,7 +335,7 @@ int ensure_graph(lmcma_b200_opt* o) {
                 rc2 = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
                 if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st, true);
                 if (!rc2) rc2 = launch_update(o, ua, true, st);
-                if (!rc2) rc2 = launch_sample(o, st, true, o->progressive);
+                if (!rc2) rc2 = launch_sample(o, st, true, o->plan.progressive);
             }
         }
         return rc2;
@@ -593,6 +481,11 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     d.pop_count = cfg->pop_count < 1 ? d.lambda : cfg->pop_count;
     if (d.pop_offset < 0 || d.pop_offset + d.pop_count > d.lambda) { return fail(LMCMA_B200_ERR_ARG, "population slice out of range"); }
     if (cfg->rng == LMCMA_B200_RNG_HANSEN && d.pop_count != d.lambda) { return fail(LMCMA_B200_ERR_ARG, "HANSEN rng cannot be split"); }
+    std::string why;
+    const PlanInput in{d.n, d.lambda, d.m, d.B, d.pop_count, cfg->rng, covariance != nullptr};
+    if (!plan_launch(in, DeviceLimits{props->sm_count, props->smem_optin}, o->tune, &o->plan, &why)) return fail(LMCMA_B200_ERR_ARG, "%s", why.c_str());
+    d.RS = o->plan.rank.slices;
+    d.rank_ftile = o->plan.rank.ftile;
     d.rng_mode = cfg->rng;
     d.record_z = cfg->record_z;
     d.seed = (unsigned long long)cfg->seed;
@@ -634,7 +527,7 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     }
     DM(d.fit, B * lam); DM(d.fit_sorted, B * lam); DM(d.prev_fit, B * lam);
     DM(d.rank, B * lam); DM(d.arindex, B * lam);
-    if (d.lambda > TELL_FTILE && d.pop_count == d.lambda) {
+    if (o->plan.rank.tile_sorted) {
         DM(d.prev_sorted, B * lam); DM(d.tile_sorted, B * lam); DM(d.tile_pos, B * lam);
     }
     DM(d.ncoll, B * pc); DM(d.nsamp, B * pc);
@@ -644,11 +537,6 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     DM(d.VPs, B * m * 2 * ns);
     DM(d.t, B * m); DM(d.vec, B * m);
     DM(d.sc, B); DM(d.best_x, B * ns); DM(d.S_count, B); DM(d.done_count, B); DM(d.progress, B * (m + 2)); DM(d.rank_ticket, B); DM(d.resident, B);
-    {   // row slices of k_tell's phase A: 32 rows per slice, at most 256 slices
-        const int rows_per = std::max(32, (d.pop_count + 255) / 256);
-        if (rows_per > TELL_MAX_ROWS) { return fail(LMCMA_B200_ERR_ARG, "population too large (max %d rows per handle)", 256 * TELL_MAX_ROWS); }
-        d.RS = (d.pop_count + rows_per - 1) / rows_per;
-    }
     if (o->tune.dbg) DM(d.dbg, 64);
     DM(d.partial, B * d.RS * ns);
 
@@ -682,14 +570,7 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     }
     CU(cudaMemcpy(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice));
 
-    rc = configure_sample(o);
-    if (!rc) rc = configure_update(o);
-    // one query with a wide sampler and the register sweep: k_sample consumes the direction pairs while k_update's sweep
-    // is still producing them (k_update.cuh / k_sample.cuh "progressive")
-    o->progressive = !rc && B == 1 && o->smp_wide && o->upd_rmax > 0 && !o->upd_gram && !o->d_Lf && o->smp_kc == 8 &&
-                     o->smp_stages >= (m + o->smp_kc - 1) / o->smp_kc && cfg->rng == LMCMA_B200_RNG_PHILOX &&
-                     o->tune.progressive != 0;
-    o->overlap = o->progressive && o->tune.overlap != 0;
+    o->overlap = o->plan.overlap;
     if (o->overlap) {
         cudaError_t e2 = cudaStreamCreateWithFlags(&o->side_stream, cudaStreamNonBlocking);
         if (e2 == cudaSuccess) e2 = cudaEventCreateWithFlags(&o->ev_fork, cudaEventDisableTiming);
@@ -706,12 +587,11 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
             else cudaMemset(o->d_spec, 0xff, B * o->spec_stride * sizeof(float));   // generation -1: matches nothing
         }
     }
-    if (!rc && o->upd_gram) {
-        rc = dmalloc(&d.G, B * GRAM_KS * m * m);
-        if (!rc) rc = dmalloc(&d.Cf, B * m * m);
-        if (!rc) rc = dmalloc(&d.gram_hdr, B);
+    if (o->plan.update.gram) {
+        DM(d.G, B * GRAM_KS * m * m);
+        DM(d.Cf, B * m * m);
+        DM(d.gram_hdr, B);
     }
-    if (rc) return rc;
     o->f_host.assign(B * lam, 0.f);
     // first population (LMCMA::init -> sample(), lmcma.cpp:298)
     if (cfg->rng == LMCMA_B200_RNG_INJECT) o->needs_sample = true;

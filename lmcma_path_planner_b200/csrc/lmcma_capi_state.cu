@@ -96,34 +96,11 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
                 out[b] = which == LMCMA_B200_I32_ITR ? sc[b].itr : (which == LMCMA_B200_I32_LIVE ? sc[b].live : (int)sc[b].counteval);
             return 0;
         }
-        case LMCMA_B200_I32_LAUNCH: {   // per handle, from the configuration create chose (configure_sample / configure_update)
+        case LMCMA_B200_I32_LAUNCH:     // per handle: the launch plan create chose (lmcma_plan.cpp)
             ARG(cap >= LMCMA_B200_LAUNCH_FIELDS, "capacity");
-            int32_t* v = out;
-            v[LMCMA_B200_LAUNCH_SAMPLER] = o->smp_rows ? 2 : (o->smp_wide ? 1 : 0);
-            v[LMCMA_B200_LAUNCH_SMP_NV] = o->smp_nv;
-            v[LMCMA_B200_LAUNCH_SMP_SPEC] = 1;
-            v[LMCMA_B200_LAUNCH_SMP_THREADS] = o->smp_rows ? 512 : (o->smp_wide ? 32 * o->smp_R * o->smp_CW : o->smp_threads);
-            v[LMCMA_B200_LAUNCH_SMP_RBW] = o->smp_wide ? o->smp_RBW : 0;
-            v[LMCMA_B200_LAUNCH_SMP_CW] = o->smp_wide ? o->smp_CW : 0;
-            v[LMCMA_B200_LAUNCH_SMP_R] = o->smp_wide ? o->smp_R : 0;
-            v[LMCMA_B200_LAUNCH_SMP_ROWS_QW] = o->smp_rows ? o->smp_rows_qw : 0;
-            v[LMCMA_B200_LAUNCH_SMP_ROWS_RL] = o->smp_rows ? o->smp_rows_rl : 0;
-            v[LMCMA_B200_LAUNCH_SMP_KC] = o->smp_rows ? o->smp_rows_kc : o->smp_kc;
-            v[LMCMA_B200_LAUNCH_SMP_STAGES] = o->smp_rows ? o->smp_rows_stages : o->smp_stages;
-            v[LMCMA_B200_LAUNCH_UPD_NVB] = o->upd_nvb;
-            v[LMCMA_B200_LAUNCH_UPD_RMAX] = o->upd_rmax;
-            v[LMCMA_B200_LAUNCH_UPD_ROWS_IN_SMEM] = o->upd_rows_in_smem ? 1 : 0;
-            v[LMCMA_B200_LAUNCH_UPD_GRAM] = o->upd_gram ? 1 : 0;
-            v[LMCMA_B200_LAUNCH_UPD_WARPS] = o->upd_warps;
-            v[LMCMA_B200_LAUNCH_UPD_SWEEP_WARPS] = o->upd_warps;
-            v[LMCMA_B200_LAUNCH_COEF_ELEMS] = o->coef_elems;
-            v[LMCMA_B200_LAUNCH_RANK_THREADS] = o->rank_threads;
-            v[LMCMA_B200_LAUNCH_RANK_FTILE] = d.rank_ftile;
-            v[LMCMA_B200_LAUNCH_RANK_TILE_SORTED] = d.tile_sorted ? 1 : 0;
-            v[LMCMA_B200_LAUNCH_PROGRESSIVE] = o->progressive ? 1 : 0;
-            v[LMCMA_B200_LAUNCH_OVERLAP] = o->overlap ? 1 : 0;
+            launch_fields(o->plan, out);
+            out[LMCMA_B200_LAUNCH_OVERLAP] = o->overlap ? 1 : 0;   // what the handle runs now, not what the plan allowed
             return 0;
-        }
         default: return fail(LMCMA_B200_ERR_ARG, "unknown i32 field %d", which);
     }
     ARG(cap >= (int64_t)cnt, "capacity");

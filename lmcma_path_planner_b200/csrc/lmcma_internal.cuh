@@ -1,6 +1,7 @@
-// lmcma_internal.cuh — what the translation units of liblmcma_b200.so share: error helpers, the create-time tuning knobs,
-// the two handle types and the launch helpers that cross a file boundary.
-//   lmcma_capi.cu        library / device queries, the optimiser entry points, launch configuration, CUDA graphs
+// lmcma_internal.cuh — what the translation units of liblmcma_b200.so share: error helpers, the two handle types and the
+// launch helpers that cross a file boundary.  The create-time tuning knobs and the launch plan: lmcma_plan.hpp.
+//   lmcma_capi.cu        library / device queries, the optimiser entry points, the launchers, CUDA graphs
+//   lmcma_plan.cpp       the launch plan of an optimiser handle: kernel builds, block sizes, grids, shared memory
 //   lmcma_capi_map.cu    cost map handles, distance transform, the cost evaluator (k_cost, k_edt, k_brick)
 //   lmcma_capi_state.cu  state getters / setters, the host-side pieces of the reference API
 #pragma once
@@ -19,6 +20,7 @@
 #include <vector>
 #include "../../include/lmcma_b200.h"
 #include "lmcma_host.hpp"
+#include "lmcma_plan.hpp"
 #include "lmcma_common.cuh"
 
 namespace lmcma_capi {
@@ -91,45 +93,6 @@ struct Graph {
     int launches = 0;
 };
 
-
-inline int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v && *v ? atoi(v) : dflt;
-}
-
-// Every LMCMA_B200_* environment knob, read ONCE when a handle (map or optimiser) is created and kept on the handle:
-// nothing on a launch path calls getenv.  The defaults are the product; each switch is a serial-order reference of the
-// bit-identity tests, a test seam, an operational override or a diagnostic (INTEGRATION.md section 5 lists them all).
-struct Tuning {
-    int cost_minb = 0 /* 0 = by launch size */, cost_tpt = 0, cost_cb = 0, zerocopy = 1;
-    int sample_rows = 0;    // 1: k_sample_rows also for one large population (else only where it pays: many rows)
-    int update_gram = 0, progressive = 1, overlap = 1, tell_overlap = 1;
-    int tell_spec = 1;      // tell_all: speculative update of the next generation at the end of the graph (LMCMA_B200_TELL_SPEC=0: off)
-    int graph_unroll = 8;   // fused generations per CUDA graph for runs of at least that many (LMCMA_B200_GRAPH_UNROLL, 1 = off)
-    int update_warps = 0;   // k_update CTA size: 0 = by batch size, 8 / 16 forced (LMCMA_B200_UPDATE_WARPS)
-    int graph_dbg = 0, dbg = 0, update_dbg = 0, cost_dbg = 0;
-    static Tuning from_env() {
-        Tuning t;
-        t.cost_minb = env_int("LMCMA_B200_COST_MINB", t.cost_minb);
-        t.cost_tpt = env_int("LMCMA_B200_COST_TPT", 0);
-        t.cost_cb = env_int("LMCMA_B200_COST_CB", 0);
-        t.zerocopy = env_int("LMCMA_B200_ZEROCOPY", 1);
-        t.sample_rows = env_int("LMCMA_B200_SAMPLE_ROWS", 0);
-        t.update_gram = env_int("LMCMA_B200_UPDATE_GRAM", 0);
-        t.progressive = env_int("LMCMA_B200_PROGRESSIVE", 1);
-        t.overlap = env_int("LMCMA_B200_OVERLAP", 1);
-        t.tell_overlap = env_int("LMCMA_B200_TELL_OVERLAP", 1);
-        t.tell_spec = env_int("LMCMA_B200_TELL_SPEC", 1);
-        t.update_warps = env_int("LMCMA_B200_UPDATE_WARPS", 0);
-        t.graph_unroll = env_int("LMCMA_B200_GRAPH_UNROLL", 8);
-        if (t.graph_unroll < 1 || t.graph_unroll > 64) t.graph_unroll = 1;
-        t.graph_dbg = env_int("LMCMA_B200_GRAPH_DBG", 0);
-        t.dbg = getenv("LMCMA_B200_DBG") ? 1 : 0;
-        t.update_dbg = getenv("LMCMA_B200_UPDATE_DBG") ? 1 : 0;
-        t.cost_dbg = getenv("LMCMA_B200_COST_DBG") ? 1 : 0;
-        return t;
-    }
-};
 
 struct DeviceProps {
     int sm_count = 0;
@@ -219,30 +182,19 @@ struct lmcma_b200_opt {
     float* f_pinned = nullptr;                // the graph's copy source (the caller's fitness array is copied here first)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool have_run_timing = false;
-    // sample launch config
-    int smp_threads = 128, smp_kc = 1, smp_nv = 1, smp_rb = 1, smp_stages = 2;
-    bool smp_wide = false; int smp_R = 1, smp_CW = 1, smp_qpw = 32, smp_RBW = 1;
-    bool smp_rows = false; int smp_rows_qw = 8, smp_rows_rl = 1, smp_rows_kc = 8, smp_rows_stages = 2, smp_rows_region = 0;   // k_sample_rows
-    size_t smp_rows_smem = 0;
+    lmcma_capi::LaunchPlan plan;       // every kernel configuration, chosen at create (lmcma_plan.hpp)
     float* d_Lf = nullptr;             // lower Cholesky factor of the smoothness prior (n x ns FP32) or null
     bool mirror_dirty = true;          // the sequence-ordered pair mirror must be rebuilt (k_pack_pairs) before sampling
-    size_t smp_smem = 0;
     lmcma::CostShape cost_shape;
-    bool progressive = false;   // k_update -> k_sample hand-over inside the fused generation (k_update.cuh)
-    bool overlap = false;       // fused generation with k_update on a side branch, concurrent with k_cost / k_rank (k_update.cuh)
+    // fused generation with k_update on a side branch, concurrent with k_cost / k_rank (k_update.cuh): plan.overlap, until
+    // something at run time rules it out (no side stream, the co-scheduling probe, a failed forked capture, check_lost)
+    bool overlap = false;
     cudaStream_t side_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     float* x_mirror = nullptr;        // page-locked, mapped host mirror of X (lmcma_b200_ask_all_view); OptDev::Xh is its device alias
     bool mirror_on = false, mirror_suppressed = false, xh_fresh = false;
     int* err_host = nullptr;          // page-locked, mapped: OptDev::err (a kernel of the overlapped generation gave up on its partner)
     long long* graph_dbg = nullptr;   // LMCMA_B200_GRAPH_DBG: k_update's timeline inside the fused generation, printed by lmcma_b200_sync
-    int upd_nvb = 4, upd_rmax = 0, upd_warps = 16;
-    bool upd_gram = false; size_t coef_smem = 0;   // Gram-matrix recompute (k_gram.cuh) for rows that fit neither registers nor smem
-    int coef_elems = 0;                            // k_coef<coef_elems>: elements per lane, ceil(m / 8) rounded up to a build
-    bool upd_rows_in_smem = true;
-    size_t upd_smem = 0, rank_smem = 0;
-    int rank_threads = 1024;
-    size_t cost_smem = 0;
 };
 
 

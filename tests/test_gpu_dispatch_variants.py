@@ -1,6 +1,6 @@
 """Every sampler / update / k_coef build the launcher can pick by default, against the FP64 oracle.
 
-The launcher picks a template instantiation from n, lambda, m and the batch size (configure_sample / configure_update /
+The launcher picks a template instantiation from n, lambda, m and the batch size (plan_launch in lmcma_plan.cpp,
 launch_sample / launch_update in lmcma_capi.cu), not from a workload name, so the shapes bench.py times leave builds
 untested that users reach just by asking for more waypoints or a larger population.  Each case below first asserts,
 through Optimizer.launch(), that it got the build it is there for, then runs the oracle comparison; the coverage test at
@@ -96,10 +96,9 @@ def _instantiations(l):
     if l["sampler"] == "rows":
         smp = "launch_sample_rows_t<%d,%d>" % (l["smp_rows_qw"], l["smp_rows_rl"])
     elif l["sampler"] == "wide":
-        smp = {2: "launch_sample_wide_t<2,1024>", 4: "launch_sample_wide_t<4,512>"}[l["smp_RBW"]]
+        smp = "launch_sample_wide_t<%d>" % l["smp_RBW"]
     else:
-        smp = {1: "<1,4,512>", 2: "<2,4,512>", 4: "<4,2,512,true>", 8: "<8,1,512>", 12: "<12,1,256>", 16: "<16,1,256>"}[l["smp_nv"]]
-        smp = "launch_sample_t" + smp
+        smp = "launch_sample_t<%d>" % l["smp_nv"]
     nvb, rmax = l["upd_nvb"], l["upd_rmax"]
     if l["upd_gram"]:
         return {smp, "launch_update_t<%d,-1,false>" % nvb, "k_coef<%d>" % l["coef_elems"]}
@@ -356,7 +355,7 @@ def test_fused_graphs_beyond_512_columns(map1024, monkeypatch):
 # ------------------------------------------------------------------------------------------------
 # 8. coverage: the table reaches every instantiation the launcher has
 # ------------------------------------------------------------------------------------------------
-def test_every_launcher_instantiation_has_a_case(monkeypatch):
+def test_every_launcher_instantiation_is_reached_by_a_case(monkeypatch):
     import importlib
     reached = {}
     for cid, c in CASES.items():
