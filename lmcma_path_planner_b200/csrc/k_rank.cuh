@@ -114,8 +114,8 @@ __device__ __forceinline__ void tell_phase_a(const OptDev& o, const float* __res
     __shared__ int sh_nsel;
     __shared__ unsigned long long sh_S;
 
-#define RNK_STAMP(k) do { if (o.dbg && threadIdx.x == 0 && blockIdx.x == 0 && b == 0) o.dbg[16 + (k)] = gtime(); } while (0)
-    RNK_STAMP(0);
+#define RNK_STAMP(k) do { if (o.dbg && threadIdx.x == 0 && blockIdx.x == 0 && b == 0) o.dbg[k] = gtime(); } while (0)
+    RNK_STAMP(TL_RANK_START);
     const bool sorted = o.tile_sorted != nullptr;                    // sorted-tile mode (k_rank_tiles ran just before this grid)
     const float* cur = f_all + (size_t)b * lambda;
     const float* cur_stage = sorted ? o.tile_sorted + (size_t)b * lambda : cur;
@@ -193,7 +193,7 @@ __device__ __forceinline__ void tell_phase_a(const OptDev& o, const float* __res
         }
     }
     __syncthreads();
-    RNK_STAMP(1);
+    RNK_STAMP(TL_RANK_RANKED);
     if (tid == 0 && sh_S) atomicAdd(o.S_count + b, sh_S);
 
     // ---- compact the selected rows (rank < mu) in row order: deterministic summation order ----
@@ -214,7 +214,7 @@ __device__ __forceinline__ void tell_phase_a(const OptDev& o, const float* __res
         if (lane == 0) sh_nsel = nsel;
     }
     __syncthreads();
-    RNK_STAMP(2);
+    RNK_STAMP(TL_RANK_COMPACTED);
     const int nsel = sh_nsel;
 
     // ---- weighted partial sums of d = x - xmean: 128 float4 columns x (nthr/128) row groups ----
@@ -242,7 +242,7 @@ __device__ __forceinline__ void tell_phase_a(const OptDev& o, const float* __res
                 }
             }
         }
-        RNK_STAMP(3);
+        RNK_STAMP(TL_RANK_GATHERED);
         if (g > 0) red[(g - 1) * 128 + tq] = acc;
         __syncthreads();
         if (g == 0 && q < nq) {
@@ -251,7 +251,7 @@ __device__ __forceinline__ void tell_phase_a(const OptDev& o, const float* __res
         }
         __syncthreads();
     }
-    RNK_STAMP(4);
+    RNK_STAMP(TL_RANK_STORED);
 #undef RNK_STAMP
 }
 
@@ -296,7 +296,7 @@ __global__ void __launch_bounds__(MAXT, 2) k_rank(OptDev o, const float* __restr
     if (threadIdx.x == 0) {
         __threadfence();
         atomicAdd(o.rank_ticket + b, 1u);
-        if (o.dbg && b == 0 && blockIdx.x == gridDim.x - 1) o.dbg[21] = gtime();
+        if (o.dbg && b == 0 && blockIdx.x == gridDim.x - 1) o.dbg[TL_RANK_LAST_SLICE] = gtime();
     }
     if (!(mode & RANK_PACK)) return;
     __threadfence();

@@ -262,8 +262,8 @@ template <int RBW, int MAXT>
 __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nstages, int R, int CW, int qpw /* float4 columns per warp */,
                                                        int progressive) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-#define SMP_STAMP(k) do { if (o.dbg && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) o.dbg[32 + k] = gtime(); } while (0)
-    SMP_STAMP(0);
+#define SMP_STAMP(k) do { if (o.dbg && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) o.dbg[k] = gtime(); } while (0)
+    SMP_STAMP(TL_SMP_START);
     const int b = blockIdx.y;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int rl = warp / CW, cw = warp - rl * CW;              // row-group within the CTA, column-warp within the row
@@ -305,7 +305,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
         if (threadIdx.x == 0) wait_flag(progressive == 2 ? flags + o.m + 1 : flags);   // (early) scalars
         __syncthreads();
     }
-    SMP_STAMP(1);
+    SMP_STAMP(TL_SMP_FLAGS);
     const float* vps = o.VPs + (size_t)b * o.m * 2 * ns;
     // one bulk async copy per chunk of consecutive pairs; sized by m, not by the live count, so that the first
     // chunks are requested before the scalar state has even been read (rows beyond `live` are never used)
@@ -322,7 +322,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
     const Scalars sc = o.sc[b];
     const int live = sc.live;
     const int nchunks = (live + kc - 1) / kc;
-    SMP_STAMP(2);
+    SMP_STAMP(TL_SMP_SCALARS);
     const float Mf = (float)o.M, Minv = 1.0f / Mf;
     // the groups of 8 start at chunk boundaries: with kc < 8 (rows longer than ~1600) pair k is element (k mod kc) of its
     // group, and the last group reads up to 7 entries past its last live pair (zeros: they scale dots of zero pairs)
@@ -413,7 +413,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
         }
         z[r] = v; az[r] = v;
     }
-    SMP_STAMP(3);
+    SMP_STAMP(TL_SMP_Z);
     __syncthreads();                                            // nj_s
     // The chunks are consumed in rounds of up to `nstages` resident chunks.  Within a round every dot product comes
     // first (all against the ORIGINAL z: no ordering between pairs), the partial sums are exchanged ONCE, then the
@@ -432,8 +432,8 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
             const int st = c % nstages;
             if (progressive && warp == 0) provide_chunk(c);
             mbar_wait(&bars[st], (unsigned)((c / nstages) & 1));
-            if (c == 0) SMP_STAMP(4);
-            if (c < 8) SMP_STAMP(7 + c);
+            if (c == 0) SMP_STAMP(TL_SMP_FIRST_PAIRS);
+            if (c < TL_SMP_CHUNKS) SMP_STAMP(TL_SMP_CHUNK + c);
             const float* sb = stage_base + st * stage_floats;
             const int cnt = min(kc, live - c * kc);
             for (int k = 0; k < cnt; k += SAMPLE_G, ++grp) {
@@ -454,10 +454,10 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
                 }
             }
         }
-        SMP_STAMP(15);
+        SMP_STAMP(TL_SMP_DOTS);
         if (CW > 1) named_bar_sync(1 + rl, CW * 32);            // the CW warps of this row-group (ids 1..15: R <= 15)
         else __syncwarp();
-        SMP_STAMP(16);
+        SMP_STAMP(TL_SMP_EXCHANGED);
         grp = grp0;
         for (int c = c0; c < c1; ++c) {
             const int st = c % nstages;
@@ -499,7 +499,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
         }
     }
     (void)gpc;
-    SMP_STAMP(5);
+    SMP_STAMP(TL_SMP_LOOP_DONE);
     double sigma = sc.sigma;
     if (progressive == 2) {                                     // step size and mean arrive after k_rank, late in k_update
         if (threadIdx.x == 0) wait_flag(flags);
@@ -515,7 +515,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
         }
     }
     if (progressive) griddep_wait();                            // stream order: this grid ends after k_update has
-    SMP_STAMP(6);
+    SMP_STAMP(TL_SMP_END);
 #undef SMP_STAMP
 }
 

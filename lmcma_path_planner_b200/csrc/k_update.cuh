@@ -33,7 +33,7 @@ struct UpdateArgs {
     int n_slices;
     long long slice_stride, inst_stride;
     int payload_mode;          // slices are all-gather payloads (S rides in the 2 floats after ns)
-    long long* dbg;            // optional: globaltimer stamps (LMCMA_B200_UPDATE_DBG)
+    long long* dbg;            // optional: OptDev::dbg + TL_UPD, the TL_UPD_* timeline slots (LMCMA_B200_DBG); null in normal runs
     int overlap;               // fused single-query generation: this kernel runs on a side branch of the graph, CONCURRENTLY
                                // with k_cost and k_rank.  Everything that does not depend on this generation's fitness —
                                // bookkeeping, and the sweep over every pending row but the newest — comes first; then it
@@ -133,7 +133,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         __syncthreads();
         if (tid == 0) { __threadfence(); st_release_gpu(o.resident + b, 1); }
     }
-    UPD_STAMP(0);
+    UPD_STAMP(TL_UPD_START);
     // =============================== prologue: independent of k_rank ===============================
     for (int i = tid; i < m; i += nthr) { order[i] = tg[i]; stamp[i] = vg[i]; ljslot[i] = (float)Ljd[i]; mbar_init(&rowbar[i], 1); mbar_init(&scalbar[i], 1); }
     if (tid == 0) { sh_key = ~0ull; if (SMEM) mbar_init(&sh_bar, 1); }
@@ -183,7 +183,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         st_release_gpu(flags + m + 1, 1);
     }
     if (first_stale == 1) first_stale = 0;                           // lmcma.cpp:373-374
-    UPD_STAMP(1);
+    UPD_STAMP(TL_UPD_BOOKKEEPING);
 
     // ---- direction rows -> shared memory by 1-D bulk async copies issued by the lanes of warp 0: final rows
     //      (i < first_stale) come from V, pending rows start as their pc_j (lmcma.cpp:376-378); the newest
@@ -262,7 +262,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         mbar_wait(&sh_bar, 0);
     }
     if (OVERLAP) __syncthreads(); else best_so_far(0, nwarps);             // overlap: k_cost is still running
-    UPD_STAMP(2);
+    UPD_STAMP(TL_UPD_PROLOGUE);
 
     // =============================== needs k_rank's partial sums ===============================
     // ---- population-success step size (lmcma.cpp:393-419), counters (lmcma.cpp:189, 423): needs only k_rank's pair
@@ -328,7 +328,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         }
     };
     auto post_rank = [&](const bool dry) {                           // block-collective; dry: same instructions, no side effects
-    if (!dry) UPD_STAMP(3);
+    if (!dry) UPD_STAMP(TL_UPD_POST);
     // overlap: the pair count is fetched here and used beside the chain, so its round trip hides behind the slice loads
     if (OVERLAP && tid == nthr - 1 && !dry && !a.payload_mode) S_early = atomicExch(o.S_count + b, 0ull);
     if (tid == 0 && !dry) o.rank_ticket[b] = 0u;                             // k_rank's CTAs of this generation have all drawn one
@@ -393,7 +393,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     }
     if (!SMEM) __threadfence();
     __syncthreads();
-    if (!dry) UPD_STAMP(4);
+    if (!dry) UPD_STAMP(TL_UPD_MEAN);
     if (a.progressive && !dry) {
         // scalars and mean are final; so are the pairs in front of the first stale position (untouched this generation;
         // overlap mode has published those before its sweep)
@@ -526,7 +526,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
             }
             __syncwarp();                                            // orders the lanes' stores before lane 0's release
             if (lane == 0) mbar_arrive(&rowbar[i]);                  // ONE arrive: 32 arrives on one mbarrier serialise (~27 cycles each)
-            if (a.dbg && lane == 0 && i < 40) a.dbg[24 + i] = gtime();
+            if (a.dbg && lane == 0 && i < TL_UPD_ROW_STAMPS) a.dbg[TL_UPD_ROWS + i] = gtime();
             float2 nn = make_float2(0.f, 0.f);                       // |v_i|^2: after the hand-over, off the chain
 #pragma unroll
             for (int it = 0; it < NVB; ++it) { nn = ffma2(lo2(x[it]), lo2(x[it]), nn); nn = ffma2(hi2(x[it]), hi2(x[it]), nn); }
@@ -633,11 +633,11 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                     const float2 l = ffma2(me, lo2(v[r]), lo2(yn)), h = ffma2(me, hi2(v[r]), hi2(yn));
                     yn = make_float4(l.x, l.y, h.x, h.y);
                 }
-                if (a.dbg && tid == 0 && OVERLAP && !dry) a.dbg[12 + (j0 >> 3)] = gtime();
+                if (a.dbg && tid == 0 && OVERLAP && !dry) a.dbg[TL_UPD_CHAIN + (j0 >> 3)] = gtime();
             }
             // pc at its position in the mirror (after the chain: nothing in it should queue behind these stores)
             if (has && !dry) reinterpret_cast<float4*>(VPb + ((size_t)(live - 1) * 2 + 1) * ns)[q] = pc4;
-            if (OVERLAP) { if (a.dbg && tid == 0 && !dry) a.dbg[18] = gtime(); __syncthreads(); }   // the other warps have copied the best-so-far candidate out of X
+            if (OVERLAP) { if (a.dbg && tid == 0 && !dry) a.dbg[TL_UPD_BEST_COPIED] = gtime(); __syncthreads(); }   // the other warps have copied the best-so-far candidate out of X
             // ---- publish: y K^(live-1) is the final v of the newest pair (what publish() does for a row held by one warp) ----
             const int i = live - 1;
             const float kf = (float)kn;
@@ -658,7 +658,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
 #pragma unroll
                 for (int w = 1; w < NVB; ++w) nv += norm_part[w];
                 mbar_arrive(&rowbar[i]);
-                if (a.dbg && i < 40) a.dbg[24 + i] = gtime();
+                if (a.dbg && i < TL_UPD_ROW_STAMPS) a.dbg[TL_UPD_ROWS + i] = gtime();
                 publish_scalars(i, nv);
                 mbar_arrive(&scalbar[i]);
                 if (a.progressive) {                                 // pair i of the mirror and Njs[i] are final
@@ -757,7 +757,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         }
         // every older row is final
         __syncthreads();
-        UPD_STAMP(7);
+        UPD_STAMP(TL_UPD_ROWS_FINAL);
         if (phase != 2) for (int k = 1 + warp; k < hi; k += WARPS) gram_row(k);  // block Gram entries for the newest row's chain
         if (phase == 1) {
             // ---- speculative pass: leave the rows, their scalars and the Gram entries for the next tell_all and stop here ----
@@ -803,7 +803,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                         __threadfence();
                     }
                     __syncthreads();
-                    UPD_STAMP(8);
+                    UPD_STAMP(TL_UPD_RANKS_SEEN);
                 }
                 if (step == 1 || step == 2) {
                     post_rank(dry);                                  // mean, step size, the new evolution path -> rows_s[live - 1]
@@ -815,7 +815,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                         if (tid == nthr - 1 && !dry) {                // the thread that took the pair count in post_rank
                             step_size_and_counters();
                             if (a.progressive) st_release_gpu(flags, 1);
-                            if (a.dbg) a.dbg[22] = gtime();
+                            if (a.dbg) a.dbg[TL_UPD_STEP_SIZE] = gtime();
                         }
                     } else if (!dry) {
                         best_so_far(NVB, nwarps - NVB - 1);
@@ -823,7 +823,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                     __syncthreads();
                 } else {
                     newest_row(dry, need);
-                    if (!dry) UPD_STAMP(9);
+                    if (!dry) UPD_STAMP(TL_UPD_NEWEST);
                 }
             }
         } else {
@@ -896,9 +896,9 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         }
     }
     __syncthreads();
-    UPD_STAMP(5);
+    UPD_STAMP(TL_UPD_TAIL);
     if (OVERLAP) copy_fitness();                                     // (post_rank leaves it to the end in this build)
-    if (a.dbg && threadIdx.x == 0) { a.dbg[10] = first_stale; a.dbg[11] = live; }
+    if (a.dbg && threadIdx.x == 0) { a.dbg[TL_UPD_FIRST_STALE] = first_stale; a.dbg[TL_UPD_LIVE] = live; }
     for (int i = first_stale + tid; i < live && RMAX >= 0; i += nthr) {   // FP64 scalar state of the recomputed rows
         const int slot = order[i];
         const double nv = (double)nv_s[i], r = o.c1 / (1.0 - o.c1), am = o.M;
@@ -906,7 +906,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         const double nj = am * r / (t + 1.0), lj = r / (am * t * (t + 1.0));
         Njd[slot] = nj; Ljd[slot] = lj; Njf[slot] = (float)nj; Njsb[i] = (float)nj;
     }
-    UPD_STAMP(6);
+    UPD_STAMP(TL_UPD_END);
 }
 
 // overlapped generation: k_cost must not be released before every k_update CTA holds its SM (a full SM: 512 threads x 128

@@ -162,6 +162,7 @@ UpdateArgs update_args_local(lmcma_b200_opt* o) {
     a.f_all = o->d.fit;
     a.slices = o->d.partial; a.n_slices = o->d.RS; a.slice_stride = o->d.ns; a.inst_stride = (long long)o->d.RS * o->d.ns;
     a.spec = o->d_spec; a.spec_stride = (long long)o->spec_stride;
+    a.dbg = o->d.dbg ? o->d.dbg + TL_UPD : nullptr;
     return a;
 }
 
@@ -247,9 +248,43 @@ int replay(const Graph& g, cudaStream_t st) {
     return 0;
 }
 
-// LMCMA_B200_GRAPH_DBG: k_update's timeline inside the graphs, printed by lmcma_b200_sync (best effort)
-void ensure_graph_dbg(lmcma_b200_opt* o) {
-    if (o->tune.graph_dbg && !o->graph_dbg && cudaMalloc(&o->graph_dbg, 64 * sizeof(long long)) == cudaSuccess) { cudaMemset(o->graph_dbg, 0, 64 * sizeof(long long)); cudaDeviceSynchronize(); }
+// LMCMA_B200_DBG: the device timeline (TimelineSlot) on stderr, in ns after its earliest stamp ("-": not stamped), then
+// cleared, so that each print shows only what ran since the last one
+int print_timeline(lmcma_b200_opt* o) {
+    long long h[TL_SLOTS];
+    CU(cudaMemcpyAsync(h, o->d.dbg, sizeof(h), cudaMemcpyDeviceToHost, o->stream));
+    CU(cudaStreamSynchronize(o->stream));
+    const long long* u = h + TL_UPD;
+    long long t0 = 0;
+    for (int i = 0; i < TL_SLOTS; ++i)
+        if (h[i] && i != TL_UPD + TL_UPD_FIRST_STALE && i != TL_UPD + TL_UPD_LIVE && (!t0 || h[i] < t0)) t0 = h[i];
+    auto at = [&](long long t) { t ? fprintf(stderr, "%lld", t - t0) : fprintf(stderr, "-"); };
+    auto named = [&](const char* section, const long long* base, std::initializer_list<std::pair<const char*, int>> slots) {
+        fprintf(stderr, "  %s:", section);
+        for (const auto& s : slots) { fprintf(stderr, " %s=", s.first); at(base[s.second]); }
+        fprintf(stderr, "\n");
+    };
+    auto series = [&](const char* name, const long long* t, int count) {
+        fprintf(stderr, "    %s:", name);
+        for (int i = 0; i < count; ++i) { fprintf(stderr, " "); at(t[i]); }
+        fprintf(stderr, "\n");
+    };
+    fprintf(stderr, "device timeline (ns after the earliest stamp)\n");
+    named("k_update", u, {{"start", TL_UPD_START}, {"bookkeeping", TL_UPD_BOOKKEEPING}, {"prologue", TL_UPD_PROLOGUE},
+                          {"rows_final", TL_UPD_ROWS_FINAL}, {"ranks_seen", TL_UPD_RANKS_SEEN}, {"post_rank", TL_UPD_POST},
+                          {"mean", TL_UPD_MEAN}, {"step_size", TL_UPD_STEP_SIZE}, {"best_copied", TL_UPD_BEST_COPIED},
+                          {"newest_row", TL_UPD_NEWEST}, {"tail", TL_UPD_TAIL}, {"end", TL_UPD_END}});
+    fprintf(stderr, "    first_stale=%lld live=%lld\n", u[TL_UPD_FIRST_STALE], u[TL_UPD_LIVE]);
+    series("chain blocks", u + TL_UPD_CHAIN, TL_UPD_CHAIN_STAMPS);
+    series("rows", u + TL_UPD_ROWS, TL_UPD_ROW_STAMPS);
+    named("k_rank CTA 0", h, {{"start", TL_RANK_START}, {"ranked", TL_RANK_RANKED}, {"compacted", TL_RANK_COMPACTED},
+                              {"gathered", TL_RANK_GATHERED}, {"stored", TL_RANK_STORED}, {"last_slice", TL_RANK_LAST_SLICE}});
+    named("k_sample_wide CTA 0", h, {{"start", TL_SMP_START}, {"flags", TL_SMP_FLAGS}, {"scalars", TL_SMP_SCALARS}, {"z", TL_SMP_Z},
+                                     {"first_pairs", TL_SMP_FIRST_PAIRS}, {"dots", TL_SMP_DOTS}, {"exchanged", TL_SMP_EXCHANGED},
+                                     {"loop_done", TL_SMP_LOOP_DONE}, {"end", TL_SMP_END}});
+    series("chunks", h + TL_SMP_CHUNK, TL_SMP_CHUNKS);
+    CU(cudaMemsetAsync(o->d.dbg, 0, sizeof(h), o->stream));
+    return 0;
 }
 
 // Do the two branches of a forked CUDA graph really run concurrently on this device, in this process?  (Not under a
@@ -310,13 +345,11 @@ int ensure_graph(lmcma_b200_opt* o) {
     if (rc) return rc;
     cudaStream_t st = o->stream;
     if ((rc = ensure_mirror(o, st))) return rc;
-    ensure_graph_dbg(o);
     // `reps` generations in ONE graph: between two graph launches the device idles for the launch latency of the next one
     // (~5 us of a 52 us generation); inside a graph a generation follows the previous one as a plain dependency
     auto body = [&](int reps) -> int {
         UpdateArgs ua = update_args_local(o);
         ua.progressive = o->plan.progressive ? 1 : 0;            // ensure_mirror above: the mirror is clean
-        ua.dbg = o->graph_dbg;
         int rc2 = 0;
         for (int g = 0; g < reps && !rc2; ++g) {
             if (o->overlap) {
@@ -373,7 +406,6 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
     // k_update would be the longer branch of the graph (measured: tell_all 57 -> 69 us)
     const bool spec = o->d_spec != nullptr && o->mirror_on && !o->mirror_suppressed;
     o->tell_graph_spec = spec;
-    ensure_graph_dbg(o);
     // resume = 0: the whole update; resume = 1: k_update picks up the rows the last graph's speculative pass left.  With the
     // scratch both graphs END with that pass for the next generation, on the side branch behind k_update
     auto body = [&](int resume) -> int {
@@ -381,7 +413,6 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
         ua.progressive = 1;
         ua.overlap = 1;
         ua.phase = resume ? 2 : 0;
-        ua.dbg = o->graph_dbg;                                   // LMCMA_B200_GRAPH_DBG: the timeline lmcma_b200_sync prints
         const bool valid_before = o->spec_valid;
         bool ok = cudaEventRecord(o->ev_fork, st) == cudaSuccess && cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) == cudaSuccess;
         if (ok) ok = launch_update(o, ua, false, o->side_stream) == 0;
@@ -537,7 +568,7 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     DM(d.VPs, B * m * 2 * ns);
     DM(d.t, B * m); DM(d.vec, B * m);
     DM(d.sc, B); DM(d.best_x, B * ns); DM(d.S_count, B); DM(d.done_count, B); DM(d.progress, B * (m + 2)); DM(d.rank_ticket, B); DM(d.resident, B);
-    if (o->tune.dbg) DM(d.dbg, 64);
+    if (o->tune.dbg) DM(d.dbg, TL_SLOTS);
     DM(d.partial, B * d.RS * ns);
 
     std::vector<float> wf(o->weights.begin(), o->weights.end());
@@ -623,7 +654,6 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     if (o->side_stream) cudaStreamDestroy(o->side_stream);
     if (o->ev_fork) cudaEventDestroy(o->ev_fork);
     if (o->ev_join) cudaEventDestroy(o->ev_join);
-    if (o->graph_dbg) cudaFree(o->graph_dbg);
     delete o;
     return 0;
 }
@@ -844,27 +874,7 @@ int lmcma_b200_sync(lmcma_b200_opt* o) {
     CU(cudaSetDevice(o->cfg.device));
     CU(cudaStreamSynchronize(o->stream));
     { int lost = check_lost(o); if (lost) return lost; }
-    if (o->graph_dbg) {
-        long long h[64];
-        cudaMemcpy(h, o->graph_dbg, sizeof(h), cudaMemcpyDeviceToHost);
-        fprintf(stderr, "fused generation, k_update (ns since its start): bookkeeping=%lld prologue=%lld sweep: warp 0 done=%lld, all done + ranks seen=%lld post start=%lld mean=%lld progress[0]=%lld newest row=%lld tail=%lld end=%lld",
-                h[1] - h[0], h[2] - h[0], h[7] - h[0], h[8] - h[0], h[3] - h[0], h[4] - h[0], h[22] - h[0], h[9] - h[0], h[5] - h[0], h[6] - h[0]);
-        fprintf(stderr, " chain blocks:");
-        for (int i = 12; i < 21; ++i) fprintf(stderr, " %lld", (h[i] - h[0]) / 100);
-        fprintf(stderr, " rows:");
-        for (int i = 0; i < 40; ++i) fprintf(stderr, " %lld", (h[24 + i] - h[0]) / 100);
-        if (o->d.dbg) {
-            long long g[64];
-            cudaMemcpy(g, o->d.dbg, sizeof(g), cudaMemcpyDeviceToHost);
-            fprintf(stderr, " | k_sample CTA 0: start=%lld flags=%lld loop done=%lld end=%lld", g[32] - h[0], g[33] - h[0], g[37] - h[0], g[38] - h[0]);
-            fprintf(stderr, " | k_rank CTA 0: start=%lld ranked=%lld compacted=%lld gathered=%lld stored=%lld", g[16] - h[0], g[17] - h[0], g[18] - h[0], g[19] - h[0], g[20] - h[0]);
-            fprintf(stderr, " last slice stored=%lld", g[21] - h[0]);
-            cudaMemset(o->d.dbg + 21, 0, sizeof(long long));
-            cudaDeviceSynchronize();
-        }
-        fprintf(stderr, "\n");
-    }
-    return 0;
+    return o->d.dbg ? print_timeline(o) : 0;
 }
 
 int lmcma_b200_last_run_ms(lmcma_b200_opt* o, float* ms) {
@@ -900,17 +910,17 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
     }
     cudaError_t se = cudaStreamSynchronize(st);
     if (!rc && se != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "profile run: %s", cudaGetErrorString(se));
-    if (!rc && o->tune.cost_dbg) {     // debug: per-CTA timeline of k_cost (phase stamps), one extra launch
+    if (!rc && o->d.dbg) rc = print_timeline(o);
+    if (!rc && o->d.dbg) {     // and the per-CTA timeline of k_cost (phase stamps): one extra launch of its TRACE build
         const size_t ctas = (size_t)o->d.pop_count * o->d.B;
         long long* dbg = nullptr;
         if (cudaMalloc(&dbg, ctas * 8 * sizeof(long long)) == cudaSuccess) {
-            cudaMemset(dbg, 0, ctas * 8 * sizeof(long long));
-            cudaDeviceSynchronize();
+            std::vector<long long> h(ctas * 8);
+            cudaMemsetAsync(dbg, 0, h.size() * sizeof(long long), st);
             CostArgs cd = ca; cd.dbg = dbg; cd.cells = nullptr; cd.max_cells = 0;
             launch_cost(o->map->dev, cd, o->d.pop_count, o->d.B, o->cost_shape, true, st);   // the TRACE build carries the stamps (no cells requested)
+            cudaMemcpyAsync(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, st);
             cudaStreamSynchronize(st);
-            std::vector<long long> h(ctas * 8);
-            cudaMemcpy(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
             long long t0 = h[0];
             for (size_t c = 0; c < ctas; ++c) t0 = std::min(t0, h[c * 8]);
             static const char* nm[] = {"start", "x loaded", "phase 1 done", "loop done", "end samples done", "end"};
@@ -933,37 +943,6 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
             fprintf(stderr, "\n");
             cudaFree(dbg);
         }
-    }
-    if (!rc && o->tune.update_dbg) {   // debug: timeline of k_update
-        long long* dbg = nullptr;
-        if (cudaMalloc(&dbg, 64 * sizeof(long long)) == cudaSuccess) {
-            cudaMemset(dbg, 0, 64 * sizeof(long long));
-            UpdateArgs ua = update_args_local(o);
-            ua.dbg = dbg;
-            launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
-            launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st);
-            launch_update(o, ua, true, st);
-            launch_sample(o, st, true);
-            cudaStreamSynchronize(st);
-            long long h[64];
-            cudaMemcpy(h, dbg, sizeof(h), cudaMemcpyDeviceToHost);
-            static const char* names[] = {"start", "bookkeeping", "prologue done", "k_rank done", "mean", "sweep", "end"};
-            fprintf(stderr, "k_update timeline (ns since start; first_stale=%lld live=%lld):", h[10], h[11]);
-            for (int k = 1; k < 7; ++k) fprintf(stderr, " %s=%lld", names[k], h[k] - h[0]);
-            fprintf(stderr, "\n");
-            cudaFree(dbg);
-        }
-    }
-    if (!rc && o->d.dbg) {
-        long long h[64];
-        cudaMemcpy(h, o->d.dbg, sizeof(h), cudaMemcpyDeviceToHost);
-        fprintf(stderr, "k_sample timeline (CTA 0, ns):");
-        static const char* nm[] = {"start", "griddep", "order", "z ready", "first pairs", "loop done", "end"};
-        for (int k = 1; k < 7; ++k) fprintf(stderr, " %s=%lld", nm[k], h[32 + k] - h[32]);
-        fprintf(stderr, " | chunk waits:");
-        for (int k = 7; k < 12; ++k) fprintf(stderr, " %lld", h[32 + k] - h[32]);
-        fprintf(stderr, " dots done=%lld exchanged=%lld", h[32 + 15] - h[32], h[32 + 16] - h[32]);
-        fprintf(stderr, "\n");
     }
     for (int k = 0; k < 4; ++k) ms4[k] = 0.f;
     if (!rc)

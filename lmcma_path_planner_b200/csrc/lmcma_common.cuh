@@ -92,10 +92,33 @@ struct OptDev {
     unsigned* done_count;          // B : tickets of k_rank (split-population payload packing)
     double c1, cc, cs, target, K, M, mueff;
     double pc_coef;    // sqrt(cc (2 - cc) mueff), lmcma.cpp:328
-    long long* dbg;    // optional 64-slot debug timeline (LMCMA_B200_DBG); null in normal runs
+    long long* dbg;    // optional device timeline of TL_SLOTS stamps (LMCMA_B200_DBG, see TimelineSlot); null in normal runs
     int* err;          // host-visible (mapped, page-locked) error word of the handle: a kernel of the overlapped generation
                        // that gives up waiting for its concurrently running partner writes a code here and carries on
                        // (never __trap: that would poison the whole CUDA context); the host checks it at every sync
+};
+
+// The slots of the device timeline OptDev::dbg (LMCMA_B200_DBG): globaltimer stamps taken by one thread of instance 0,
+// printed and cleared by print_timeline (lmcma_capi.cu).  k_rank and k_sample_wide stamp [0, TL_UPD) through
+// OptDev::dbg; k_update stamps through UpdateArgs::dbg = OptDev::dbg + TL_UPD, so the TL_UPD_* slots count from there.
+enum TimelineSlot : int {
+    // k_rank, CTA 0: start, ranks stored, selected rows compacted, partial sums gathered / stored; the last CTA's ticket
+    TL_RANK_START = 16, TL_RANK_RANKED, TL_RANK_COMPACTED, TL_RANK_GATHERED, TL_RANK_STORED, TL_RANK_LAST_SLICE,
+    // k_sample_wide, CTA 0: start, flags / griddep, scalars read, z ready, first pairs, loop done, end; chunk c < 8
+    // arrived; last round's dots done and exchanged
+    TL_SMP_START = 32, TL_SMP_FLAGS, TL_SMP_SCALARS, TL_SMP_Z, TL_SMP_FIRST_PAIRS, TL_SMP_LOOP_DONE, TL_SMP_END,
+    TL_SMP_CHUNK, TL_SMP_CHUNKS = 8, TL_SMP_DOTS = TL_SMP_CHUNK + TL_SMP_CHUNKS, TL_SMP_EXCHANGED,
+    TL_UPD = 64,
+    // k_update, relative to TL_UPD: start, bookkeeping, prologue, post-rank start, mean, tail start, end, every older row
+    // final, ranks seen, newest row done (overlapped build)
+    TL_UPD_START = 0, TL_UPD_BOOKKEEPING, TL_UPD_PROLOGUE, TL_UPD_POST, TL_UPD_MEAN, TL_UPD_TAIL, TL_UPD_END,
+    TL_UPD_ROWS_FINAL, TL_UPD_RANKS_SEEN, TL_UPD_NEWEST,
+    TL_UPD_FIRST_STALE = 10, TL_UPD_LIVE = 11,          // values, not stamps
+    TL_UPD_BEST_COPIED = 18,                            // overlapped build: the best-so-far candidate is copied out of X
+    TL_UPD_STEP_SIZE = 22,                              // overlapped build: step size released (progress[0])
+    TL_UPD_ROWS = 24, TL_UPD_ROW_STAMPS = 40,           // row i < 40 published
+    TL_UPD_CHAIN = 64, TL_UPD_CHAIN_STAMPS = 10,        // overlapped build: block j0 / UPD_BLK of the newest row's chain (m <= 80)
+    TL_SLOTS = TL_UPD + TL_UPD_CHAIN + TL_UPD_CHAIN_STAMPS
 };
 
 // codes written to OptDev::err
@@ -132,7 +155,7 @@ struct CostArgs {
     long long max_cells;
     int cb;                    // capacity of the per-block record stage (32-sample blocks), set by the launcher
     int spt;                   // segments per thread = ceil((W + 1) / threads per trajectory), set by the launcher
-    long long* dbg;            // optional (LMCMA_B200_COST_DBG): 8 globaltimer stamps per CTA, [cta * 8 + k]
+    long long* dbg;            // optional (LMCMA_B200_DBG, profile_kernels): 8 globaltimer stamps per CTA, [cta * 8 + k]
 };
 
 struct CostShape { int tpt = 128, cb = 256, minb = 0; };   // launch shape of k_cost: threads per trajectory, block-record capacity, CTAs per SM of the build to launch (0 = chosen by the launch size)

@@ -194,7 +194,6 @@ struct lmcma_b200_opt {
     float* x_mirror = nullptr;        // page-locked, mapped host mirror of X (lmcma_b200_ask_all_view); OptDev::Xh is its device alias
     bool mirror_on = false, mirror_suppressed = false, xh_fresh = false;
     int* err_host = nullptr;          // page-locked, mapped: OptDev::err (a kernel of the overlapped generation gave up on its partner)
-    long long* graph_dbg = nullptr;   // LMCMA_B200_GRAPH_DBG: k_update's timeline inside the fused generation, printed by lmcma_b200_sync
 };
 
 

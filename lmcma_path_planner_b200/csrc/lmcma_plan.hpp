@@ -47,7 +47,7 @@ struct Tuning {
     int tell_spec = 1;      // tell_all: speculative update of the next generation at the end of the graph (LMCMA_B200_TELL_SPEC=0: off)
     int graph_unroll = 8;   // fused generations per CUDA graph for runs of at least that many (LMCMA_B200_GRAPH_UNROLL, 1 = off)
     int update_warps = 0;   // k_update CTA size: 0 = by batch size, 8 / 16 forced (LMCMA_B200_UPDATE_WARPS)
-    int graph_dbg = 0, dbg = 0, update_dbg = 0, cost_dbg = 0;
+    int dbg = 0;            // device timelines, printed by lmcma_b200_sync and profile_kernels (LMCMA_B200_DBG set)
     static Tuning from_env() {
         Tuning t;
         t.cost_minb = env_int("LMCMA_B200_COST_MINB", t.cost_minb);
@@ -63,10 +63,7 @@ struct Tuning {
         t.update_warps = env_int("LMCMA_B200_UPDATE_WARPS", 0);
         t.graph_unroll = env_int("LMCMA_B200_GRAPH_UNROLL", 8);
         if (t.graph_unroll < 1 || t.graph_unroll > 64) t.graph_unroll = 1;
-        t.graph_dbg = env_int("LMCMA_B200_GRAPH_DBG", 0);
         t.dbg = getenv("LMCMA_B200_DBG") ? 1 : 0;
-        t.update_dbg = getenv("LMCMA_B200_UPDATE_DBG") ? 1 : 0;
-        t.cost_dbg = getenv("LMCMA_B200_COST_DBG") ? 1 : 0;
         return t;
     }
 };

@@ -1,8 +1,8 @@
-"""Per-CTA phase timeline of k_cost on the C2 shape (LMCMA_B200_COST_DBG=1) and, optionally, a C3-shaped batch.
-  LMCMA_B200_COST_DBG=1 python tools/cost_timeline.py [batch]"""
+"""Per-CTA phase timeline of k_cost on the C2 shape (LMCMA_B200_DBG=1) and, optionally, a C3-shaped batch.
+  LMCMA_B200_DBG=1 python tools/cost_timeline.py [batch]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-os.environ.setdefault("LMCMA_B200_COST_DBG", "1")
+os.environ.setdefault("LMCMA_B200_DBG", "1")
 import numpy as np
 import lmcma_path_planner_b200 as L
 from lmcma_path_planner_b200 import maps

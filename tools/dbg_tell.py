@@ -1,5 +1,5 @@
 """Device timeline of tell_all on the C2 shape (k_update / k_rank / k_sample globaltimer stamps, printed by lmcma_b200_sync):
-  LMCMA_B200_GRAPH_DBG=1 LMCMA_B200_DBG=1 python tools/dbg_tell.py [flush]     flush: 256 MiB fill before every generation"""
+  LMCMA_B200_DBG=1 python tools/dbg_tell.py [flush]     flush: 256 MiB fill before every generation"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, bench
