@@ -99,7 +99,7 @@ __global__ void __launch_bounds__(64 * TMAX) k_coef(OptDev o) {
     const int* order = o.t + (size_t)b * m;
     const int sub = tid & 7, i = tid >> 3;                        // this thread's row (8 aligned lanes of one warp per row)
     const bool row_on = i < L;
-    const double Kd = o.K, invK = 1.0 / o.K, r = o.c1 / (1.0 - o.c1), am = o.M;
+    const double Kd = o.K, invK = 1.0 / o.K, r = nj_ratio(o), am = o.M;
     double c[TMAX], u[TMAX];
 #pragma unroll
     for (int t = 0; t < TMAX; ++t) {
@@ -187,8 +187,7 @@ __global__ void __launch_bounds__(64 * TMAX) k_coef(OptDev o) {
     for (int e = tid; e < L * L; e += nthr) { const int i2 = e / L, k = e - i2 * L; if (i2 >= first_stale) Cf[(size_t)i2 * m + k] = (k <= i2) ? Cs[i2 * LP + k] : 0.0; }
     for (int i2 = first_stale + tid; i2 < L; i2 += nthr) {
         const int slot = order[i2];
-        const double nv = nv_s[i2], t2 = sqrt(1.0 + r * nv);
-        const double nj = am * r / (t2 + 1.0);
+        const double nj = nj_form(r, am, nv_s[i2]).nj;
         o.Nj[(size_t)b * m + slot] = nj; o.Lj[(size_t)b * m + slot] = lj_s[i2] * Kd;
         o.Njf[(size_t)b * m + slot] = (float)nj; o.Njs[(size_t)b * m + i2] = (float)nj;
     }

@@ -8,17 +8,13 @@
 
 namespace lmcma {
 
-// Z <- N(0,1) from the same counter-based generator k_sample uses (so that a prior run and a plain run see the
-// same raw deviates): grid = (ceil(nq / 128), pop_count, B)
+// Z <- N(0,1), the samplers' deviates (philox_deviate4): grid = (ceil(nq / 128), pop_count, B)
 __global__ void __launch_bounds__(128) k_gauss(OptDev o) {
     const int q = blockIdx.x * 128 + threadIdx.x, row = blockIdx.y, b = blockIdx.z, nq = o.ns >> 2;
     if (q >= nq) return;
     const int itr = o.sc[b].itr;
-    float4 v = philox_normal4((unsigned)q, (unsigned)(o.pop_offset + row), (unsigned)itr, (unsigned)b, o.seed);
-    const int e = q * 4;
-    if (e + 1 >= o.n) v.y = 0.f;
-    if (e + 2 >= o.n) v.z = 0.f;
-    if (e + 3 >= o.n) v.w = 0.f;
+    float4 v;
+    philox_deviate4(o, b, row, q, itr, v);
     reinterpret_cast<float4*>(o.Z + ((size_t)b * o.pop_count + row) * o.ns)[q] = v;
 }
 

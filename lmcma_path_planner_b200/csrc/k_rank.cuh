@@ -288,7 +288,7 @@ __global__ void __launch_bounds__(MAXT, 2) k_rank(OptDev o, const float* __restr
     griddep_launch_dependents();
     const int b = blockIdx.y;
     // the hand-over flags of this generation's k_update -> k_sample (both start after this grid has completed)
-    if (blockIdx.x == 0 && !(mode & RANK_KEEP_FLAGS)) for (int i = threadIdx.x; i < o.m + 2; i += blockDim.x) o.progress[(size_t)b * (o.m + 2) + i] = 0;
+    if (blockIdx.x == 0 && !(mode & RANK_KEEP_FLAGS)) for (int i = threadIdx.x; i < progress_len(o.m); i += blockDim.x) progress_flags(o.progress, o.m, b)[i] = 0;
     tell_phase_a(o, f_all, b, blockIdx.x, smem_raw, prev_staged);
     // one ticket per CTA once its ranks / partial sums are stored: the overlapped generation's k_update (not a stream
     // successor of this grid) waits for RS of them; every k_update resets the counter

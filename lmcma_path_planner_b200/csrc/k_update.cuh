@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     // classic: k_sample may be scheduled right away; it waits for this grid to complete before reading anything.
     // progressive: it is released after this kernel's own wait (k_rank has reset the hand-over flags by then)
     if (!a.progressive) griddep_launch_dependents();
-    int* flags = o.progress + (size_t)b * (m + 2);                 // [0] scalars + mean, [1 + i] pair i, [m + 1] early scalars (itr, live)
+    int* flags = progress_flags(o.progress, m, b);
     const Scalars sc0 = *scp;
     float* const spec = OVERLAP && a.spec ? a.spec + (size_t)b * a.spec_stride : nullptr;
     int phase = OVERLAP ? a.phase : 0;
@@ -129,7 +129,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     if (OVERLAP && phase != 1) {
         // the previous generation's sampler has completed (graph order): reset its flags, then tell k_gate that this CTA
         // holds its SM (k_cost is released only then and fills the other SMs)
-        for (int i = tid; i < m + 2; i += nthr) flags[i] = 0;
+        for (int i = tid; i < progress_len(m); i += nthr) flags[i] = 0;
         __syncthreads();
         if (tid == 0) { __threadfence(); st_release_gpu(o.resident + b, 1); }
     }
@@ -180,7 +180,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     const int slot_new = order[live - 1];
     if (OVERLAP && tid == 0 && phase != 1) {                       // what the sampler needs to start on the finished pairs
         scp->itr = itr + 1; scp->live = live;
-        st_release_gpu(flags + m + 1, 1);
+        st_release_gpu(flag_early(flags, m), 1);
     }
     if (first_stale == 1) first_stale = 0;                           // lmcma.cpp:373-374
     UPD_STAMP(TL_UPD_BOOKKEEPING);
@@ -397,8 +397,8 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     if (a.progressive && !dry) {
         // scalars and mean are final; so are the pairs in front of the first stale position (untouched this generation;
         // overlap mode has published those before its sweep)
-        if (!OVERLAP) for (int i = tid; i < first_stale; i += nthr) st_release_gpu(flags + 1 + i, 1);
-        if (tid == 0 && !OVERLAP) st_release_gpu(flags, 1);      // overlap: with the step size, beside the chain
+        if (!OVERLAP) for (int i = tid; i < first_stale; i += nthr) st_release_gpu(flag_pair(flags, i), 1);
+        if (tid == 0 && !OVERLAP) st_release_gpu(flag_mean(flags), 1);   // overlap: with the step size, beside the chain
     }
     };
     if (!OVERLAP) {
@@ -406,7 +406,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         if (a.progressive) griddep_launch_dependents();
         post_rank(false);
     } else {
-        if (phase != 1) for (int i = tid; i < first_stale; i += nthr) st_release_gpu(flags + 1 + i, 1);   // untouched pairs: final already
+        if (phase != 1) for (int i = tid; i < first_stale; i += nthr) st_release_gpu(flag_pair(flags, i), 1);   // untouched pairs: final already
     }
 
     // ---- recompute v from the first stale position (lmcma.cpp:373-390) ----
@@ -433,6 +433,10 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
         const float t = sqrtf(fmaf(r_f, nv, 1.0f));
         nv_s[i] = nv;
         lj_s[i] = __fdividef(r_f, a_f * t * (t + 1.0f)) * invK;
+    };
+    auto pair_final = [&](int i, float nv) {                        // one thread: pair i of the mirror and Njs[i] are final
+        Njsb[i] = (float)nj_form(nj_ratio(o), o.M, nv).nj;
+        st_release_gpu(flag_pair(flags, i), 1);
     };
 
     if (RMAX < 0) {
@@ -542,13 +546,9 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                 const int q = lane + 32 * it;
                 if (q < nq && phase != 1) { dst[q] = x[it]; dst2[q] = x[it]; }
             }
-            if (a.progressive && phase != 1) {                       // pair i of the mirror and Njs[i] are final
+            if (a.progressive && phase != 1) {
                 __syncwarp();
-                if (lane == 0) {
-                    const double r = o.c1 / (1.0 - o.c1), t = sqrt(1.0 + r * (double)nv);
-                    Njsb[i] = (float)(o.M * r / (t + 1.0));          // the value the epilogue stores, too
-                    st_release_gpu(flags + 1 + i, 1);
-                }
+                if (lane == 0) pair_final(i, nv);
             }
         };
         // ---- the newest row: this generation's evolution path through the factors 0 .. live-2 (lmcma.cpp:375-382), a block of
@@ -661,11 +661,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                 if (a.dbg && i < TL_UPD_ROW_STAMPS) a.dbg[TL_UPD_ROWS + i] = gtime();
                 publish_scalars(i, nv);
                 mbar_arrive(&scalbar[i]);
-                if (a.progressive) {                                 // pair i of the mirror and Njs[i] are final
-                    const double r = o.c1 / (1.0 - o.c1), t = sqrt(1.0 + r * (double)nv);
-                    Njsb[i] = (float)(o.M * r / (t + 1.0));          // the value the epilogue stores, too
-                    st_release_gpu(flags + 1 + i, 1);
-                }
+                if (a.progressive) pair_final(i, nv);
             }
         };
         if (first_stale == 0 && warp == 0 && hi > 0 && phase != 2) { publish(y[0], 0, 1.0); retire_first(); }   // row 0 has no factors (v_0 = pc_0)
@@ -748,11 +744,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                 float4* dst2 = reinterpret_cast<float4*>(VPb + (size_t)i * 2 * ns);
                 for (int q = lane; q < nq; q += 32) { const float4 x = srow[q]; dst[q] = x; dst2[q] = x; dst2[nq + q] = __ldcg(prow + q); }
                 __syncwarp();
-                if (lane == 0) {
-                    const double r = o.c1 / (1.0 - o.c1), t = sqrt(1.0 + r * (double)nv_s[i]);
-                    Njsb[i] = (float)(o.M * r / (t + 1.0));
-                    st_release_gpu(flags + 1 + i, 1);
-                }
+                if (lane == 0) pair_final(i, nv_s[i]);
             }
         }
         // every older row is final
@@ -814,7 +806,7 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
                     if (warp == nwarps - 1) {
                         if (tid == nthr - 1 && !dry) {                // the thread that took the pair count in post_rank
                             step_size_and_counters();
-                            if (a.progressive) st_release_gpu(flags, 1);
+                            if (a.progressive) st_release_gpu(flag_mean(flags), 1);
                             if (a.dbg) a.dbg[TL_UPD_STEP_SIZE] = gtime();
                         }
                     } else if (!dry) {
@@ -901,9 +893,9 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == UPD_WARPS ? 1 : 2) k_upda
     if (a.dbg && threadIdx.x == 0) { a.dbg[TL_UPD_FIRST_STALE] = first_stale; a.dbg[TL_UPD_LIVE] = live; }
     for (int i = first_stale + tid; i < live && RMAX >= 0; i += nthr) {   // FP64 scalar state of the recomputed rows
         const int slot = order[i];
-        const double nv = (double)nv_s[i], r = o.c1 / (1.0 - o.c1), am = o.M;
-        const double t = sqrt(1.0 + r * nv);
-        const double nj = am * r / (t + 1.0), lj = r / (am * t * (t + 1.0));
+        const double r = nj_ratio(o), am = o.M;
+        const NjForm f = nj_form(r, am, (double)nv_s[i]);
+        const double nj = f.nj, lj = r / (am * f.t * (f.t + 1.0));
         Njd[slot] = nj; Ljd[slot] = lj; Njf[slot] = (float)nj; Njsb[i] = (float)nj;
     }
     UPD_STAMP(TL_UPD_END);

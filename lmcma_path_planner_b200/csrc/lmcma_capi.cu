@@ -567,7 +567,7 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     DM(d.Nj, B * m); DM(d.Lj, B * m); DM(d.Njf, B * m); DM(d.Njs, B * m);
     DM(d.VPs, B * m * 2 * ns);
     DM(d.t, B * m); DM(d.vec, B * m);
-    DM(d.sc, B); DM(d.best_x, B * ns); DM(d.S_count, B); DM(d.done_count, B); DM(d.progress, B * (m + 2)); DM(d.rank_ticket, B); DM(d.resident, B);
+    DM(d.sc, B); DM(d.best_x, B * ns); DM(d.S_count, B); DM(d.done_count, B); DM(d.progress, B * progress_len(m)); DM(d.rank_ticket, B); DM(d.resident, B);
     if (o->tune.dbg) DM(d.dbg, TL_SLOTS);
     DM(d.partial, B * d.RS * ns);
 

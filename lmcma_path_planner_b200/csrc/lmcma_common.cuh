@@ -72,10 +72,9 @@ struct OptDev {
     double* G;         // B x m x m
     double* Cf;        // B x m x m
     int2* gram_hdr;    // B : {first_stale, live} handed from k_update to k_gram / k_coef / k_combine
-    // progressive hand-over k_update -> k_sample inside one generation (see k_update.cuh): [0] = scalars and mean are
-    // final, [1 + i] = pair i of the sequence-ordered mirror (and Njs[i]) is final.  Reset by k_rank (by k_update itself
-    // in the overlapped generation).
-    int* progress;     // B x (m + 2): [0] scalars + mean, [1 + i] pair i, [m + 1] early scalars (itr, live) of the overlapped generation
+    // progressive hand-over k_update -> k_sample inside one generation (see k_update.cuh).  Reset by k_rank (by k_update
+    // itself in the overlapped generation).
+    int* progress;     // B x (m + 2): slots named by progress_len, progress_flags and flag_* below
     unsigned* rank_ticket;   // B : one ticket per k_rank CTA after its last store; k_update waits for RS of them in the overlapped generation
     int* resident;     // B : k_update (overlapped generation) holds its SM; k_gate releases k_cost
     int* t;            // B x m   slot order, oldest -> newest
@@ -97,6 +96,15 @@ struct OptDev {
                        // that gives up waiting for its concurrently running partner writes a code here and carries on
                        // (never __trap: that would poison the whole CUDA context); the host checks it at every sync
 };
+
+// The hand-over flags OptDev::progress of instance b: progress_len(m) = m + 2 ints, [0] scalars and mean are final
+// (flag_mean), [1 + i] pair i of the sequence-ordered mirror and Njs[i] are final (flag_pair), [m + 1] the early scalars
+// (itr, live) of the overlapped generation are final (flag_early).
+__host__ __device__ __forceinline__ int progress_len(int m) { return m + 2; }
+__device__ __forceinline__ int* progress_flags(int* progress, int m, int b) { return progress + (size_t)b * progress_len(m); }
+__device__ __forceinline__ int* flag_mean(int* flags) { return flags; }
+__device__ __forceinline__ int* flag_pair(int* flags, int i) { return flags + 1 + i; }
+__device__ __forceinline__ int* flag_early(int* flags, int m) { return flags + m + 1; }
 
 // The slots of the device timeline OptDev::dbg (LMCMA_B200_DBG): globaltimer stamps taken by one thread of instance 0,
 // printed and cleared by print_timeline (lmcma_capi.cu).  k_rank and k_sample_wide stamp [0, TL_UPD) through
@@ -290,6 +298,26 @@ __device__ __forceinline__ float4 philox_normal4(unsigned q, unsigned row, unsig
     __sincosf(6.283185307179586f * u1, &s0, &c0);
     __sincosf(6.283185307179586f * u3, &s1, &c1);
     return make_float4(ra * c0, ra * s0, rb * c1, rb * s1);
+}
+// The generator's deviates v of float4 column q of local row `row` of instance b in generation itr, padding lanes zeroed:
+// what the samplers draw (sample_deviate4, k_sample.cuh) and k_gauss materialises for the prior, so that a prior run and
+// a plain run see the same raw deviates.
+__device__ __forceinline__ void philox_deviate4(const OptDev& o, int b, int row, int q, int itr, float4& v) {
+    v = philox_normal4((unsigned)q, (unsigned)(o.pop_offset + row), (unsigned)itr, (unsigned)b, o.seed);
+    const int e = q * 4;
+    if (e + 1 >= o.n) v.y = 0.f;
+    if (e + 2 >= o.n) v.z = 0.f;
+    if (e + 3 >= o.n) v.w = 0.f;
+}
+
+// Nj from |v|^2 in FP64 (lmcma.cpp:386-387, cancellation-free form: see the sweep in k_update.cuh): with r = nj_ratio(o),
+// t = sqrt(1 + r |v|^2) and Nj = M r / (t + 1).  t comes back too: k_update's closed form of Lj is built on it.  Every
+// store of Nj (k_update's hand-over and epilogue, k_coef) goes through here, so that all of them round alike.
+__device__ __forceinline__ double nj_ratio(const OptDev& o) { return o.c1 / (1.0 - o.c1); }
+struct NjForm { double t, nj; };
+__device__ __forceinline__ NjForm nj_form(double r, double M, double nv) {
+    const double t = sqrt(1.0 + r * nv);
+    return {t, M * r / (t + 1.0)};
 }
 
 }  // namespace lmcma
