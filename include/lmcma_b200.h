@@ -19,8 +19,8 @@
  * optimiser handles and host threads: lmcma_b200_cost_evaluate_dev may be called concurrently from several threads and
  * on several streams for different queries (the end points travel by value with each launch; no per-map device state is
  * written); lmcma_b200_cost_evaluate and lmcma_b200_cost_trace (host buffers) serialise on a per-map lock because they
- * share the map's staging buffers and private stream.  lmcma_b200_map_set_l2_persist and lmcma_b200_map_destroy must not
- * race with evaluations on the same map.
+ * share the map's staging buffers and private stream.  lmcma_b200_map_set_l2_persist, lmcma_b200_map_update_occupancy and
+ * lmcma_b200_map_destroy must not race with evaluations on the same map.
  *
  * Environment knobs (LMCMA_B200_*, experiments / debugging only) are read once when a handle is created, never on a
  * launch path.  The overlapped single-query generation (a forked CUDA graph whose branches must run concurrently) is
@@ -89,6 +89,17 @@ int lmcma_b200_edt(int device, int dims, const int32_t* shape_xyz, const uint8_t
 /* map_create fed by an occupancy grid: distance transform + conversion to the map storage, all on the device */
 int lmcma_b200_map_create_from_occupancy(int device, int dims, const int32_t* shape_xyz, const uint8_t* occ_host, float clamp,
                                          int storage, float u8_scale, float c_min, lmcma_b200_map** map_out);
+/* Replace the occupancy of the box [lo, lo + size) (cells, x y [z]; occ_box row-major [sz][sy][sx], non-zero = obstacle)
+ * of a map built by lmcma_b200_map_create_from_occupancy, and bring its storage up to date on the device.  Afterwards the
+ * map holds, bit for bit, what map_create_from_occupancy of the edited grid with the same clamp / storage / u8_scale /
+ * c_min would hold.  Synchronous.  Must not race with evaluations of this map (like map_destroy).  Optimiser handles
+ * attached to the map, including their captured graphs, read the new contents on their next launch: no re-attach.
+ * With clamp > 0 only the cells closer than the clamp to the box are recomputed, from a window of the grid around them;
+ * with clamp <= 0 the whole grid is (one obstacle removed can change any distance), from the occupancy the map storage
+ * encodes, so only the box crosses PCIe either way.
+ * LMCMA_B200_ERR_STATE: a map made by lmcma_b200_map_create (a caller's distance field has no occupancy behind it).
+ * LMCMA_B200_ERR_ARG: a null pointer, a size below 1, or a box not inside the grid.  A refused call changes nothing. */
+int lmcma_b200_map_update_occupancy(lmcma_b200_map* map, const int32_t* lo_xyz, const int32_t* size_xyz, const uint8_t* occ_box_host);
 int lmcma_b200_map_destroy(lmcma_b200_map* map);
 /* the distance field the evaluator effectively uses, back on the host: U8 storage gives E_q = q * u8_scale; F32 storage
  * gives 1 / (1 / max(E, c_min)) in FP32, i.e. the clearance with the c_min floor (up to the rounding of the two
@@ -219,6 +230,13 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* opt, int32_t generations, float* 
 
 /* best evaluated candidate so far per instance (the reference keeps only BestF, lmcma.cpp:192-194) */
 int lmcma_b200_best(lmcma_b200_opt* opt, float* x_best_host /* batch x n */, float* f_best_host /* batch */);
+/* Re-evaluate each instance's best-so-far candidate (lmcma_b200_best) on the attached map as it is now, and make its
+ * cost the new best_f.  Needed after a map update: otherwise a stale best_f from the old map keeps a path that now
+ * collides as "best" for good.  Instances with no evaluation yet are left as they are.  best_x and counteval do not
+ * change; PREV_FIT keeps the previous generation's fitness on the old map, which the next update compares once in its
+ * step-size rule (the reference has no notion of a changing cost).  Synchronous.
+ * LMCMA_B200_ERR_STATE without an attached cost, and on a split-population handle (best_x may hold a peer's row there). */
+int lmcma_b200_rescore_best(lmcma_b200_opt* opt);
 
 /* ---- state access (parity / teacher forcing / checkpointing) ---- */
 enum {

@@ -200,6 +200,12 @@ public:
         check(lmcma_b200_cost_evaluate(h_, &obj, &e, X, count, f, ncoll, nsamp));
     }
 
+    // replanning on a changing map built from occupancy: replace the occupancy of the box [lo, lo + size) (occ row-major
+    // [sz][sy][sx], non-zero = obstacle); optimiser handles attached to the map see the update on their next run
+    void updateOccupancy(const int32_t* lo_xyz, const int32_t* size_xyz, const uint8_t* occ) {
+        check(lmcma_b200_map_update_occupancy(h_, lo_xyz, size_xyz, occ));
+    }
+
 private:
     int dims_;
     lmcma_b200_map* h_;

@@ -61,6 +61,7 @@ SIGNATURES = {
     "lmcma_b200_load_binvox": (C.c_int, [C.c_char_p, C.POINTER(C.c_uint8), _i64, _pi, _pd, _pd]),
     "lmcma_b200_load_bt": (C.c_int, [C.c_char_p, C.POINTER(C.c_uint8), _i64, _pi, _pi, _pd]),
     "lmcma_b200_load_text_matrix": (C.c_int, [C.c_char_p, _pd, _i64, _pi, _pi]),
+    "lmcma_b200_map_update_occupancy": (C.c_int, [_vp, _pi, _pi, C.POINTER(C.c_uint8)]),
     "lmcma_b200_map_destroy": (C.c_int, [_vp]),
     "lmcma_b200_map_dequantized": (C.c_int, [_vp, _pf]),
     "lmcma_b200_map_set_l2_persist": (C.c_int, [_vp, C.c_int]),
@@ -87,6 +88,7 @@ SIGNATURES = {
     "lmcma_b200_last_run_ms": (C.c_int, [_vp, _pf]),
     "lmcma_b200_profile_kernels": (C.c_int, [_vp, _i32, _pf]),
     "lmcma_b200_best": (C.c_int, [_vp, _pf, _pf]),
+    "lmcma_b200_rescore_best": (C.c_int, [_vp]),
     "lmcma_b200_get_f64": (C.c_int, [_vp, _i32, _pd, _i64]),
     "lmcma_b200_get_f32": (C.c_int, [_vp, _i32, _pf, _i64]),
     "lmcma_b200_get_i32": (C.c_int, [_vp, _i32, _pi, _i64]),

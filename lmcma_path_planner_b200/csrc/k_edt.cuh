@@ -6,11 +6,23 @@
 //            one thread per line, lines laid out so that the threads of a warp touch consecutive addresses
 // then dist = sqrt(d2) (FP64 sqrt, rounded once to FP32 — what scipy's exact EDT gives), optional clamp, and the
 // conversion to the bricked map storage k_cost reads (k_brick) without a host round trip.
+// An in-place occupancy update (lmcma_b200_map_update_occupancy) runs the same passes on a window of the grid: k_occ_gather
+// decodes the window's occupancy from the map storage, and k_edt_finish / k_brick write only the cells whose value can
+// change (DESIGN.md, "In-place occupancy updates").  A map build passes the whole grid as both windows.
 #pragma once
 #include <cfloat>
 #include "lmcma_common.cuh"
 
 namespace lmcma {
+
+struct Box3 { int x0, y0, z0, nx, ny, nz; };   // the cells [x0, x0 + nx) x [y0, y0 + ny) x [z0, z0 + nz) of a grid
+__host__ __device__ __forceinline__ long long box_cells(const Box3& b) { return (long long)b.nx * b.ny * b.nz; }
+// grid coordinates of cell i of box b, row-major [z][y][x] inside the box
+__device__ __forceinline__ void box_cell(const Box3& b, long long i, int& x, int& y, int& z) {
+    x = b.x0 + (int)(i % b.nx);
+    y = b.y0 + (int)((i / b.nx) % b.ny);
+    z = b.z0 + (int)(i / ((long long)b.nx * b.ny));
+}
 
 // Squared distances are unsigned 32-bit: the largest one an accepted grid holds (axes <= 32767 cells) is 3 * 32766^2 =
 // 3 220 832 268, past INT_MAX but below EDT_NONE, the "no obstacle" sentinel.  Envelope arithmetic is 64-bit.
@@ -95,27 +107,30 @@ __global__ void __launch_bounds__(128) k_edt_axis(unsigned* __restrict__ d2, int
     }
 }
 
-// ---- d2 -> distance in cells (FP32), optional clamp; no obstacle anywhere -> clamp (or EDT_EMPTY = FLT_MAX when unclamped)
-__global__ void __launch_bounds__(256) k_edt_finish(const unsigned* __restrict__ d2, float* __restrict__ dist, long long cells, float clamp) {
+// ---- d2 -> distance in cells (FP32), optional clamp; no obstacle anywhere -> clamp (or EDT_EMPTY = FLT_MAX when unclamped).
+//      d2 is row-major over the window `win`; dist receives the cells of `out` (inside win), row-major over out.
+__global__ void __launch_bounds__(256) k_edt_finish(const unsigned* __restrict__ d2, Box3 win, float* __restrict__ dist, Box3 out, float clamp) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= cells) return;
-    const unsigned v = d2[i];
+    if (i >= box_cells(out)) return;
+    int x, y, z;
+    box_cell(out, i, x, y, z);
+    const unsigned v = d2[((long long)(z - win.z0) * win.ny + (y - win.y0)) * win.nx + (x - win.x0)];
     float d = v == EDT_NONE ? EDT_EMPTY : (float)sqrt((double)v);
     if (clamp > 0.f) d = fminf(d, clamp);
     dist[i] = d;
 }
 
-// ---- row-major distance field -> the bricked storage of the cost map (lmcma_layout.hpp):
-//      F32: sign-tagged reciprocal clearance (negative on obstacles); U8: quantised distance
+// ---- distance field of the cells of `out` (row-major over out) -> those cells of the bricked storage of the cost map
+//      (lmcma_layout.hpp): F32: sign-tagged reciprocal clearance (negative on obstacles); U8: quantised distance
 template <int DIMS, int STORAGE>
-__global__ void __launch_bounds__(256) k_brick(const float* __restrict__ dist, float* __restrict__ g32, unsigned char* __restrict__ q8,
-                                               int nx, int ny, int nz, unsigned nbx, unsigned nby, float c_min, float u8_scale) {
+__global__ void __launch_bounds__(256) k_brick(const float* __restrict__ dist, Box3 out, float* __restrict__ g32, unsigned char* __restrict__ q8,
+                                               unsigned nbx, unsigned nby, float c_min, float u8_scale) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long cells = (long long)nx * ny * nz;
-    if (i >= cells) return;
-    const unsigned x = (unsigned)(i % nx), y = (unsigned)((i / nx) % ny), z = (unsigned)(i / ((long long)nx * ny));
+    if (i >= box_cells(out)) return;
+    int x, y, z;
+    box_cell(out, i, x, y, z);
     const float e = dist[i];
-    const unsigned o = brick_offset<DIMS, STORAGE>(x, y, z, nbx, nby);
+    const unsigned o = brick_offset<DIMS, STORAGE>((unsigned)x, (unsigned)y, (unsigned)z, nbx, nby);
     if (STORAGE == 0) {
         g32[o] = (e > 0.f) ? 1.0f / fmaxf(e, c_min) : -1.0f / c_min;
     } else {
@@ -123,6 +138,27 @@ __global__ void __launch_bounds__(256) k_brick(const float* __restrict__ dist, f
         if (e > 0.f) { v = (int)floorf(e / u8_scale); v = min(255, max(1, v)); }
         q8[o] = (unsigned char)v;
     }
+}
+
+// ---- occupancy of the window `win` of a map built from occupancy, row-major over win (1 = obstacle), with the cells of
+//      `box` taken from box_occ (row-major over box, non-zero = obstacle) instead.  Outside the box the storage encodes the
+//      occupancy: the distance is 0 exactly on obstacles, so k_brick stored a negative value (F32) or q = 0 (U8) there.
+template <int DIMS, int STORAGE>
+__global__ void __launch_bounds__(256) k_occ_gather(const float* __restrict__ g32, const unsigned char* __restrict__ q8, unsigned nbx,
+                                                    unsigned nby, Box3 win, const unsigned char* __restrict__ box_occ, Box3 box,
+                                                    unsigned char* __restrict__ occ) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= box_cells(win)) return;
+    int x, y, z;
+    box_cell(win, i, x, y, z);
+    bool obstacle;
+    if (x >= box.x0 && x < box.x0 + box.nx && y >= box.y0 && y < box.y0 + box.ny && z >= box.z0 && z < box.z0 + box.nz) {
+        obstacle = box_occ[((long long)(z - box.z0) * box.ny + (y - box.y0)) * box.nx + (x - box.x0)] != 0;
+    } else {
+        const unsigned o = brick_offset<DIMS, STORAGE>((unsigned)x, (unsigned)y, (unsigned)z, nbx, nby);
+        obstacle = STORAGE == 0 ? g32[o] < 0.f : q8[o] == 0;
+    }
+    occ[i] = obstacle ? 1 : 0;
 }
 
 }  // namespace lmcma

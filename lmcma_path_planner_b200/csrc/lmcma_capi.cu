@@ -177,6 +177,13 @@ int cost_args_for(lmcma_b200_opt* o, CostArgs* a) {
     return 0;
 }
 
+// lmcma_b200_rescore_best: best_f <- the cost of best_x on the map as it is now, for every instance that has been evaluated
+// (canonicalised as k_update canonicalises a fitness before it compares it with best_f)
+__global__ void k_set_best_f(Scalars* sc, const float* f, int B) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < B && sc[b].counteval > 0) sc[b].best_f = (double)canon_fitness(f[b]);
+}
+
 // generate / stage deviates on the host for HANSEN mode, then sample
 int host_rng_and_sample(lmcma_b200_opt* o, cudaStream_t st, bool progressive = false) {
     if (o->cfg.rng == LMCMA_B200_RNG_HANSEN) {
@@ -640,7 +647,7 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     if (o->stream) cudaStreamSynchronize(o->stream);
     OptDev& d = o->d;
     void* ptrs[] = {d.prev_sorted, d.tile_sorted, d.tile_pos, d.X, d.D, d.Z, d.Zc, o->d_Lf, d.fit, d.fit_sorted, d.prev_fit, d.rank, d.arindex, d.ncoll, d.nsamp, d.xmean, d.pc, d.V, d.P,
-                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends};
+                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore};
     for (void* p : ptrs) cudaFree(p);
     drop_fused_graphs(o);
     drop_tell_graphs(o);
@@ -971,6 +978,26 @@ int lmcma_b200_best(lmcma_b200_opt* o, float* x_best, float* f_best) {
         CU(cudaStreamSynchronize(o->stream));
         for (int b = 0; b < d.B; ++b) f_best[b] = (float)sc[b].best_f;
     }
+    return 0;
+}
+
+int lmcma_b200_rescore_best(lmcma_b200_opt* o) {
+    ARG(o, "null handle");
+    if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached (call lmcma_b200_attach_cost)");
+    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles: best_x may hold a peer's row");
+    CU(cudaSetDevice(o->cfg.device));
+    const OptDev& d = o->d;
+    if (!o->d_rescore) DM(o->d_rescore, (size_t)d.B);
+    CostArgs ca;
+    int rc = cost_args_for(o, &ca);
+    if (rc) return rc;
+    ca.X = d.best_x; ca.inst_rows = 1;                           // one row per instance, the instance's own end points
+    ca.f = o->d_rescore; ca.f_stride = 1; ca.f_offset = 0; ca.ncoll = nullptr; ca.nsamp = nullptr;
+    if ((rc = apply_l2_window(o->map, o->stream))) return rc;
+    if ((rc = launch_cost(o->map->dev, ca, 1, d.B, o->cost_shape, false, o->stream))) return rc;
+    if ((rc = launch(k_set_best_f, (unsigned)((d.B + 127) / 128), 128, 0, o->stream, false, d.sc, (const float*)o->d_rescore, d.B))) return rc;
+    o->spec_valid = false;                                       // like the state setters: tell_all's speculative pass saw the old best
+    CU(cudaStreamSynchronize(o->stream));
     return 0;
 }
 

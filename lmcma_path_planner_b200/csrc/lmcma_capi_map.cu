@@ -167,35 +167,51 @@ static int map_alloc(int device, int dims, const int32_t* shape, int storage, fl
     return 0;
 }
 
-// row-major distance field on the device -> the bricked storage (values + layout, lmcma_layout.hpp)
-static int map_fill_from_dist_dev(lmcma_b200_map* m, const float* d_dist, cudaStream_t st) {
+static Box3 grid_box(int dims, const int32_t* shape) { return Box3{0, 0, 0, shape[0], shape[1], dims == 3 ? shape[2] : 1}; }
+
+// distance field of the cells of `out` on the device (row-major over out) -> those cells of the bricked storage (values +
+// layout, lmcma_layout.hpp)
+static int map_fill_from_dist_dev(lmcma_b200_map* m, const float* d_dist, const Box3& out, cudaStream_t st) {
     const MapDev& d = m->dev;
-    const unsigned blocks = (unsigned)((m->cells + 255) / 256);
+    const unsigned blocks = (unsigned)((box_cells(out) + 255) / 256);
     auto kern = d.dims == 2 ? (m->storage == 0 ? k_brick<2, 0> : k_brick<2, 1>) : (m->storage == 0 ? k_brick<3, 0> : k_brick<3, 1>);
-    return launch(kern, blocks, 256, 0, st, false, d_dist, m->d_g32, m->d_q8, d.nx, d.ny, d.nz, d.nbx, d.nby, m->c_min, m->scale);
+    return launch(kern, blocks, 256, 0, st, false, d_dist, out, m->d_g32, m->d_q8, d.nbx, d.nby, m->c_min, m->scale);
 }
 
-// exact Euclidean distance transform on the device (k_edt.cuh): d_occ (1 = obstacle) -> d_dist, both row-major [z][y][x]
-static int edt_device(int dims, const int32_t* shape, const unsigned char* d_occ, float clamp, float* d_dist, cudaStream_t st) {
-    const int nx = shape[0], ny = shape[1], nz = dims == 3 ? shape[2] : 1;
-    ARG(nx <= 32767 && ny <= 32767 && nz <= 32767, "axis longer than 32767 cells");
-    const size_t cells = (size_t)nx * ny * nz;
-    unsigned *d2 = nullptr, *gh = nullptr;   // squared distances (k_edt.cuh)
-    int *s = nullptr, *t = nullptr;
-    int rc = dmalloc(&d2, cells);
-    if (!rc) rc = dmalloc(&s, cells);
-    if (!rc) rc = dmalloc(&t, cells);
-    if (!rc) rc = dmalloc(&gh, cells);
+// scratch of the distance transform (k_edt.cuh): the squared distances and the three arrays of the lower envelope, one entry
+// per cell of the transformed window each
+struct EdtScratch { unsigned* d2; int* s; int* t; unsigned* gh; };
+
+// exact Euclidean distance transform on the device (k_edt.cuh) of the window `win` of a grid, every cell outside it taken as
+// free: d_occ (1 = obstacle, row-major over win) -> d_dist, the distances of the cells of `out` (inside win, row-major over
+// out).  Enqueued on `st`; returns without waiting.
+static int edt_device(const unsigned char* d_occ, const Box3& win, const Box3& out, float clamp, float* d_dist, const EdtScratch& w,
+                      cudaStream_t st) {
+    const int nx = win.nx, ny = win.ny, nz = win.nz;
+    const long long nlines = (long long)ny * nz, ylines = (long long)nx * nz, zlines = (long long)nx * ny;
+    int rc = launch(k_edt_x, (unsigned)((nlines + 7) / 8), 256, 0, st, false, d_occ, w.d2, nx, nlines);
+    if (!rc && ny > 1) rc = launch(k_edt_axis, (unsigned)((ylines + 127) / 128), 128, 0, st, false, w.d2, ny, nx, nx, nz, (long long)nx * ny, w.s, w.t, w.gh);
+    if (!rc && nz > 1) rc = launch(k_edt_axis, (unsigned)((zlines + 127) / 128), 128, 0, st, false, w.d2, nz, (long long)nx * ny, nx * ny, 1, 0, w.s, w.t, w.gh);
+    if (!rc) rc = launch(k_edt_finish, (unsigned)((box_cells(out) + 255) / 256), 256, 0, st, false, w.d2, win, d_dist, out, clamp);
+    return rc;
+}
+
+// the distance transform of a whole grid (the map builds, lmcma_b200_edt), with scratch of its own; finished on return
+static int edt_grid(int dims, const int32_t* shape, const unsigned char* d_occ, float clamp, float* d_dist, cudaStream_t st) {
+    const Box3 grid = grid_box(dims, shape);
+    ARG(grid.nx <= 32767 && grid.ny <= 32767 && grid.nz <= 32767, "axis longer than 32767 cells");
+    const size_t cells = (size_t)box_cells(grid);
+    EdtScratch w{};
+    int rc = dmalloc(&w.d2, cells);
+    if (!rc) rc = dmalloc(&w.s, cells);
+    if (!rc) rc = dmalloc(&w.t, cells);
+    if (!rc) rc = dmalloc(&w.gh, cells);
     if (!rc) {
-        const long long nlines = (long long)ny * nz, ylines = (long long)nx * nz, zlines = (long long)nx * ny;
-        rc = launch(k_edt_x, (unsigned)((nlines + 7) / 8), 256, 0, st, false, d_occ, d2, nx, nlines);
-        if (!rc && ny > 1) rc = launch(k_edt_axis, (unsigned)((ylines + 127) / 128), 128, 0, st, false, d2, ny, nx, nx, nz, (long long)nx * ny, s, t, gh);
-        if (!rc && nz > 1) rc = launch(k_edt_axis, (unsigned)((zlines + 127) / 128), 128, 0, st, false, d2, nz, (long long)nx * ny, nx * ny, 1, 0, s, t, gh);
-        if (!rc) rc = launch(k_edt_finish, (unsigned)((cells + 255) / 256), 256, 0, st, false, d2, d_dist, (long long)cells, clamp);
+        rc = edt_device(d_occ, grid, grid, clamp, d_dist, w, st);
         cudaError_t e = cudaStreamSynchronize(st);
         if (!rc && e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "distance transform: %s", cudaGetErrorString(e));
     }
-    cudaFree(d2); cudaFree(s); cudaFree(t); cudaFree(gh);
+    cudaFree(w.d2); cudaFree(w.s); cudaFree(w.t); cudaFree(w.gh);
     return rc;
 }
 
@@ -211,7 +227,7 @@ int lmcma_b200_map_create(int device, int dims, const int32_t* shape, const floa
         cudaError_t e = cudaMemcpyAsync(d_dist, dist, m->cells * sizeof(float), cudaMemcpyHostToDevice, m->stream);
         if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e));
     }
-    if (!rc) rc = map_fill_from_dist_dev(m, d_dist, m->stream);
+    if (!rc) rc = map_fill_from_dist_dev(m, d_dist, grid_box(dims, shape), m->stream);
     if (!rc) { cudaError_t e = cudaStreamSynchronize(m->stream); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "map upload: %s", cudaGetErrorString(e)); }
     cudaFree(d_dist);
     if (rc) { lmcma_b200_map_destroy(m); return rc; }
@@ -232,7 +248,7 @@ int lmcma_b200_edt(int device, int dims, const int32_t* shape, const uint8_t* oc
     rc = dmalloc(&d_occ, cells);
     if (!rc) rc = dmalloc(&d_dist, cells);
     if (!rc) { cudaError_t e = cudaMemcpy(d_occ, occ_host, cells, cudaMemcpyHostToDevice); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e)); }
-    if (!rc) rc = edt_device(dims, shape, d_occ, clamp, d_dist, 0);
+    if (!rc) rc = edt_grid(dims, shape, d_occ, clamp, d_dist, 0);
     if (!rc) { cudaError_t e = cudaMemcpy(dist_host_out, d_dist, cells * sizeof(float), cudaMemcpyDeviceToHost); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e)); }
     cudaFree(d_occ); cudaFree(d_dist);
     return rc;
@@ -248,13 +264,82 @@ int lmcma_b200_map_create_from_occupancy(int device, int dims, const int32_t* sh
     rc = dmalloc(&d_occ, m->cells);
     if (!rc) rc = dmalloc(&d_dist, m->cells);
     if (!rc) { cudaError_t e = cudaMemcpy(d_occ, occ_host, m->cells, cudaMemcpyHostToDevice); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "cudaMemcpy: %s", cudaGetErrorString(e)); }
-    if (!rc) rc = edt_device(dims, shape, d_occ, clamp, d_dist, m->stream);
-    if (!rc) rc = map_fill_from_dist_dev(m, d_dist, m->stream);
+    if (!rc) rc = edt_grid(dims, shape, d_occ, clamp, d_dist, m->stream);
+    if (!rc) rc = map_fill_from_dist_dev(m, d_dist, grid_box(dims, shape), m->stream);
     if (!rc) { cudaError_t e = cudaStreamSynchronize(m->stream); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "map build: %s", cudaGetErrorString(e)); }
     cudaFree(d_occ); cudaFree(d_dist);
     if (rc) { lmcma_b200_map_destroy(m); return rc; }
+    m->from_occupancy = true;
+    m->clamp = clamp;
     *out = m;
     return 0;
+}
+
+// b grown by r cells on every side along the first `dims` axes (Chebyshev dilation), clipped to the grid [0, n)
+static Box3 dilate(const Box3& b, int r, int dims, const int* n) {
+    int lo[3] = {b.x0, b.y0, b.z0}, ext[3] = {b.nx, b.ny, b.nz};
+    for (int c = 0; c < dims; ++c) {
+        const long long a = std::max(0LL, (long long)lo[c] - r), e = std::min((long long)n[c], (long long)lo[c] + ext[c] + r);
+        lo[c] = (int)a; ext[c] = (int)(e - a);
+    }
+    return Box3{lo[0], lo[1], lo[2], ext[0], ext[1], ext[2]};
+}
+
+int lmcma_b200_map_update_occupancy(lmcma_b200_map* m, const int32_t* lo_xyz, const int32_t* size_xyz, const uint8_t* occ_box_host) {
+    ARG(m && lo_xyz && size_xyz && occ_box_host, "null pointer");
+    if (!m->from_occupancy)
+        return fail(LMCMA_B200_ERR_STATE, "the map holds a caller's distance field, no occupancy: only maps built by "
+                                          "lmcma_b200_map_create_from_occupancy can be updated");
+    const int dims = m->dev.dims;
+    const int n[3] = {m->dev.nx, m->dev.ny, m->dev.nz};
+    int b0[3] = {0, 0, 0}, bn[3] = {1, 1, 1};
+    for (int c = 0; c < dims; ++c) {
+        ARG(size_xyz[c] >= 1, "box size below 1");
+        ARG(lo_xyz[c] >= 0 && (long long)lo_xyz[c] + size_xyz[c] <= n[c], "box not inside the grid");
+        b0[c] = lo_xyz[c]; bn[c] = size_xyz[c];
+    }
+    const Box3 box{b0[0], b0[1], b0[2], bn[0], bn[1], bn[2]};
+    // A: the cells whose value can change, I: the window transformed for them (DESIGN.md, "In-place occupancy updates").
+    // Clamped: a cell farther than the clamp from the box keeps its value, and every obstacle closer than the clamp to a
+    // cell of A lies in I.  Unclamped: removing an obstacle can change any cell.
+    Box3 A{0, 0, 0, n[0], n[1], n[2]}, I = A;
+    if (m->clamp > 0.f) {
+        const int r = (int)std::min(std::ceil((double)m->clamp), 65536.0);   // past every axis: the whole grid
+        A = dilate(box, r, dims, n);
+        I = dilate(A, r, dims, n);
+    }
+    std::lock_guard<std::mutex> lock(m->host_path);   // the private stream and the scratch
+    CU(cudaSetDevice(m->device));
+    // grow-only scratch: d2, s, t, gh over I, the distances of A, the occupancy of I, the uploaded box
+    auto aligned = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+    const size_t ni = (size_t)box_cells(I), na = (size_t)box_cells(A), nb = (size_t)box_cells(box);
+    const size_t need = 4 * aligned(ni * 4) + aligned(na * 4) + aligned(ni) + aligned(nb);
+    if (m->d_update_cap < need) {
+        if (m->d_update) CU(cudaFreeAsync(m->d_update, m->stream));
+        m->d_update = nullptr; m->d_update_cap = 0;
+        cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&m->d_update), need, m->stream);
+        if (e != cudaSuccess) { m->d_update = nullptr; return fail(LMCMA_B200_ERR_NOMEM, "cudaMallocAsync(%zu bytes): %s", need, cudaGetErrorString(e)); }
+        m->d_update_cap = need;
+    }
+    char* p = m->d_update;
+    EdtScratch w;
+    w.d2 = reinterpret_cast<unsigned*>(p); p += aligned(ni * 4);
+    w.s = reinterpret_cast<int*>(p); p += aligned(ni * 4);
+    w.t = reinterpret_cast<int*>(p); p += aligned(ni * 4);
+    w.gh = reinterpret_cast<unsigned*>(p); p += aligned(ni * 4);
+    float* d_dist = reinterpret_cast<float*>(p); p += aligned(na * 4);
+    unsigned char* d_occ = reinterpret_cast<unsigned char*>(p); p += aligned(ni);
+    unsigned char* d_box = reinterpret_cast<unsigned char*>(p);
+    const cudaStream_t st = m->stream;
+    CU(cudaMemcpyAsync(d_box, occ_box_host, nb, cudaMemcpyHostToDevice, st));
+    const MapDev& d = m->dev;
+    auto gather = dims == 2 ? (m->storage == 0 ? k_occ_gather<2, 0> : k_occ_gather<2, 1>) : (m->storage == 0 ? k_occ_gather<3, 0> : k_occ_gather<3, 1>);
+    int rc = launch(gather, (unsigned)((ni + 255) / 256), 256, 0, st, false, m->d_g32, m->d_q8, d.nbx, d.nby, I, d_box, box, d_occ);
+    if (!rc) rc = edt_device(d_occ, I, A, m->clamp, d_dist, w, st);
+    if (!rc) rc = map_fill_from_dist_dev(m, d_dist, A, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (!rc && e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "occupancy update: %s", cudaGetErrorString(e));
+    return rc;
 }
 
 int lmcma_b200_map_destroy(lmcma_b200_map* m) {
@@ -262,6 +347,7 @@ int lmcma_b200_map_destroy(lmcma_b200_map* m) {
     cudaSetDevice(m->device);
     cudaFree(m->d_g32); cudaFree(m->d_q8); cudaFree(m->d_lut); cudaFree(m->d_X); cudaFree(m->d_f);
     cudaFree(m->d_nc); cudaFree(m->d_ns);
+    if (m->d_update) { cudaFreeAsync(m->d_update, m->stream); cudaStreamSynchronize(m->stream); }
     if (m->stream) cudaStreamDestroy(m->stream);
     delete m;
     return 0;

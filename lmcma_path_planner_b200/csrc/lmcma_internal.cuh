@@ -140,7 +140,14 @@ struct lmcma_b200_map {
     // staging for the host-buffer evaluate path
     float* d_X = nullptr; size_t d_X_cap = 0;
     float* d_f = nullptr; int* d_nc = nullptr; int* d_ns = nullptr; size_t d_out_cap = 0;
-    std::mutex host_path;            // lmcma_b200_cost_evaluate / cost_trace share the staging buffers and the private stream
+    // built by lmcma_b200_map_create_from_occupancy (with this clamp): the storage encodes the occupancy, and
+    // lmcma_b200_map_update_occupancy may edit it
+    bool from_occupancy = false;
+    float clamp = 0.f;
+    // grow-only scratch of lmcma_b200_map_update_occupancy (stream-ordered on `stream`: growing it never synchronises the device)
+    char* d_update = nullptr; size_t d_update_cap = 0;
+    std::mutex host_path;            // lmcma_b200_cost_evaluate / cost_trace / map_update_occupancy share the staging buffers
+                                     // and the private stream
 };
 
 struct lmcma_b200_opt {
@@ -165,6 +172,7 @@ struct lmcma_b200_opt {
     lmcma_b200_map* map = nullptr;
     lmcma_b200_objective obj{};
     float* d_ends = nullptr;
+    float* d_rescore = nullptr;        // B costs of best_x on the attached map (lmcma_b200_rescore_best)
     // graph
     lmcma_capi::Graph graph;                  // one fused generation (lmcma_b200_run)
     lmcma_capi::Graph graph_multi;            // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)

@@ -69,6 +69,17 @@ class CostMap:
         self.bytes_per_cell = 4 if self.storage == K.MAP_F32 else 1
         return self
 
+    def update_occupancy(self, lo_xyz, occ_box):
+        """Replace the occupancy of a box of a map built by from_occupancy (non-zero = obstacle): occ_box is [sz, sy, sx]
+        or [sy, sx] like the grid, lo_xyz its first cell (x, y[, z]).  Afterwards the map holds what from_occupancy of the
+        edited grid would hold; optimisers attached to it see the new map on their next run.  Synchronise them first."""
+        o = np.ascontiguousarray(np.asarray(occ_box) != 0, np.uint8)
+        if o.ndim != self.dims:
+            raise ValueError("occ_box has %d dimensions, the map %d" % (o.ndim, self.dims))
+        lo = np.array(lo_xyz, np.int32).reshape(self.dims)
+        size = np.array(o.shape[::-1], np.int32)
+        K.check(K.lib().lmcma_b200_map_update_occupancy(self._h, K.iptr(lo), K.iptr(size), o.ctypes.data_as(C.POINTER(C.c_uint8))))
+
     def close(self):
         if getattr(self, "_h", None):
             K.lib().lmcma_b200_map_destroy(self._h)
@@ -236,6 +247,11 @@ class Optimizer:
         f = np.zeros(self.batch, np.float32)
         K.check(K.lib().lmcma_b200_best(self._h, K.fptr(x), K.fptr(f)))
         return x, f
+
+    def rescore_best(self):
+        """best_f <- the cost of best_x on the attached map as it is now (after CostMap.update_occupancy), for every
+        instance evaluated at least once."""
+        K.check(K.lib().lmcma_b200_rescore_best(self._h))
 
     # ---- state ----
     def _shape_of(self, name):
