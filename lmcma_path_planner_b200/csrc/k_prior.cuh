@@ -8,9 +8,12 @@
 
 namespace lmcma {
 
-// Z <- N(0,1), the samplers' deviates (philox_deviate4): grid = (ceil(nq / 128), pop_count, B)
+// Z <- N(0,1), the samplers' deviates (philox_deviate4): grid = (ceil(nq / 128) x pop_count, 1, B), the column tile
+// fastest.  The rows share grid x with the column tiles, in the order a (tiles, rows) grid would launch them: pop_count
+// reaches 65 536, past the 65 535 that y and z take
 __global__ void __launch_bounds__(128) k_gauss(OptDev o) {
-    const int q = blockIdx.x * 128 + threadIdx.x, row = blockIdx.y, b = blockIdx.z, nq = o.ns >> 2;
+    const int nq = o.ns >> 2, tiles = (nq + 127) >> 7;
+    const int row = blockIdx.x / tiles, q = (blockIdx.x - row * tiles) * 128 + threadIdx.x, b = blockIdx.z;
     if (q >= nq) return;
     const int itr = o.sc[b].itr;
     float4 v;
@@ -19,12 +22,14 @@ __global__ void __launch_bounds__(128) k_gauss(OptDev o) {
 }
 
 // Zc[r][i] = sum_{k <= i} L[i][k] Z[r][k];  L: n x ns row-major FP32 (zero above the diagonal and in the padding)
-// grid = (ceil(ns / 64), ceil(rows / 64)), 256 threads
+// grid = ceil(ns / 64) x ceil(rows / 64) blocks on x, the column tile fastest (the order of a (columns, rows) grid, which
+// keeps the long last column tiles apart), 256 threads: rows = B x pop_count can pass the 65 535 x 64 that y would take
 __global__ void __launch_bounds__(256) k_prior(const float* __restrict__ Z, const float* __restrict__ Lf, float* __restrict__ Zc,
                                                int rows, int n, int ns) {
     __shared__ float zs[16][64 + 4];      // [k][r]
     __shared__ float ls[16][64 + 4];      // [k][i]
-    const int i0 = blockIdx.x * 64, r0 = blockIdx.y * 64;
+    const int tiles = (ns + 63) >> 6, rt = blockIdx.x / tiles;
+    const int r0 = rt * 64, i0 = (blockIdx.x - rt * tiles) * 64;
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;          // 16 x 16 threads, 4 x 4 outputs each
     float acc[4][4];
 #pragma unroll

@@ -81,9 +81,9 @@ int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool pro
     if (o->d_Lf) {   // smoothness prior: z <- L z for the whole population before computeAz (lmcma.cpp:216-217)
         const OptDev& d = o->d;
         int rc = 0;
-        if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) rc = launch(k_gauss, dim3((d.ns / 4 + 127) / 128, d.pop_count, d.B), 128, 0, st, false, d);
+        if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) rc = launch(k_gauss, dim3((d.ns / 4 + 127) / 128 * d.pop_count, 1, d.B), 128, 0, st, false, d);
         const int rows = d.B * d.pop_count;
-        if (!rc) rc = launch(k_prior, dim3((d.ns + 63) / 64, (rows + 63) / 64), 256, 0, st, false, d.Z, o->d_Lf, d.Zc, rows, d.n, d.ns);
+        if (!rc) rc = launch(k_prior, dim3((d.ns + 63) / 64 * ((rows + 63) / 64)), 256, 0, st, false, d.Z, o->d_Lf, d.Zc, rows, d.n, d.ns);
         if (rc) return rc;
         pdl = false;
     }

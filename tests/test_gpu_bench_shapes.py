@@ -8,7 +8,7 @@ import pytest
 
 import lmcma_path_planner_b200 as L
 from lmcma_path_planner_b200 import maps
-from test_gpu_parity import _teacher_forced, rel_err, COST_RTOL
+from test_gpu_parity import _teacher_forced, prior_deviates, rel_err, COST_RTOL
 
 pytestmark = pytest.mark.gpu
 
@@ -254,14 +254,16 @@ def _device_state(dev, b):
     return st
 
 
-def _sampler_matches_oracle(po, dev, n, lam, m, lo, hi, instances):
-    """The population the device has just sampled == the oracle's sample() from the device's own state and deviates."""
+def _sampler_matches_oracle(po, dev, n, lam, m, lo, hi, instances, L64=None):
+    """The population the device has just sampled == the oracle's sample() from the device's own state and deviates.
+    L64: the FP64 Cholesky factor of the handle's covariance prior (test_gpu_parity.prior_factor); "Z" holds the deviates
+    before the prior, so the oracle is fed z L^T."""
     worst = 0.0
     Z, X = dev.get("Z"), dev.get("X")
     for b in instances:
         st = _device_state(dev, b)
         ora = po.OracleLMCMA(n, x0=np.zeros(n), lam=lam, m=m, lo=lo, hi=hi, sigma=1.0)
-        ora.load_state(st, np.zeros(lam), Z[b].astype(np.float64))
+        ora.load_state(st, np.zeros(lam), prior_deviates(Z[b], L64))
         Xo = ora.array("X")
         scale = max(1.0, float(np.abs(Xo).max()))
         worst = max(worst, float(np.abs(X[b] - Xo).max()) / scale)

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import lmcma_path_planner_b200 as L
+from lmcma_path_planner_b200 import _capi as K
 from lmcma_path_planner_b200 import maps
 from conftest import weighted_sphere
 
@@ -142,22 +143,38 @@ def test_cost_full_size_properties(po):
 # ------------------------------------------------------------------------------------------------
 # optimiser: teacher-forced generations against the FP64 oracle (SURVEY 7.2 #3)
 # ------------------------------------------------------------------------------------------------
+def prior_factor(covariance):
+    """The FP64 lower Cholesky factor of a covariance prior: the factor the library rounds to FP32 for its deviates L z."""
+    n = covariance.shape[0]
+    L64 = np.zeros(n * n)
+    K.check(K.lib().lmcma_b200_cholesky(n, K.dptr(np.ascontiguousarray(covariance, np.float64).ravel()), K.dptr(L64)))
+    return L64.reshape(n, n)
+
+
+def prior_deviates(Z, L64=None):
+    """The deviates the samplers combine, in FP64: Z itself, or L z for every row (Z L^T) with a covariance prior."""
+    Z = np.asarray(Z, np.float64)
+    return Z if L64 is None else Z @ L64.T
+
+
 def _teacher_forced(po, n, lam, m, gens, seed, lo=None, hi=None, sigma=1.0, fobj=weighted_sphere, x0=None,
-                    tol=2e-5, tol_v=None, warm=None):
+                    tol=2e-5, tol_v=None, warm=None, covariance=None):
     """`gens` teacher-forced generations.  warm: an oracle state of the same (n, m) (OracleLMCMA.state(), e.g. from a cheap
     small-population run) to start from instead of the empty state, so that a few generations have every slot live and
-    being recycled; the previous fitness is then the sorted fitness of the first population."""
+    being recycled; the previous fitness is then the sorted fitness of the first population.  covariance: the device
+    handle gets this smoothness prior and the oracle, which has none, is fed z L^T in FP64 wherever it takes deviates."""
     rng = np.random.default_rng(seed)
     x0 = np.full(n, 0.5) if x0 is None else x0
-    dev = L.Optimizer(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma0=sigma, rng="inject")
+    L64 = None if covariance is None else prior_factor(covariance)
+    dev = L.Optimizer(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma0=sigma, rng="inject", covariance=covariance)
     lam = dev.lam
     zs = rng.standard_normal((gens + 1, lam, n)).astype(np.float32)
-    ora = po.OracleLMCMA(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma=sigma, seed=1, Z0=zs[0].astype(np.float64))
+    ora = po.OracleLMCMA(n, x0=x0, lam=lam, m=m, lo=lo, hi=hi, sigma=sigma, seed=1, Z0=prior_deviates(zs[0], L64))
     dev.inject_z(zs[0])
     if warm is not None:
-        ora.load_state(warm, np.zeros(lam), zs[0].astype(np.float64))
+        ora.load_state(warm, np.zeros(lam), prior_deviates(zs[0], L64))
         prev = np.sort(fobj(ora.array("X")).astype(np.float32))
-        ora.load_state(warm, prev.astype(np.float64), zs[0].astype(np.float64))
+        ora.load_state(warm, prev.astype(np.float64), prior_deviates(zs[0], L64))
         dev.load_state(dict(warm, prev_fit=prev))
         dev.resample()
     worst = {}
@@ -167,7 +184,7 @@ def _teacher_forced(po, n, lam, m, gens, seed, lo=None, hi=None, sigma=1.0, fobj
         xs = max(1e-3, float(np.abs(Xo).max()))               # waypoint-coordinate scale
         worst["X"] = max(worst.get("X", 0), float(np.abs(Xd - Xo).max()) / xs)
         f = fobj(Xo).astype(np.float32)            # both sides are told the same FP32 fitness
-        ora.tell_all(f.astype(np.float64), zs[g + 1].astype(np.float64))
+        ora.tell_all(f.astype(np.float64), prior_deviates(zs[g + 1], L64))
         dev.inject_z(zs[g + 1])
         dev.tell_all(f)
         so = ora.state()
