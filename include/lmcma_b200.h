@@ -20,7 +20,9 @@
  * on several streams for different queries (the end points travel by value with each launch; no per-map device state is
  * written); lmcma_b200_cost_evaluate and lmcma_b200_cost_trace (host buffers) serialise on a per-map lock because they
  * share the map's staging buffers and private stream.  lmcma_b200_map_set_l2_persist, lmcma_b200_map_update_occupancy and
- * lmcma_b200_map_destroy must not race with evaluations on the same map.
+ * lmcma_b200_map_destroy must not race with evaluations on the same map.  lmcma_b200_tell_all_dev enqueues on the
+ * handle's stream only and returns without waiting: the caller's cost, and every later call on the handle, are ordered
+ * after it by that stream (call lmcma_b200_set_stream with the stream the cost runs on, never NULL).
  *
  * Environment knobs (LMCMA_B200_*, experiments / debugging only) are read once when a handle is created, never on a
  * launch path.  The overlapped single-query generation (a forked CUDA graph whose branches must run concurrently) is
@@ -200,6 +202,27 @@ int lmcma_b200_tell_all(lmcma_b200_opt* opt, const float* f_host);
  * H2D of the candidates).  Same contents as lmcma_b200_ask_all. */
 int lmcma_b200_ask_all_view(lmcma_b200_opt* opt, const float** X_host_view, int64_t* ld_out);
 
+/* Device-resident batched protocol, for a cost the caller computes on the GPU.
+ * X_dev: the current population, batch x pop_count rows of n FP32, row stride *ld_out floats (>= n).  Read-only.
+ * f_dev: the handle's fitness buffer, batch x lambda FP32, dense.  The caller writes it, then calls tell_all_dev.
+ * Both pointers stay valid and unchanged for the handle's lifetime.  Any handle may call this.  Nothing is allocated, so
+ * a stream capture may begin right after it. */
+int lmcma_b200_device_buffers(lmcma_b200_opt* opt, const float** X_dev, int64_t* ld_out, float** f_dev);
+/* update() + sample() from the fitness in f_dev, enqueued on the handle's stream (lmcma_b200_set_stream).  Returns without
+ * waiting.  Later work on that stream sees the next population in X_dev.  The same bits as lmcma_b200_tell_all given the
+ * same fitness.  Capturable into the caller's stream capture (torch.cuda.graph, cudaStreamBeginCapture): under a capture
+ * it enqueues the stream-ordered generation, builds and replays no graph of its own, allocates nothing and never waits.
+ * Uncaptured, one query with the overlapped generation replays tell_all's forked graph without its fitness copy; other
+ * handles enqueue the stream-ordered generation.  A lost co-scheduling is reported by the next synchronising call.
+ * The handle's stream must be one the caller's cost is ordered with: set_stream with the cost's own stream.  NULL selects
+ * the handle's private non-blocking stream, which neither the caller's streams nor the legacy default stream wait for.
+ * Replays of a caller's graph advance the state without this library seeing them: once a generation has been recorded,
+ * ask_all_view and ask_one always read the population from the device, and the setters of V, P, NJ, LJ, T and VEC
+ * rebuild the pair mirror the sampler reads at once.  Order the replays with later calls on the handle (replay on the
+ * handle's stream, or synchronise).
+ * LMCMA_B200_ERR_STATE: rng != PHILOX, a split-population handle. */
+int lmcma_b200_tell_all_dev(lmcma_b200_opt* opt);
+
 /* deviates for the NEXT sample(): batch x pop_count x n FP32 (rng == INJECT).  The first call after
  * create builds the first population immediately; later calls are consumed by the next tell. */
 int lmcma_b200_inject_z(lmcma_b200_opt* opt, const float* Z_host);
@@ -220,7 +243,9 @@ int lmcma_b200_attach_cost(lmcma_b200_opt* opt, lmcma_b200_map* map, const lmcma
 int lmcma_b200_run(lmcma_b200_opt* opt, int32_t generations);
 int lmcma_b200_sync(lmcma_b200_opt* opt);
 /* number of kernels this library has launched so far (all handles, this process).  A replay of one of its CUDA graphs
- * (lmcma_b200_run, lmcma_b200_tell_all) counts the kernels the graph holds; building a graph counts none. */
+ * (lmcma_b200_run, lmcma_b200_tell_all, lmcma_b200_tell_all_dev) counts the kernels the graph holds; building a graph
+ * counts none.  Kernels lmcma_b200_tell_all_dev enqueues into the caller's stream capture count none either: they run
+ * when the caller replays its graph, which this library does not see. */
 int64_t lmcma_b200_launch_count(void);
 /* CUDA-event timing of everything enqueued by the last lmcma_b200_run on this handle (ms) */
 int lmcma_b200_last_run_ms(lmcma_b200_opt* opt, float* ms_out);

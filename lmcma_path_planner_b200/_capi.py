@@ -78,6 +78,8 @@ SIGNATURES = {
     "lmcma_b200_ask_all": (C.c_int, [_vp, _pf]),
     "lmcma_b200_tell_all": (C.c_int, [_vp, _pf]),
     "lmcma_b200_ask_all_view": (C.c_int, [_vp, C.POINTER(_pf), _pl]),
+    "lmcma_b200_device_buffers": (C.c_int, [_vp, C.POINTER(_vp), _pl, C.POINTER(_vp)]),
+    "lmcma_b200_tell_all_dev": (C.c_int, [_vp]),
     "lmcma_b200_inject_z": (C.c_int, [_vp, _pf]),
     "lmcma_b200_resample": (C.c_int, [_vp]),
     "lmcma_b200_is_done": (C.c_int, [_vp, _pi]),

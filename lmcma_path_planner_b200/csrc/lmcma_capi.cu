@@ -224,10 +224,15 @@ void drop_fused_graphs(lmcma_b200_opt* o) {
     drop(o->graph_multi);
 }
 // the tell graphs, and with them what their speculative pass left behind
-void drop_tell_graphs(lmcma_b200_opt* o) {
-    drop(o->tell_graph);
-    drop(o->tell_graph_resume);
+void drop_tell_graphs(lmcma_b200_opt* o, TellGraphs& tg) {
+    drop(tg.whole);
+    drop(tg.resume);
+    tg.built_for = nullptr;
     o->spec_valid = false;
+}
+void drop_tell_graphs(lmcma_b200_opt* o) {
+    drop_tell_graphs(o, o->tell_host);
+    drop_tell_graphs(o, o->tell_dev);
 }
 
 // Records what body() enqueues on `st` (and on the streams it forks from `st`) into *g, which is empty.  Capture enqueues
@@ -335,12 +340,21 @@ int lmcma_capi::check_lost(lmcma_b200_opt* o) {
     o->props->cosched = 0;
     drop_fused_graphs(o);
     drop_tell_graphs(o);
-    o->tell_graph_failed = true;
+    o->tell_host.failed = o->tell_dev.failed = true;
     o->mirror_dirty = true;
     return fail(LMCMA_B200_ERR_CUDA, "overlapped generation lost co-scheduling (%s): the branches of the CUDA graph did not run "
                 "concurrently (profiler / sanitizer / SMs held elsewhere).  This handle now uses the linear graph; the generation in "
                 "flight is void - restore the state or recreate the handle (LMCMA_B200_OVERLAP=0 avoids the overlapped graph)",
                 code == LOST_UPDATE_WAITING_FOR_RANK ? "k_update timed out waiting for k_rank" : "k_sample timed out waiting for k_update");
+}
+// After a state setter: on a handle whose generations replay in a caller's graph (caller_graphs), rebuild the pair mirror
+// now, because the next sampler to read it may be a replay that never passes through ensure_mirror
+int lmcma_capi::settle_mirror(lmcma_b200_opt* o) {
+    if (!o->caller_graphs || !o->mirror_dirty) return 0;
+    int rc = ensure_mirror(o, o->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(o->stream));
+    return 0;
 }
 namespace {
 
@@ -397,22 +411,26 @@ int ensure_graph(lmcma_b200_opt* o) {
     return 0;
 }
 
-// tell_all of one query as a forked graph (see lmcma_b200_tell_all); on failure the caller takes the stream-ordered path
-int ensure_tell_graph(lmcma_b200_opt* o) {
-    if (o->tell_graph.exec && o->tell_graph_for == o->stream) return ensure_mirror(o, o->stream);
-    drop_tell_graphs(o);
+// The tell of one query as a forked graph (see lmcma_b200_tell_all).  dev: the graph of lmcma_b200_tell_all_dev, which
+// finds the fitness in d.fit already (no H2D node) and never writes the host mirror.  On failure the caller takes the
+// stream-ordered path.
+int ensure_tell_graph(lmcma_b200_opt* o, bool dev) {
+    TellGraphs& tg = dev ? o->tell_dev : o->tell_host;
+    if (tg.whole.exec && tg.built_for == o->stream) return ensure_mirror(o, o->stream);
+    drop_tell_graphs(o, tg);
     cudaStream_t st = o->stream;
     const OptDev& d = o->d;
     int rc = ensure_mirror(o, st);
     if (rc) return rc;
-    if (!o->f_pinned && cudaHostAlloc(&o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaHostAllocDefault) != cudaSuccess) {
-        cudaGetLastError(); o->f_pinned = nullptr; o->tell_graph_failed = true; return 0;
+    if (!dev && !o->f_pinned && cudaHostAlloc(&o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaHostAllocDefault) != cudaSuccess) {
+        cudaGetLastError(); o->f_pinned = nullptr; tg.failed = true; return 0;
     }
     // the speculative pass pays only where something hides it: with the host mirror on, the candidates' trip across PCIe
     // (35 us behind the sampler).  Without the mirror tell_all returns when the sampler is done, and a 25 us kernel behind
-    // k_update would be the longer branch of the graph (measured: tell_all 57 -> 69 us)
-    const bool spec = o->d_spec != nullptr && o->mirror_on && !o->mirror_suppressed;
-    o->tell_graph_spec = spec;
+    // k_update would be the longer branch of the graph (measured: tell_all 57 -> 69 us).  tell_all_dev: not even when it
+    // is left running beside the caller's cost (DESIGN.md 4.4)
+    const bool spec = !dev && o->d_spec != nullptr && o->mirror_on && !o->mirror_suppressed;
+    tg.spec = spec;
     // resume = 0: the whole update; resume = 1: k_update picks up the rows the last graph's speculative pass left.  With the
     // scratch both graphs END with that pass for the next generation, on the side branch behind k_update
     auto body = [&](int resume) -> int {
@@ -426,7 +444,7 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
         if (ok && spec) { UpdateArgs us = ua; us.phase = 1; us.dbg = nullptr; ok = launch_update(o, us, false, o->side_stream) == 0; }
         o->spec_valid = valid_before;                            // capture enqueues nothing
         if (ok) ok = cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess;
-        if (ok) ok = cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st) == cudaSuccess;
+        if (ok && !dev) ok = cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st) == cudaSuccess;
         if (ok) ok = launch(k_gate, (d.B + 31) / 32, 32, 0, st, false, d) == 0;   // k_update has reset the flags and holds its SM
         // the sampler is released when k_rank starts: the pairs it needs first are final (resume: at once; else as the sweep goes)
         if (ok) ok = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, false) == 0;
@@ -434,15 +452,18 @@ int ensure_tell_graph(lmcma_b200_opt* o) {
         if (ok) ok = cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
         return ok ? 0 : LMCMA_B200_ERR_CUDA;
     };
-    rc = capture(st, [&] { return body(0); }, &o->tell_graph);
-    if (!rc && spec) rc = capture(st, [&] { return body(1); }, &o->tell_graph_resume);
+    const bool suppressed = o->mirror_suppressed;
+    if (dev) o->mirror_suppressed = true;                        // the device protocol keeps the candidates on the device
+    rc = capture(st, [&] { return body(0); }, &tg.whole);
+    if (!rc && spec) rc = capture(st, [&] { return body(1); }, &tg.resume);
+    o->mirror_suppressed = suppressed;
     if (rc) {
         cudaGetLastError();
-        drop_tell_graphs(o);
-        o->tell_graph_failed = true;
+        drop_tell_graphs(o, tg);
+        tg.failed = true;
         return 0;
     }
-    o->tell_graph_for = st;
+    tg.built_for = st;
     return 0;
 }
 
@@ -736,7 +757,9 @@ int lmcma_b200_ask_all_view(lmcma_b200_opt* o, const float** X_view, int64_t* ld
         // the captured graphs carry the old kernel parameters (OptDev by value): rebuild them on next use
         drop_tell_graphs(o);
     }
-    if (!o->xh_fresh) {                                  // first use / after a fused run or a state setter: one ordinary copy
+    // first use / after a fused run, a state setter or a tell_all_dev (or, once the caller has recorded generations: every
+    // time): one ordinary copy
+    if (!o->xh_fresh || o->caller_graphs) {
         CU(cudaMemcpyAsync(o->x_mirror, d.X, floats * sizeof(float), cudaMemcpyDeviceToHost, o->stream));
         o->xh_fresh = true;
     }
@@ -753,18 +776,18 @@ int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     int rc;
-    if (o->overlap && !o->tell_graph_failed && o->tune.tell_overlap != 0) {
+    if (o->overlap && !o->tell_host.failed && o->tune.tell_overlap != 0) {
         // One query (the conditions of the overlapped generation, DESIGN.md 4.3): everything in update() that does not
         // depend on this generation's fitness — slot bookkeeping, the sweep over every pending row but the newest — runs on
         // a side branch while the fitness crosses PCIe and k_rank runs; k_update then waits for k_rank's tickets and
         // k_sample follows its hand-over flags.  Same kernels and arithmetic as the fused generation (bit-identical to the
         // serial order), replayed as one CUDA graph: launched kernel by kernel, the fork / join costs more host time than
         // the overlap saves.
-        if ((rc = ensure_tell_graph(o)) == 0 && o->tell_graph.exec) {
+        if ((rc = ensure_tell_graph(o, false)) == 0 && o->tell_host.whole.exec) {
             memcpy(o->f_pinned, f, (size_t)d.B * d.lambda * sizeof(float));
-            const bool resume = o->spec_valid && o->tell_graph_resume.exec;   // the last tell_all graph left the next update's rows behind
-            if ((rc = replay(resume ? o->tell_graph_resume : o->tell_graph, o->stream))) return rc;
-            o->spec_valid = o->tell_graph_spec;                   // ... and so does this one
+            const bool resume = o->spec_valid && o->tell_host.resume.exec;   // the last tell left the next update's rows behind
+            if ((rc = replay(resume ? o->tell_host.resume : o->tell_host.whole, o->stream))) return rc;
+            o->spec_valid = o->tell_host.spec;                    // ... and so does this one
             o->xh_fresh = o->mirror_on;                          // the captured sampler writes the host mirror when it is on
             o->x_cache_valid = false;
             o->sample_idx = 0;
@@ -781,11 +804,53 @@ int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
     return 0;
 }
 
+int lmcma_b200_device_buffers(lmcma_b200_opt* o, const float** X_dev, int64_t* ld_out, float** f_dev) {
+    ARG(o && X_dev && ld_out && f_dev, "null pointer");
+    *X_dev = o->d.X;
+    *ld_out = o->d.ns;
+    *f_dev = o->d.fit;
+    return 0;
+}
+
+int lmcma_b200_tell_all_dev(lmcma_b200_opt* o) {
+    ARG(o, "null handle");
+    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "tell_all_dev needs the PHILOX rng (HANSEN / INJECT: tell_all)");
+    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles use the mg_* entry points");
+    CU(cudaSetDevice(o->cfg.device));
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    CU(cudaStreamIsCapturing(o->stream, &cs));
+    int rc = 0;
+    o->mirror_suppressed = true;                                 // the candidates stay on the device
+    if (cs != cudaStreamCaptureStatusNone) {
+        // the caller's capture: no library graph is replayed or built, nothing allocated or synchronised.  The linear
+        // generation (same bits as the forked one) keeps kernels that spin on a partner out of a graph the library does not
+        // control.  Its kernels are counted by nobody: they run when the caller replays the graph
+        long long uncounted = 0;
+        g_capture_launches = &uncounted;
+        rc = generation_tail(o, o->stream);
+        g_capture_launches = nullptr;
+        o->caller_graphs = true;
+    } else if (o->overlap && !o->tell_dev.failed && o->tune.tell_overlap != 0 && (rc = ensure_tell_graph(o, true)) == 0 &&
+               o->tell_dev.whole.exec) {
+        // one query: the forked graph of tell_all without the fitness copy (and without the speculative pass, DESIGN.md 4.4)
+        rc = replay(o->tell_dev.whole, o->stream);
+        o->spec_valid = false;
+    } else if (!rc) {
+        rc = generation_tail(o, o->stream);
+    }
+    o->mirror_suppressed = false;
+    o->x_cache_valid = false;
+    o->sample_idx = 0;
+    o->xh_fresh = false;
+    o->pending_z = false;
+    return rc;
+}
+
 int lmcma_b200_ask_one(lmcma_b200_opt* o, double* params, int32_t n) {
     ARG(o && params, "null pointer");
     ARG(n == o->d.n, "N mismatch");
     if (o->d.B != 1 || o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "ask_one needs batch == 1 and an unsplit population");
-    if (!o->x_cache_valid) {
+    if (!o->x_cache_valid || o->caller_graphs) {                  // a replay of the caller's graph may have moved on
         o->x_cache.resize((size_t)o->d.lambda * o->d.n);
         int rc = lmcma_b200_ask_all(o, o->x_cache.data());
         if (rc) return rc;

@@ -139,7 +139,7 @@ int lmcma_b200_set_f64(lmcma_b200_opt* o, int32_t which, const double* in, int64
                 CU(cudaStreamSynchronize(o->stream));
             }
             CU(cudaStreamSynchronize(o->stream));
-            return 0;
+            return settle_mirror(o);
         }
     }
     return fail(LMCMA_B200_ERR_ARG, "f64 field %d is not settable", which);
@@ -158,7 +158,10 @@ int lmcma_b200_set_f32(lmcma_b200_opt* o, int32_t which, const float* in, int64_
         case LMCMA_B200_F32_V: case LMCMA_B200_F32_P:
             ARG(count == (int64_t)(B * d.m * d.n), "count");
             o->mirror_dirty = true;
-            return h2d_rows(which == LMCMA_B200_F32_V ? d.V : d.P, in, B * d.m, w, p, o->stream);
+            {
+                int rc = h2d_rows(which == LMCMA_B200_F32_V ? d.V : d.P, in, B * d.m, w, p, o->stream);
+                return rc ? rc : settle_mirror(o);
+            }
         case LMCMA_B200_F32_X: {
             ARG(count == (int64_t)(B * d.pop_count * d.n), "count");
             o->x_cache_valid = false;
@@ -203,7 +206,7 @@ int lmcma_b200_set_i32(lmcma_b200_opt* o, int32_t which, const int32_t* in, int6
             o->mirror_dirty = true;
             CU(cudaMemcpyAsync(which == LMCMA_B200_I32_T ? d.t : d.vec, in, B * d.m * sizeof(int), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));
-            return 0;
+            return settle_mirror(o);
         case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: {
             ARG(count == (int64_t)B, "count");
             std::vector<Scalars> sc(B);

@@ -93,6 +93,15 @@ struct Graph {
     int launches = 0;
 };
 
+// the forked graphs of one query's tell (lmcma_capi.cu: ensure_tell_graph): the whole update, and the one that resumes from
+// the rows a speculative pass left in d_spec
+struct TellGraphs {
+    Graph whole, resume;
+    cudaStream_t built_for = nullptr;
+    bool spec = false;                 // the graphs end with the speculative pass (tell_all with the host mirror on)
+    bool failed = false;               // could not be built here: this tell takes the stream-ordered path for good
+};
+
 
 struct DeviceProps {
     int sm_count = 0;
@@ -177,16 +186,18 @@ struct lmcma_b200_opt {
     lmcma_capi::Graph graph;                  // one fused generation (lmcma_b200_run)
     lmcma_capi::Graph graph_multi;            // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)
     cudaStream_t graph_built_for = nullptr;
-    lmcma_capi::Graph tell_graph;             // tell_all of one query: H2D fitness -> k_rank -> k_sample, k_update on a side branch
-    cudaStream_t tell_graph_for = nullptr;
-    bool tell_graph_failed = false;
-    // speculative update (k_update.cuh, UpdateArgs::phase): every tell_all graph ends with the fitness-independent part of the
-    // NEXT generation's update (into d_spec, beside the sampler's tail and the candidates' trip across PCIe); the next tell_all
-    // resumes from it (tell_graph_resume) unless anything else touched the optimiser's state in between
-    lmcma_capi::Graph tell_graph_resume;
+    // tell of one query: [H2D fitness ->] k_gate -> k_rank -> k_sample, k_update on a side branch.  tell_host: tell_all;
+    // tell_dev: tell_all_dev (the fitness is in d.fit already, the host mirror is not written)
+    lmcma_capi::TellGraphs tell_host, tell_dev;
+    // lmcma_b200_tell_all_dev recorded generations into a caller's stream capture.  Their replays advance the state without
+    // this library seeing them, so from then on no host-side record of the population is trusted (ask_all_view copies,
+    // ask_one reloads) and a state setter rebuilds the pair mirror at once instead of at the next library launch
+    bool caller_graphs = false;
+    // speculative update (k_update.cuh, UpdateArgs::phase): with the host mirror on, every tell_all graph ends with the
+    // fitness-independent part of the NEXT generation's update (into d_spec, beside the sampler's tail and the candidates' trip
+    // across PCIe); the next tell_all resumes from it (tell_host.resume) unless anything else touched the state in between
     float* d_spec = nullptr; size_t spec_stride = 0;
     bool spec_valid = false;
-    bool tell_graph_spec = false;             // the tell graphs were captured with the speculative pass (host mirror on)
     float* f_pinned = nullptr;                // the graph's copy source (the caller's fitness array is copied here first)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool have_run_timing = false;
@@ -215,6 +226,7 @@ void register_mirror(const void* host, size_t bytes, const float* dev, long long
 void unregister_mirror(const void* host);
 // ---- defined in lmcma_capi.cu ----
 int check_lost(lmcma_b200_opt* o);
+int settle_mirror(lmcma_b200_opt* o);
 
 // dense <-> pitched copies
 inline int d2h_rows(void* dst, const void* src, size_t rows, size_t width_bytes, size_t src_pitch_bytes, cudaStream_t st) {

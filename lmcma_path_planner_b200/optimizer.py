@@ -129,6 +129,18 @@ class CostMap:
         return cells[:min(n_out.value, max_cells)].copy()
 
 
+class _DeviceBuffer:
+    """One of an optimiser's device buffers as a __cuda_array_interface__ (FP32).  A tensor made from it holds a reference to
+    it, and through `owner` to the optimiser, so garbage collection cannot free the memory under it (close() still does).
+    torch takes no read-only flag: that
+    X must not be written is the caller's part (device_tensors)."""
+
+    def __init__(self, owner, ptr, shape, strides):
+        self.owner = owner
+        self.__cuda_array_interface__ = {"shape": shape, "strides": strides, "typestr": "<f4", "data": (ptr, False),
+                                         "version": 2}
+
+
 class Optimizer:
     """B independent LM-CMA instances of one shape on one device."""
 
@@ -152,7 +164,9 @@ class Optimizer:
         shp = np.zeros(8, np.int32)
         K.check(K.lib().lmcma_b200_shape(h, K.iptr(shp)))
         self.n, self.lam, self.mu, self.m, self.batch, self.pop_offset, self.pop_count, self.ld = (int(v) for v in shp)
+        self.device = int(device)
         self._map = None
+        self._stream = None          # set_stream: None = the handle's own non-blocking stream
 
     def close(self):
         if getattr(self, "_h", None):
@@ -182,6 +196,37 @@ class Optimizer:
     def tell_all(self, f):
         f = K.f32c(f).reshape(self.batch, self.lam)
         K.check(K.lib().lmcma_b200_tell_all(self._h, K.fptr(f)))
+
+    def device_tensors(self):
+        """torch views (X [batch, pop_count, n], F [batch, lambda]) over the handle's device buffers, for a cost computed on
+        the GPU: read the population from X, write every fitness into F, then call tell_all_dev.  X is READ-ONLY (its rows
+        have stride ld floats); F must be fully written before each tell.  The views keep this optimiser from being garbage
+        collected, but close() frees the buffers under them: do not use them after close().
+
+        The handle's work must be ordered with the cost's: run the cost on a torch.cuda.Stream() (not the default stream)
+        and put the handle on it first, set_stream(s.cuda_stream).  The default stream's cuda_stream is 0, which selects the
+        handle's own non-blocking stream, and nothing torch enqueues is ordered with that one; tell_all_dev refuses it.
+        Nothing is allocated, so a torch.cuda.graph capture may follow at once."""
+        import torch                                             # only this method needs torch
+        xp, fp, ld = C.c_void_p(), C.c_void_p(), C.c_int64(0)
+        K.check(K.lib().lmcma_b200_device_buffers(self._h, C.byref(xp), C.byref(ld), C.byref(fp)))
+        ld = int(ld.value)
+        X = _DeviceBuffer(self, xp.value, (self.batch, self.pop_count, self.n), (self.pop_count * ld * 4, ld * 4, 4))
+        F = _DeviceBuffer(self, fp.value, (self.batch, self.lam), (self.lam * 4, 4))
+        dev = torch.device("cuda", self.device)
+        return torch.as_tensor(X, device=dev), torch.as_tensor(F, device=dev)
+
+    def tell_all_dev(self):
+        """update() + sample() from the fitness in device_tensors()'s F, enqueued on the handle's stream; returns without
+        waiting.  Same bits as tell_all with the same fitness.  Capturable in torch.cuda.graph (with the handle on the
+        capture stream).  PHILOX handles of one unsplit population only.
+
+        Raises (ERR_STATE, nothing enqueued) while the handle runs on its own stream: Python code cannot enqueue a cost on
+        that stream, so the tell could not be ordered after it (see device_tensors)."""
+        if self._stream is None:
+            raise K.LmcmaError(K.ERR_STATE, "tell_all_dev on the handle's own stream: no cost can be ordered before it; "
+                               "set_stream(s.cuda_stream) with the (non-default) torch stream the cost runs on")
+        K.check(K.lib().lmcma_b200_tell_all_dev(self._h))
 
     def ask_one(self):
         x = np.zeros(self.n, np.float64)
@@ -230,7 +275,9 @@ class Optimizer:
         K.check(K.lib().lmcma_b200_sync(self._h))
 
     def set_stream(self, stream):
+        """int cudaStream_t to run on; None or 0 = the handle's own non-blocking stream"""
         K.check(K.lib().lmcma_b200_set_stream(self._h, stream))
+        self._stream = stream or None
 
     def last_run_ms(self):
         ms = C.c_float(0)
