@@ -74,9 +74,11 @@ int ensure_mirror(lmcma_b200_opt* o, cudaStream_t st) {
     return 0;
 }
 
+// mirror: write the host mirror of X too (if any, lmcma_b200_ask_all_view): the host-buffer protocol does; the fused
+// generations (lmcma_b200_run), the device-resident tell and the split-population stages keep the candidates on the device
 // pdl: launched as a programmatic dependent of the kernel enqueued just before it on `st` (k_update)
 // progressive: that k_update was launched with UpdateArgs::progressive (only meaningful with pdl)
-int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool progressive = false, int progressive_mode = 1) {
+int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool mirror, bool pdl = false, bool progressive = false, int progressive_mode = 1) {
     if (o->mirror_dirty) { int rc = ensure_mirror(o, st); if (rc) return rc; pdl = false; }
     if (o->d_Lf) {   // smoothness prior: z <- L z for the whole population before computeAz (lmcma.cpp:216-217)
         const OptDev& d = o->d;
@@ -87,11 +89,8 @@ int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool pdl = false, bool pro
         if (rc) return rc;
         pdl = false;
     }
-    // the host mirror of X (lmcma_b200_ask_all_view) is written by the samplers of the host-buffer protocol only: the fused
-    // on-device generations (lmcma_b200_run) and the split-population stages keep the candidates on the device
     OptDev d = o->d;
-    if (!o->mirror_on || o->mirror_suppressed) d.Xh = nullptr;
-    o->xh_fresh = d.Xh != nullptr;
+    if (!mirror) d.Xh = nullptr;
     if (o->plan.sample.kind == Sampler::ROWS) return launch_sample_rows(o, d, pdl, st);
     if (o->plan.sample.kind == Sampler::WIDE)
         return launch_sample_wide(o, d, pdl, st, (pdl && progressive && o->plan.progressive) ? progressive_mode : 0);
@@ -126,7 +125,6 @@ int launch_update_t(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream
 // the serial part of update() (k_update.cuh).  pdl: launched as a programmatic dependent of the kernel enqueued just
 // before it on `st` (k_rank), so that its prologue overlaps that kernel
 int launch_update(lmcma_b200_opt* o, const UpdateArgs& a, bool pdl, cudaStream_t st) {
-    if (a.phase == 0) o->spec_valid = false;                        // a whole update: whatever the speculative pass left is stale
     const auto& u = o->plan.update;
     if (u.gram) {
         int rc = u.nvb == 4 ? launch_update_t<4, -1, false>(o, a, pdl, st) : launch_update_t<16, -1, false>(o, a, pdl, st);
@@ -185,7 +183,7 @@ __global__ void k_set_best_f(Scalars* sc, const float* f, int B) {
 }
 
 // generate / stage deviates on the host for HANSEN mode, then sample
-int host_rng_and_sample(lmcma_b200_opt* o, cudaStream_t st, bool progressive = false) {
+int host_rng_and_sample(lmcma_b200_opt* o, cudaStream_t st, bool mirror, bool progressive = false) {
     if (o->cfg.rng == LMCMA_B200_RNG_HANSEN) {
         const size_t rows = (size_t)o->d.pop_count;
         o->z_host.assign(rows * o->d.ns, 0.f);
@@ -195,23 +193,83 @@ int host_rng_and_sample(lmcma_b200_opt* o, cudaStream_t st, bool progressive = f
         CU(cudaMemcpyAsync(o->d.Z, o->z_host.data(), o->z_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
         CU(cudaStreamSynchronize(st));   // z_host is pageable and reused
     }
-    return launch_sample(o, st, o->cfg.rng != LMCMA_B200_RNG_HANSEN, progressive);
+    return launch_sample(o, st, mirror, o->cfg.rng != LMCMA_B200_RNG_HANSEN, progressive);
 }
 
-// update() + sample() after the fitness of a generation is in d.fit
-int generation_tail(lmcma_b200_opt* o, cudaStream_t st) {
+// a sampler has been enqueued or replayed (mirror: it wrote the host mirror): the host's record of the population is stale
+void new_population(lmcma_b200_opt* o, bool mirror) {
+    o->x_cache_valid = false;
+    o->sample_idx = 0;
+    o->xh_fresh = mirror && o->x_mirror;
+}
+
+// where a generation's fitness comes from: k_cost on the attached map, a copy from f_pinned, or d.fit as it is
+enum class Fit { COST, FROM_HOST, IN_PLACE };
+
+int launch_own_cost(lmcma_b200_opt* o, cudaStream_t st) {
+    CostArgs ca;
+    int rc = cost_args_for(o, &ca);
+    return rc ? rc : launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
+}
+
+// One generation in stream order (fit: COST or IN_PLACE): [k_cost ->] k_rank -> k_update -> [HANSEN deviates ->] the
+// sampler, or without the sampler (sample = false).  k_rank is a programmatic dependent of k_cost only.
+int enqueue_linear(lmcma_b200_opt* o, cudaStream_t st, Fit fit, bool mirror, bool sample = true) {
     int rc;
-    if ((rc = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st))) return rc;
+    if (fit == Fit::COST && (rc = launch_own_cost(o, st))) return rc;
+    if ((rc = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st, fit == Fit::COST))) return rc;
     // device RNG: k_sample follows k_update directly and can take its outputs as they become final
     const bool prog = o->plan.progressive && o->cfg.rng == LMCMA_B200_RNG_PHILOX && !o->mirror_dirty;
     UpdateArgs ua = update_args_local(o);
     ua.progressive = prog ? 1 : 0;
     if ((rc = launch_update(o, ua, true, st))) return rc;
-    o->x_cache_valid = false;
-    o->sample_idx = 0;
-    if (o->cfg.rng == LMCMA_B200_RNG_INJECT && !o->pending_z) { o->needs_sample = true; return 0; }
+    return sample ? host_rng_and_sample(o, st, mirror, prog) : 0;
+}
+
+// the two branches of a forked graph: the side stream starts behind `st`, and `st` ends behind the side stream
+int fork_side(lmcma_b200_opt* o, cudaStream_t st) {
+    CU(cudaEventRecord(o->ev_fork, st));
+    CU(cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0));
+    return 0;
+}
+int join_side(lmcma_b200_opt* o, cudaStream_t st) {
+    CU(cudaEventRecord(o->ev_join, o->side_stream));
+    CU(cudaStreamWaitEvent(st, o->ev_join, 0));
+    return 0;
+}
+
+// One overlapped generation (DESIGN.md 4.3) for a graph.  Side branch: k_update [-> the speculative pass of the next one
+// (spec)]; main branch: [the fitness from f_pinned ->] k_gate -> [k_cost ->] k_rank -> the sampler; joined at the end.
+// phase: k_update's UpdateArgs::phase (0: the whole update; 2: resume from the rows the last speculative pass left)
+int enqueue_forked(lmcma_b200_opt* o, cudaStream_t st, Fit fit, bool mirror, int phase = 0, bool spec = false) {
+    const OptDev& d = o->d;
+    UpdateArgs ua = update_args_local(o);
+    ua.progressive = 1;                                          // the overlapped generation is a progressive one (plan_launch)
+    ua.overlap = 1;
+    ua.phase = phase;
+    int rc;
+    if ((rc = fork_side(o, st)) || (rc = launch_update(o, ua, false, o->side_stream))) return rc;
+    if (spec) { UpdateArgs us = ua; us.phase = 1; us.dbg = nullptr; if ((rc = launch_update(o, us, false, o->side_stream))) return rc; }
+    if (fit == Fit::FROM_HOST) CU(cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st));
+    if ((rc = launch(k_gate, (d.B + 31) / 32, 32, 0, st, false, d))) return rc;   // until k_update has reset the flags and holds its SM
+    if (fit == Fit::COST && (rc = launch_own_cost(o, st))) return rc;
+    // the sampler is released when k_rank starts: the pairs it needs first are final (resume: at once; else as the sweep goes)
+    if ((rc = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, fit == Fit::COST))) return rc;
+    if ((rc = launch_sample(o, st, mirror, true, true, 2))) return rc;
+    return join_side(o, st);
+}
+
+// update() + sample() after the fitness of a generation is in d.fit.  INJECT without the next deviates stops after the
+// update: inject_z samples
+int generation_tail(lmcma_b200_opt* o, cudaStream_t st, bool mirror) {
+    const bool sample = o->cfg.rng != LMCMA_B200_RNG_INJECT || o->pending_z;
+    int rc = enqueue_linear(o, st, Fit::IN_PLACE, mirror, sample);
+    if (rc) return rc;
+    o->spec_valid = false;                                       // a whole update: whatever the speculative pass left is stale
+    if (!sample) o->needs_sample = true;
     o->pending_z = false;
-    return host_rng_and_sample(o, st, prog);
+    new_population(o, sample && mirror);
+    return 0;
 }
 
 // ---- CUDA graphs: built by capture(), replayed by replay(), freed by drop_fused_graphs / drop_tell_graphs ----
@@ -235,16 +293,21 @@ void drop_tell_graphs(lmcma_b200_opt* o) {
     drop_tell_graphs(o, o->tell_dev);
 }
 
+// while it lives, this thread's kernel launches are counted in *count instead of g_launches
+struct CountLaunchesIn {
+    explicit CountLaunchesIn(long long* count) { g_capture_launches = count; }
+    ~CountLaunchesIn() { g_capture_launches = nullptr; }
+};
+
 // Records what body() enqueues on `st` (and on the streams it forks from `st`) into *g, which is empty.  Capture enqueues
 // nothing: the kernels the body launches are counted in g->launches, and each replay adds them to g_launches.
 template <class Body>
 int capture(cudaStream_t st, Body&& body, Graph* g) {
     cudaGraph_t graph = nullptr;
     long long launches = 0;
+    CountLaunchesIn counted(&launches);
     CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    g_capture_launches = &launches;
     int rc = body();
-    g_capture_launches = nullptr;
     cudaError_t e = cudaStreamEndCapture(st, &graph);
     if (!rc && e == cudaSuccess) e = cudaGraphInstantiate(&g->exec, graph, 0);
     if (graph) cudaGraphDestroy(graph);
@@ -310,10 +373,10 @@ int probe_coschedule(lmcma_b200_opt* o) {
     cudaStream_t st = o->own_stream;
     if (cudaMalloc(&d, 4 * sizeof(int)) != cudaSuccess) { cudaGetLastError(); return 0; }
     bool ok = capture(st, [&] {
-        bool ok2 = cudaEventRecord(o->ev_fork, st) == cudaSuccess && cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) == cudaSuccess;
-        if (ok2) ok2 = launch(k_probe, 1, 1, 0, o->side_stream, false, d, d + 2, 0, 5000000ll) == 0 && cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess;
-        if (ok2) ok2 = launch(k_probe, 1, 1, 0, st, false, d, d + 2, 1, 5000000ll) == 0 && cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
-        return ok2 ? 0 : LMCMA_B200_ERR_CUDA;
+        int rc = fork_side(o, st);
+        if (!rc) rc = launch(k_probe, 1, 1, 0, o->side_stream, false, d, d + 2, 0, 5000000ll);
+        if (!rc) rc = launch(k_probe, 1, 1, 0, st, false, d, d + 2, 1, 5000000ll);
+        return rc ? rc : join_side(o, st);
     }, &probe) == 0;
     for (int attempt = 0; attempt < 2 && ok; ++attempt) {
         int h[4] = {0, 0, 0, 0};
@@ -340,7 +403,6 @@ int lmcma_capi::check_lost(lmcma_b200_opt* o) {
     o->props->cosched = 0;
     drop_fused_graphs(o);
     drop_tell_graphs(o);
-    o->tell_host.failed = o->tell_dev.failed = true;
     o->mirror_dirty = true;
     return fail(LMCMA_B200_ERR_CUDA, "overlapped generation lost co-scheduling (%s): the branches of the CUDA graph did not run "
                 "concurrently (profiler / sanitizer / SMs held elsewhere).  This handle now uses the linear graph; the generation in "
@@ -358,47 +420,23 @@ int lmcma_capi::settle_mirror(lmcma_b200_opt* o) {
 }
 namespace {
 
+// the fused graphs for o->stream, and the pair mirror their samplers read (a state setter since the last run made it dirty)
 int ensure_graph(lmcma_b200_opt* o) {
-    if (o->graph.exec && o->graph_built_for == o->stream) return 0;
-    drop_fused_graphs(o);
-    CostArgs ca;
-    int rc = cost_args_for(o, &ca);
-    if (rc) return rc;
     cudaStream_t st = o->stream;
-    if ((rc = ensure_mirror(o, st))) return rc;
+    int rc = ensure_mirror(o, st);
+    if (rc || (o->graph.exec && o->graph_built_for == st)) return rc;
+    drop_fused_graphs(o);
     // `reps` generations in ONE graph: between two graph launches the device idles for the launch latency of the next one
     // (~5 us of a 52 us generation); inside a graph a generation follows the previous one as a plain dependency
     auto body = [&](int reps) -> int {
-        UpdateArgs ua = update_args_local(o);
-        ua.progressive = o->plan.progressive ? 1 : 0;            // ensure_mirror above: the mirror is clean
         int rc2 = 0;
-        for (int g = 0; g < reps && !rc2; ++g) {
-            if (o->overlap) {
-                // side branch: k_update starts with the generation; main branch: k_gate (waits until k_update holds its SM) ->
-                // k_cost -> k_rank -> k_sample (released by k_rank, follows k_update's flags); join before the generation ends
-                ua.overlap = 1;
-                if (cudaEventRecord(o->ev_fork, st) != cudaSuccess || cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph fork failed");
-                if (!rc2) rc2 = launch_update(o, ua, false, o->side_stream);
-                if (!rc2 && cudaEventRecord(o->ev_join, o->side_stream) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph join record failed");
-                if (!rc2) rc2 = launch(k_gate, (o->d.B + 31) / 32, 32, 0, st, false, o->d);
-                if (!rc2) rc2 = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
-                if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, true);
-                if (!rc2) rc2 = launch_sample(o, st, true, true, 2);
-                if (!rc2 && cudaStreamWaitEvent(st, o->ev_join, 0) != cudaSuccess) rc2 = fail(LMCMA_B200_ERR_CUDA, "graph join failed");
-            } else {
-                rc2 = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
-                if (!rc2) rc2 = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st, true);
-                if (!rc2) rc2 = launch_update(o, ua, true, st);
-                if (!rc2) rc2 = launch_sample(o, st, true, o->plan.progressive);
-            }
-        }
+        for (int g = 0; g < reps && !rc2; ++g)
+            rc2 = o->overlap ? enqueue_forked(o, st, Fit::COST, false) : enqueue_linear(o, st, Fit::COST, false);
         return rc2;
     };
-    o->mirror_suppressed = true;                                 // fused generations keep the candidates on the device
     rc = capture(st, [&] { return body(1); }, &o->graph);
     if (!rc && o->tune.graph_unroll > 1 && capture(st, [&] { return body(o->tune.graph_unroll); }, &o->graph_multi) != 0)
         cudaGetLastError();                                      // optional: the single one still works
-    o->mirror_suppressed = false;
     if (rc && o->overlap) {
         // the forked graph could not be built here (capture / instantiation of the side branch): fall back to the linear one
         cudaGetLastError();
@@ -411,17 +449,19 @@ int ensure_graph(lmcma_b200_opt* o) {
     return 0;
 }
 
+// Does this tell replay a forked graph?  One query with the overlapped generation, unless its graphs could not be built here
+bool forked_tell(const lmcma_b200_opt* o, const TellGraphs& tg) { return o->overlap && !tg.failed && o->tune.tell_overlap != 0; }
+
 // The tell of one query as a forked graph (see lmcma_b200_tell_all).  dev: the graph of lmcma_b200_tell_all_dev, which
 // finds the fitness in d.fit already (no H2D node) and never writes the host mirror.  On failure the caller takes the
 // stream-ordered path.
 int ensure_tell_graph(lmcma_b200_opt* o, bool dev) {
     TellGraphs& tg = dev ? o->tell_dev : o->tell_host;
-    if (tg.whole.exec && tg.built_for == o->stream) return ensure_mirror(o, o->stream);
-    drop_tell_graphs(o, tg);
     cudaStream_t st = o->stream;
-    const OptDev& d = o->d;
     int rc = ensure_mirror(o, st);
-    if (rc) return rc;
+    if (rc || (tg.whole.exec && tg.built_for == st)) return rc;
+    drop_tell_graphs(o, tg);
+    const OptDev& d = o->d;
     if (!dev && !o->f_pinned && cudaHostAlloc(&o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaHostAllocDefault) != cudaSuccess) {
         cudaGetLastError(); o->f_pinned = nullptr; tg.failed = true; return 0;
     }
@@ -429,34 +469,10 @@ int ensure_tell_graph(lmcma_b200_opt* o, bool dev) {
     // (35 us behind the sampler).  Without the mirror tell_all returns when the sampler is done, and a 25 us kernel behind
     // k_update would be the longer branch of the graph (measured: tell_all 57 -> 69 us).  tell_all_dev: not even when it
     // is left running beside the caller's cost (DESIGN.md 4.4)
-    const bool spec = !dev && o->d_spec != nullptr && o->mirror_on && !o->mirror_suppressed;
-    tg.spec = spec;
-    // resume = 0: the whole update; resume = 1: k_update picks up the rows the last graph's speculative pass left.  With the
-    // scratch both graphs END with that pass for the next generation, on the side branch behind k_update
-    auto body = [&](int resume) -> int {
-        UpdateArgs ua = update_args_local(o);
-        ua.progressive = 1;
-        ua.overlap = 1;
-        ua.phase = resume ? 2 : 0;
-        const bool valid_before = o->spec_valid;
-        bool ok = cudaEventRecord(o->ev_fork, st) == cudaSuccess && cudaStreamWaitEvent(o->side_stream, o->ev_fork, 0) == cudaSuccess;
-        if (ok) ok = launch_update(o, ua, false, o->side_stream) == 0;
-        if (ok && spec) { UpdateArgs us = ua; us.phase = 1; us.dbg = nullptr; ok = launch_update(o, us, false, o->side_stream) == 0; }
-        o->spec_valid = valid_before;                            // capture enqueues nothing
-        if (ok) ok = cudaEventRecord(o->ev_join, o->side_stream) == cudaSuccess;
-        if (ok && !dev) ok = cudaMemcpyAsync(d.fit, o->f_pinned, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, st) == cudaSuccess;
-        if (ok) ok = launch(k_gate, (d.B + 31) / 32, 32, 0, st, false, d) == 0;   // k_update has reset the flags and holds its SM
-        // the sampler is released when k_rank starts: the pairs it needs first are final (resume: at once; else as the sweep goes)
-        if (ok) ok = launch_rank(o, d.fit, RANK_PLAIN | RANK_KEEP_FLAGS, nullptr, st, false) == 0;
-        if (ok) ok = launch_sample(o, st, true, true, 2) == 0;
-        if (ok) ok = cudaStreamWaitEvent(st, o->ev_join, 0) == cudaSuccess;
-        return ok ? 0 : LMCMA_B200_ERR_CUDA;
-    };
-    const bool suppressed = o->mirror_suppressed;
-    if (dev) o->mirror_suppressed = true;                        // the device protocol keeps the candidates on the device
-    rc = capture(st, [&] { return body(0); }, &tg.whole);
-    if (!rc && spec) rc = capture(st, [&] { return body(1); }, &tg.resume);
-    o->mirror_suppressed = suppressed;
+    tg.spec = !dev && o->d_spec != nullptr && o->x_mirror != nullptr;
+    const Fit fit = dev ? Fit::IN_PLACE : Fit::FROM_HOST;
+    rc = capture(st, [&] { return enqueue_forked(o, st, fit, !dev, 0, tg.spec); }, &tg.whole);
+    if (!rc && tg.spec) rc = capture(st, [&] { return enqueue_forked(o, st, fit, !dev, 2, tg.spec); }, &tg.resume);
     if (rc) {
         cudaGetLastError();
         drop_tell_graphs(o, tg);
@@ -655,9 +671,10 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     // first population (LMCMA::init -> sample(), lmcma.cpp:298)
     if (cfg->rng == LMCMA_B200_RNG_INJECT) o->needs_sample = true;
     else {
-        rc = host_rng_and_sample(o, o->stream);
+        rc = host_rng_and_sample(o, o->stream, true);
         if (!rc) { cudaError_t e = cudaStreamSynchronize(o->stream); if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "first sample: %s", cudaGetErrorString(e)); }
         if (rc) return rc;
+        new_population(o, true);
     }
     return 0;
 }
@@ -710,8 +727,9 @@ int lmcma_b200_inject_z(lmcma_b200_opt* o, const float* Z) {
     if (rc) return rc;
     if (o->needs_sample) {
         o->needs_sample = false;
-        rc = launch_sample(o, o->stream);
+        rc = launch_sample(o, o->stream, true);
         if (rc) return rc;
+        new_population(o, true);
         CU(cudaStreamSynchronize(o->stream));
     } else {
         o->pending_z = true;
@@ -724,10 +742,10 @@ int lmcma_b200_resample(lmcma_b200_opt* o) {
     if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no deviates yet: inject_z first");
     if (o->cfg.rng == LMCMA_B200_RNG_HANSEN) return fail(LMCMA_B200_ERR_STATE, "resample would advance the serial HANSEN stream");
     CU(cudaSetDevice(o->cfg.device));
-    int rc = launch_sample(o, o->stream);
+    int rc = launch_sample(o, o->stream, true);
     if (rc) return rc;
+    new_population(o, true);
     CU(cudaStreamSynchronize(o->stream));
-    o->x_cache_valid = false;
     return 0;
 }
 
@@ -751,8 +769,6 @@ int lmcma_b200_ask_all_view(lmcma_b200_opt* o, const float** X_view, int64_t* ld
         CU(cudaHostAlloc(&o->x_mirror, floats * sizeof(float), cudaHostAllocMapped));
         cudaError_t e = cudaHostGetDevicePointer(&d.Xh, o->x_mirror, 0);
         if (e != cudaSuccess) { cudaFreeHost(o->x_mirror); o->x_mirror = nullptr; d.Xh = nullptr; return fail(LMCMA_B200_ERR_CUDA, "cudaHostGetDevicePointer: %s", cudaGetErrorString(e)); }
-        o->mirror_on = true;
-        o->xh_fresh = false;
         register_mirror(o->x_mirror, floats * sizeof(float), d.X, d.ns, o->cfg.device);
         // the captured graphs carry the old kernel parameters (OptDev by value): rebuild them on next use
         drop_tell_graphs(o);
@@ -776,7 +792,7 @@ int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     int rc;
-    if (o->overlap && !o->tell_host.failed && o->tune.tell_overlap != 0) {
+    if (forked_tell(o, o->tell_host)) {
         // One query (the conditions of the overlapped generation, DESIGN.md 4.3): everything in update() that does not
         // depend on this generation's fitness — slot bookkeeping, the sweep over every pending row but the newest — runs on
         // a side branch while the fitness crosses PCIe and k_rank runs; k_update then waits for k_rank's tickets and
@@ -788,18 +804,14 @@ int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
             const bool resume = o->spec_valid && o->tell_host.resume.exec;   // the last tell left the next update's rows behind
             if ((rc = replay(resume ? o->tell_host.resume : o->tell_host.whole, o->stream))) return rc;
             o->spec_valid = o->tell_host.spec;                    // ... and so does this one
-            o->xh_fresh = o->mirror_on;                          // the captured sampler writes the host mirror when it is on
-            o->x_cache_valid = false;
-            o->sample_idx = 0;
-            o->pending_z = false;
+            new_population(o, true);
             CU(cudaStreamSynchronize(o->stream));
             return check_lost(o);
         }
         if (rc) return rc;
     }
     CU(cudaMemcpyAsync(d.fit, f, (size_t)d.B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, o->stream));
-    rc = generation_tail(o, o->stream);
-    if (rc) return rc;
+    if ((rc = generation_tail(o, o->stream, true))) return rc;
     CU(cudaStreamSynchronize(o->stream));
     return 0;
 }
@@ -820,29 +832,22 @@ int lmcma_b200_tell_all_dev(lmcma_b200_opt* o) {
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     CU(cudaStreamIsCapturing(o->stream, &cs));
     int rc = 0;
-    o->mirror_suppressed = true;                                 // the candidates stay on the device
     if (cs != cudaStreamCaptureStatusNone) {
         // the caller's capture: no library graph is replayed or built, nothing allocated or synchronised.  The linear
         // generation (same bits as the forked one) keeps kernels that spin on a partner out of a graph the library does not
         // control.  Its kernels are counted by nobody: they run when the caller replays the graph
         long long uncounted = 0;
-        g_capture_launches = &uncounted;
-        rc = generation_tail(o, o->stream);
-        g_capture_launches = nullptr;
+        CountLaunchesIn counted(&uncounted);
+        rc = generation_tail(o, o->stream, false);
         o->caller_graphs = true;
-    } else if (o->overlap && !o->tell_dev.failed && o->tune.tell_overlap != 0 && (rc = ensure_tell_graph(o, true)) == 0 &&
-               o->tell_dev.whole.exec) {
+    } else if (forked_tell(o, o->tell_dev) && (rc = ensure_tell_graph(o, true)) == 0 && o->tell_dev.whole.exec) {
         // one query: the forked graph of tell_all without the fitness copy (and without the speculative pass, DESIGN.md 4.4)
         rc = replay(o->tell_dev.whole, o->stream);
         o->spec_valid = false;
+        new_population(o, false);
     } else if (!rc) {
-        rc = generation_tail(o, o->stream);
+        rc = generation_tail(o, o->stream, false);
     }
-    o->mirror_suppressed = false;
-    o->x_cache_valid = false;
-    o->sample_idx = 0;
-    o->xh_fresh = false;
-    o->pending_z = false;
     return rc;
 }
 
@@ -915,7 +920,6 @@ int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
     o->spec_valid = false;                                       // the fused generations advance the state past what tell_all's speculative pass saw
     if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) {
         if ((rc = ensure_graph(o))) return rc;
-        if ((rc = ensure_mirror(o, o->stream))) return rc;       // a state setter since the last run: the graph's sampler reads the mirror
         CU(cudaEventRecord(o->ev0, o->stream));                  // after the (host-side) graph build: last_run_ms is device time
         const int unroll = o->graph_multi.exec ? o->tune.graph_unroll : 0;
         for (int g = 0; g < generations;) {
@@ -923,21 +927,16 @@ int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
             if ((rc = replay(multi ? o->graph_multi : o->graph, o->stream))) return rc;
             g += multi ? unroll : 1;
         }
+        if (generations > 0) new_population(o, false);           // the graph's sampler does not write the host mirror
     } else {
         if (o->cfg.rng == LMCMA_B200_RNG_INJECT && generations > 1)
             return fail(LMCMA_B200_ERR_STATE, "INJECT rng: run one generation per injected Z");
-        CostArgs ca;
-        if ((rc = cost_args_for(o, &ca))) return rc;
         CU(cudaEventRecord(o->ev0, o->stream));
-        for (int g = 0; g < generations; ++g) {
-            if ((rc = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, o->stream))) return rc;
-            if ((rc = generation_tail(o, o->stream))) return rc;
-        }
+        for (int g = 0; g < generations; ++g)
+            if ((rc = launch_own_cost(o, o->stream)) || (rc = generation_tail(o, o->stream, true))) return rc;
     }
     CU(cudaEventRecord(o->ev1, o->stream));
     o->have_run_timing = true;
-    o->x_cache_valid = false;
-    if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) o->xh_fresh = false;    // the graph's sampler does not write the host mirror
     return 0;
 }
 
@@ -977,9 +976,11 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
         cudaEventRecord(e[2], st);
         if (!rc) rc = launch_update(o, update_args_local(o), false, st);   // serialised here so that the events separate the kernels
         cudaEventRecord(e[3], st);
-        if (!rc) rc = launch_sample(o, st);
+        if (!rc) rc = launch_sample(o, st, true);
         cudaEventRecord(e[4], st);
     }
+    o->spec_valid = false;
+    new_population(o, true);
     cudaError_t se = cudaStreamSynchronize(st);
     if (!rc && se != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "profile run: %s", cudaGetErrorString(se));
     if (!rc && o->d.dbg) rc = print_timeline(o);
@@ -1025,7 +1026,6 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
                 ms4[k] += ms / generations;
             }
     for (auto& e : ev) cudaEventDestroy(e);
-    o->x_cache_valid = false;
     return rc;
 }
 
@@ -1108,11 +1108,9 @@ int lmcma_b200_mg_update(lmcma_b200_opt* o, const float* payload_all_dev, int32_
     a.f_all = o->d.fit; a.slices = payload_all_dev; a.n_slices = world;
     a.slice_stride = (long long)o->d.B * pf; a.inst_stride = pf; a.payload_mode = 1;
     int rc = launch_update(o, a, false, st);
-    if (rc) return rc;
-    o->x_cache_valid = false;
-    o->mirror_suppressed = true;
-    rc = launch_sample(o, st, true);
-    o->mirror_suppressed = false;
+    if (!rc) rc = launch_sample(o, st, false, true);
+    o->spec_valid = false;
+    new_population(o, false);
     return rc;
 }
 

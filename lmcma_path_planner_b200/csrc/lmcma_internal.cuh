@@ -186,9 +186,7 @@ struct lmcma_b200_opt {
     lmcma_capi::Graph graph;                  // one fused generation (lmcma_b200_run)
     lmcma_capi::Graph graph_multi;            // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)
     cudaStream_t graph_built_for = nullptr;
-    // tell of one query: [H2D fitness ->] k_gate -> k_rank -> k_sample, k_update on a side branch.  tell_host: tell_all;
-    // tell_dev: tell_all_dev (the fitness is in d.fit already, the host mirror is not written)
-    lmcma_capi::TellGraphs tell_host, tell_dev;
+    lmcma_capi::TellGraphs tell_host, tell_dev;  // the forked tell graphs of tell_all and of tell_all_dev (ensure_tell_graph)
     // lmcma_b200_tell_all_dev recorded generations into a caller's stream capture.  Their replays advance the state without
     // this library seeing them, so from then on no host-side record of the population is trusted (ask_all_view copies,
     // ask_one reloads) and a state setter rebuilds the pair mirror at once instead of at the next library launch
@@ -211,7 +209,7 @@ struct lmcma_b200_opt {
     cudaStream_t side_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     float* x_mirror = nullptr;        // page-locked, mapped host mirror of X (lmcma_b200_ask_all_view); OptDev::Xh is its device alias
-    bool mirror_on = false, mirror_suppressed = false, xh_fresh = false;
+    bool xh_fresh = false;            // x_mirror holds the population (the last sampler wrote it)
     int* err_host = nullptr;          // page-locked, mapped: OptDev::err (a kernel of the overlapped generation gave up on its partner)
 };
 
