@@ -223,6 +223,36 @@ int lmcma_b200_device_buffers(lmcma_b200_opt* opt, const float** X_dev, int64_t*
  * LMCMA_B200_ERR_STATE: rng != PHILOX, a split-population handle. */
 int lmcma_b200_tell_all_dev(lmcma_b200_opt* opt);
 
+/* Restart chosen instances of a live batch in place, for a planning service or a restart policy whose queries finish at
+ * different times.  Each reset instance gets exactly what lmcma_b200_create leaves for a start x0 and step size sigma0 (mean
+ * x0, every path, direction pair, slot, fitness and best-so-far cleared, itr = counteval = 0), with its deviate stream moved
+ * on by one epoch (LMCMA_B200_I32_EPOCH), so a restart from the same start does not repeat the earlier run; then its first
+ * population is drawn.  The other instances, the handle's CUDA graphs and its kernel configuration are untouched: the
+ * next run / tell replays the graphs it has.  The cost's launch shape stays what attach_cost chose from the end points
+ * of instance 0; it only sizes k_cost's launch, so longer trajectories of reset instances take more rounds and stay
+ * correct.
+ *
+ * Host: synchronous.  idx: count distinct instance indices; x0: count x n; sigma0: count, or NULL for cfg.sigma0; ends:
+ * count new end-point pairs, or NULL to keep them (needs an attached cost).  count == 0 does nothing.  The flagged rows of
+ * the host mirror (ask_all_view) are rewritten, so the mirror stays as current as it was.
+ * LMCMA_B200_ERR_ARG: an index out of range or repeated, a null idx / x0, a non-finite x0, a sigma0 not finite or <= 0,
+ * count < 0.  LMCMA_B200_ERR_STATE: rng HANSEN or INJECT, a split-population handle, ends without an attached cost.  A
+ * refused call changes nothing. */
+int lmcma_b200_reset_instances(lmcma_b200_opt* opt, int32_t count, const int32_t* idx, const double* x0,
+                               const double* sigma0, const lmcma_b200_endpoints* ends);
+/* Device: the same reset from flags the caller computed on the device.  flags_dev: batch int32, non-zero = reset;
+ * x0_dev: batch x n FP64 dense (rows of unflagged instances are not read); sigma0_dev: batch FP64 or NULL (cfg.sigma0);
+ * ends_dev: batch x 6 FP32 {start xyz, goal xyz} or NULL (keep); best_x_out_dev: batch x n FP32 and best_f_out_dev: batch
+ * FP64, or NULL: the retiring instance's best_x and best_f (as stored) before the reset, written for flagged rows only.
+ * Enqueued on the handle's stream (as lmcma_b200_tell_all_dev, set_stream with the stream the flags are computed on);
+ * never waits and allocates nothing.  Capturable: under the caller's stream capture it records into that capture, and its
+ * kernels are not counted by lmcma_b200_launch_count.  The inputs are trusted as tell_all_dev trusts f_dev: values are not
+ * checked (sigma0 > 0, finite x0 are the caller's part).  The host mirror is stale afterwards (ask_all_view copies).
+ * LMCMA_B200_ERR_ARG: a null flags_dev / x0_dev.  LMCMA_B200_ERR_STATE: as the host variant. */
+int lmcma_b200_reset_instances_dev(lmcma_b200_opt* opt, const int32_t* flags_dev, const double* x0_dev,
+                                   const double* sigma0_dev, const float* ends_dev, float* best_x_out_dev,
+                                   double* best_f_out_dev);
+
 /* deviates for the NEXT sample(): batch x pop_count x n FP32 (rng == INJECT).  The first call after
  * create builds the first population immediately; later calls are consumed by the next tell. */
 int lmcma_b200_inject_z(lmcma_b200_opt* opt, const float* Z_host);
@@ -294,8 +324,11 @@ enum {
     LMCMA_B200_I32_COUNTEVAL = 6,  /* batch       (CMABase::counteval) */
     LMCMA_B200_I32_NCOLL = 7,      /* batch x pop_count colliding samples of the last evaluated population */
     LMCMA_B200_I32_NSAMP = 8,      /* batch x pop_count map samples of the last evaluated population */
-    LMCMA_B200_I32_LAUNCH = 9      /* LMCMA_B200_LAUNCH_FIELDS values per HANDLE (not per instance), read-only: the launch
+    LMCMA_B200_I32_LAUNCH = 9,     /* LMCMA_B200_LAUNCH_FIELDS values per HANDLE (not per instance), read-only: the launch
                                       configuration chosen at create, indexed by LMCMA_B200_LAUNCH_* below */
+    LMCMA_B200_I32_EPOCH = 10      /* batch       deviate stream of the instance: 0 at create, + 1 per reset_instances.  The
+                                      PHILOX key is (lo32(seed), hi32(seed) + epoch) mod 2^32, so seed s at epoch e draws what
+                                      seed s + e 2^32 draws at epoch 0.  A checkpoint that restores ITR restores this too */
 };
 /* fields of LMCMA_B200_I32_LAUNCH.  Sampler kernels: 0 = k_sample<NV> (narrow), 1 = k_sample_wide<RBW> (a row split over CW
  * column-warps, R row groups per CTA), 2 = k_sample_rows<QW, RL> (rows on lanes).  KC / STAGES are those of the chosen
@@ -318,7 +351,7 @@ int lmcma_b200_get_f64(lmcma_b200_opt* opt, int32_t which, double* out, int64_t 
 int lmcma_b200_get_f32(lmcma_b200_opt* opt, int32_t which, float* out, int64_t capacity);
 int lmcma_b200_get_i32(lmcma_b200_opt* opt, int32_t which, int32_t* out, int64_t capacity);
 /* teacher forcing: overwrite optimiser state (same `which` / layouts as the getters; XMEAN, SIGMA, S,
- * NJ, LJ | PC, V, P, PREV_FIT | T, VEC, ITR, LIVE are settable) */
+ * NJ, LJ | PC, V, P, PREV_FIT | T, VEC, ITR, LIVE, EPOCH are settable) */
 int lmcma_b200_set_f64(lmcma_b200_opt* opt, int32_t which, const double* in, int64_t count);
 int lmcma_b200_set_f32(lmcma_b200_opt* opt, int32_t which, const float* in, int64_t count);
 int lmcma_b200_set_i32(lmcma_b200_opt* opt, int32_t which, const int32_t* in, int64_t count);

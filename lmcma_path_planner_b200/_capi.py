@@ -14,7 +14,7 @@ MAP_F32, MAP_U8 = 0, 1
 
 F64 = {"xmean": 0, "sigma": 1, "s": 2, "best_f": 3, "consts": 4, "weights": 5, "Nj": 6, "Lj": 7}
 F32 = {"X": 0, "pc": 1, "V": 2, "P": 3, "fit": 4, "fit_sorted": 5, "prev_fit": 6, "Z": 7}
-I32 = {"t": 0, "vec": 1, "arindex": 2, "rank": 3, "itr": 4, "live": 5, "counteval": 6, "ncoll": 7, "nsamp": 8}
+I32 = {"t": 0, "vec": 1, "arindex": 2, "rank": 3, "itr": 4, "live": 5, "counteval": 6, "ncoll": 7, "nsamp": 8, "epoch": 10}
 I32_LAUNCH = 9
 # the fields of LMCMA_B200_I32_LAUNCH in order (LMCMA_B200_LAUNCH_*)
 LAUNCH_FIELDS = ("sampler", "smp_nv", "smp_spec", "smp_threads", "smp_RBW", "smp_CW", "smp_R", "smp_rows_qw", "smp_rows_rl",
@@ -80,6 +80,8 @@ SIGNATURES = {
     "lmcma_b200_ask_all_view": (C.c_int, [_vp, C.POINTER(_pf), _pl]),
     "lmcma_b200_device_buffers": (C.c_int, [_vp, C.POINTER(_vp), _pl, C.POINTER(_vp)]),
     "lmcma_b200_tell_all_dev": (C.c_int, [_vp]),
+    "lmcma_b200_reset_instances": (C.c_int, [_vp, _i32, _pi, _pd, _pd, C.POINTER(Endpoints)]),
+    "lmcma_b200_reset_instances_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "lmcma_b200_inject_z": (C.c_int, [_vp, _pf]),
     "lmcma_b200_resample": (C.c_int, [_vp]),
     "lmcma_b200_is_done": (C.c_int, [_vp, _pi]),

@@ -10,14 +10,14 @@ namespace lmcma {
 
 // Z <- N(0,1), the samplers' deviates (philox_deviate4): grid = (ceil(nq / 128) x pop_count, 1, B), the column tile
 // fastest.  The rows share grid x with the column tiles, in the order a (tiles, rows) grid would launch them: pop_count
-// reaches 65 536, past the 65 535 that y and z take
+// reaches 65 536, past the 65 535 that y and z take.  With OptDev::only, the instances it does not flag keep their Z.
 __global__ void __launch_bounds__(128) k_gauss(OptDev o) {
     const int nq = o.ns >> 2, tiles = (nq + 127) >> 7;
     const int row = blockIdx.x / tiles, q = (blockIdx.x - row * tiles) * 128 + threadIdx.x, b = blockIdx.z;
-    if (q >= nq) return;
-    const int itr = o.sc[b].itr;
+    if (q >= nq || (o.only && o.only[b] == 0)) return;
+    const int itr = o.sc[b].itr, epoch = o.sc[b].epoch;
     float4 v;
-    philox_deviate4(o, b, row, q, itr, v);
+    philox_deviate4(o, b, row, q, itr, epoch, v);
     reinterpret_cast<float4*>(o.Z + ((size_t)b * o.pop_count + row) * o.ns)[q] = v;
 }
 

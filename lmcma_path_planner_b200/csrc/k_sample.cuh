@@ -44,11 +44,11 @@ __device__ __forceinline__ float reduce_scatter8(const float (&v)[SAMPLE_G], int
 
 // The deviate v of float4 column q of local row `row` of instance b, whose offset in Z / Zc is roff: the prior's L z
 // (k_prior has formed it), the generator's (recorded into Z when Z is kept), or the injected Z.
-__device__ __forceinline__ void sample_deviate4(const OptDev& o, int b, int row, size_t roff, int q, int itr, float4& v) {
+__device__ __forceinline__ void sample_deviate4(const OptDev& o, int b, int row, size_t roff, int q, int itr, int epoch, float4& v) {
     if (o.Zc) {
         v = reinterpret_cast<const float4*>(o.Zc + roff)[q];
     } else if (o.rng_mode == 0) {
-        philox_deviate4(o, b, row, q, itr, v);
+        philox_deviate4(o, b, row, q, itr, epoch, v);
         if (o.Z) reinterpret_cast<float4*>(o.Z + roff)[q] = v;
     } else {
         v = reinterpret_cast<const float4*>(o.Z + roff)[q];
@@ -110,6 +110,7 @@ template <int NV, int RB, int MAXT, bool SPEC = false>
 __global__ void __launch_bounds__(MAXT) k_sample(OptDev o, int kc /* pairs per stage, multiple of 8 */, int nstages) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int b = blockIdx.y;
+    if (o.only && o.only[b] == 0) return;                     // an instance the reset leaves alone (OptDev::only)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int ns = o.ns, nq = ns >> 2;
     float* stage_base = reinterpret_cast<float*>(smem_raw);
@@ -142,7 +143,7 @@ __global__ void __launch_bounds__(MAXT) k_sample(OptDev o, int kc /* pairs per s
         for (int i = 0; i < NV; ++i) {
             const int q = lane + 32 * i;
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (rv && q < nq) sample_deviate4(o, b, row, roff, q, sc.itr, v);
+            if (rv && q < nq) sample_deviate4(o, b, row, roff, q, sc.itr, sc.epoch, v);
             z[r][i] = v;
             az[r][i] = v;
         }
@@ -273,9 +274,10 @@ template <int RBW, int MAXT>
 __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nstages, int R, int CW, int qpw /* float4 columns per warp */,
                                                        int progressive) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int b = blockIdx.y;
+    if (o.only && o.only[b] == 0) return;                       // an instance the reset leaves alone (OptDev::only)
 #define SMP_STAMP(k) do { if (o.dbg && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) o.dbg[k] = gtime(); } while (0)
     SMP_STAMP(TL_SMP_START);
-    const int b = blockIdx.y;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int rl = warp / CW, cw = warp - rl * CW;              // row-group within the CTA, column-warp within the row
     const int ns = o.ns, nq = ns >> 2;
@@ -396,7 +398,7 @@ __global__ void __launch_bounds__(MAXT) k_sample_wide(OptDev o, int kc, int nsta
         const bool on = qon && row < o.pop_count;
         const size_t roff = ((size_t)b * o.pop_count + (row < o.pop_count ? row : 0)) * ns;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (on) sample_deviate4(o, b, row, roff, q, sc.itr, v);
+        if (on) sample_deviate4(o, b, row, roff, q, sc.itr, sc.epoch, v);
         z[r] = v; az[r] = v;
     }
     SMP_STAMP(TL_SMP_Z);
@@ -532,6 +534,7 @@ template <int QW, int RL>
 __global__ void __launch_bounds__(512, 1) k_sample_rows(OptDev o, int kc, int nstages, int region_floats /* >= stages, >= transposition tile */) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int b = blockIdx.y;
+    if (o.only && o.only[b] == 0) return;                     // an instance the reset leaves alone (OptDev::only)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5, nthr = blockDim.x;
     const int ns = o.ns, nq = ns >> 2, m = o.m;
     constexpr int ROWS = 32 * RL;
@@ -578,7 +581,7 @@ __global__ void __launch_bounds__(512, 1) k_sample_rows(OptDev o, int kc, int ns
         for (int i = 0; i < QW; ++i) {
             const int q = q0 + i;
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (rv && i < qper && q < nq) sample_deviate4(o, b, row, roff, q, sc.itr, v);
+            if (rv && i < qper && q < nq) sample_deviate4(o, b, row, roff, q, sc.itr, sc.epoch, v);
             acc[r][i] = v;
         }
     }

@@ -9,6 +9,7 @@
 #include "k_update.cuh"
 #include "k_prior.cuh"
 #include "k_gram.cuh"
+#include "k_reset.cuh"
 
 using namespace lmcma;
 using namespace lmcma_capi;
@@ -78,18 +79,21 @@ int ensure_mirror(lmcma_b200_opt* o, cudaStream_t st) {
 // generations (lmcma_b200_run), the device-resident tell and the split-population stages keep the candidates on the device
 // pdl: launched as a programmatic dependent of the kernel enqueued just before it on `st` (k_update)
 // progressive: that k_update was launched with UpdateArgs::progressive (only meaningful with pdl)
-int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool mirror, bool pdl = false, bool progressive = false, int progressive_mode = 1) {
+// only: OptDev::only, the instances to draw (the plain launch of lmcma_b200_reset_instances), or null for all of them
+int launch_sample(lmcma_b200_opt* o, cudaStream_t st, bool mirror, bool pdl = false, bool progressive = false, int progressive_mode = 1,
+                  const int* only = nullptr) {
     if (o->mirror_dirty) { int rc = ensure_mirror(o, st); if (rc) return rc; pdl = false; }
+    OptDev d = o->d;
+    d.only = only;
     if (o->d_Lf) {   // smoothness prior: z <- L z for the whole population before computeAz (lmcma.cpp:216-217)
-        const OptDev& d = o->d;
         int rc = 0;
         if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) rc = launch(k_gauss, dim3((d.ns / 4 + 127) / 128 * d.pop_count, 1, d.B), 128, 0, st, false, d);
+        // every row: an instance k_gauss skipped still holds this generation's deviates in Z, so its Zc comes out unchanged
         const int rows = d.B * d.pop_count;
         if (!rc) rc = launch(k_prior, dim3((d.ns + 63) / 64 * ((rows + 63) / 64)), 256, 0, st, false, d.Z, o->d_Lf, d.Zc, rows, d.n, d.ns);
         if (rc) return rc;
         pdl = false;
     }
-    OptDev d = o->d;
     if (!mirror) d.Xh = nullptr;
     if (o->plan.sample.kind == Sampler::ROWS) return launch_sample_rows(o, d, pdl, st);
     if (o->plan.sample.kind == Sampler::WIDE)
@@ -201,6 +205,23 @@ void new_population(lmcma_b200_opt* o, bool mirror) {
     o->x_cache_valid = false;
     o->sample_idx = 0;
     o->xh_fresh = mirror && o->x_mirror;
+}
+
+// lmcma_b200_reset_instances(_dev): k_reset, then the sampler for the flagged instances only, a plain launch (the
+// generation's PDL and hand-over pair a sampler with the k_update before it).  mirror: the sampler writes the flagged rows
+// of the host mirror, so the mirror is as fresh as it was; without it the mirror is stale.  No graph is dropped: the
+// captured ones read the state, the end points and the flags through pointers.
+int enqueue_reset(lmcma_b200_opt* o, cudaStream_t st, ResetArgs a, bool mirror) {
+    a.sigma_default = o->cfg.sigma0;
+    a.d_ends = o->d_ends;
+    int rc = launch(k_reset, o->d.B, 256, 0, st, false, o->d, a);
+    if (!rc) rc = launch_sample(o, st, mirror, false, false, 1, a.flags);
+    if (rc) return rc;
+    o->spec_valid = false;                                       // the speculative pass saw the retired instances
+    o->x_cache_valid = false;
+    o->sample_idx = 0;
+    o->xh_fresh = o->xh_fresh && mirror;
+    return 0;
 }
 
 // where a generation's fitness comes from: k_cost on the attached map, a copy from f_pinned, or d.fit as it is
@@ -685,7 +706,7 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     if (o->stream) cudaStreamSynchronize(o->stream);
     OptDev& d = o->d;
     void* ptrs[] = {d.prev_sorted, d.tile_sorted, d.tile_pos, d.X, d.D, d.Z, d.Zc, o->d_Lf, d.fit, d.fit_sorted, d.prev_fit, d.rank, d.arindex, d.ncoll, d.nsamp, d.xmean, d.pc, d.V, d.P,
-                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore};
+                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore, o->d_reset};
     for (void* p : ptrs) cudaFree(p);
     drop_fused_graphs(o);
     drop_tell_graphs(o);
@@ -848,6 +869,101 @@ int lmcma_b200_tell_all_dev(lmcma_b200_opt* o) {
     } else if (!rc) {
         rc = generation_tail(o, o->stream, false);
     }
+    return rc;
+}
+
+// what lmcma_b200_reset_instances(_dev) refuses with ERR_STATE: HANSEN / INJECT draw their deviates on the host, a split
+// population's best and slots live on several handles, and end points need the device end points of an attached cost
+static int reset_refused(const lmcma_b200_opt* o, bool ends) {
+    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "reset_instances needs the PHILOX rng");
+    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "reset_instances: split-population handles are not supported");
+    if (ends && !o->d_ends) return fail(LMCMA_B200_ERR_STATE, "reset_instances: end points need an attached cost (lmcma_b200_attach_cost)");
+    return 0;
+}
+
+// o->d_reset: sigma0 (B doubles), x0 (B x n doubles), ends (B x 6 floats), flags (B ints), each at a 16-byte boundary
+struct ResetLayout { size_t sigma0, x0, ends, flags, bytes; };
+static ResetLayout reset_layout(const OptDev& d) {
+    auto up = [](size_t v) { return (v + 15) & ~(size_t)15; };
+    ResetLayout l;
+    l.sigma0 = 0;
+    l.x0 = up(l.sigma0 + (size_t)d.B * sizeof(double));
+    l.ends = up(l.x0 + (size_t)d.B * d.n * sizeof(double));
+    l.flags = up(l.ends + (size_t)d.B * 6 * sizeof(float));
+    l.bytes = l.flags + (size_t)d.B * sizeof(int);
+    return l;
+}
+
+int lmcma_b200_reset_instances(lmcma_b200_opt* o, int32_t count, const int32_t* idx, const double* x0, const double* sigma0,
+                               const lmcma_b200_endpoints* ends) {
+    ARG(o, "null handle");
+    int rc = reset_refused(o, ends != nullptr);
+    if (rc) return rc;
+    ARG(count >= 0, "count must be >= 0");
+    if (count == 0) return 0;
+    ARG(idx && x0, "null pointer");
+    const OptDev& d = o->d;
+    const int n = d.n;
+    std::vector<int> flags(d.B, 0);
+    int lo = d.B, hi = -1;                                       // the rows the call touches: [lo, hi]
+    for (int i = 0; i < count; ++i) {
+        ARG(idx[i] >= 0 && idx[i] < d.B, "instance index out of range");
+        ARG(flags[idx[i]] == 0, "instance index repeated");
+        flags[idx[i]] = 1;
+        lo = std::min(lo, idx[i]);
+        hi = std::max(hi, idx[i]);
+        ARG(!sigma0 || (std::isfinite(sigma0[i]) && sigma0[i] > 0.0), "sigma0 must be finite and > 0");
+        for (int k = 0; k < n; ++k) ARG(std::isfinite(x0[(size_t)i * n + k]), "x0 must be finite");
+    }
+    CU(cudaSetDevice(o->cfg.device));
+    const ResetLayout l = reset_layout(d);
+    if (!o->d_reset) DM(o->d_reset, l.bytes);
+    // only rows [lo, hi] of x0, sigma0 and the end points cross PCIe; the flags of every instance do
+    const size_t rows = (size_t)(hi - lo + 1);
+    std::vector<double> xs(rows * n), ss(rows, o->cfg.sigma0);
+    std::vector<float> es(ends ? rows * 6 : 0);
+    for (int i = 0; i < count; ++i) {
+        const size_t r = (size_t)(idx[i] - lo);
+        std::copy(x0 + (size_t)i * n, x0 + (size_t)(i + 1) * n, xs.begin() + r * n);
+        if (sigma0) ss[r] = sigma0[i];
+        if (ends)
+            for (int c = 0; c < 3; ++c) { es[r * 6 + c] = ends[i].start[c]; es[r * 6 + 3 + c] = ends[i].goal[c]; }
+    }
+    ResetArgs a;
+    memset(&a, 0, sizeof(a));
+    a.flags = reinterpret_cast<const int*>(o->d_reset + l.flags);
+    a.x0 = reinterpret_cast<const double*>(o->d_reset + l.x0);
+    a.sigma0 = reinterpret_cast<const double*>(o->d_reset + l.sigma0);
+    a.ends = ends ? reinterpret_cast<const float*>(o->d_reset + l.ends) : nullptr;
+    cudaStream_t st = o->stream;
+    CU(cudaMemcpyAsync(o->d_reset + l.flags, flags.data(), flags.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(o->d_reset + l.x0 + (size_t)lo * n * sizeof(double), xs.data(), xs.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(o->d_reset + l.sigma0 + (size_t)lo * sizeof(double), ss.data(), ss.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (ends) CU(cudaMemcpyAsync(o->d_reset + l.ends + (size_t)lo * 6 * sizeof(float), es.data(), es.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    if ((rc = enqueue_reset(o, st, a, true))) return rc;
+    CU(cudaStreamSynchronize(st));                               // the staging vectors are pageable
+    return check_lost(o);
+}
+
+int lmcma_b200_reset_instances_dev(lmcma_b200_opt* o, const int32_t* flags_dev, const double* x0_dev, const double* sigma0_dev,
+                                   const float* ends_dev, float* best_x_out_dev, double* best_f_out_dev) {
+    ARG(o, "null handle");
+    int rc = reset_refused(o, ends_dev != nullptr);
+    if (rc) return rc;
+    ARG(flags_dev && x0_dev, "null pointer");
+    CU(cudaSetDevice(o->cfg.device));
+    ResetArgs a;
+    memset(&a, 0, sizeof(a));
+    a.flags = flags_dev; a.x0 = x0_dev; a.sigma0 = sigma0_dev; a.ends = ends_dev;
+    a.best_x_out = best_x_out_dev; a.best_f_out = best_f_out_dev;
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    CU(cudaStreamIsCapturing(o->stream, &cs));
+    if (cs == cudaStreamCaptureStatusNone) return enqueue_reset(o, o->stream, a, false);
+    // the caller's capture, as in lmcma_b200_tell_all_dev: its kernels run, uncounted, when the caller replays the graph
+    long long uncounted = 0;
+    CountLaunchesIn counted(&uncounted);
+    rc = enqueue_reset(o, o->stream, a, false);
+    o->caller_graphs = true;
     return rc;
 }
 

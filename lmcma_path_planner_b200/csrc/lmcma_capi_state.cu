@@ -87,13 +87,14 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
         case LMCMA_B200_I32_RANK: src = d.rank; cnt = B * d.lambda; break;
         case LMCMA_B200_I32_NCOLL: src = d.ncoll; cnt = B * d.pop_count; break;
         case LMCMA_B200_I32_NSAMP: src = d.nsamp; cnt = B * d.pop_count; break;
-        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: {
+        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH: {
             ARG(cap >= (int64_t)B, "capacity");
             std::vector<Scalars> sc(B);
             CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
             CU(cudaStreamSynchronize(o->stream));
             for (size_t b = 0; b < B; ++b)
-                out[b] = which == LMCMA_B200_I32_ITR ? sc[b].itr : (which == LMCMA_B200_I32_LIVE ? sc[b].live : (int)sc[b].counteval);
+                out[b] = which == LMCMA_B200_I32_ITR ? sc[b].itr : (which == LMCMA_B200_I32_LIVE ? sc[b].live :
+                         (which == LMCMA_B200_I32_EPOCH ? sc[b].epoch : (int)sc[b].counteval));
             return 0;
         }
         case LMCMA_B200_I32_LAUNCH:     // per handle: the launch plan create chose (lmcma_plan.cpp)
@@ -207,7 +208,7 @@ int lmcma_b200_set_i32(lmcma_b200_opt* o, int32_t which, const int32_t* in, int6
             CU(cudaMemcpyAsync(which == LMCMA_B200_I32_T ? d.t : d.vec, in, B * d.m * sizeof(int), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));
             return settle_mirror(o);
-        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: {
+        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH: {
             ARG(count == (int64_t)B, "count");
             std::vector<Scalars> sc(B);
             CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
@@ -215,6 +216,7 @@ int lmcma_b200_set_i32(lmcma_b200_opt* o, int32_t which, const int32_t* in, int6
             for (size_t b = 0; b < B; ++b) {
                 if (which == LMCMA_B200_I32_ITR) sc[b].itr = in[b];
                 else if (which == LMCMA_B200_I32_LIVE) sc[b].live = in[b];
+                else if (which == LMCMA_B200_I32_EPOCH) sc[b].epoch = in[b];
                 else sc[b].counteval = in[b];
             }
             CU(cudaMemcpyAsync(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice, o->stream));

@@ -27,7 +27,7 @@ struct Scalars {          // per-instance scalar state
     int itr;              // CMABase::itr
     int live;             // LMCMA::iterator_sz
     int best_local;       // 1 if best_x holds the row that achieved best_f (split mode: may live on a peer)
-    int pad;
+    int epoch;            // deviate stream of the instance: 0 at create, + 1 at every lmcma_b200_reset_instances (philox_deviate4)
 };
 
 struct OptDev {
@@ -95,6 +95,8 @@ struct OptDev {
     int* err;          // host-visible (mapped, page-locked) error word of the handle: a kernel of the overlapped generation
                        // that gives up waiting for its concurrently running partner writes a code here and carries on
                        // (never __trap: that would poison the whole CUDA context); the host checks it at every sync
+    const int* only;   // B flags or null: the samplers and k_gauss draw only the instances b with only[b] != 0, the others'
+                       // CTAs return at entry (the sampler launch of lmcma_b200_reset_instances; null in every generation)
 };
 
 // The hand-over flags OptDev::progress of instance b: progress_len(m) = m + 2 ints, [0] scalars and mean are final
@@ -287,8 +289,11 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
     }
     return c;
 }
-__device__ __forceinline__ float4 philox_normal4(unsigned q, unsigned row, unsigned gen, unsigned inst, unsigned long long seed) {
-    const uint4 r = philox4x32_10(make_uint4(q, row, gen, inst), make_uint2((unsigned)seed, (unsigned)(seed >> 32)));
+// Key (lo32(seed), hi32(seed) + epoch) mod 2^32: epoch 0 is the plain seed, and seed s at epoch e draws what seed
+// s + e 2^32 draws at epoch 0.
+__device__ __forceinline__ float4 philox_normal4(unsigned q, unsigned row, unsigned gen, unsigned inst, unsigned long long seed,
+                                                 unsigned epoch) {
+    const uint4 r = philox4x32_10(make_uint4(q, row, gen, inst), make_uint2((unsigned)seed, (unsigned)(seed >> 32) + epoch));
     const float s = 2.3283064365386963e-10f;   // 2^-32
     const float u0 = r.x * s + 1.1641532182693481e-10f, u1 = r.y * s + 1.1641532182693481e-10f;
     const float u2 = r.z * s + 1.1641532182693481e-10f, u3 = r.w * s + 1.1641532182693481e-10f;
@@ -299,11 +304,11 @@ __device__ __forceinline__ float4 philox_normal4(unsigned q, unsigned row, unsig
     __sincosf(6.283185307179586f * u3, &s1, &c1);
     return make_float4(ra * c0, ra * s0, rb * c1, rb * s1);
 }
-// The generator's deviates v of float4 column q of local row `row` of instance b in generation itr, padding lanes zeroed:
-// what the samplers draw (sample_deviate4, k_sample.cuh) and k_gauss materialises for the prior, so that a prior run and
-// a plain run see the same raw deviates.
-__device__ __forceinline__ void philox_deviate4(const OptDev& o, int b, int row, int q, int itr, float4& v) {
-    v = philox_normal4((unsigned)q, (unsigned)(o.pop_offset + row), (unsigned)itr, (unsigned)b, o.seed);
+// The generator's deviates v of float4 column q of local row `row` of instance b in generation itr of stream epoch `epoch`
+// (Scalars::epoch), padding lanes zeroed: what the samplers draw (sample_deviate4, k_sample.cuh) and k_gauss materialises
+// for the prior, so that a prior run and a plain run see the same raw deviates.
+__device__ __forceinline__ void philox_deviate4(const OptDev& o, int b, int row, int q, int itr, int epoch, float4& v) {
+    v = philox_normal4((unsigned)q, (unsigned)(o.pop_offset + row), (unsigned)itr, (unsigned)b, o.seed, (unsigned)epoch);
     const int e = q * 4;
     if (e + 1 >= o.n) v.y = 0.f;
     if (e + 2 >= o.n) v.z = 0.f;

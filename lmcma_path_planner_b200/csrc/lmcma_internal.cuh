@@ -182,6 +182,7 @@ struct lmcma_b200_opt {
     lmcma_b200_objective obj{};
     float* d_ends = nullptr;
     float* d_rescore = nullptr;        // B costs of best_x on the attached map (lmcma_b200_rescore_best)
+    char* d_reset = nullptr;           // lmcma_b200_reset_instances stages its ResetArgs arrays here (reset_layout), from the first call on
     // graph
     lmcma_capi::Graph graph;                  // one fused generation (lmcma_b200_run)
     lmcma_capi::Graph graph_multi;            // Tuning::graph_unroll generations in one graph (lmcma_b200_run of many generations)

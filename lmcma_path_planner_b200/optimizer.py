@@ -228,6 +228,58 @@ class Optimizer:
                                "set_stream(s.cuda_stream) with the (non-default) torch stream the cost runs on")
         K.check(K.lib().lmcma_b200_tell_all_dev(self._h))
 
+    def reset_instances(self, idx, x0, sigma0=None, starts=None, goals=None):
+        """Restart the instances idx in place, as a fresh create would start them from x0 [len(idx), n] (or one row for
+        all) with step size sigma0 (per instance, one value, or None for the handle's sigma0), on a new deviate stream.
+        starts / goals: new end points, one row per instance or one for all (needs an attached cost), or None to keep
+        them.  Synchronous; the other instances and the handle's graphs are untouched."""
+        idx = np.ascontiguousarray(np.atleast_1d(np.asarray(idx)), np.int32)
+        count = len(idx)
+        x0a = K.f64c(np.broadcast_to(np.asarray(x0, np.float64), (count, self.n)) if np.ndim(x0) == 1 else x0)
+        sg = None if sigma0 is None else K.f64c(np.broadcast_to(np.asarray(sigma0, np.float64), (count,)))
+        ends = None
+        if starts is not None or goals is not None:
+            starts = np.asarray(starts, np.float32).reshape(-1, np.shape(starts)[-1])
+            goals = np.asarray(goals, np.float32).reshape(-1, np.shape(goals)[-1])
+            if starts.shape[0] == 1 and count > 1:
+                starts = np.repeat(starts, count, 0)
+                goals = np.repeat(goals, count, 0)
+            assert starts.shape[0] == count and goals.shape[0] == count
+            ends = (K.Endpoints * count)(*[_endpoints(starts[i], goals[i]) for i in range(count)])
+        K.check(K.lib().lmcma_b200_reset_instances(self._h, count, K.iptr(idx), K.dptr(x0a),
+                                                   None if sg is None else K.dptr(sg), ends))
+
+    def reset_instances_dev(self, flags, x0, sigma0=None, ends=None, best_x_out=None, best_f_out=None):
+        """The reset from flags computed on the device, enqueued on the handle's stream without waiting (capturable in
+        torch.cuda.graph, like tell_all_dev).  torch CUDA tensors on this handle's device, contiguous: flags int32 [batch]
+        (non-zero = reset), x0 float64 [batch, n] (rows of unflagged instances unused), sigma0 float64 [batch] or None,
+        ends float32 [batch, 6] (start xyz, goal xyz) or None; best_x_out float32 [batch, n] / best_f_out float64 [batch]
+        or None receive each reset instance's best before the reset.  The library trusts the values (finite x0,
+        sigma0 > 0); this method checks dtypes, shapes, devices and contiguity only, without a synchronise."""
+        import torch                                             # only the device path needs torch
+        if self._stream is None:
+            raise K.LmcmaError(K.ERR_STATE, "reset_instances_dev on the handle's own stream: nothing torch enqueues is ordered "
+                               "with it; set_stream(s.cuda_stream) with the (non-default) torch stream the flags come from")
+        B, n = self.batch, self.n
+        want = dict(flags=(torch.int32, (B,)), x0=(torch.float64, (B, n)), sigma0=(torch.float64, (B,)),
+                    ends=(torch.float32, (B, 6)), best_x_out=(torch.float32, (B, n)), best_f_out=(torch.float64, (B,)))
+        given = dict(flags=flags, x0=x0, sigma0=sigma0, ends=ends, best_x_out=best_x_out, best_f_out=best_f_out)
+        ptr = {}
+        for name, t in given.items():
+            if t is None:
+                if name in ("flags", "x0"):
+                    raise ValueError("%s is required" % name)
+                ptr[name] = None
+                continue
+            dtype, shape = want[name]
+            if not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != shape:
+                raise ValueError("%s must be a %s tensor of shape %s" % (name, dtype, shape))
+            if t.device != torch.device("cuda", self.device) or not t.is_contiguous():
+                raise ValueError("%s must be contiguous on cuda:%d" % (name, self.device))
+            ptr[name] = t.data_ptr()
+        K.check(K.lib().lmcma_b200_reset_instances_dev(self._h, ptr["flags"], ptr["x0"], ptr["sigma0"], ptr["ends"],
+                                                       ptr["best_x_out"], ptr["best_f_out"]))
+
     def ask_one(self):
         x = np.zeros(self.n, np.float64)
         K.check(K.lib().lmcma_b200_ask_one(self._h, K.dptr(x), self.n))
@@ -307,7 +359,7 @@ class Optimizer:
                 "Nj": (B, m), "Lj": (B, m), "X": (B, pc, n), "Z": (B, pc, n), "pc": (B, n), "V": (B, m, n),
                 "P": (B, m, n), "fit": (B, lam), "fit_sorted": (B, lam), "prev_fit": (B, lam), "t": (B, m),
                 "vec": (B, m), "arindex": (B, lam), "rank": (B, lam), "itr": (B,), "live": (B,),
-                "counteval": (B,), "ncoll": (B, pc), "nsamp": (B, pc)}[name]
+                "counteval": (B,), "ncoll": (B, pc), "nsamp": (B, pc), "epoch": (B,)}[name]
 
     def get(self, name):
         shp = self._shape_of(name)
