@@ -107,7 +107,8 @@ int lmcma_b200_map_destroy(lmcma_b200_map* map);
  * gives 1 / (1 / max(E, c_min)) in FP32, i.e. the clearance with the c_min floor (up to the rounding of the two
  * reciprocals), and 0 on obstacles */
 int lmcma_b200_map_dequantized(const lmcma_b200_map* map, float* dist_host_out);
-/* pin the map in L2 (cudaAccessPolicyWindow, persisting) for the launches of this library */
+/* pin the map in L2 (cudaAccessPolicyWindow, persisting) for the launches of this library.  An optimiser handle attached
+ * to several maps (lmcma_b200_attach_cost_maps) sets no window: one window covers one address range */
 int lmcma_b200_map_set_l2_persist(lmcma_b200_map* map, int enable);
 
 /* A planning query: fixed end points (planner.cpp:701-711) and the objective weights
@@ -268,6 +269,28 @@ int lmcma_b200_is_done(lmcma_b200_opt* opt, int32_t* done_host);
 /* ends: batch end-point pairs (one query per instance).  The map must live on the same device. */
 int lmcma_b200_attach_cost(lmcma_b200_opt* opt, lmcma_b200_map* map, const lmcma_b200_objective* obj,
                            const lmcma_b200_endpoints* ends);
+/* One handle on several maps (several floors or sites, a coarse map beside a fine one), so that one batch and one launch
+ * of each kernel serve queries on all of them: instance b is evaluated on maps[map_of[b]] (map_of: batch entries).  Every
+ * map must live on the handle's device and share dims and storage; shape, u8_scale, c_min and clamp may differ.  One
+ * objective for the whole handle; the end points stay per instance.  The box bounds stay per handle: samples of an
+ * instance that leave its map are collisions, so maps padded to one shape give every instance a tight box.
+ * map_of is per-instance state: LMCMA_B200_I32_MAP_OF (get / set) and lmcma_b200_instance_maps_dev change it without
+ * rebuilding a graph, and reset_instances leaves it alone.  The maps must outlive the attachment, as with attach_cost, and
+ * an occupancy update of any of them is seen by the next launch.  L2 persistence (lmcma_b200_map_set_l2_persist) is not
+ * applied on a handle with several maps: an access-policy window covers one address range.  map_count == 1 attaches
+ * maps[0] exactly as lmcma_b200_attach_cost does.
+ * LMCMA_B200_ERR_ARG: a null pointer, map_count < 1, maps of different devices / dims / storage, dims * waypoints != n, a
+ * map_of entry outside [0, map_count).  LMCMA_B200_ERR_STATE: a split-population handle (the mg_* entry points take one
+ * map).  A refused call changes nothing. */
+int lmcma_b200_attach_cost_maps(lmcma_b200_opt* opt, int32_t map_count, lmcma_b200_map* const* maps,
+                                const int32_t* map_of /* batch */, const lmcma_b200_objective* obj,
+                                const lmcma_b200_endpoints* ends /* batch */);
+/* The handle's device copy of map_of (batch int32), stable for the handle's lifetime.  The caller may write it on the
+ * handle's stream, also inside its stream capture, as it writes f_dev of lmcma_b200_device_buffers; the next cost launch
+ * reads it.  Values are trusted, with one exception: k_cost gives an instance whose entry lies outside [0, map_count)
+ * f = +inf and ncoll = nsamp = 0 and reads no map for it.  LMCMA_B200_ERR_STATE on a handle not attached to several
+ * maps. */
+int lmcma_b200_instance_maps_dev(lmcma_b200_opt* opt, int32_t** map_of_dev);
 /* `generations` x [cost -> rank -> update -> sample] replayed from a CUDA graph with no
  * host round trip (the loop of example_lmcma.cpp:49-55 with the cost on the device). Asynchronous. */
 int lmcma_b200_run(lmcma_b200_opt* opt, int32_t generations);
@@ -326,9 +349,11 @@ enum {
     LMCMA_B200_I32_NSAMP = 8,      /* batch x pop_count map samples of the last evaluated population */
     LMCMA_B200_I32_LAUNCH = 9,     /* LMCMA_B200_LAUNCH_FIELDS values per HANDLE (not per instance), read-only: the launch
                                       configuration chosen at create, indexed by LMCMA_B200_LAUNCH_* below */
-    LMCMA_B200_I32_EPOCH = 10      /* batch       deviate stream of the instance: 0 at create, + 1 per reset_instances.  The
+    LMCMA_B200_I32_EPOCH = 10,     /* batch      deviate stream of the instance: 0 at create, + 1 per reset_instances.  The
                                       PHILOX key is (lo32(seed), hi32(seed) + epoch) mod 2^32, so seed s at epoch e draws what
                                       seed s + e 2^32 draws at epoch 0.  A checkpoint that restores ITR restores this too */
+    LMCMA_B200_I32_MAP_OF = 11     /* batch       map of the instance (lmcma_b200_attach_cost_maps); all zeros on a handle on one
+                                      map.  Settable with entries in [0, map_count); no graph is rebuilt */
 };
 /* fields of LMCMA_B200_I32_LAUNCH.  Sampler kernels: 0 = k_sample<NV> (narrow), 1 = k_sample_wide<RBW> (a row split over CW
  * column-warps, R row groups per CTA), 2 = k_sample_rows<QW, RL> (rows on lanes).  KC / STAGES are those of the chosen
@@ -351,7 +376,7 @@ int lmcma_b200_get_f64(lmcma_b200_opt* opt, int32_t which, double* out, int64_t 
 int lmcma_b200_get_f32(lmcma_b200_opt* opt, int32_t which, float* out, int64_t capacity);
 int lmcma_b200_get_i32(lmcma_b200_opt* opt, int32_t which, int32_t* out, int64_t capacity);
 /* teacher forcing: overwrite optimiser state (same `which` / layouts as the getters; XMEAN, SIGMA, S,
- * NJ, LJ | PC, V, P, PREV_FIT | T, VEC, ITR, LIVE, EPOCH are settable) */
+ * NJ, LJ | PC, V, P, PREV_FIT | T, VEC, ITR, LIVE, EPOCH, MAP_OF are settable) */
 int lmcma_b200_set_f64(lmcma_b200_opt* opt, int32_t which, const double* in, int64_t count);
 int lmcma_b200_set_f32(lmcma_b200_opt* opt, int32_t which, const float* in, int64_t count);
 int lmcma_b200_set_i32(lmcma_b200_opt* opt, int32_t which, const int32_t* in, int64_t count);

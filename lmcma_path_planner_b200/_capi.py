@@ -14,7 +14,8 @@ MAP_F32, MAP_U8 = 0, 1
 
 F64 = {"xmean": 0, "sigma": 1, "s": 2, "best_f": 3, "consts": 4, "weights": 5, "Nj": 6, "Lj": 7}
 F32 = {"X": 0, "pc": 1, "V": 2, "P": 3, "fit": 4, "fit_sorted": 5, "prev_fit": 6, "Z": 7}
-I32 = {"t": 0, "vec": 1, "arindex": 2, "rank": 3, "itr": 4, "live": 5, "counteval": 6, "ncoll": 7, "nsamp": 8, "epoch": 10}
+I32 = {"t": 0, "vec": 1, "arindex": 2, "rank": 3, "itr": 4, "live": 5, "counteval": 6, "ncoll": 7, "nsamp": 8, "epoch": 10,
+       "map_of": 11}
 I32_LAUNCH = 9
 # the fields of LMCMA_B200_I32_LAUNCH in order (LMCMA_B200_LAUNCH_*)
 LAUNCH_FIELDS = ("sampler", "smp_nv", "smp_spec", "smp_threads", "smp_RBW", "smp_CW", "smp_R", "smp_rows_qw", "smp_rows_rl",
@@ -86,6 +87,8 @@ SIGNATURES = {
     "lmcma_b200_resample": (C.c_int, [_vp]),
     "lmcma_b200_is_done": (C.c_int, [_vp, _pi]),
     "lmcma_b200_attach_cost": (C.c_int, [_vp, _vp, C.POINTER(Objective), C.POINTER(Endpoints)]),
+    "lmcma_b200_attach_cost_maps": (C.c_int, [_vp, _i32, C.POINTER(_vp), _pi, C.POINTER(Objective), C.POINTER(Endpoints)]),
+    "lmcma_b200_instance_maps_dev": (C.c_int, [_vp, C.POINTER(_vp)]),
     "lmcma_b200_run": (C.c_int, [_vp, _i32]),
     "lmcma_b200_sync": (C.c_int, [_vp]),
     "lmcma_b200_launch_count": (C.c_int64, []),

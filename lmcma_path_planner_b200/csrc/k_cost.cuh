@@ -45,12 +45,16 @@ constexpr int COST_MAX_WARPS = 8;
 template <int STORAGE> struct RawCell { typedef float type; };
 template <> struct RawCell<1> { typedef unsigned char type; };
 
-template <int DIMS, int STORAGE, bool TRACE, int MINB = 7>
+template <int DIMS, int STORAGE, bool TRACE, int MINB = 7, bool MULTI = false>
 // 8 warps per CTA, 7 CTAs per SM: 32 registers per thread, every trajectory of a 1024-wide population resident at once.
 // MINB = 6 (LMCMA_B200_COST_MINB=6: 40 registers, no local-memory spill, 1.17 waves at lambda = 1024) is compiled
 // beside it; measured slower on the single C2 query (33.9 vs 31.0 us, profiles/r1g_minb_compare.txt), kept for the
 // many-wave batched shapes.
-__global__ void __launch_bounds__(COST_MAX_WARPS * 32, MINB) k_cost(MapDev mp, CostArgs a) {
+// MULTI (lmcma_b200_attach_cost_maps; DESIGN.md 4.7): the map of instance b is a.maps[a.map_of[b]], loaded by every CTA
+// (one uniform address) instead of `mp0`, whose fields the single-map builds read from the parameter bank.  An index
+// outside [0, a.map_count) gives the trajectory f = +inf, ncoll = nsamp = 0: the CTA stores that and returns before any
+// barrier, without reading the table.
+__global__ void __launch_bounds__(COST_MAX_WARPS * 32, MINB) k_cost(MapDev mp0, CostArgs a) {
     typedef typename RawCell<STORAGE>::type raw_t;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int W = a.W, NSEG = W + 1;
@@ -67,6 +71,19 @@ __global__ void __launch_bounds__(COST_MAX_WARPS * 32, MINB) k_cost(MapDev mp, C
 
     griddep_launch_dependents();          // k_rank may become resident as this grid drains; it waits for completion
     const int row = blockIdx.x, b = blockIdx.y;
+    int mi = 0;
+    if (MULTI) {
+        mi = a.map_of[b];
+        if ((unsigned)mi >= (unsigned)a.map_count) {              // the whole CTA leaves here: no barrier has been reached
+            if (threadIdx.x == 0) {
+                a.f[(size_t)b * a.f_stride + a.f_offset + row] = __int_as_float(0x7f800000);
+                if (a.ncoll) a.ncoll[(size_t)b * a.inst_rows + row] = 0;
+                if (a.nsamp) a.nsamp[(size_t)b * a.inst_rows + row] = 0;
+            }
+            return;
+        }
+    }
+    const MapDev mp = MULTI ? a.maps[mi] : mp0;
 #define COST_STAMP(k) do { if (TRACE && a.dbg && (threadIdx.x & 31) == 0) { const long long t__ = gtime(); if ((k) == 0 || (k) == 1 || (k) == 2) { if (threadIdx.x == 0) a.dbg[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8 + (k)] = t__; } else atomicMax(reinterpret_cast<unsigned long long*>(a.dbg + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8 + (k)), (unsigned long long)t__); } } while (0)
     COST_STAMP(0);
     const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = nthr >> 5;

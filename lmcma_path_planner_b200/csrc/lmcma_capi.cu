@@ -176,7 +176,20 @@ int cost_args_for(lmcma_b200_opt* o, CostArgs* a) {
     a->ends = o->d_ends; a->ends_per_instance = 1;
     a->f = o->d.fit; a->f_stride = o->d.lambda; a->f_offset = o->d.pop_offset;
     a->ncoll = o->d.ncoll; a->nsamp = o->d.nsamp;
+    if (o->maps.size() > 1) { a->maps = o->d_maps; a->map_of = o->d_map_of; a->map_count = (int)o->maps.size(); }
     return 0;
+}
+
+// every launch of the attached cost (the generations, rescore_best, profile_kernels): the map passed by value gives the
+// build's dims and storage; with several maps k_cost reads each instance's map from the table in `a` (cost_args_for)
+int launch_attached_cost(lmcma_b200_opt* o, const CostArgs& a, int rows, cudaStream_t st) {
+    return launch_cost(o->map->dev, a, rows, o->d.B, o->cost_shape, false, st);
+}
+
+// the L2 persistence window of the attached map on `st`.  An access-policy window covers one address range: a handle on
+// several maps sets none
+int attached_l2_window(lmcma_b200_opt* o, cudaStream_t st) {
+    return o->maps.size() > 1 ? 0 : apply_l2_window(o->map, st);
 }
 
 // lmcma_b200_rescore_best: best_f <- the cost of best_x on the map as it is now, for every instance that has been evaluated
@@ -230,7 +243,7 @@ enum class Fit { COST, FROM_HOST, IN_PLACE };
 int launch_own_cost(lmcma_b200_opt* o, cudaStream_t st) {
     CostArgs ca;
     int rc = cost_args_for(o, &ca);
-    return rc ? rc : launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
+    return rc ? rc : launch_attached_cost(o, ca, o->d.pop_count, st);
 }
 
 // One generation in stream order (fit: COST or IN_PLACE): [k_cost ->] k_rank -> k_update -> [HANSEN deviates ->] the
@@ -706,7 +719,7 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     if (o->stream) cudaStreamSynchronize(o->stream);
     OptDev& d = o->d;
     void* ptrs[] = {d.prev_sorted, d.tile_sorted, d.tile_pos, d.X, d.D, d.Z, d.Zc, o->d_Lf, d.fit, d.fit_sorted, d.prev_fit, d.rank, d.arindex, d.ncoll, d.nsamp, d.xmean, d.pc, d.V, d.P,
-                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore, o->d_reset};
+                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore, o->d_reset, o->d_maps, o->d_map_of};
     for (void* p : ptrs) cudaFree(p);
     drop_fused_graphs(o);
     drop_tell_graphs(o);
@@ -1006,13 +1019,9 @@ int lmcma_b200_is_done(lmcma_b200_opt* o, int32_t* done) {
     return 0;
 }
 
-int lmcma_b200_attach_cost(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b200_objective* obj,
-                           const lmcma_b200_endpoints* ends) {
-    ARG(o && ends, "null pointer");
-    int rc = check_obj(map, obj);
-    if (rc) return rc;
-    ARG(map->device == o->cfg.device, "map and optimiser live on different devices");
-    ARG(map->dev.dims * obj->waypoints == o->d.n, "n != dims * waypoints");
+// what attach_cost and attach_cost_maps share once their arguments are checked: the objective, the end points, the cost's
+// launch shape, and the graphs that launched the previous cost
+static int attach_body(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b200_objective* obj, const lmcma_b200_endpoints* ends) {
     CU(cudaSetDevice(o->cfg.device));
     o->map = map; o->obj = *obj;
     std::vector<float> e6((size_t)o->d.B * 6);
@@ -1025,13 +1034,67 @@ int lmcma_b200_attach_cost(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b
     return 0;
 }
 
+int lmcma_b200_attach_cost(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b200_objective* obj,
+                           const lmcma_b200_endpoints* ends) {
+    ARG(o && ends, "null pointer");
+    int rc = check_obj(map, obj);
+    if (rc) return rc;
+    ARG(map->device == o->cfg.device, "map and optimiser live on different devices");
+    ARG(map->dev.dims * obj->waypoints == o->d.n, "n != dims * waypoints");
+    o->maps.assign(1, map);
+    return attach_body(o, map, obj, ends);
+}
+
+int lmcma_b200_attach_cost_maps(lmcma_b200_opt* o, int32_t map_count, lmcma_b200_map* const* maps, const int32_t* map_of,
+                                const lmcma_b200_objective* obj, const lmcma_b200_endpoints* ends) {
+    ARG(o && maps && map_of && obj && ends, "null pointer");
+    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "attach_cost_maps: split-population handles take one map (attach_cost)");
+    ARG(map_count >= 1, "map_count must be >= 1");
+    for (int k = 0; k < map_count; ++k) {
+        ARG(maps[k], "null map");
+        ARG(maps[k]->device == o->cfg.device, "map and optimiser live on different devices");
+        ARG(maps[k]->dev.dims == maps[0]->dev.dims && maps[k]->storage == maps[0]->storage, "maps of different dims or storage");
+    }
+    int rc = check_obj(maps[0], obj);
+    if (rc) return rc;
+    ARG(maps[0]->dev.dims * obj->waypoints == o->d.n, "n != dims * waypoints");
+    for (int b = 0; b < o->d.B; ++b) ARG(map_of[b] >= 0 && map_of[b] < map_count, "map_of entry outside [0, map_count)");
+    if (map_count == 1) {                                        // a single-map handle, as attach_cost makes it
+        o->maps.assign(1, maps[0]);
+        return attach_body(o, maps[0], obj, ends);
+    }
+    CU(cudaSetDevice(o->cfg.device));
+    // the table: MapDev is written by the map builds only (an occupancy update rewrites the storage it points to), so the
+    // copy stays current for as long as the maps live
+    std::vector<MapDev> table((size_t)map_count);
+    for (int k = 0; k < map_count; ++k) table[k] = maps[k]->dev;
+    if (o->d_maps_cap < (size_t)map_count) {
+        cudaFree(o->d_maps); o->d_maps = nullptr; o->d_maps_cap = 0;
+        DM(o->d_maps, (size_t)map_count);
+        o->d_maps_cap = (size_t)map_count;
+    }
+    if (!o->d_map_of) DM(o->d_map_of, (size_t)o->d.B);
+    CU(cudaMemcpyAsync(o->d_maps, table.data(), table.size() * sizeof(MapDev), cudaMemcpyHostToDevice, o->stream));
+    CU(cudaMemcpyAsync(o->d_map_of, map_of, (size_t)o->d.B * sizeof(int), cudaMemcpyHostToDevice, o->stream));
+    CU(cudaStreamSynchronize(o->stream));
+    o->maps.assign(maps, maps + map_count);
+    return attach_body(o, maps[0], obj, ends);
+}
+
+int lmcma_b200_instance_maps_dev(lmcma_b200_opt* o, int32_t** map_of_dev) {
+    ARG(o && map_of_dev, "null pointer");
+    if (o->maps.size() < 2) return fail(LMCMA_B200_ERR_STATE, "instance_maps_dev: the handle is not attached to several maps (attach_cost_maps)");
+    *map_of_dev = o->d_map_of;
+    return 0;
+}
+
 int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
     ARG(o && generations >= 0, "bad argument");
     if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached");
     if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet: inject_z first");
     if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles use the mg_* entry points");
     CU(cudaSetDevice(o->cfg.device));
-    int rc = apply_l2_window(o->map, o->stream);
+    int rc = attached_l2_window(o, o->stream);
     if (rc) return rc;
     o->spec_valid = false;                                       // the fused generations advance the state past what tell_all's speculative pass saw
     if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) {
@@ -1086,7 +1149,7 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
     for (int g = 0; g < generations && !rc; ++g) {
         cudaEvent_t* e = &ev[(size_t)g * 5];
         cudaEventRecord(e[0], st);
-        rc = launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
+        rc = launch_attached_cost(o, ca, o->d.pop_count, st);
         cudaEventRecord(e[1], st);
         if (!rc) rc = launch_rank(o, o->d.fit, RANK_PLAIN, nullptr, st);
         cudaEventRecord(e[2], st);
@@ -1100,7 +1163,9 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
     cudaError_t se = cudaStreamSynchronize(st);
     if (!rc && se != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "profile run: %s", cudaGetErrorString(se));
     if (!rc && o->d.dbg) rc = print_timeline(o);
-    if (!rc && o->d.dbg) {     // and the per-CTA timeline of k_cost (phase stamps): one extra launch of its TRACE build
+    if (!rc && o->d.dbg && o->maps.size() > 1)
+        fprintf(stderr, "k_cost timeline: skipped, a handle on several maps has no TRACE build of k_cost\n");
+    else if (!rc && o->d.dbg) {     // and the per-CTA timeline of k_cost (phase stamps): one extra launch of its TRACE build
         const size_t ctas = (size_t)o->d.pop_count * o->d.B;
         long long* dbg = nullptr;
         if (cudaMalloc(&dbg, ctas * 8 * sizeof(long long)) == cudaSuccess) {
@@ -1174,8 +1239,8 @@ int lmcma_b200_rescore_best(lmcma_b200_opt* o) {
     if (rc) return rc;
     ca.X = d.best_x; ca.inst_rows = 1;                           // one row per instance, the instance's own end points
     ca.f = o->d_rescore; ca.f_stride = 1; ca.f_offset = 0; ca.ncoll = nullptr; ca.nsamp = nullptr;
-    if ((rc = apply_l2_window(o->map, o->stream))) return rc;
-    if ((rc = launch_cost(o->map->dev, ca, 1, d.B, o->cost_shape, false, o->stream))) return rc;
+    if ((rc = attached_l2_window(o, o->stream))) return rc;
+    if ((rc = launch_attached_cost(o, ca, 1, o->stream))) return rc;   // each instance's best_x on its own map
     if ((rc = launch(k_set_best_f, (unsigned)((d.B + 127) / 128), 128, 0, o->stream, false, d.sc, (const float*)o->d_rescore, d.B))) return rc;
     o->spec_valid = false;                                       // like the state setters: tell_all's speculative pass saw the old best
     CU(cudaStreamSynchronize(o->stream));

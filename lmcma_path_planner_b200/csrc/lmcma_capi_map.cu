@@ -8,7 +8,7 @@ using namespace lmcma;
 using namespace lmcma_capi;
 
 namespace {
-template <int DIMS, int STORAGE, bool TRACE, int MINB = 7>
+template <int DIMS, int STORAGE, bool TRACE, int MINB = 7, bool MULTI = false>
 int launch_cost_t(const MapDev& mp, const CostArgs& a0, int rows, int B, CostShape shape, cudaStream_t st) {
     CostArgs a = a0;
     a.spt = (a.W + 1 + shape.tpt - 1) / shape.tpt;
@@ -17,7 +17,18 @@ int launch_cost_t(const MapDev& mp, const CostArgs& a0, int rows, int B, CostSha
     // + the candidate row (16-byte aligned)
     const size_t smem = (size_t)36 * (a.W + 1) + sizeof(int) * (a.W + 2) + 28 + (size_t)8 * shape.cb + (STORAGE == 1 ? 1024 : 0) +
                         sizeof(float) * DIMS * ((size_t)a.W + 2) + 16;
-    return launch(k_cost<DIMS, STORAGE, TRACE, MINB>, dim3(rows, B), shape.tpt, smem, st, false, mp, a);
+    return launch(k_cost<DIMS, STORAGE, TRACE, MINB, MULTI>, dim3(rows, B), shape.tpt, smem, st, false, mp, a);
+}
+
+// the non-TRACE builds at `minb` CTAs per SM, single-map or multi-map (CostArgs::maps)
+template <bool MULTI>
+int launch_cost_minb(const MapDev& mp, const CostArgs& a, int rows, int B, CostShape shape, int minb, cudaStream_t st) {
+    if (minb == 6) {
+        if (mp.dims == 2) return mp.storage == 0 ? launch_cost_t<2, 0, false, 6, MULTI>(mp, a, rows, B, shape, st) : launch_cost_t<2, 1, false, 6, MULTI>(mp, a, rows, B, shape, st);
+        return mp.storage == 0 ? launch_cost_t<3, 0, false, 6, MULTI>(mp, a, rows, B, shape, st) : launch_cost_t<3, 1, false, 6, MULTI>(mp, a, rows, B, shape, st);
+    }
+    if (mp.dims == 2) return mp.storage == 0 ? launch_cost_t<2, 0, false, 7, MULTI>(mp, a, rows, B, shape, st) : launch_cost_t<2, 1, false, 7, MULTI>(mp, a, rows, B, shape, st);
+    return mp.storage == 0 ? launch_cost_t<3, 0, false, 7, MULTI>(mp, a, rows, B, shape, st) : launch_cost_t<3, 1, false, 7, MULTI>(mp, a, rows, B, shape, st);
 }
 
 }  // namespace
@@ -26,20 +37,20 @@ namespace lmcma_capi {
 int launch_cost(const MapDev& mp, const CostArgs& a, int rows, int B, CostShape shape, bool trace, cudaStream_t st) {
     if (rows <= 0 || B <= 0) return 0;
     if (trace) {
+        if (a.maps) return fail(LMCMA_B200_ERR_STATE, "k_cost has no TRACE build for several maps");
         if (mp.dims == 2) return mp.storage == 0 ? launch_cost_t<2, 0, true>(mp, a, rows, B, shape, st) : launch_cost_t<2, 1, true>(mp, a, rows, B, shape, st);
         return mp.storage == 0 ? launch_cost_t<3, 0, true>(mp, a, rows, B, shape, st) : launch_cost_t<3, 1, true>(mp, a, rows, B, shape, st);
     }
     // seven CTAs per SM (32 registers, 28 / 36 B of spills outside the sample loop) keep a 1024-trajectory population resident in
     // ONE wave.  The 40-register build at six per SM was 7 % faster from four waves on in round 1 (0.280 -> 0.261 ms for 16384
     // trajectories); after round 2's instruction diet of the phases around the loop it is the other way round in 2-D (C3 batch
-    // of 262144 trajectories: 3.39 ms at seven per SM, 3.47 ms at six), so 2-D launches always take the seven-per-SM build
+    // of 262144 trajectories: 3.39 ms at seven per SM, 3.47 ms at six), so 2-D launches always take the seven-per-SM build.
+    // The multi-map builds (several maps, mp: their common dims and storage) follow the same rule.  Their map pitches, bounds
+    // and base pointers are registers, not parameter-bank operands: at seven per SM they stay at 32 registers with 28-44 B
+    // of spill stores, at six per SM at 40 with 0-24 B.  Measured on a B200 (tools/multi_map_timing.py, 4096 queries x
+    // lambda 64 on four 4096^2 u8 maps): k_cost 3.33 ms at seven per SM, 3.41 ms at six (DESIGN.md 4.7)
     const int minb = shape.minb ? shape.minb : (mp.dims == 3 && (long long)rows * B >= 4LL * 7 * 148 ? 6 : 7);
-    if (minb == 6) {
-        if (mp.dims == 2) return mp.storage == 0 ? launch_cost_t<2, 0, false, 6>(mp, a, rows, B, shape, st) : launch_cost_t<2, 1, false, 6>(mp, a, rows, B, shape, st);
-        return mp.storage == 0 ? launch_cost_t<3, 0, false, 6>(mp, a, rows, B, shape, st) : launch_cost_t<3, 1, false, 6>(mp, a, rows, B, shape, st);
-    }
-    if (mp.dims == 2) return mp.storage == 0 ? launch_cost_t<2, 0, false>(mp, a, rows, B, shape, st) : launch_cost_t<2, 1, false>(mp, a, rows, B, shape, st);
-    return mp.storage == 0 ? launch_cost_t<3, 0, false>(mp, a, rows, B, shape, st) : launch_cost_t<3, 1, false>(mp, a, rows, B, shape, st);
+    return a.maps ? launch_cost_minb<true>(mp, a, rows, B, shape, minb, st) : launch_cost_minb<false>(mp, a, rows, B, shape, minb, st);
 }
 
 // CTA width and per-block record capacity of k_cost from the expected samples per trajectory

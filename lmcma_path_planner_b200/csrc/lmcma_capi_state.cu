@@ -97,6 +97,11 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
                          (which == LMCMA_B200_I32_EPOCH ? sc[b].epoch : (int)sc[b].counteval));
             return 0;
         }
+        case LMCMA_B200_I32_MAP_OF:     // the map of every instance: all zeros unless the handle is on several maps
+            if (o->maps.size() > 1) { src = o->d_map_of; cnt = B; break; }
+            ARG(cap >= (int64_t)B, "capacity");
+            std::fill(out, out + B, 0);
+            return 0;
         case LMCMA_B200_I32_LAUNCH:     // per handle: the launch plan create chose (lmcma_plan.cpp)
             ARG(cap >= LMCMA_B200_LAUNCH_FIELDS, "capacity");
             launch_fields(o->plan, out);
@@ -220,6 +225,16 @@ int lmcma_b200_set_i32(lmcma_b200_opt* o, int32_t which, const int32_t* in, int6
                 else sc[b].counteval = in[b];
             }
             CU(cudaMemcpyAsync(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice, o->stream));
+            CU(cudaStreamSynchronize(o->stream));
+            return 0;
+        }
+        case LMCMA_B200_I32_MAP_OF: {   // read by k_cost through a pointer: no graph is rebuilt
+            if (!o->map) return fail(LMCMA_B200_ERR_STATE, "map_of: no cost attached");
+            ARG(count == (int64_t)B, "count");
+            const int64_t maps = (int64_t)o->maps.size();
+            for (size_t b = 0; b < B; ++b) ARG(in[b] >= 0 && in[b] < maps, "map_of entry outside [0, map_count)");
+            if (maps == 1) return 0;                             // a single-map handle: all zeros, nothing stored
+            CU(cudaMemcpyAsync(o->d_map_of, in, B * sizeof(int), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));
             return 0;
         }

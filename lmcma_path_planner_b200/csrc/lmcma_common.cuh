@@ -166,6 +166,11 @@ struct CostArgs {
     int cb;                    // capacity of the per-block record stage (32-sample blocks), set by the launcher
     int spt;                   // segments per thread = ceil((W + 1) / threads per trajectory), set by the launcher
     long long* dbg;            // optional (LMCMA_B200_DBG, profile_kernels): 8 globaltimer stamps per CTA, [cta * 8 + k]
+    // several maps (lmcma_b200_attach_cost_maps): instance b is evaluated on maps[map_of[b]], map_count entries of one
+    // dims / storage.  Null maps: every instance on the map passed by value (the single-map builds)
+    const MapDev* maps;
+    const int* map_of;
+    int map_count;
 };
 
 struct CostShape { int tpt = 128, cb = 256, minb = 0; };   // launch shape of k_cost: threads per trajectory, block-record capacity, CTAs per SM of the build to launch (0 = chosen by the launch size)

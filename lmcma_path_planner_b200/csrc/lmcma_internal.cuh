@@ -177,8 +177,14 @@ struct lmcma_b200_opt {
     int sample_idx = 0;
     std::vector<float> x_cache; bool x_cache_valid = false;
     std::vector<float> f_host;
-    // attached cost
+    // attached cost.  map: the map of a single-map handle, maps[0] of a multi-map one (lmcma_b200_attach_cost_maps), whose
+    // dims, storage and device every map shares.  A multi-map handle (maps.size() > 1) keeps the MapDev table of its maps
+    // (d_maps) and the map index of every instance (d_map_of, B ints, allocated at the first such attach and kept for the
+    // handle's lifetime); cost_args_for hands both to k_cost
     lmcma_b200_map* map = nullptr;
+    std::vector<lmcma_b200_map*> maps;
+    lmcma::MapDev* d_maps = nullptr; size_t d_maps_cap = 0;
+    int* d_map_of = nullptr;
     lmcma_b200_objective obj{};
     float* d_ends = nullptr;
     float* d_rescore = nullptr;        // B costs of best_x on the attached map (lmcma_b200_rescore_best)

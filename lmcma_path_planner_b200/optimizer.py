@@ -130,14 +130,14 @@ class CostMap:
 
 
 class _DeviceBuffer:
-    """One of an optimiser's device buffers as a __cuda_array_interface__ (FP32).  A tensor made from it holds a reference to
-    it, and through `owner` to the optimiser, so garbage collection cannot free the memory under it (close() still does).
-    torch takes no read-only flag: that
+    """One of an optimiser's device buffers as a __cuda_array_interface__ (FP32, or typestr).  A tensor made from it holds a
+    reference to it, and through `owner` to the optimiser, so garbage collection cannot free the memory under it (close()
+    still does).  torch takes no read-only flag: that
     X must not be written is the caller's part (device_tensors)."""
 
-    def __init__(self, owner, ptr, shape, strides):
+    def __init__(self, owner, ptr, shape, strides, typestr="<f4"):
         self.owner = owner
-        self.__cuda_array_interface__ = {"shape": shape, "strides": strides, "typestr": "<f4", "data": (ptr, False),
+        self.__cuda_array_interface__ = {"shape": shape, "strides": strides, "typestr": typestr, "data": (ptr, False),
                                          "version": 2}
 
 
@@ -302,21 +302,51 @@ class Optimizer:
         return d.astype(bool)
 
     # ---- fused planning ----
-    def attach_cost(self, cmap, starts, goals, waypoints, weights=LONGSAFE, w_col=1e4):
-        starts = np.asarray(starts, np.float32).reshape(-1, cmap.dims)
-        goals = np.asarray(goals, np.float32).reshape(-1, cmap.dims)
+    def attach_cost(self, cmap_or_maps, starts, goals, waypoints, weights=LONGSAFE, w_col=1e4, map_of=None):
+        """The fused generations' cost: one CostMap, or a sequence of CostMaps of one dims and storage with map_of [batch]
+        naming each instance's map (lmcma_b200_attach_cost_maps; map_of may be omitted for a single map).  starts / goals:
+        one row per instance or one for all.  The handle keeps its maps alive."""
+        several = not isinstance(cmap_or_maps, CostMap)
+        cmaps = list(cmap_or_maps) if several else [cmap_or_maps]
+        if not cmaps:
+            raise ValueError("attach_cost needs at least one map")
+        dims = cmaps[0].dims
+        starts = np.asarray(starts, np.float32).reshape(-1, dims)
+        goals = np.asarray(goals, np.float32).reshape(-1, dims)
         if starts.shape[0] == 1 and self.batch > 1:
             starts = np.repeat(starts, self.batch, 0)
             goals = np.repeat(goals, self.batch, 0)
         assert starts.shape[0] == self.batch
         ends = (K.Endpoints * self.batch)()
         for b in range(self.batch):
-            for c in range(cmap.dims):
+            for c in range(dims):
                 ends[b].start[c] = float(starts[b, c])
                 ends[b].goal[c] = float(goals[b, c])
         obj = _objective(waypoints, weights, w_col)
-        K.check(K.lib().lmcma_b200_attach_cost(self._h, cmap._h, C.byref(obj), ends))
-        self._map = cmap   # keep alive
+        if not several:
+            if map_of is not None and np.any(np.asarray(map_of) != 0):
+                raise ValueError("map_of names maps other than the one given")
+            K.check(K.lib().lmcma_b200_attach_cost(self._h, cmap_or_maps._h, C.byref(obj), ends))
+        else:
+            if map_of is None:
+                if len(cmaps) > 1:
+                    raise ValueError("map_of is required with several maps")
+                map_of = 0
+            mo = np.ascontiguousarray(np.broadcast_to(np.asarray(map_of, np.int32), (self.batch,)))
+            hs = (C.c_void_p * len(cmaps))(*[m._h for m in cmaps])
+            K.check(K.lib().lmcma_b200_attach_cost_maps(self._h, len(cmaps), hs, K.iptr(mo), C.byref(obj), ends))
+        self._map = cmaps[0] if not several else cmaps   # keep alive
+
+    def device_map_index(self):
+        """torch int32 view [batch] over the handle's map index of every instance (a handle attached to several maps): write
+        it on the handle's stream, also inside a torch.cuda.graph capture, and the next cost launch evaluates each instance
+        on its new map.  Values must lie in [0, number of maps); an instance whose entry does not gets f = +inf.  Same
+        ownership rules as device_tensors."""
+        import torch                                             # only this method needs torch
+        p = C.c_void_p()
+        K.check(K.lib().lmcma_b200_instance_maps_dev(self._h, C.byref(p)))
+        buf = _DeviceBuffer(self, p.value, (self.batch,), (4,), "<i4")
+        return torch.as_tensor(buf, device=torch.device("cuda", self.device))
 
     def run(self, generations, sync=True):
         K.check(K.lib().lmcma_b200_run(self._h, int(generations)))
@@ -349,7 +379,7 @@ class Optimizer:
 
     def rescore_best(self):
         """best_f <- the cost of best_x on the attached map as it is now (after CostMap.update_occupancy), for every
-        instance evaluated at least once."""
+        instance evaluated at least once; on a handle with several maps each instance's own map."""
         K.check(K.lib().lmcma_b200_rescore_best(self._h))
 
     # ---- state ----
@@ -359,7 +389,7 @@ class Optimizer:
                 "Nj": (B, m), "Lj": (B, m), "X": (B, pc, n), "Z": (B, pc, n), "pc": (B, n), "V": (B, m, n),
                 "P": (B, m, n), "fit": (B, lam), "fit_sorted": (B, lam), "prev_fit": (B, lam), "t": (B, m),
                 "vec": (B, m), "arindex": (B, lam), "rank": (B, lam), "itr": (B,), "live": (B,),
-                "counteval": (B,), "ncoll": (B, pc), "nsamp": (B, pc), "epoch": (B,)}[name]
+                "counteval": (B,), "ncoll": (B, pc), "nsamp": (B, pc), "epoch": (B,), "map_of": (B,)}[name]
 
     def get(self, name):
         shp = self._shape_of(name)
