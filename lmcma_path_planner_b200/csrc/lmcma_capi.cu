@@ -168,16 +168,17 @@ UpdateArgs update_args_local(lmcma_b200_opt* o) {
     return a;
 }
 
-int cost_args_for(lmcma_b200_opt* o, CostArgs* a) {
-    if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached (call lmcma_b200_attach_cost)");
-    memset(a, 0, sizeof(*a));
-    a->W = o->obj.waypoints; a->w_len = o->obj.w_len; a->w_clr = o->obj.w_clr; a->w_col = o->obj.w_col;
-    a->X = o->d.X; a->ld = o->d.ns; a->inst_rows = o->d.pop_count;
-    a->ends = o->d_ends; a->ends_per_instance = 1;
-    a->f = o->d.fit; a->f_stride = o->d.lambda; a->f_offset = o->d.pop_offset;
-    a->ncoll = o->d.ncoll; a->nsamp = o->d.nsamp;
-    if (o->maps.size() > 1) { a->maps = o->d_maps; a->map_of = o->d_map_of; a->map_count = (int)o->maps.size(); }
-    return 0;
+// the k_cost arguments of the attached cost (callers have checked need_cost)
+CostArgs cost_args_for(const lmcma_b200_opt* o) {
+    CostArgs a;
+    memset(&a, 0, sizeof(a));
+    a.W = o->obj.waypoints; a.w_len = o->obj.w_len; a.w_clr = o->obj.w_clr; a.w_col = o->obj.w_col;
+    a.X = o->d.X; a.ld = o->d.ns; a.inst_rows = o->d.pop_count;
+    a.ends = o->d_ends; a.ends_per_instance = 1;
+    a.f = o->d.fit; a.f_stride = o->d.lambda; a.f_offset = o->d.pop_offset;
+    a.ncoll = o->d.ncoll; a.nsamp = o->d.nsamp;
+    if (o->maps.size() > 1) { a.maps = o->d_maps; a.map_of = o->d_map_of; a.map_count = (int)o->maps.size(); }
+    return a;
 }
 
 // every launch of the attached cost (the generations, rescore_best, profile_kernels): the map passed by value gives the
@@ -213,27 +214,17 @@ int host_rng_and_sample(lmcma_b200_opt* o, cudaStream_t st, bool mirror, bool pr
     return launch_sample(o, st, mirror, o->cfg.rng != LMCMA_B200_RNG_HANSEN, progressive);
 }
 
-// a sampler has been enqueued or replayed (mirror: it wrote the host mirror): the host's record of the population is stale
-void new_population(lmcma_b200_opt* o, bool mirror) {
-    o->x_cache_valid = false;
-    o->sample_idx = 0;
-    o->xh_fresh = mirror && o->x_mirror;
-}
-
 // lmcma_b200_reset_instances(_dev): k_reset, then the sampler for the flagged instances only, a plain launch (the
 // generation's PDL and hand-over pair a sampler with the k_update before it).  mirror: the sampler writes the flagged rows
-// of the host mirror, so the mirror is as fresh as it was; without it the mirror is stale.  No graph is dropped: the
-// captured ones read the state, the end points and the flags through pointers.
+// of the host mirror.  No graph is dropped: the captured ones read the state, the end points and the flags through pointers.
 int enqueue_reset(lmcma_b200_opt* o, cudaStream_t st, ResetArgs a, bool mirror) {
     a.sigma_default = o->cfg.sigma0;
     a.d_ends = o->d_ends;
+    state_written(o);                                            // the speculative pass saw the retired instances
     int rc = launch(k_reset, o->d.B, 256, 0, st, false, o->d, a);
     if (!rc) rc = launch_sample(o, st, mirror, false, false, 1, a.flags);
     if (rc) return rc;
-    o->spec_valid = false;                                       // the speculative pass saw the retired instances
-    o->x_cache_valid = false;
-    o->sample_idx = 0;
-    o->xh_fresh = o->xh_fresh && mirror;
+    new_population(o, mirror && o->xh_fresh);                    // the other instances keep their rows
     return 0;
 }
 
@@ -241,9 +232,7 @@ int enqueue_reset(lmcma_b200_opt* o, cudaStream_t st, ResetArgs a, bool mirror) 
 enum class Fit { COST, FROM_HOST, IN_PLACE };
 
 int launch_own_cost(lmcma_b200_opt* o, cudaStream_t st) {
-    CostArgs ca;
-    int rc = cost_args_for(o, &ca);
-    return rc ? rc : launch_attached_cost(o, ca, o->d.pop_count, st);
+    return launch_attached_cost(o, cost_args_for(o), o->d.pop_count, st);
 }
 
 // One generation in stream order (fit: COST or IN_PLACE): [k_cost ->] k_rank -> k_update -> [HANSEN deviates ->] the
@@ -297,9 +286,9 @@ int enqueue_forked(lmcma_b200_opt* o, cudaStream_t st, Fit fit, bool mirror, int
 // update: inject_z samples
 int generation_tail(lmcma_b200_opt* o, cudaStream_t st, bool mirror) {
     const bool sample = o->cfg.rng != LMCMA_B200_RNG_INJECT || o->pending_z;
+    state_written(o);                                            // a whole update
     int rc = enqueue_linear(o, st, Fit::IN_PLACE, mirror, sample);
     if (rc) return rc;
-    o->spec_valid = false;                                       // a whole update: whatever the speculative pass left is stale
     if (!sample) o->needs_sample = true;
     o->pending_z = false;
     new_population(o, sample && mirror);
@@ -355,6 +344,22 @@ int replay(const Graph& g, cudaStream_t st) {
     CU(cudaGraphLaunch(g.exec, st));
     g_launches += g.launches;
     return 0;
+}
+
+// The device-side entry points (tell_all_dev, reset_instances_dev) enqueue through here: enqueue(captured) on o->stream,
+// captured when o->stream is in the caller's stream capture.  Then enqueue must replay or build no library graph and
+// allocate or synchronise nothing; its kernels are counted by nobody (they run when the caller replays the graph), and
+// the handle has caller_graphs from then on.
+template <class Enqueue>
+int enqueue_dev(lmcma_b200_opt* o, Enqueue&& enqueue) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    CU(cudaStreamIsCapturing(o->stream, &cs));
+    if (cs == cudaStreamCaptureStatusNone) return enqueue(false);
+    long long uncounted = 0;
+    CountLaunchesIn counted(&uncounted);
+    const int rc = enqueue(true);
+    o->caller_graphs = true;
+    return rc;
 }
 
 // LMCMA_B200_DBG: the device timeline (TimelineSlot) on stderr, in ns after its earliest stamp ("-": not stamped), then
@@ -443,10 +448,9 @@ int lmcma_capi::check_lost(lmcma_b200_opt* o) {
                 "flight is void - restore the state or recreate the handle (LMCMA_B200_OVERLAP=0 avoids the overlapped graph)",
                 code == LOST_UPDATE_WAITING_FOR_RANK ? "k_update timed out waiting for k_rank" : "k_sample timed out waiting for k_update");
 }
-// After a state setter: on a handle whose generations replay in a caller's graph (caller_graphs), rebuild the pair mirror
-// now, because the next sampler to read it may be a replay that never passes through ensure_mirror
-int lmcma_capi::settle_mirror(lmcma_b200_opt* o) {
-    if (!o->caller_graphs || !o->mirror_dirty) return 0;
+int lmcma_capi::pairs_written(lmcma_b200_opt* o) {
+    o->mirror_dirty = true;
+    if (!o->caller_graphs) return 0;                             // the next library sampler rebuilds it (ensure_mirror)
     int rc = ensure_mirror(o, o->stream);
     if (rc) return rc;
     CU(cudaStreamSynchronize(o->stream));
@@ -620,50 +624,50 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     CU(cudaEventCreate(&o->ev1));
 
     const size_t B = d.B, ns = d.ns, lam = d.lambda, pc = d.pop_count, m = d.m;
-    DM(d.X, B * pc * ns);
-    DM(d.D, B * pc * ns);
-    if (cfg->rng != LMCMA_B200_RNG_PHILOX || cfg->record_z || covariance) DM(d.Z, B * pc * ns);
+    DM(o, d.X, B * pc * ns);
+    DM(o, d.D, B * pc * ns);
+    if (cfg->rng != LMCMA_B200_RNG_PHILOX || cfg->record_z || covariance) DM(o, d.Z, B * pc * ns);
     if (covariance) {   // CMABase::init factors the prior once (cholesky, lmcma.cpp:165-169)
         std::vector<double> Ld((size_t)d.n * d.n);
         if (!cholesky_lower(covariance, d.n, Ld.data())) { return fail(LMCMA_B200_ERR_ARG, "covariance prior is not symmetric positive definite"); }
         std::vector<float> Lf((size_t)d.n * ns, 0.f);
         for (int i = 0; i < d.n; ++i)
             for (int k = 0; k <= i; ++k) Lf[(size_t)i * ns + k] = (float)Ld[(size_t)i * d.n + k];
-        DM(o->d_Lf, (size_t)d.n * ns);
+        DM(o, o->d_Lf, (size_t)d.n * ns);
         CU(cudaMemcpy(o->d_Lf, Lf.data(), Lf.size() * sizeof(float), cudaMemcpyHostToDevice));
         d.Lf = o->d_Lf;
-        DM(d.Zc, B * pc * ns);
+        DM(o, d.Zc, B * pc * ns);
     }
-    DM(d.fit, B * lam); DM(d.fit_sorted, B * lam); DM(d.prev_fit, B * lam);
-    DM(d.rank, B * lam); DM(d.arindex, B * lam);
+    DM(o, d.fit, B * lam); DM(o, d.fit_sorted, B * lam); DM(o, d.prev_fit, B * lam);
+    DM(o, d.rank, B * lam); DM(o, d.arindex, B * lam);
     if (o->plan.rank.tile_sorted) {
-        DM(d.prev_sorted, B * lam); DM(d.tile_sorted, B * lam); DM(d.tile_pos, B * lam);
+        DM(o, d.prev_sorted, B * lam); DM(o, d.tile_sorted, B * lam); DM(o, d.tile_pos, B * lam);
     }
-    DM(d.ncoll, B * pc); DM(d.nsamp, B * pc);
-    DM(d.xmean, B * ns); DM(d.pc, B * ns);
-    DM(d.V, B * m * ns); DM(d.P, B * m * ns);
-    DM(d.Nj, B * m); DM(d.Lj, B * m); DM(d.Njf, B * m); DM(d.Njs, B * m);
-    DM(d.VPs, B * m * 2 * ns);
-    DM(d.t, B * m); DM(d.vec, B * m);
-    DM(d.sc, B); DM(d.best_x, B * ns); DM(d.S_count, B); DM(d.done_count, B); DM(d.progress, B * progress_len(m)); DM(d.rank_ticket, B); DM(d.resident, B);
-    if (o->tune.dbg) DM(d.dbg, TL_SLOTS);
-    DM(d.partial, B * d.RS * ns);
+    DM(o, d.ncoll, B * pc); DM(o, d.nsamp, B * pc);
+    DM(o, d.xmean, B * ns); DM(o, d.pc, B * ns);
+    DM(o, d.V, B * m * ns); DM(o, d.P, B * m * ns);
+    DM(o, d.Nj, B * m); DM(o, d.Lj, B * m); DM(o, d.Njf, B * m); DM(o, d.Njs, B * m);
+    DM(o, d.VPs, B * m * 2 * ns);
+    DM(o, d.t, B * m); DM(o, d.vec, B * m);
+    DM(o, d.sc, B); DM(o, d.best_x, B * ns); DM(o, d.S_count, B); DM(o, d.done_count, B); DM(o, d.progress, B * progress_len(m)); DM(o, d.rank_ticket, B); DM(o, d.resident, B);
+    if (o->tune.dbg) DM(o, d.dbg, TL_SLOTS);
+    DM(o, d.partial, B * d.RS * ns);
 
     std::vector<float> wf(o->weights.begin(), o->weights.end());
-    DM(o->d_w, d.mu);
+    DM(o, o->d_w, d.mu);
     CU(cudaMemcpy(o->d_w, wf.data(), d.mu * sizeof(float), cudaMemcpyHostToDevice));
     d.w = o->d_w;
     if (lo) {   // padded to the row stride so that the kernels clamp whole float4 columns
         o->lo_f.assign(d.ns, -std::numeric_limits<float>::max());
         for (int k = 0; k < d.n; ++k) o->lo_f[k] = (float)lo[k];
-        DM(o->d_lo, d.ns);
+        DM(o, o->d_lo, d.ns);
         CU(cudaMemcpy(o->d_lo, o->lo_f.data(), d.ns * sizeof(float), cudaMemcpyHostToDevice));
         d.lo = o->d_lo;
     }
     if (hi) {
         o->hi_f.assign(d.ns, std::numeric_limits<float>::max());
         for (int k = 0; k < d.n; ++k) o->hi_f[k] = (float)hi[k];
-        DM(o->d_hi, d.ns);
+        DM(o, o->d_hi, d.ns);
         CU(cudaMemcpy(o->d_hi, o->hi_f.data(), d.ns * sizeof(float), cudaMemcpyHostToDevice));
         d.hi = o->d_hi;
     }
@@ -672,12 +676,11 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
     for (size_t b = 0; b < B; ++b)
         for (int k = 0; k < d.n; ++k) xm[b * ns + k] = x0 ? x0[b * d.n + k] : o->hansen.uniform();
     CU(cudaMemcpy(d.xmean, xm.data(), xm.size() * sizeof(double), cudaMemcpyHostToDevice));
-    std::vector<Scalars> sc(B);
-    for (auto& s : sc) {
+    rc = write_scalars(o, [&](int, Scalars& s) {
         memset(&s, 0, sizeof(s));
         s.sigma = cfg->sigma0; s.s = 0.0; s.best_f = std::numeric_limits<double>::max();
-    }
-    CU(cudaMemcpy(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice));
+    });
+    if (rc) return rc;
 
     o->overlap = o->plan.overlap;
     if (o->overlap) {
@@ -692,14 +695,14 @@ static int create_body(lmcma_b200_opt* o, DeviceProps* props, const lmcma_b200_c
         if (o->overlap && o->tune.overlap != 2 && probe_coschedule(o) != 1) o->overlap = false;
         if (o->overlap && o->tune.tell_spec != 0) {              // scratch of the speculative update (best effort)
             o->spec_stride = (spec_floats(m, d.ns) + 3) & ~(size_t)3;
-            if (cudaMalloc(&o->d_spec, B * o->spec_stride * sizeof(float)) != cudaSuccess) { cudaGetLastError(); o->d_spec = nullptr; }
+            if (o->buffers.alloc(&o->d_spec, B * o->spec_stride)) { cudaGetLastError(); o->d_spec = nullptr; }
             else cudaMemset(o->d_spec, 0xff, B * o->spec_stride * sizeof(float));   // generation -1: matches nothing
         }
     }
     if (o->plan.update.gram) {
-        DM(d.G, B * GRAM_KS * m * m);
-        DM(d.Cf, B * m * m);
-        DM(d.gram_hdr, B);
+        DM(o, d.G, B * GRAM_KS * m * m);
+        DM(o, d.Cf, B * m * m);
+        DM(o, d.gram_hdr, B);
     }
     o->f_host.assign(B * lam, 0.f);
     // first population (LMCMA::init -> sample(), lmcma.cpp:298)
@@ -717,13 +720,9 @@ int lmcma_b200_destroy(lmcma_b200_opt* o) {
     if (!o) return 0;
     cudaSetDevice(o->cfg.device);
     if (o->stream) cudaStreamSynchronize(o->stream);
-    OptDev& d = o->d;
-    void* ptrs[] = {d.prev_sorted, d.tile_sorted, d.tile_pos, d.X, d.D, d.Z, d.Zc, o->d_Lf, d.fit, d.fit_sorted, d.prev_fit, d.rank, d.arindex, d.ncoll, d.nsamp, d.xmean, d.pc, d.V, d.P,
-                    d.Nj, d.Lj, d.Njf, d.Njs, d.VPs, d.dbg, d.G, d.Cf, d.gram_hdr, d.t, d.vec, d.sc, d.best_x, d.S_count, d.done_count, d.progress, d.rank_ticket, d.resident, d.partial, o->d_lo, o->d_hi, o->d_w, o->d_ends, o->d_rescore, o->d_reset, o->d_maps, o->d_map_of};
-    for (void* p : ptrs) cudaFree(p);
+    o->buffers.free_all();
     drop_fused_graphs(o);
     drop_tell_graphs(o);
-    cudaFree(o->d_spec);
     if (o->f_pinned) cudaFreeHost(o->f_pinned);
     if (o->err_host) cudaFreeHost(o->err_host);
     if (o->x_mirror) { unregister_mirror(o->x_mirror); cudaFreeHost(o->x_mirror); }
@@ -773,7 +772,7 @@ int lmcma_b200_inject_z(lmcma_b200_opt* o, const float* Z) {
 
 int lmcma_b200_resample(lmcma_b200_opt* o) {
     ARG(o, "null handle");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no deviates yet: inject_z first");
+    TRY(need_population(o, "resample"));
     if (o->cfg.rng == LMCMA_B200_RNG_HANSEN) return fail(LMCMA_B200_ERR_STATE, "resample would advance the serial HANSEN stream");
     CU(cudaSetDevice(o->cfg.device));
     int rc = launch_sample(o, o->stream, true);
@@ -785,7 +784,7 @@ int lmcma_b200_resample(lmcma_b200_opt* o) {
 
 int lmcma_b200_ask_all(lmcma_b200_opt* o, float* X) {
     ARG(o && X, "null pointer");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet: inject_z first");
+    TRY(need_population(o, "ask_all"));
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     int rc = d2h_rows(X, d.X, (size_t)d.B * d.pop_count, d.n * sizeof(float), d.ns * sizeof(float), o->stream);
@@ -794,7 +793,7 @@ int lmcma_b200_ask_all(lmcma_b200_opt* o, float* X) {
 
 int lmcma_b200_ask_all_view(lmcma_b200_opt* o, const float** X_view, int64_t* ld_out) {
     ARG(o && X_view, "null pointer");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet: inject_z first");
+    TRY(need_population(o, "ask_all_view"));
     CU(cudaSetDevice(o->cfg.device));
     OptDev& d = o->d;
     const size_t floats = (size_t)d.B * d.pop_count * d.ns;
@@ -821,8 +820,8 @@ int lmcma_b200_ask_all_view(lmcma_b200_opt* o, const float** X_view, int64_t* ld
 
 int lmcma_b200_tell_all(lmcma_b200_opt* o, const float* f) {
     ARG(o && f, "null pointer");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet: inject_z first");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles use the mg_* entry points");
+    TRY(need_population(o, "tell_all"));
+    TRY(need_unsplit(o, "tell_all"));
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     int rc;
@@ -860,38 +859,33 @@ int lmcma_b200_device_buffers(lmcma_b200_opt* o, const float** X_dev, int64_t* l
 
 int lmcma_b200_tell_all_dev(lmcma_b200_opt* o) {
     ARG(o, "null handle");
-    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "tell_all_dev needs the PHILOX rng (HANSEN / INJECT: tell_all)");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles use the mg_* entry points");
+    TRY(need_philox(o, "tell_all_dev"));                         // HANSEN / INJECT: tell_all
+    TRY(need_unsplit(o, "tell_all_dev"));
     CU(cudaSetDevice(o->cfg.device));
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    CU(cudaStreamIsCapturing(o->stream, &cs));
-    int rc = 0;
-    if (cs != cudaStreamCaptureStatusNone) {
-        // the caller's capture: no library graph is replayed or built, nothing allocated or synchronised.  The linear
-        // generation (same bits as the forked one) keeps kernels that spin on a partner out of a graph the library does not
-        // control.  Its kernels are counted by nobody: they run when the caller replays the graph
-        long long uncounted = 0;
-        CountLaunchesIn counted(&uncounted);
-        rc = generation_tail(o, o->stream, false);
-        o->caller_graphs = true;
-    } else if (forked_tell(o, o->tell_dev) && (rc = ensure_tell_graph(o, true)) == 0 && o->tell_dev.whole.exec) {
-        // one query: the forked graph of tell_all without the fitness copy (and without the speculative pass, DESIGN.md 4.4)
-        rc = replay(o->tell_dev.whole, o->stream);
-        o->spec_valid = false;
-        new_population(o, false);
-    } else if (!rc) {
-        rc = generation_tail(o, o->stream, false);
-    }
-    return rc;
+    return enqueue_dev(o, [&](bool captured) {
+        // in the caller's capture, the linear generation (same bits as the forked one) keeps kernels that spin on a partner
+        // out of a graph the library does not control
+        if (!captured && forked_tell(o, o->tell_dev)) {
+            // one query: the forked graph of tell_all without the fitness copy (and without the speculative pass, DESIGN.md 4.4)
+            int rc = ensure_tell_graph(o, true);
+            if (rc) return rc;
+            if (o->tell_dev.whole.exec) {
+                rc = replay(o->tell_dev.whole, o->stream);
+                state_written(o);
+                new_population(o, false);
+                return rc;
+            }
+        }
+        return generation_tail(o, o->stream, false);
+    });
 }
 
 // what lmcma_b200_reset_instances(_dev) refuses with ERR_STATE: HANSEN / INJECT draw their deviates on the host, a split
 // population's best and slots live on several handles, and end points need the device end points of an attached cost
 static int reset_refused(const lmcma_b200_opt* o, bool ends) {
-    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "reset_instances needs the PHILOX rng");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "reset_instances: split-population handles are not supported");
-    if (ends && !o->d_ends) return fail(LMCMA_B200_ERR_STATE, "reset_instances: end points need an attached cost (lmcma_b200_attach_cost)");
-    return 0;
+    TRY(need_philox(o, "reset_instances"));
+    TRY(need_unsplit(o, "reset_instances"));
+    return ends ? need_cost(o, "reset_instances with end points") : 0;
 }
 
 // o->d_reset: sigma0 (B doubles), x0 (B x n doubles), ends (B x 6 floats), flags (B ints), each at a 16-byte boundary
@@ -930,7 +924,7 @@ int lmcma_b200_reset_instances(lmcma_b200_opt* o, int32_t count, const int32_t* 
     }
     CU(cudaSetDevice(o->cfg.device));
     const ResetLayout l = reset_layout(d);
-    if (!o->d_reset) DM(o->d_reset, l.bytes);
+    if (!o->d_reset) DM(o, o->d_reset, l.bytes);
     // only rows [lo, hi] of x0, sigma0 and the end points cross PCIe; the flags of every instance do
     const size_t rows = (size_t)(hi - lo + 1);
     std::vector<double> xs(rows * n), ss(rows, o->cfg.sigma0);
@@ -939,8 +933,7 @@ int lmcma_b200_reset_instances(lmcma_b200_opt* o, int32_t count, const int32_t* 
         const size_t r = (size_t)(idx[i] - lo);
         std::copy(x0 + (size_t)i * n, x0 + (size_t)(i + 1) * n, xs.begin() + r * n);
         if (sigma0) ss[r] = sigma0[i];
-        if (ends)
-            for (int c = 0; c < 3; ++c) { es[r * 6 + c] = ends[i].start[c]; es[r * 6 + 3 + c] = ends[i].goal[c]; }
+        if (ends) pack_ends(ends + i, 1, &es[r * 6]);
     }
     ResetArgs a;
     memset(&a, 0, sizeof(a));
@@ -969,21 +962,14 @@ int lmcma_b200_reset_instances_dev(lmcma_b200_opt* o, const int32_t* flags_dev, 
     memset(&a, 0, sizeof(a));
     a.flags = flags_dev; a.x0 = x0_dev; a.sigma0 = sigma0_dev; a.ends = ends_dev;
     a.best_x_out = best_x_out_dev; a.best_f_out = best_f_out_dev;
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    CU(cudaStreamIsCapturing(o->stream, &cs));
-    if (cs == cudaStreamCaptureStatusNone) return enqueue_reset(o, o->stream, a, false);
-    // the caller's capture, as in lmcma_b200_tell_all_dev: its kernels run, uncounted, when the caller replays the graph
-    long long uncounted = 0;
-    CountLaunchesIn counted(&uncounted);
-    rc = enqueue_reset(o, o->stream, a, false);
-    o->caller_graphs = true;
-    return rc;
+    return enqueue_dev(o, [&](bool) { return enqueue_reset(o, o->stream, a, false); });
 }
 
 int lmcma_b200_ask_one(lmcma_b200_opt* o, double* params, int32_t n) {
     ARG(o && params, "null pointer");
     ARG(n == o->d.n, "N mismatch");
-    if (o->d.B != 1 || o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "ask_one needs batch == 1 and an unsplit population");
+    TRY(need_batch_of_one(o, "ask_one"));
+    TRY(need_unsplit(o, "ask_one"));
     if (!o->x_cache_valid || o->caller_graphs) {                  // a replay of the caller's graph may have moved on
         o->x_cache.resize((size_t)o->d.lambda * o->d.n);
         int rc = lmcma_b200_ask_all(o, o->x_cache.data());
@@ -996,7 +982,8 @@ int lmcma_b200_ask_one(lmcma_b200_opt* o, double* params, int32_t n) {
 
 int lmcma_b200_tell_one(lmcma_b200_opt* o, const double* feedbacks, int32_t num) {
     ARG(o && (feedbacks || num == 0) && num >= 0, "null pointer");
-    if (o->d.B != 1 || o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "tell_one needs batch == 1 and an unsplit population");
+    TRY(need_batch_of_one(o, "tell_one"));
+    TRY(need_unsplit(o, "tell_one"));
     double f = 0.0;                                    // lmcma.cpp:186-188
     for (int i = 0; i < num; ++i) f += feedbacks[i];
     // the device ranks FP32 values: keep huge penalties finite and ordered instead of letting them round to +-inf
@@ -1012,23 +999,19 @@ int lmcma_b200_tell_one(lmcma_b200_opt* o, const double* feedbacks, int32_t num)
 int lmcma_b200_is_done(lmcma_b200_opt* o, int32_t* done) {
     ARG(o && done, "null pointer");
     CU(cudaSetDevice(o->cfg.device));
-    std::vector<Scalars> sc(o->d.B);
-    CU(cudaMemcpyAsync(sc.data(), o->d.sc, sc.size() * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-    CU(cudaStreamSynchronize(o->stream));
-    for (int b = 0; b < o->d.B; ++b) done[b] = sc[b].sigma < 1e-20 ? 1 : 0;   // lmcma.cpp:426-429
-    return 0;
+    return read_scalars(o, [&](int b, const Scalars& s) { done[b] = s.sigma < 1e-20 ? 1 : 0; });   // lmcma.cpp:426-429
 }
 
 // what attach_cost and attach_cost_maps share once their arguments are checked: the objective, the end points, the cost's
-// launch shape, and the graphs that launched the previous cost
+// launch shape, and the graphs that launched the previous cost.  The end points are on the device before o->map is set
+// (need_cost: an attached cost has them)
 static int attach_body(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b200_objective* obj, const lmcma_b200_endpoints* ends) {
     CU(cudaSetDevice(o->cfg.device));
-    o->map = map; o->obj = *obj;
     std::vector<float> e6((size_t)o->d.B * 6);
-    for (int b = 0; b < o->d.B; ++b)
-        for (int c = 0; c < 3; ++c) { e6[b * 6 + c] = ends[b].start[c]; e6[b * 6 + 3 + c] = ends[b].goal[c]; }
-    if (!o->d_ends) DM(o->d_ends, (size_t)o->d.B * 6);
+    pack_ends(ends, o->d.B, e6.data());
+    if (!o->d_ends) DM(o, o->d_ends, (size_t)o->d.B * 6);
     CU(cudaMemcpy(o->d_ends, e6.data(), e6.size() * sizeof(float), cudaMemcpyHostToDevice));
+    o->map = map; o->obj = *obj;
     o->cost_shape = pick_cost_shape(obj->waypoints, ends[0].start, ends[0].goal, map->dev.dims, o->tune);
     drop_fused_graphs(o);
     return 0;
@@ -1048,7 +1031,7 @@ int lmcma_b200_attach_cost(lmcma_b200_opt* o, lmcma_b200_map* map, const lmcma_b
 int lmcma_b200_attach_cost_maps(lmcma_b200_opt* o, int32_t map_count, lmcma_b200_map* const* maps, const int32_t* map_of,
                                 const lmcma_b200_objective* obj, const lmcma_b200_endpoints* ends) {
     ARG(o && maps && map_of && obj && ends, "null pointer");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "attach_cost_maps: split-population handles take one map (attach_cost)");
+    TRY(need_unsplit(o, "attach_cost_maps"));                    // a split population takes one map: attach_cost
     ARG(map_count >= 1, "map_count must be >= 1");
     for (int k = 0; k < map_count; ++k) {
         ARG(maps[k], "null map");
@@ -1069,11 +1052,11 @@ int lmcma_b200_attach_cost_maps(lmcma_b200_opt* o, int32_t map_count, lmcma_b200
     std::vector<MapDev> table((size_t)map_count);
     for (int k = 0; k < map_count; ++k) table[k] = maps[k]->dev;
     if (o->d_maps_cap < (size_t)map_count) {
-        cudaFree(o->d_maps); o->d_maps = nullptr; o->d_maps_cap = 0;
-        DM(o->d_maps, (size_t)map_count);
+        o->d_maps_cap = 0;
+        DM(o, o->d_maps, (size_t)map_count);
         o->d_maps_cap = (size_t)map_count;
     }
-    if (!o->d_map_of) DM(o->d_map_of, (size_t)o->d.B);
+    if (!o->d_map_of) DM(o, o->d_map_of, (size_t)o->d.B);
     CU(cudaMemcpyAsync(o->d_maps, table.data(), table.size() * sizeof(MapDev), cudaMemcpyHostToDevice, o->stream));
     CU(cudaMemcpyAsync(o->d_map_of, map_of, (size_t)o->d.B * sizeof(int), cudaMemcpyHostToDevice, o->stream));
     CU(cudaStreamSynchronize(o->stream));
@@ -1090,13 +1073,15 @@ int lmcma_b200_instance_maps_dev(lmcma_b200_opt* o, int32_t** map_of_dev) {
 
 int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
     ARG(o && generations >= 0, "bad argument");
-    if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet: inject_z first");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles use the mg_* entry points");
+    TRY(need_cost(o, "run"));
+    TRY(need_population(o, "run"));
+    TRY(need_unsplit(o, "run"));
+    if (o->cfg.rng == LMCMA_B200_RNG_INJECT && generations > 1)
+        return fail(LMCMA_B200_ERR_STATE, "INJECT rng: run one generation per injected Z");
     CU(cudaSetDevice(o->cfg.device));
+    state_written(o);
     int rc = attached_l2_window(o, o->stream);
     if (rc) return rc;
-    o->spec_valid = false;                                       // the fused generations advance the state past what tell_all's speculative pass saw
     if (o->cfg.rng == LMCMA_B200_RNG_PHILOX) {
         if ((rc = ensure_graph(o))) return rc;
         CU(cudaEventRecord(o->ev0, o->stream));                  // after the (host-side) graph build: last_run_ms is device time
@@ -1108,8 +1093,6 @@ int lmcma_b200_run(lmcma_b200_opt* o, int32_t generations) {
         }
         if (generations > 0) new_population(o, false);           // the graph's sampler does not write the host mirror
     } else {
-        if (o->cfg.rng == LMCMA_B200_RNG_INJECT && generations > 1)
-            return fail(LMCMA_B200_ERR_STATE, "INJECT rng: run one generation per injected Z");
         CU(cudaEventRecord(o->ev0, o->stream));
         for (int g = 0; g < generations; ++g)
             if ((rc = launch_own_cost(o, o->stream)) || (rc = generation_tail(o, o->stream, true))) return rc;
@@ -1137,15 +1120,15 @@ int lmcma_b200_last_run_ms(lmcma_b200_opt* o, float* ms) {
 
 int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms4) {
     ARG(o && ms4 && generations >= 1, "bad argument");
-    if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached");
-    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "profile_kernels needs the PHILOX rng");
+    TRY(need_cost(o, "profile_kernels"));
+    TRY(need_philox(o, "profile_kernels"));
     CU(cudaSetDevice(o->cfg.device));
-    CostArgs ca;
-    int rc = cost_args_for(o, &ca);
-    if (rc) return rc;
+    const CostArgs ca = cost_args_for(o);
     cudaStream_t st = o->stream;
     std::vector<cudaEvent_t> ev((size_t)generations * 5);
     for (auto& e : ev) CU(cudaEventCreate(&e));
+    state_written(o);
+    int rc = 0;
     for (int g = 0; g < generations && !rc; ++g) {
         cudaEvent_t* e = &ev[(size_t)g * 5];
         cudaEventRecord(e[0], st);
@@ -1158,7 +1141,6 @@ int lmcma_b200_profile_kernels(lmcma_b200_opt* o, int32_t generations, float* ms
         if (!rc) rc = launch_sample(o, st, true);
         cudaEventRecord(e[4], st);
     }
-    o->spec_valid = false;
     new_population(o, true);
     cudaError_t se = cudaStreamSynchronize(st);
     if (!rc && se != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "profile run: %s", cudaGetErrorString(se));
@@ -1218,31 +1200,24 @@ int lmcma_b200_best(lmcma_b200_opt* o, float* x_best, float* f_best) {
         int rc = d2h_rows(x_best, d.best_x, d.B, d.n * sizeof(float), d.ns * sizeof(float), o->stream);
         if (rc) return rc;
     }
-    if (f_best) {
-        std::vector<Scalars> sc(d.B);
-        CU(cudaMemcpyAsync(sc.data(), d.sc, sc.size() * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-        CU(cudaStreamSynchronize(o->stream));
-        for (int b = 0; b < d.B; ++b) f_best[b] = (float)sc[b].best_f;
-    }
-    return 0;
+    return f_best ? read_scalars(o, [&](int b, const Scalars& s) { f_best[b] = (float)s.best_f; }) : 0;
 }
 
 int lmcma_b200_rescore_best(lmcma_b200_opt* o) {
     ARG(o, "null handle");
-    if (!o->map) return fail(LMCMA_B200_ERR_STATE, "no cost attached (call lmcma_b200_attach_cost)");
-    if (o->d.pop_count != o->d.lambda) return fail(LMCMA_B200_ERR_STATE, "split-population handles: best_x may hold a peer's row");
+    TRY(need_cost(o, "rescore_best"));
+    TRY(need_unsplit(o, "rescore_best"));                        // best_x may hold a peer's row
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
-    if (!o->d_rescore) DM(o->d_rescore, (size_t)d.B);
-    CostArgs ca;
-    int rc = cost_args_for(o, &ca);
-    if (rc) return rc;
+    if (!o->d_rescore) DM(o, o->d_rescore, (size_t)d.B);
+    state_written(o);                                            // like the state setters: tell_all's speculative pass saw the old best
+    CostArgs ca = cost_args_for(o);
     ca.X = d.best_x; ca.inst_rows = 1;                           // one row per instance, the instance's own end points
     ca.f = o->d_rescore; ca.f_stride = 1; ca.f_offset = 0; ca.ncoll = nullptr; ca.nsamp = nullptr;
-    if ((rc = attached_l2_window(o, o->stream))) return rc;
+    int rc = attached_l2_window(o, o->stream);
+    if (rc) return rc;
     if ((rc = launch_attached_cost(o, ca, 1, o->stream))) return rc;   // each instance's best_x on its own map
     if ((rc = launch(k_set_best_f, (unsigned)((d.B + 127) / 128), 128, 0, o->stream, false, d.sc, (const float*)o->d_rescore, d.B))) return rc;
-    o->spec_valid = false;                                       // like the state setters: tell_all's speculative pass saw the old best
     CU(cudaStreamSynchronize(o->stream));
     return 0;
 }
@@ -1256,21 +1231,21 @@ int lmcma_b200_mg_payload_floats(lmcma_b200_opt* o, int32_t* floats_out) {
 
 int lmcma_b200_mg_evaluate(lmcma_b200_opt* o, float* f_local_dev, void* stream) {
     ARG(o && f_local_dev, "null pointer");
-    if (o->d.B != 1) return fail(LMCMA_B200_ERR_STATE, "split-population mode needs batch == 1");
-    if (o->needs_sample) return fail(LMCMA_B200_ERR_STATE, "no population yet");
+    TRY(need_batch_of_one(o, "mg_evaluate"));
+    TRY(need_population(o, "mg_evaluate"));
+    TRY(need_cost(o, "mg_evaluate"));
     CU(cudaSetDevice(o->cfg.device));
-    CostArgs ca;
-    int rc = cost_args_for(o, &ca);
-    if (rc) return rc;
+    CostArgs ca = cost_args_for(o);
     ca.f = f_local_dev; ca.f_stride = o->d.pop_count; ca.f_offset = 0;
     cudaStream_t st = stream ? (cudaStream_t)stream : o->stream;
-    if ((rc = apply_l2_window(o->map, st))) return rc;
+    int rc = apply_l2_window(o->map, st);
+    if (rc) return rc;
     return launch_cost(o->map->dev, ca, o->d.pop_count, o->d.B, o->cost_shape, false, st);
 }
 
 int lmcma_b200_mg_rank(lmcma_b200_opt* o, const float* f_all_dev, float* payload_dev, void* stream) {
     ARG(o && f_all_dev && payload_dev, "null pointer");
-    if (o->d.B != 1) return fail(LMCMA_B200_ERR_STATE, "split-population mode needs batch == 1");
+    TRY(need_batch_of_one(o, "mg_rank"));
     CU(cudaSetDevice(o->cfg.device));
     cudaStream_t st = stream ? (cudaStream_t)stream : o->stream;
     // keep the gathered fitness: k_update needs it for prev_fit / best tracking
@@ -1280,7 +1255,7 @@ int lmcma_b200_mg_rank(lmcma_b200_opt* o, const float* f_all_dev, float* payload
 
 int lmcma_b200_mg_update(lmcma_b200_opt* o, const float* payload_all_dev, int32_t world, void* stream) {
     ARG(o && payload_all_dev && world >= 1, "bad argument");
-    if (o->cfg.rng != LMCMA_B200_RNG_PHILOX) return fail(LMCMA_B200_ERR_STATE, "split-population mode needs the PHILOX rng");   // before anything is launched
+    TRY(need_philox(o, "mg_update"));
     CU(cudaSetDevice(o->cfg.device));
     cudaStream_t st = stream ? (cudaStream_t)stream : o->stream;
     const long long pf = o->d.ns + 4;
@@ -1288,9 +1263,9 @@ int lmcma_b200_mg_update(lmcma_b200_opt* o, const float* payload_all_dev, int32_
     memset(&a, 0, sizeof(a));
     a.f_all = o->d.fit; a.slices = payload_all_dev; a.n_slices = world;
     a.slice_stride = (long long)o->d.B * pf; a.inst_stride = pf; a.payload_mode = 1;
+    state_written(o);
     int rc = launch_update(o, a, false, st);
     if (!rc) rc = launch_sample(o, st, false, true);
-    o->spec_valid = false;
     new_population(o, false);
     return rc;
 }

@@ -160,10 +160,10 @@ static int map_alloc(int device, int dims, const int32_t* shape, int storage, fl
     rc = 0;
     cudaError_t e = cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) rc = fail(LMCMA_B200_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
-    if (!rc && storage == LMCMA_B200_MAP_F32) { rc = dmalloc(&m->d_g32, m->stored); m->dev.g32 = m->d_g32; }   // padding cells are never addressed
+    if (!rc && storage == LMCMA_B200_MAP_F32) { rc = m->buffers.alloc(&m->d_g32, m->stored); m->dev.g32 = m->d_g32; }   // padding cells are never addressed
     if (!rc && storage == LMCMA_B200_MAP_U8) {
-        rc = dmalloc(&m->d_q8, m->stored);
-        if (!rc) rc = dmalloc(&m->d_lut, 256);
+        rc = m->buffers.alloc(&m->d_q8, m->stored);
+        if (!rc) rc = m->buffers.alloc(&m->d_lut, 256);
         if (!rc) {
             float lut[256];
             lut[0] = -m->dev.g_coll;
@@ -356,8 +356,7 @@ int lmcma_b200_map_update_occupancy(lmcma_b200_map* m, const int32_t* lo_xyz, co
 int lmcma_b200_map_destroy(lmcma_b200_map* m) {
     if (!m) return 0;
     cudaSetDevice(m->device);
-    cudaFree(m->d_g32); cudaFree(m->d_q8); cudaFree(m->d_lut); cudaFree(m->d_X); cudaFree(m->d_f);
-    cudaFree(m->d_nc); cudaFree(m->d_ns);
+    m->buffers.free_all();
     if (m->d_update) { cudaFreeAsync(m->d_update, m->stream); cudaStreamSynchronize(m->stream); }
     if (m->stream) cudaStreamDestroy(m->stream);
     delete m;
@@ -429,6 +428,11 @@ int lmcma_capi::check_obj(const lmcma_b200_map* m, const lmcma_b200_objective* o
     ARG(obj->waypoints >= 1 && obj->waypoints <= 8190, "waypoints out of range");
     return 0;
 }
+// the end points of `count` queries as k_cost reads them (CostArgs::ends, ends0): start xyz then goal xyz, six floats each
+void lmcma_capi::pack_ends(const lmcma_b200_endpoints* ends, int count, float* out) {
+    for (int i = 0; i < count; ++i)
+        for (int c = 0; c < 3; ++c) { out[i * 6 + c] = ends[i].start[c]; out[i * 6 + 3 + c] = ends[i].goal[c]; }
+}
 extern "C" {
 
 int lmcma_b200_cost_evaluate_dev(lmcma_b200_map* m, const lmcma_b200_objective* obj, const lmcma_b200_endpoints* ends,
@@ -445,7 +449,7 @@ int lmcma_b200_cost_evaluate_dev(lmcma_b200_map* m, const lmcma_b200_objective* 
     memset(&a, 0, sizeof(a));
     a.W = obj->waypoints; a.w_len = obj->w_len; a.w_clr = obj->w_clr; a.w_col = obj->w_col;
     a.X = X_dev; a.ld = ld; a.inst_rows = count; a.ends = nullptr; a.ends_per_instance = 0;
-    for (int c = 0; c < 3; ++c) { a.ends0[c] = ends->start[c]; a.ends0[3 + c] = ends->goal[c]; }   // by value: nothing shared between callers
+    pack_ends(ends, 1, a.ends0);                                 // by value: nothing shared between callers
     a.f = f_dev; a.f_stride = count; a.f_offset = 0; a.ncoll = ncoll_dev; a.nsamp = nsamp_dev;
     if ((rc = apply_l2_window(m, st))) return rc;
     return launch_cost(m->dev, a, count, 1, pick_cost_shape(a.W, ends->start, ends->goal, m->dev.dims, m->tune), false, st);
@@ -480,8 +484,8 @@ int lmcma_b200_cost_evaluate(lmcma_b200_map* m, const lmcma_b200_objective* obj,
     const bool out_direct = f_dev && (!ncoll_host || nc_dev) && (!nsamp_host || ns_dev);
     if (!X_dev) {
         if (m->d_X_cap < (size_t)count * n) {
-            cudaFree(m->d_X); m->d_X = nullptr; m->d_X_cap = 0;
-            DM(m->d_X, (size_t)count * n);
+            m->d_X_cap = 0;
+            DM(m, m->d_X, (size_t)count * n);
             m->d_X_cap = (size_t)count * n;
         }
         CU(cudaMemcpyAsync(m->d_X, X_host, (size_t)count * n * sizeof(float), cudaMemcpyHostToDevice, m->stream));
@@ -489,9 +493,8 @@ int lmcma_b200_cost_evaluate(lmcma_b200_map* m, const lmcma_b200_objective* obj,
     }
     if (!out_direct) {
         if (m->d_out_cap < (size_t)count) {
-            cudaFree(m->d_f); cudaFree(m->d_nc); cudaFree(m->d_ns);
-            m->d_f = nullptr; m->d_nc = nullptr; m->d_ns = nullptr; m->d_out_cap = 0;
-            DM(m->d_f, count); DM(m->d_nc, count); DM(m->d_ns, count);
+            m->d_out_cap = 0;
+            DM(m, m->d_f, count); DM(m, m->d_nc, count); DM(m, m->d_ns, count);
             m->d_out_cap = count;
         }
         f_dev = m->d_f; nc_dev = m->d_nc; ns_dev = m->d_ns;
@@ -532,7 +535,7 @@ int lmcma_b200_cost_trace(lmcma_b200_map* m, const lmcma_b200_objective* obj, co
     memset(&a, 0, sizeof(a));
     a.W = obj->waypoints; a.w_len = obj->w_len; a.w_clr = obj->w_clr; a.w_col = obj->w_col;
     a.X = dX; a.ld = (long long)n; a.inst_rows = 1; a.ends = nullptr; a.ends_per_instance = 0;
-    for (int c = 0; c < 3; ++c) { a.ends0[c] = ends->start[c]; a.ends0[3 + c] = ends->goal[c]; }
+    pack_ends(ends, 1, a.ends0);
     a.f = df; a.f_stride = 1; a.nsamp = dns; a.cells = dcells; a.max_cells = max_cells;
     rc = launch_cost(m->dev, a, 1, 1, pick_cost_shape(a.W, ends->start, ends->goal, m->dev.dims, m->tune), true, m->stream);
     if (!rc) {

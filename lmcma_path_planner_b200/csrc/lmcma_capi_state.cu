@@ -16,15 +16,11 @@ int lmcma_b200_get_f64(lmcma_b200_opt* o, int32_t which, double* out, int64_t ca
         case LMCMA_B200_F64_XMEAN:
             ARG(cap >= (int64_t)(B * d.n), "capacity");
             return d2h_rows(out, d.xmean, B, d.n * sizeof(double), d.ns * sizeof(double), o->stream);
-        case LMCMA_B200_F64_SIGMA: case LMCMA_B200_F64_S: case LMCMA_B200_F64_BESTF: {
+        case LMCMA_B200_F64_SIGMA: case LMCMA_B200_F64_S: case LMCMA_B200_F64_BESTF:
             ARG(cap >= (int64_t)B, "capacity");
-            std::vector<Scalars> sc(B);
-            CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            for (size_t b = 0; b < B; ++b)
-                out[b] = which == LMCMA_B200_F64_SIGMA ? sc[b].sigma : (which == LMCMA_B200_F64_S ? sc[b].s : sc[b].best_f);
-            return 0;
-        }
+            return read_scalars(o, [&](int b, const Scalars& s) {
+                out[b] = which == LMCMA_B200_F64_SIGMA ? s.sigma : (which == LMCMA_B200_F64_S ? s.s : s.best_f);
+            });
         case LMCMA_B200_F64_CONSTS:
             ARG(cap >= 7, "capacity");
             out[0] = d.c1; out[1] = d.cc; out[2] = d.cs; out[3] = d.target; out[4] = d.K; out[5] = d.M; out[6] = d.mueff;
@@ -87,16 +83,12 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
         case LMCMA_B200_I32_RANK: src = d.rank; cnt = B * d.lambda; break;
         case LMCMA_B200_I32_NCOLL: src = d.ncoll; cnt = B * d.pop_count; break;
         case LMCMA_B200_I32_NSAMP: src = d.nsamp; cnt = B * d.pop_count; break;
-        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH: {
+        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH:
             ARG(cap >= (int64_t)B, "capacity");
-            std::vector<Scalars> sc(B);
-            CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            for (size_t b = 0; b < B; ++b)
-                out[b] = which == LMCMA_B200_I32_ITR ? sc[b].itr : (which == LMCMA_B200_I32_LIVE ? sc[b].live :
-                         (which == LMCMA_B200_I32_EPOCH ? sc[b].epoch : (int)sc[b].counteval));
-            return 0;
-        }
+            return read_scalars(o, [&](int b, const Scalars& s) {
+                out[b] = which == LMCMA_B200_I32_ITR ? s.itr : (which == LMCMA_B200_I32_LIVE ? s.live :
+                         (which == LMCMA_B200_I32_EPOCH ? s.epoch : (int)s.counteval));
+            });
         case LMCMA_B200_I32_MAP_OF:     // the map of every instance: all zeros unless the handle is on several maps
             if (o->maps.size() > 1) { src = o->d_map_of; cnt = B; break; }
             ARG(cap >= (int64_t)B, "capacity");
@@ -117,27 +109,21 @@ int lmcma_b200_get_i32(lmcma_b200_opt* o, int32_t which, int32_t* out, int64_t c
 
 int lmcma_b200_set_f64(lmcma_b200_opt* o, int32_t which, const double* in, int64_t count) {
     ARG(o && in, "null pointer");
-    o->spec_valid = false;                              // tell_all's speculative update saw the state before this call
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     const size_t B = d.B;
     switch (which) {
         case LMCMA_B200_F64_XMEAN:
             ARG(count == (int64_t)(B * d.n), "count");
+            state_written(o);
             return h2d_rows(d.xmean, in, B, d.n * sizeof(double), d.ns * sizeof(double), o->stream);
-        case LMCMA_B200_F64_SIGMA: case LMCMA_B200_F64_S: {
+        case LMCMA_B200_F64_SIGMA: case LMCMA_B200_F64_S:
             ARG(count == (int64_t)B, "count");
-            std::vector<Scalars> sc(B);
-            CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            for (size_t b = 0; b < B; ++b) (which == LMCMA_B200_F64_SIGMA ? sc[b].sigma : sc[b].s) = in[b];
-            CU(cudaMemcpyAsync(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            return 0;
-        }
+            state_written(o);
+            return write_scalars(o, [&](int b, Scalars& s) { (which == LMCMA_B200_F64_SIGMA ? s.sigma : s.s) = in[b]; });
         case LMCMA_B200_F64_NJ: case LMCMA_B200_F64_LJ: {
             ARG(count == (int64_t)(B * d.m), "count");
-            o->mirror_dirty = true;
+            state_written(o);
             CU(cudaMemcpyAsync(which == LMCMA_B200_F64_NJ ? d.Nj : d.Lj, in, B * d.m * sizeof(double), cudaMemcpyHostToDevice, o->stream));
             if (which == LMCMA_B200_F64_NJ) {
                 std::vector<float> f(in, in + B * d.m);
@@ -145,7 +131,7 @@ int lmcma_b200_set_f64(lmcma_b200_opt* o, int32_t which, const double* in, int64
                 CU(cudaStreamSynchronize(o->stream));
             }
             CU(cudaStreamSynchronize(o->stream));
-            return settle_mirror(o);
+            return pairs_written(o);
         }
     }
     return fail(LMCMA_B200_ERR_ARG, "f64 field %d is not settable", which);
@@ -153,25 +139,24 @@ int lmcma_b200_set_f64(lmcma_b200_opt* o, int32_t which, const double* in, int64
 
 int lmcma_b200_set_f32(lmcma_b200_opt* o, int32_t which, const float* in, int64_t count) {
     ARG(o && in, "null pointer");
-    o->spec_valid = false;                              // tell_all's speculative update saw the state before this call
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     const size_t B = d.B, w = d.n * sizeof(float), p = d.ns * sizeof(float);
     switch (which) {
         case LMCMA_B200_F32_PC:
             ARG(count == (int64_t)(B * d.n), "count");
+            state_written(o);
             return h2d_rows(d.pc, in, B, w, p, o->stream);
-        case LMCMA_B200_F32_V: case LMCMA_B200_F32_P:
+        case LMCMA_B200_F32_V: case LMCMA_B200_F32_P: {
             ARG(count == (int64_t)(B * d.m * d.n), "count");
-            o->mirror_dirty = true;
-            {
-                int rc = h2d_rows(which == LMCMA_B200_F32_V ? d.V : d.P, in, B * d.m, w, p, o->stream);
-                return rc ? rc : settle_mirror(o);
-            }
+            state_written(o);
+            int rc = h2d_rows(which == LMCMA_B200_F32_V ? d.V : d.P, in, B * d.m, w, p, o->stream);
+            return rc ? rc : pairs_written(o);
+        }
         case LMCMA_B200_F32_X: {
             ARG(count == (int64_t)(B * d.pop_count * d.n), "count");
-            o->x_cache_valid = false;
-            o->xh_fresh = false;
+            state_written(o);
+            rows_written(o, false);
             // keep the offsets d = x - xmean consistent with the overwritten candidates
             std::vector<double> xm(B * d.n);
             int rc = d2h_rows(xm.data(), d.xmean, B, d.n * sizeof(double), d.ns * sizeof(double), o->stream);
@@ -188,6 +173,7 @@ int lmcma_b200_set_f32(lmcma_b200_opt* o, int32_t which, const float* in, int64_
         }
         case LMCMA_B200_F32_PREV_FIT:
             ARG(count == (int64_t)(B * d.lambda), "count");
+            state_written(o);
             CU(cudaMemcpyAsync(d.prev_fit, in, B * d.lambda * sizeof(float), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));
             if (d.prev_sorted) {                                  // the sorted-tile ranking searches an ascending copy
@@ -202,37 +188,31 @@ int lmcma_b200_set_f32(lmcma_b200_opt* o, int32_t which, const float* in, int64_
 
 int lmcma_b200_set_i32(lmcma_b200_opt* o, int32_t which, const int32_t* in, int64_t count) {
     ARG(o && in, "null pointer");
-    o->spec_valid = false;                              // tell_all's speculative update saw the state before this call
     CU(cudaSetDevice(o->cfg.device));
     const OptDev& d = o->d;
     const size_t B = d.B;
     switch (which) {
         case LMCMA_B200_I32_T: case LMCMA_B200_I32_VEC:
             ARG(count == (int64_t)(B * d.m), "count");
-            o->mirror_dirty = true;
+            state_written(o);
             CU(cudaMemcpyAsync(which == LMCMA_B200_I32_T ? d.t : d.vec, in, B * d.m * sizeof(int), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));
-            return settle_mirror(o);
-        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH: {
+            return pairs_written(o);
+        case LMCMA_B200_I32_ITR: case LMCMA_B200_I32_LIVE: case LMCMA_B200_I32_COUNTEVAL: case LMCMA_B200_I32_EPOCH:
             ARG(count == (int64_t)B, "count");
-            std::vector<Scalars> sc(B);
-            CU(cudaMemcpyAsync(sc.data(), d.sc, B * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            for (size_t b = 0; b < B; ++b) {
-                if (which == LMCMA_B200_I32_ITR) sc[b].itr = in[b];
-                else if (which == LMCMA_B200_I32_LIVE) sc[b].live = in[b];
-                else if (which == LMCMA_B200_I32_EPOCH) sc[b].epoch = in[b];
-                else sc[b].counteval = in[b];
-            }
-            CU(cudaMemcpyAsync(d.sc, sc.data(), B * sizeof(Scalars), cudaMemcpyHostToDevice, o->stream));
-            CU(cudaStreamSynchronize(o->stream));
-            return 0;
-        }
+            state_written(o);
+            return write_scalars(o, [&](int b, Scalars& s) {
+                if (which == LMCMA_B200_I32_ITR) s.itr = in[b];
+                else if (which == LMCMA_B200_I32_LIVE) s.live = in[b];
+                else if (which == LMCMA_B200_I32_EPOCH) s.epoch = in[b];
+                else s.counteval = in[b];
+            });
         case LMCMA_B200_I32_MAP_OF: {   // read by k_cost through a pointer: no graph is rebuilt
-            if (!o->map) return fail(LMCMA_B200_ERR_STATE, "map_of: no cost attached");
+            TRY(need_cost(o, "set map_of"));
             ARG(count == (int64_t)B, "count");
             const int64_t maps = (int64_t)o->maps.size();
             for (size_t b = 0; b < B; ++b) ARG(in[b] >= 0 && in[b] < maps, "map_of entry outside [0, map_count)");
+            state_written(o);
             if (maps == 1) return 0;                             // a single-map handle: all zeros, nothing stored
             CU(cudaMemcpyAsync(o->d_map_of, in, B * sizeof(int), cudaMemcpyHostToDevice, o->stream));
             CU(cudaStreamSynchronize(o->stream));

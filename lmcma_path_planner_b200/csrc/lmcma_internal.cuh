@@ -62,10 +62,35 @@ inline int dmalloc(T** p, size_t count) {
     if (e != cudaSuccess) return fail(LMCMA_B200_ERR_CUDA, "cudaMemset: %s", cudaGetErrorString(e));
     return 0;
 }
-#define DM(ptr, count)                              \
-    do {                                            \
-        int rc__ = dmalloc(&(ptr), (count));        \
-        if (rc__) return rc__;                      \
+
+// The device buffers of a handle.  alloc fills a member slot of the handle (zeroed, as dmalloc), freeing what the slot
+// held before, and records the slot; free_all releases every recorded slot, so a buffer cannot be left off a list at destroy.
+struct DeviceBuffers {
+    std::vector<void**> slots;
+    template <class T>
+    int alloc(T** slot, size_t count) {
+        void** s = reinterpret_cast<void**>(slot);
+        if (std::find(slots.begin(), slots.end(), s) == slots.end()) slots.push_back(s);
+        if (*s) cudaFree(*s);
+        *s = nullptr;
+        return dmalloc(slot, count);
+    }
+    void free_all() {
+        for (void** s : slots) { if (*s) cudaFree(*s); *s = nullptr; }
+        slots.clear();
+    }
+};
+// a device buffer of the handle `owner` into its member `slot`
+#define DM(owner, slot, count)                                  \
+    do {                                                        \
+        int rc__ = (owner)->buffers.alloc(&(slot), (count));    \
+        if (rc__) return rc__;                                  \
+    } while (0)
+// returns the code of an int-returning call that failed
+#define TRY(call)                   \
+    do {                            \
+        int rc__ = (call);          \
+        if (rc__) return rc__;      \
     } while (0)
 
 // Every kernel of the library is launched here.  Dynamic shared memory above 48 KiB is opted into; pdl makes the kernel a
@@ -138,6 +163,7 @@ struct lmcma_b200_map {
     int device = 0;
     lmcma_capi::Tuning tune;
     lmcma::MapDev dev{};
+    lmcma_capi::DeviceBuffers buffers;   // every device buffer below but d_update (lmcma_b200_map_destroy frees them all)
     int storage = 0;
     float c_min = 0.5f, scale = 1.f;
     size_t cells = 0, stored = 0;   // logical cells / stored elements (bricked, padded)
@@ -163,6 +189,7 @@ struct lmcma_b200_opt {
     lmcma_b200_config cfg{};
     lmcma_capi::Tuning tune;
     lmcma::OptDev d{};
+    lmcma_capi::DeviceBuffers buffers;    // every device buffer of the handle, d and the d_* members (DM)
     lmcma_capi::DeviceProps* props = nullptr;
     cudaStream_t own_stream = nullptr, stream = nullptr;
     // host mirrors
@@ -173,6 +200,10 @@ struct lmcma_b200_opt {
     lmcma::HansenStream hansen{1};
     std::vector<float> z_host;         // staging for HANSEN
     bool needs_sample = false, pending_z = false;
+    // The host's view of the device state: spec_valid, x_cache_valid, xh_fresh, sample_idx and mirror_dirty.  Entry points
+    // change it through the transitions below (new_population, rows_written, state_written, pairs_written); besides those,
+    // only the code that consumes a flag writes it: ensure_mirror, tell_all's replay, ask_all_view, ask_one / tell_one,
+    // check_lost and the graph drop.
     // reference one-at-a-time protocol
     int sample_idx = 0;
     std::vector<float> x_cache; bool x_cache_valid = false;
@@ -201,6 +232,7 @@ struct lmcma_b200_opt {
     // speculative update (k_update.cuh, UpdateArgs::phase): with the host mirror on, every tell_all graph ends with the
     // fitness-independent part of the NEXT generation's update (into d_spec, beside the sampler's tail and the candidates' trip
     // across PCIe); the next tell_all resumes from it (tell_host.resume) unless anything else touched the state in between
+    // (state_written)
     float* d_spec = nullptr; size_t spec_stride = 0;
     bool spec_valid = false;
     float* f_pinned = nullptr;                // the graph's copy source (the caller's fitness array is copied here first)
@@ -208,7 +240,7 @@ struct lmcma_b200_opt {
     bool have_run_timing = false;
     lmcma_capi::LaunchPlan plan;       // every kernel configuration, chosen at create (lmcma_plan.hpp)
     float* d_Lf = nullptr;             // lower Cholesky factor of the smoothness prior (n x ns FP32) or null
-    bool mirror_dirty = true;          // the sequence-ordered pair mirror must be rebuilt (k_pack_pairs) before sampling
+    bool mirror_dirty = true;          // the sequence-ordered pair mirror must be rebuilt (k_pack_pairs) before sampling (pairs_written)
     lmcma::CostShape cost_shape;
     // fused generation with k_update on a side branch, concurrent with k_cost / k_rank (k_update.cuh): plan.overlap, until
     // something at run time rules it out (no side stream, the co-scheduling probe, a failed forked capture, check_lost)
@@ -216,7 +248,7 @@ struct lmcma_b200_opt {
     cudaStream_t side_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     float* x_mirror = nullptr;        // page-locked, mapped host mirror of X (lmcma_b200_ask_all_view); OptDev::Xh is its device alias
-    bool xh_fresh = false;            // x_mirror holds the population (the last sampler wrote it)
+    bool xh_fresh = false;            // x_mirror holds the population (the last sampler wrote it, or ask_all_view copied it)
     int* err_host = nullptr;          // page-locked, mapped: OptDev::err (a kernel of the overlapped generation gave up on its partner)
 };
 
@@ -227,11 +259,72 @@ int launch_cost(const MapDev& mp, const CostArgs& a, int rows, int B, CostShape 
 CostShape pick_cost_shape(int W, const float* start, const float* goal, int dims, const Tuning& tune);
 int apply_l2_window(lmcma_b200_map* m, cudaStream_t st);
 int check_obj(const lmcma_b200_map* m, const lmcma_b200_objective* obj);
+void pack_ends(const lmcma_b200_endpoints* ends, int count, float* out);
 void register_mirror(const void* host, size_t bytes, const float* dev, long long ld, int device);
 void unregister_mirror(const void* host);
 // ---- defined in lmcma_capi.cu ----
 int check_lost(lmcma_b200_opt* o);
-int settle_mirror(lmcma_b200_opt* o);
+
+// ---- the transitions of the host's view of the device state ----
+// The optimiser state was written by something other than the forked tell: whatever tell_all's speculative pass left in
+// d_spec is stale.  Every entry point that writes the state calls it once its checks have passed.
+inline void state_written(lmcma_b200_opt* o) { o->spec_valid = false; }
+// d.X was written: ask_one's cache no longer holds it, nor does the host mirror unless the sampler that wrote d.X wrote the
+// mirror too (mirror)
+inline void rows_written(lmcma_b200_opt* o, bool mirror) {
+    o->x_cache_valid = false;
+    o->xh_fresh = mirror && o->x_mirror;
+}
+// A sampler has been enqueued or replayed (mirror: it wrote the host mirror): rows_written, and the one-at-a-time protocol
+// starts at the first row.  A sampler that redraws some instances only (lmcma_b200_reset_instances) leaves the mirror fresh
+// only if it was fresh before: it passes mirror && xh_fresh.
+inline void new_population(lmcma_b200_opt* o, bool mirror) {
+    rows_written(o, mirror);
+    o->sample_idx = 0;
+}
+// The direction pairs (V, P, Nj, Lj, t, vec) were written from the host: the pair mirror is rebuilt before the next
+// library sampler, or at once on a handle whose generations replay in a caller's graph (caller_graphs), because the next
+// sampler to read it may be such a replay.  Defined in lmcma_capi.cu.
+int pairs_written(lmcma_b200_opt* o);
+
+// ---- the ERR_STATE preconditions several entry points share (`who`: the entry point, for the message) ----
+inline int need_population(const lmcma_b200_opt* o, const char* who) {
+    return o->needs_sample ? fail(LMCMA_B200_ERR_STATE, "%s: no population yet (rng INJECT: inject_z first)", who) : 0;
+}
+inline int need_unsplit(const lmcma_b200_opt* o, const char* who) {
+    return o->d.pop_count != o->d.lambda
+               ? fail(LMCMA_B200_ERR_STATE, "%s: not supported on a split-population handle (it takes the mg_* entry points)", who) : 0;
+}
+inline int need_philox(const lmcma_b200_opt* o, const char* who) {
+    return o->cfg.rng != LMCMA_B200_RNG_PHILOX ? fail(LMCMA_B200_ERR_STATE, "%s needs the PHILOX rng", who) : 0;
+}
+// an attached cost: o->map, and with it the device end points d_ends (attach_body)
+inline int need_cost(const lmcma_b200_opt* o, const char* who) {
+    return o->map ? 0 : fail(LMCMA_B200_ERR_STATE, "%s: no cost attached (lmcma_b200_attach_cost)", who);
+}
+inline int need_batch_of_one(const lmcma_b200_opt* o, const char* who) {
+    return o->d.B != 1 ? fail(LMCMA_B200_ERR_STATE, "%s needs batch == 1", who) : 0;
+}
+
+// The B Scalars of the handle through the host, in order on o->stream; both return when their copies are done.
+// read_scalars calls f(b, const Scalars&) for every instance b; write_scalars lets f(b, Scalars&) edit a copy of every
+// instance's Scalars and writes the copies back.
+template <class F>
+int read_scalars(lmcma_b200_opt* o, F&& f) {
+    std::vector<Scalars> sc(o->d.B);
+    CU(cudaMemcpyAsync(sc.data(), o->d.sc, sc.size() * sizeof(Scalars), cudaMemcpyDeviceToHost, o->stream));
+    CU(cudaStreamSynchronize(o->stream));
+    for (int b = 0; b < o->d.B; ++b) f(b, sc[b]);
+    return 0;
+}
+template <class F>
+int write_scalars(lmcma_b200_opt* o, F&& f) {
+    std::vector<Scalars> sc(o->d.B);
+    TRY(read_scalars(o, [&](int b, const Scalars& s) { sc[b] = s; f(b, sc[b]); }));
+    CU(cudaMemcpyAsync(o->d.sc, sc.data(), sc.size() * sizeof(Scalars), cudaMemcpyHostToDevice, o->stream));
+    CU(cudaStreamSynchronize(o->stream));
+    return 0;
+}
 
 // dense <-> pitched copies
 inline int d2h_rows(void* dst, const void* src, size_t rows, size_t width_bytes, size_t src_pitch_bytes, cudaStream_t st) {
